@@ -368,6 +368,28 @@ def train_bytes_per_sample(D):
     return 2 * 3 * fwd_rows * 512
 
 
+DUMP_ENVS, DUMP_SEED = 32, 0    # 32 of 4096 envs keep the dump at ~41 MiB, most of it the two [T+D,B,N,128] embedding histories
+
+
+def dump_outputs(batch, out_dir):
+    """Writes the TrainBatch that `MAPPO.explore_batched` returned for the last timed episode as <out_dir>/<key>.npy, restricted to
+    a fixed, seeded sample of DUMP_ENVS envs (axis 1 of every key, in ascending env order).  float32, except the bit-packed
+    adjacency words (int32), which are written as float64 so that they stay exact."""
+    import numpy as np
+    import torch
+    from distributed_multi_agent_reinforcement_learning_b200.mappo_parallel import TrainBatch
+    envs = np.sort(np.random.default_rng(DUMP_SEED).choice(batch.B, size=min(DUMP_ENVS, batch.B), replace=False))
+    idx = torch.from_numpy(envs).to(batch.p.device)
+    out = {}
+    for k in TrainBatch.KEYS:
+        a = getattr(batch, k).index_select(1, idx).cpu().numpy()
+        out[k] = a.astype(np.float64 if a.dtype == np.int32 else np.float32)
+    assert sum(a.nbytes for a in out.values()) <= 64e6
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def _popcount_mean(torch, words):
     """Mean number of set bits per row of a packed int32 [..., W] tensor."""
     w = words.to(torch.int64) & 0xFFFFFFFF
@@ -458,6 +480,8 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     status = int(env.evader_status.max().item())
     assert status == 0, f"evader status {status}: search overflow or target tape exhausted"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(pol.batch, args.dump_outputs)      # before e2e: it replays the same graph into the same buffers
     per_rank_ms = {"value": [x / args.steps for x in per_rank(ms_total)]}
     ms_total = parallel.max_over_ranks(ms_total, dev)
     value = world * B * N * T * args.steps / (ms_total * 1e-3)
@@ -647,7 +671,13 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed episode's rollout batch (a fixed sample of envs) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
