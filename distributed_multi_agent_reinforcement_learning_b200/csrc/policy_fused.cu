@@ -27,6 +27,7 @@
 #include "common.cuh"
 #include <cuda_fp16.h>
 #include <stdlib.h>
+#include <type_traits>
 
 namespace marl {
 namespace pf {
@@ -105,7 +106,7 @@ struct NetArgs {
 struct StepArgs {
     int B, N, O, NW, OW, depth, rows_per_tile, n_tiles, A;
     int64_t R;
-    const double *p_state, *e_state;
+    const void *p_state, *e_state;   // double, or float in the STATE_F32 instantiations
     const int32_t *oxy, *map_id, *o_count;
     const uint32_t *p_adj;
     const uint8_t *e_adj;
@@ -315,21 +316,26 @@ __device__ __forceinline__ bool row_info(const Ctx &c, int r, int64_t &gr, int &
     i = ok ? (int)(gr - (int64_t)env * c.a->N) : 0;
     return ok;
 }
-__device__ __forceinline__ float4 load_p(const StepArgs *a, int64_t gr)
+// F32 (MARL_POLICY_STATE_F32): the states are already (float) of the fp64 state - the rollout arena's records - and are read as is
+template <bool F32>
+__device__ __forceinline__ float4 load_state4(const void *base, int64_t idx)
 {
-    const double2 *q = reinterpret_cast<const double2 *>(a->p_state + gr * 4);
-    const double2 u = q[0], v = q[1];
-    return make_float4((float)u.x, (float)u.y, (float)v.x, (float)v.y);
+    if constexpr (F32) {
+        return reinterpret_cast<const float4 *>(base)[idx];
+    } else {
+        const double2 *q = reinterpret_cast<const double2 *>(static_cast<const double *>(base) + idx * 4);
+        const double2 u = q[0], v = q[1];
+        return make_float4((float)u.x, (float)u.y, (float)v.x, (float)v.y);
+    }
 }
-__device__ __forceinline__ float4 load_e(const StepArgs *a, int env)
-{
-    const double2 *q = reinterpret_cast<const double2 *>(a->e_state + (int64_t)env * 4);
-    const double2 u = q[0], v = q[1];
-    return make_float4((float)u.x, (float)u.y, (float)v.x, (float)v.y);
-}
+template <bool F32>
+__device__ __forceinline__ float4 load_p(const StepArgs *a, int64_t gr) { return load_state4<F32>(a->p_state, gr); }
+template <bool F32>
+__device__ __forceinline__ float4 load_e(const StepArgs *a, int env) { return load_state4<F32>(a->e_state, env); }
+template <bool F32>
 __device__ __forceinline__ float4 e_of(const Ctx &c, int r, int env)
 {
-    return (ROWS / c.a->N <= 32) ? c.s_e[r / c.a->N] : load_e(c.a, env);
+    return (ROWS / c.a->N <= 32) ? c.s_e[r / c.a->N] : load_e<F32>(c.a, env);
 }
 __device__ __forceinline__ float dot4w(const float (&w)[4], float a0, float a1, float a2, float a3, float b)
 {
@@ -386,7 +392,7 @@ __device__ __forceinline__ void load_msg_weights(const NetArgs *na, int rel, int
 
 // ---- DHGN.message + mean aggregation, generic per-row path (any N) -> X ----------------------------------------------------
 // Same arithmetic as msg_agg_fwd_kernel (policy_kernels.cu).  lane l owns channels 4l..4l+3.
-template <int WW>
+template <int WW, bool F32>
 __device__ void phase_msg_generic(const Ctx &c, int rel)
 {
     constexpr int RPW = Lay<WW>::RPW;
@@ -403,7 +409,7 @@ __device__ void phase_msg_generic(const Ctx &c, int rel)
         const bool ok = row_info(c, r, gr, env, i);
         float out[4] = {0.f, 0.f, 0.f, 0.f};
         if (ok) {
-            const float4 pi = c.s_p[r], ev = e_of(c, r, env);
+            const float4 pi = c.s_p[r], ev = e_of<F32>(c, r, env);
             const float dex = pi.x - ev.x, dey = pi.y - ev.y, dez = pi.z - ev.z, dew = pi.w - ev.w;
             if (rel == 0) {
                 int cnt = 0;
@@ -664,10 +670,10 @@ __device__ __forceinline__ bool fast_env_path(const Ctx &c)
     return (a->N == 4 || a->N == 8 || a->N == 16) && a->N <= Lay<WW>::RPW && a->O <= c.oxy_cap;
 }
 
-template <int WW>
+template <int WW, bool F32>
 __device__ void phase_msg(const Ctx &c, int rel)
 {
-    if (!fast_env_path<WW>(c)) phase_msg_generic<WW>(c, rel);
+    if (!fast_env_path<WW>(c)) phase_msg_generic<WW, F32>(c, rel);
     else if (c.a->N == 8) phase_msg_fast<8, WW>(c, rel);
     else if (c.a->N == 4) phase_msg_fast<4, WW>(c, rel);
     else if constexpr (WW == 8) phase_msg_fast<16, WW>(c, rel);
@@ -1052,11 +1058,14 @@ __device__ void epi_head(const Ctx &c)
     if (c.a->logp) c.a->logp[gr] = lpa;
 }
 
-template <int WW, bool DUAL>
+// FL: marl_policy_step.flags (MARL_POLICY_STATE_F32 / MARL_POLICY_EMBED_ONLY), one instantiation per combination
+template <int WW, bool DUAL, int FL>
 __global__ void __launch_bounds__(Lay<WW>::THREADS, DUAL ? 2 : 1)
 policy_step_kernel(const __grid_constant__ StepArgs a)
 {
     static_assert(!DUAL || WW == 8, "the two-CTA variant runs 8 worker warps");
+    static_assert(!DUAL || FL == 0, "the two-CTA variant has no flag instantiations");
+    constexpr bool F32 = (FL & MARL_POLICY_STATE_F32) != 0, EMB = (FL & MARL_POLICY_EMBED_ONLY) != 0;
     using M = Mem<DUAL>;
     constexpr int RPW = Lay<WW>::RPW, NST = M::NST;
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -1103,10 +1112,10 @@ policy_step_kernel(const __grid_constant__ StepArgs a)
             if (t < ROWS) {
                 int64_t gr;
                 int env, i;
-                s_p[t] = row_info(c, t, gr, env, i) ? load_p(&a, gr) : make_float4(0.f, 0.f, 0.f, 0.f);
+                s_p[t] = row_info(c, t, gr, env, i) ? load_p<F32>(&a, gr) : make_float4(0.f, 0.f, 0.f, 0.f);
             } else if (t < ROWS + 32) {
                 const int64_t env = c.row0 / a.N + (t - ROWS);
-                s_e[t - ROWS] = (ROWS / a.N <= 32 && t - ROWS < ROWS / a.N && env < a.B) ? load_e(&a, (int)env) : make_float4(0.f, 0.f, 0.f, 0.f);
+                s_e[t - ROWS] = (ROWS / a.N <= 32 && t - ROWS < ROWS / a.N && env < a.B) ? load_e<F32>(&a, (int)env) : make_float4(0.f, 0.f, 0.f, 0.f);
             }
             worker_sync<WW>();
         }
@@ -1125,7 +1134,7 @@ policy_step_kernel(const __grid_constant__ StepArgs a)
         }
 #define PF_TICK(slot) do { const long long now_ = clock64(); tk[slot] += now_ - t_prev; t_prev = now_; } while (0)
         for (int r = 0; r < 3; ++r) {
-            phase_msg<WW>(c, r);
+            phase_msg<WW, F32>(c, r);
             PF_TICK(0 + r);
             hand_over(c);                                              // AGG_vertex_0 -> acc @0
             PF_TICK(11);
@@ -1154,7 +1163,9 @@ policy_step_kernel(const __grid_constant__ StepArgs a)
             epi_store<WW>(c, 128, na->b_f[k], true, nullptr, 0, k == a.depth - 1 ? na->emb_out : nullptr);
             PF_TICK(7);
         }
-        if constexpr (!DUAL) {
+        if constexpr (EMB) {
+            // embeddings only: the unit program ends with the FCRA chain (fill_net), nothing is left to hand over
+        } else if constexpr (!DUAL) {
             for (int l = 0; l < 2; ++l) {
                 signal_ready(c);                                           // W_ih: r @0, z @128, n @256
                 hidden_prefetch<WW>(c, l, pre);                                //   ... while it runs: h_prev of this layer
@@ -1210,7 +1221,7 @@ policy_step_kernel(const __grid_constant__ StepArgs a)
                 PF_TICK(8);
             }
         }
-        if (net == 0) {
+        if (!EMB && net == 0) {
             hand_over(c);                                              // actor head, n_out = 16 -> acc @0
             PF_TICK(11);
             epi_head<MARL_NUM_ACTIONS>(c);
@@ -1509,10 +1520,11 @@ constexpr int PAIR8_WORKER_REGS = 232, PAIR8_OTHER_REGS = 40;     //  8 worker w
 // PROF: per-phase cycle counters in registers (tools/fused_phase_profile.py, MARL_POLICY_PROFILE=1); the production instantiation
 // only writes the CTA's start / end %globaltimer, SM id and total cycles when a debug buffer is given, and keeps nothing live for it.
 #define PP_TICK(slot) do { if constexpr (PROF) { const long long now_ = clock64(); tk[slot] += now_ - t_prev; t_prev = now_; } } while (0)
-template <int WW, bool PROF>
+template <int WW, bool PROF, int FL>
 __global__ void __launch_bounds__((WW + 4) * 32, 1)
 policy_pair_kernel(const __grid_constant__ StepArgs a)
 {
+    constexpr bool F32 = (FL & MARL_POLICY_STATE_F32) != 0, EMB = (FL & MARL_POLICY_EMBED_ONLY) != 0;
     using M = MemPair;
     extern __shared__ __align__(1024) unsigned char smem[];
     if ((smem_u32(smem) & 1023u) != 0u) __trap();
@@ -1559,10 +1571,10 @@ policy_pair_kernel(const __grid_constant__ StepArgs a)
             if (t < ROWS) {
                 int64_t gr;
                 int env, i;
-                s_p[t] = row_info(c, t, gr, env, i) ? load_p(&a, gr) : make_float4(0.f, 0.f, 0.f, 0.f);
+                s_p[t] = row_info(c, t, gr, env, i) ? load_p<F32>(&a, gr) : make_float4(0.f, 0.f, 0.f, 0.f);
             } else if (t < ROWS + 32) {
                 const int64_t env = c.row0 / a.N + (t - ROWS);
-                s_e[t - ROWS] = (ROWS / a.N <= 32 && t - ROWS < ROWS / a.N && env < a.B) ? load_e(&a, (int)env) : make_float4(0.f, 0.f, 0.f, 0.f);
+                s_e[t - ROWS] = (ROWS / a.N <= 32 && t - ROWS < ROWS / a.N && env < a.B) ? load_e<F32>(&a, (int)env) : make_float4(0.f, 0.f, 0.f, 0.f);
             }
             worker_sync<WW>();
         }
@@ -1581,7 +1593,8 @@ policy_pair_kernel(const __grid_constant__ StepArgs a)
             d[13] = (long long)gt;
             d[15] = (long long)smid;
         }
-        const int D = a.depth, G0 = 7 + 3 * D, S_ACTOR = G0 + 9, S_CRITIC = G0 + 8;
+        // EMB: both chains stop after the FCRA chain's last epilogue (step G0 - 1, which stores the embedding)
+        const int D = a.depth, G0 = 7 + 3 * D, S_ACTOR = EMB ? G0 : G0 + 9, S_CRITIC = EMB ? G0 : G0 + 8;
         constexpr int NA_BIG = Lay<WW>::RPW;                           // env size whose rows fill a warp: 8 (16 worker warps) or 16 (8)
         const bool pair01 = (a.N == NA_BIG || (WW == 16 && a.N == 4)) && a.NW == 1;      // relations 0 and 1 computed once for both chains
         const uint32_t bar_ready0 = smem_u32(&bars[M::BAR_READY]), bar_done0 = smem_u32(&bars[M::BAR_DONE]);
@@ -1626,6 +1639,7 @@ policy_pair_kernel(const __grid_constant__ StepArgs a)
                     else if (s > 6) { acc_col = 128; bias = na->b_f[fk]; gout = fk == D - 1 ? na->emb_out : nullptr; }
                     wait_prev();
                     epi_store<WW>(c, acc_col, bias, relu, wp, na->sem_ld, gout);
+                    if (EMB && s == G0 - 1) signal = false;
                     PP_TICK(1);
                 } else if (is_msg) {                           // messages of relation s/2 -> X
                     if (pair01 && a.O <= OXY_CAP) {
@@ -1643,7 +1657,7 @@ policy_pair_kernel(const __grid_constant__ StepArgs a)
                         }
                     } else {
                         wait_prev();
-                        phase_msg<WW>(c, s >> 1);
+                        phase_msg<WW, F32>(c, s >> 1);
                     }
                     PP_TICK(0);
                 } else if (is_fcra_fill) {
@@ -2009,14 +2023,16 @@ extern "C" int marl_policy_pack(const marl_dhgn_weights *w, int32_t depth, int32
     return MARL_OK;
 }
 
-static int fill_net(pf::NetArgs &na, const marl_dhgn_weights *w, const marl_policy_net_io *io, int depth, int is_actor, int A, int mode)
+static int fill_net(pf::NetArgs &na, const marl_dhgn_weights *w, const marl_policy_net_io *io, int depth, int is_actor, int A, int mode,
+                    bool embed_only)
 {
     int rc = pf::check_weights(w, depth, is_actor);
     if (rc) return rc;
-    MARL_REQUIRE(io->d_packed && io->d_hidden && io->d_emb_out, "marl_policy_rollout_step: null packed / hidden / emb_out (%s)",
+    MARL_REQUIRE(io->d_packed && (embed_only || io->d_hidden) && io->d_emb_out, "marl_policy_rollout_step: null packed / hidden / emb_out (%s)",
                  is_actor ? "actor" : "critic");
     pf::UnitSrc us[pf::MAX_UNITS];
     na.n_units = pf::build_units(w, depth, is_actor, A, us, mode);
+    if (embed_only) na.n_units = 6 + 3 * depth;           // the encoder and FCRA units lead the program (build_units)
     uint32_t off = (uint32_t)(mode * pf::layout_bytes(depth, is_actor));
     for (int u = 0; u < na.n_units; ++u) {
         na.u[u] = pf::Unit{off, (uint16_t)us[u].n_out, (uint16_t)us[u].acc_col, (uint8_t)us[u].accumulate, (uint8_t)us[u].last, 0};
@@ -2054,6 +2070,10 @@ extern "C" int marl_policy_rollout_step(const marl_policy_step *s, const marl_dh
     MARL_REQUIRE(s->d_p_state && s->d_e_state && s->d_oxy && s->d_o_count && s->d_p_adj_bits && s->d_e_adj && s->d_o_adj_bits,
                  "marl_policy_rollout_step: null observation pointer");
     MARL_REQUIRE((actor_w && actor_io) || (critic_w && critic_io), "marl_policy_rollout_step: no network given");
+    MARL_REQUIRE((s->flags & ~(MARL_POLICY_STATE_F32 | MARL_POLICY_EMBED_ONLY)) == 0, "marl_policy_rollout_step: unknown flags 0x%x",
+                 (unsigned)s->flags);
+    MARL_REQUIRE(s->variant != 2 || s->flags == 0, "marl_policy_rollout_step: variant 2 runs without flags (flags=0x%x)", (unsigned)s->flags);
+    const bool embed_only = (s->flags & MARL_POLICY_EMBED_ONLY) != 0;
     pf::StepArgs a{};
     a.B = s->B; a.N = s->N; a.O = s->O; a.NW = (s->N + 31) / 32; a.OW = (s->O + 31) / 32; a.depth = s->depth; a.A = s->action_dim;
     a.R = (int64_t)s->B * s->N;
@@ -2067,7 +2087,7 @@ extern "C" int marl_policy_rollout_step(const marl_policy_step *s, const marl_dh
     MARL_REQUIRE(s->variant != 2 || pingpong, "marl_policy_rollout_step: variant 2 needs d_hidden_out != d_hidden");
     MARL_REQUIRE(s->variant != 3 || (has_a && has_c), "marl_policy_rollout_step: variant 3 (actor + critic chains in one CTA) needs both networks");
     const bool pair = s->variant == 3;
-    const bool dual = !pair && (s->variant == 2 || (s->variant == 0 && pingpong && pf::kDualByDefault && s->O <= pf::Mem<true>::OXY));
+    const bool dual = !pair && (s->variant == 2 || (s->variant == 0 && s->flags == 0 && pingpong && pf::kDualByDefault && s->O <= pf::Mem<true>::OXY));
     const int mode = pair ? 2 : (dual ? 1 : 0);
     a.rows_per_tile = pf::choose_rows_per_tile(a.R, s->N, pair ? 1 : nets, dual ? 2 : 1, s->tile_rows);
     a.n_tiles = (int)((a.R + a.rows_per_tile - 1) / a.rows_per_tile);
@@ -2077,8 +2097,8 @@ extern "C" int marl_policy_rollout_step(const marl_policy_step *s, const marl_dh
     a.row_offset = s->row_offset;
     a.dbg = static_cast<long long *>(s->d_debug);
     int rc;
-    if (has_a) { rc = fill_net(a.net[0], actor_w, actor_io, s->depth, 1, s->action_dim, mode); if (rc) return rc; }
-    if (has_c) { rc = fill_net(a.net[1], critic_w, critic_io, s->depth, 0, s->action_dim, mode); if (rc) return rc; }
+    if (has_a) { rc = fill_net(a.net[0], actor_w, actor_io, s->depth, 1, s->action_dim, mode, embed_only); if (rc) return rc; }
+    if (has_c) { rc = fill_net(a.net[1], critic_w, critic_io, s->depth, 0, s->action_dim, mode, embed_only); if (rc) return rc; }
     a.net_count = nets;
     a.net_first = has_a ? 0 : 1;
     const unsigned grid = (unsigned)(a.n_tiles * (pair ? 1 : a.net_count));
@@ -2091,12 +2111,25 @@ extern "C" int marl_policy_rollout_step(const marl_policy_step *s, const marl_dh
     };
     // one CTA per SM: 16 worker warps unless the env-grouped message path needs a whole 16-agent env per warp
     const bool pair8 = pair && s->N == 16 && s->O <= pf::OXY_CAP;       // 16-agent envs: a whole env per warp needs 8 worker warps
-    if (pair8) rc = launch(pf::policy_pair_kernel<8, false>, (8 + 4) * 32, pf::MemPair::BYTES, false);
-    else if (pair && getenv("MARL_POLICY_PROFILE")) rc = launch(pf::policy_pair_kernel<16, true>, (16 + 4) * 32, pf::MemPair::BYTES, false);
-    else if (pair) rc = launch(pf::policy_pair_kernel<16, false>, (16 + 4) * 32, pf::MemPair::BYTES, false);
-    else if (dual) rc = launch(pf::policy_step_kernel<8, true>, pf::Lay<8>::THREADS, pf::Mem<true>::BYTES, true);
-    else if (!(s->N == 16 && s->O <= pf::OXY_CAP)) rc = launch(pf::policy_step_kernel<16, false>, pf::Lay<16>::THREADS, pf::Mem<false>::BYTES, false);
-    else rc = launch(pf::policy_step_kernel<8, false>, pf::Lay<8>::THREADS, pf::Mem<false>::BYTES, false);
+    const bool step8 = s->N == 16 && s->O <= pf::OXY_CAP;
+    // the flags select a kernel instantiation (no runtime branch in the phases); flags = 0 is the default kernels
+    auto dispatch = [&](auto fl) -> int {
+        constexpr int FL = decltype(fl)::value;
+        if (pair8) return launch(pf::policy_pair_kernel<8, false, FL>, (8 + 4) * 32, pf::MemPair::BYTES, false);
+        if constexpr (FL == 0) {
+            if (pair && getenv("MARL_POLICY_PROFILE")) return launch(pf::policy_pair_kernel<16, true, 0>, (16 + 4) * 32, pf::MemPair::BYTES, false);
+            if (dual) return launch(pf::policy_step_kernel<8, true, 0>, pf::Lay<8>::THREADS, pf::Mem<true>::BYTES, true);
+        }
+        if (pair) return launch(pf::policy_pair_kernel<16, false, FL>, (16 + 4) * 32, pf::MemPair::BYTES, false);
+        if (!step8) return launch(pf::policy_step_kernel<16, false, FL>, pf::Lay<16>::THREADS, pf::Mem<false>::BYTES, false);
+        return launch(pf::policy_step_kernel<8, false, FL>, pf::Lay<8>::THREADS, pf::Mem<false>::BYTES, false);
+    };
+    switch (s->flags) {
+    case 0: rc = dispatch(std::integral_constant<int, 0>{}); break;
+    case MARL_POLICY_STATE_F32: rc = dispatch(std::integral_constant<int, MARL_POLICY_STATE_F32>{}); break;
+    case MARL_POLICY_EMBED_ONLY: rc = dispatch(std::integral_constant<int, MARL_POLICY_EMBED_ONLY>{}); break;
+    default: rc = dispatch(std::integral_constant<int, MARL_POLICY_STATE_F32 | MARL_POLICY_EMBED_ONLY>{}); break;
+    }
     if (rc) return rc;
     return check_launch("policy_step_kernel");
 }

@@ -2,7 +2,9 @@
 the heads of the actor AND the critic for all B envs of a step (DHGN/mappo_parallel.py:758-801, network half).
 
 `FusedRolloutStep` owns the packed (hi/lo TF32, pre-swizzled) weight images and the ctypes structs; it is rebuilt (re-packed)
-whenever the weights change, i.e. once per rollout."""
+whenever the weights change, i.e. once per rollout.  Built with `snapshot=True` it also keeps its own copy of every weight the
+kernel reads unpacked (message layers, biases, head rows), so it keeps computing the rollout-time networks after the optimizer
+has stepped the live parameters - what a replay of the episode's history embeddings needs."""
 import ctypes as C
 import os
 
@@ -30,7 +32,12 @@ class PolicyStep(C.Structure):
                [("seed", C.c_uint64)] + \
                [(n, C.c_void_p) for n in ("d_p_state", "d_e_state", "d_oxy", "d_map_id", "d_o_count", "d_p_adj_bits",
                                           "d_e_adj", "d_o_adj_bits", "d_action", "d_logp", "d_value", "d_debug")] + \
-               [("row_offset", C.c_int64), ("tile_rows", C.c_int32), ("reserved", C.c_int32)]
+               [("row_offset", C.c_int64), ("tile_rows", C.c_int32), ("flags", C.c_int32)]
+
+
+# marl_policy_step.flags (include/marl_b200.h)
+STATE_F32 = 1       # d_p_state / d_e_state are float [B,N,4] / [B,4] (the rollout arena's records) instead of double
+EMBED_ONLY = 2      # encoder + FCRA chain only: write the embeddings; hidden states, actions, log-probs and values untouched
 
 
 # Kernel variant used when the caller does not ask for one (marl_policy_step.variant): 3 = the actor and the critic chain of a row
@@ -50,8 +57,9 @@ def _c(t):
 
 
 class FusedRolloutStep:
-    def __init__(self, mappo, critic_w_eff):
-        """critic_w_eff: effective [E] critic head row (weight_orig / sigma), constant while the weights are fixed."""
+    def __init__(self, mappo, critic_w_eff, snapshot=False):
+        """critic_w_eff: effective [E] critic head row (weight_orig / sigma), constant while the weights are fixed.
+        snapshot: copy the weights instead of pointing at the live parameters (see the module docstring)."""
         if not supported(mappo):
             raise _lib.MarlError("fused rollout step needs embedding_dim = rnn_hidden_dim = 128, 2 GRU layers, depth 1..3")
         self.lib = _lib.lib()
@@ -65,7 +73,7 @@ class FusedRolloutStep:
         keep = self._keep
 
         def P(t):
-            keep.append(_c(t))
+            keep.append(_c(t).clone() if snapshot else _c(t))
             return keep[-1].data_ptr()
 
         for name, net in (("actor", mappo.actor), ("critic", mappo.critic)):
@@ -96,9 +104,11 @@ class FusedRolloutStep:
             keep.append(buf)
 
     def step(self, engine, oxy_i32, o_count, t, seed, deterministic, hist_a, hist_c, emb_a, emb_c, ha, hc, action, logp, value,
-             nets=("actor", "critic"), force_action=False, debug=None, variant=0, row_offset=0, tile_rows=0):
+             nets=("actor", "critic"), force_action=False, debug=None, variant=0, row_offset=0, tile_rows=0, flags=0):
         """hist_*: list (k = 0 newest) of [B,N,E] tensors or None (zeros); emb_*: [B,N,E] outputs; ha/hc: [2,B*N,E] in/out;
         action i32 [B,N], logp / value f32 [B,N] outputs.
+        flags: STATE_F32 (engine.p_state / e_state are the fp32 records [B,N,4] / [B,4]) | EMBED_ONLY (ha / hc / action / logp /
+        value may be None and are not touched).
         variant: 0 = DEFAULT_VARIANT, 1 = one (tile, network) item per CTA (hidden state updated in place), 2 = two such CTAs per
         SM, 3 = both networks' chains of a tile interleaved in one CTA.  Variant 2 reads the previous hidden state from one
         buffer and writes the new one to another; afterwards the two tensors trade their storage, so for the caller `ha` / `hc`
@@ -114,6 +124,7 @@ class FusedRolloutStep:
         s.variant = int(variant)
         s.row_offset = int(row_offset)
         s.tile_rows = int(tile_rows)
+        s.flags = int(flags)
         P = _lib.ptr
         s.d_debug = P(debug) if debug is not None else None
         s.d_p_state, s.d_e_state, s.d_oxy, s.d_map_id, s.d_o_count = (P(engine.p_state), P(engine.e_state), P(oxy_i32),
@@ -128,7 +139,7 @@ class FusedRolloutStep:
             io.d_packed = self.packed[name].data_ptr()
             for k in range(self.depth):
                 io.d_hist[k] = P(hist[k]) if hist[k] is not None else None
-            assert hid.is_contiguous()
+            assert hid is None or hid.is_contiguous()
             io.d_emb_out, io.d_hidden, io.d_hidden_out = P(emb), P(hid), None
             if int(variant) == 2:                            # the two-CTA-per-SM kernel re-reads the previous state: separate output buffer
                 # the partner buffer belongs to THIS hidden-state tensor (env-group pipelines step their own states concurrently)

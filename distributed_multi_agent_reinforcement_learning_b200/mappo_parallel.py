@@ -35,6 +35,30 @@ PIPELINE_STAGGER = 0        # env steps by which consecutive env-group pipelines
 TWO_STREAM_TRAIN = True     # actor and critic branches of a training minibatch on two CUDA streams
 import os as _os
 CONCURRENT_MINIBATCHES = int(_os.environ.get("MARL_CONCURRENT_MB", "3"))  # minibatches of an epoch in flight at once (their clip-accumulate order is replayed afterwards)
+# A rollout stores the full [T+D,B,N,E] history of both networks when it takes at most this share of the device memory free at the
+# call (free to the driver plus what the caching allocator holds unused); otherwise it keeps a ring of D+1 slabs per network and
+# training regenerates each minibatch's history (HistoryReplay).  The share leaves the rest for the arena and the training epoch.
+STORE_HISTORY_SHARE = 0.5
+REPLAY_EMBED_ONLY = True    # the replay runs the embeddings-only fused step (MARL_POLICY_EMBED_ONLY), not the full step
+
+
+def history_bytes(T, B, N, E, D):
+    """Bytes of the stored history of both networks, [T+D,B,N,E] fp32 each."""
+    return 2 * (T + D) * B * N * E * 4
+
+
+def _history_inputs(hist_a, hist_c, t, D, quirks, net, slot, sl=slice(None)):
+    """The D history inputs of step t for `net` (k = 0 newest; None = zeros, before the episode's first step), read from the
+    [*, B, N, E] buffers at index slot(i) for history step i (t + D is what step t writes).  reference_quirks: the ONE list actor and
+    critic alias (:750-752), C(t-1), A(t-1), C(t-2), ...; otherwise each network's own embeddings."""
+    out = []
+    for k in range(D):
+        if quirks:
+            back, src = k // 2 + 1, (hist_c if k % 2 == 0 else hist_a)
+        else:
+            back, src = k + 1, (hist_a if net == "actor" else hist_c)
+        out.append(src[slot(t - back + D)][sl] if t - back >= 0 else None)
+    return out
 
 
 def orthogonal_init(layer, gain=1.0):
@@ -317,6 +341,8 @@ class TrainBatch:
     dict (`from_reference`, [B,T,...] dense fp32 as in DHGN/replay_buffer.py:28-40) or directly from a rollout."""
 
     KEYS = ("p", "e", "p_adj_bits", "e_adj", "o_adj_bits", "hist_a", "hist_c", "v", "a", "logp", "r", "active")
+    replay = None       # HistoryReplay of a batch whose history was not stored (hist_a = hist_c = None); minibatches regenerate it
+    map_id = None       # i32 [B] (replay only)
 
     def __init__(self, **kw):
         self.__dict__.update(kw)
@@ -337,12 +363,16 @@ class TrainBatch:
                    logp=tm(d["a_logprob_n"]).float(), r=tm(d["r"]).float(), active=tm(d["active"]).float(), depth=depth)
 
     def minibatch(self, lo, hi):
-        """Envs [lo, hi): contiguous copies of the time-major slabs (the reference's sequential `batch[key][index]`)."""
-        s = lambda x: x[:, lo:hi].contiguous()
+        """Envs [lo, hi): contiguous copies of the time-major slabs (the reference's sequential `batch[key][index]`).  A replay-mode
+        batch regenerates the minibatch's history from its slabs (on the current stream)."""
+        s = lambda x: None if x is None else x[:, lo:hi].contiguous()     # noqa: E731
         mb = TrainBatch(p=s(self.p), e=s(self.e), oxy=self.oxy[lo:hi].contiguous(),
                         o_count_train=self.o_count_train[lo:hi].contiguous(), p_adj_bits=s(self.p_adj_bits),
                         e_adj=s(self.e_adj), o_adj_bits=s(self.o_adj_bits), hist_a=s(self.hist_a), hist_c=s(self.hist_c),
                         v=s(self.v), a=s(self.a), logp=s(self.logp), r=s(self.r), active=s(self.active), depth=self.depth)
+        if self.replay is not None:
+            mb.replay, mb.map_id = self.replay, self.map_id[lo:hi].contiguous()
+            self.replay.regenerate(mb)
         return mb
 
     def minibatch_indexed(self, index):
@@ -366,10 +396,15 @@ class TrainBatch:
                                                    _lib.stream_ptr()), "marl_gather_rows")
             return out
 
-        return TrainBatch(p=g(self.p), e=g(self.e), oxy=g(self.oxy, False), o_count_train=g(self.o_count_train, False),
-                          p_adj_bits=g(self.p_adj_bits), e_adj=g(self.e_adj), o_adj_bits=g(self.o_adj_bits), hist_a=g(self.hist_a),
-                          hist_c=g(self.hist_c), v=g(self.v), a=g(self.a), logp=g(self.logp), r=g(self.r), active=g(self.active),
-                          depth=self.depth), g
+        gh = lambda x: None if x is None else g(x)      # noqa: E731
+        out = TrainBatch(p=g(self.p), e=g(self.e), oxy=g(self.oxy, False), o_count_train=g(self.o_count_train, False),
+                         p_adj_bits=g(self.p_adj_bits), e_adj=g(self.e_adj), o_adj_bits=g(self.o_adj_bits), hist_a=gh(self.hist_a),
+                         hist_c=gh(self.hist_c), v=g(self.v), a=g(self.a), logp=g(self.logp), r=g(self.r), active=g(self.active),
+                         depth=self.depth)
+        if self.replay is not None:
+            out.replay, out.map_id = self.replay, g(self.map_id, False)
+            self.replay.regenerate(out)
+        return out, g
 
     def graph(self):
         T, B, N = self.T, self.B, self.N
@@ -387,6 +422,44 @@ class TrainBatch:
         return [(h[D - 1 - k:], N * E, E) for k in range(D)]
 
 
+class HistoryReplay:
+    """What regenerating a rollout's history embeddings needs, carried by a replay-mode TrainBatch: the rollout-time weights (a
+    snapshot FusedRolloutStep, so the batch stays valid after `update()` steps the optimizer), the per-map boundary cells (i32) with the
+    rollout's REAL cell counts, and the aliasing rule.  The per-env inputs - fp32 states, packed adjacency, actions, map ids - are the
+    minibatch's own slabs.  The fused step's per-row output does not depend on how the batch is split into launches, and the arena
+    records are (float) of the fp64 states the rollout's step converted, so the regenerated history is the stored one bit for bit."""
+
+    def __init__(self, fused, oxy_i32, o_count, quirks):
+        self.fused, self.oxy_i32, self.o_count, self.quirks = fused, oxy_i32, o_count, bool(quirks)
+
+    def regenerate(self, mb, embed_only=None):
+        """Fills mb.hist_a / mb.hist_c [T+D, mb, N, E] with T fused steps on the current stream (forced actions, history read from the
+        tensors being filled).  embed_only (default REPLAY_EMBED_ONLY) False runs the full step from zero hidden states and returns the
+        replayed (log-prob, value) [T, mb, N] - the same numbers the rollout stored."""
+        from types import SimpleNamespace
+        embed_only = REPLAY_EMBED_ONLY if embed_only is None else embed_only
+        T, B, N, D, E = mb.T, mb.B, mb.N, mb.depth, self.fused.E
+        f32 = dict(dtype=torch.float32, device=mb.p.device)
+        mb.hist_a, mb.hist_c = torch.zeros(T + D, B, N, E, **f32), torch.zeros(T + D, B, N, E, **f32)
+        flags = fused_policy.STATE_F32 | (fused_policy.EMBED_ONLY if embed_only else 0)
+        ha = hc = act = logp = v = None
+        if not embed_only:
+            ha, hc = torch.zeros(2, B * N, E, **f32), torch.zeros(2, B * N, E, **f32)
+            act = mb.a.to(torch.int32)
+            logp, v = torch.empty(T, B, N, **f32), torch.empty(T, B, N, **f32)
+        view = SimpleNamespace(B=B, N=N, O=self.oxy_i32.shape[1], map_id=mb.map_id)
+        ident = lambda i: i      # noqa: E731
+        for t in range(T):
+            view.p_state, view.e_state = mb.p[t], mb.e[t]
+            view.p_adj_bits, view.e_adj, view.o_adj_bits = mb.p_adj_bits[t], mb.e_adj[t], mb.o_adj_bits[t]
+            h_a = _history_inputs(mb.hist_a, mb.hist_c, t, D, self.quirks, "actor", ident)
+            h_c = _history_inputs(mb.hist_a, mb.hist_c, t, D, self.quirks, "critic", ident)
+            self.fused.step(view, self.oxy_i32, self.o_count, t, 0, True, h_a, h_c, mb.hist_a[t + D], mb.hist_c[t + D], ha, hc,
+                            None if act is None else act[t], None if logp is None else logp[t], None if v is None else v[t],
+                            force_action=True, flags=flags)
+        return None if embed_only else (logp, v)
+
+
 class RolloutGraph:
     # (policy_dbg: see MAPPO._rollout_pipelined - an instrumented capture for measurements, not for production replays)
     """`MAPPO.rollout_batched` for all envs of an engine (networks in the loop) captured as ONE CUDA graph: per env step
@@ -394,10 +467,12 @@ class RolloutGraph:
     fused evader-move / step / reward-norm / store kernel; no host involvement on replay.  The engine state the episode starts
     from is whatever the engine holds at replay time."""
 
-    def __init__(self, mappo, engine, arena, T, seed, policy_dbg=None):
+    def __init__(self, mappo, engine, arena, T, seed, policy_dbg=None, history=None):
         snap = engine.snapshot()
         kw = {} if policy_dbg is None else dict(timers={"_policy_dbg": policy_dbg}, pipelines=policy_dbg.shape[1])
-        mappo.rollout_batched(engine, arena, T, seed=seed)           # eager warm-up (kernel attributes, stream pool)
+        # decided once: the warm-up's allocations would otherwise change the free memory the captured rollout sees
+        kw["history"] = history or mappo.history_mode(T, engine.B, engine.N)
+        mappo.rollout_batched(engine, arena, T, seed=seed, history=kw["history"])   # eager warm-up (kernel attributes, stream pool)
         torch.cuda.synchronize()
         engine.restore(snap)
         self.graph = torch.cuda.CUDAGraph()
@@ -635,21 +710,45 @@ class MAPPO:
         torch.save(self.critic.state_dict(), cwd + "critic.pth")
 
     # ------------------------------------------------------------------------------------------------ rollout
+    def history_mode(self, T, B, N):
+        """'store' when the full history of both networks fits STORE_HISTORY_SHARE of the free device memory, else 'replay'."""
+        free = torch.cuda.mem_get_info(self.device)[0] + torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
+        return "store" if history_bytes(T, B, N, self.embedding_dim, self.depth) <= STORE_HISTORY_SHARE * free else "replay"
+
     @torch.no_grad()
     def rollout_batched(self, engine, arena, T=None, seed=0, deterministic=False, groups=1, use_fused=None, timers=None,
-                        pipelines=None, actor_only=False):
+                        pipelines=None, actor_only=False, history=None):
         """MAPPO.run_episode (:742-827) for all B envs of a BatchedPursuitEnv at once, entirely on the GPU.
         Per step: observe kernel -> fused encoder (actor, then critic with all-ones adjacency) -> GRU cell -> heads ->
         closed-loop env kernel (evader move + pursuer step + reward-norm + store).  Fills `arena` plus the history /
         value / log-prob slabs and returns a TrainBatch ready for `train`.
 
         actor_only=True is the EVALUATOR's episode (evaluator.py:118-156): no critic, and the actor's history is its OWN
-        embeddings A(t-1), A(t-2), ... (its dataset is not aliased with a critic's there); values / bootstrap stay zero."""
+        embeddings A(t-1), A(t-2), ... (its dataset is not aliased with a critic's there); values / bootstrap stay zero.
+
+        history: 'store' keeps the full [T+D,B,N,E] history of both networks in the batch; 'replay' keeps only a ring of D+1 slabs
+        per network during the episode (step t reads at most D steps back) and returns a batch with hist_a = hist_c = None that
+        regenerates each minibatch's history in training (HistoryReplay).  None chooses with `history_mode` (store when it fits
+        comfortably).  Replay needs the fused step; actor_only rollouts always store."""
         T = T or arena.T
         B, N, E, D, L = engine.B, engine.N, self.embedding_dim, self.depth, self.num_layers
         dev = self.device
         f32 = dict(dtype=torch.float32, device=dev)
-        hist_a, hist_c = torch.zeros(T + D, B, N, E, **f32), torch.zeros(T + D, B, N, E, **f32)
+        if use_fused is None:
+            use_fused = fused_policy.supported(self)
+        if history not in (None, "store", "replay"):
+            raise ValueError(f"history={history!r}: None, 'store' or 'replay'")
+        if actor_only:
+            history = "store"
+        elif history is None:
+            history = self.history_mode(T, B, N)
+        replay = history == "replay"
+        if replay and not use_fused:
+            raise _lib.MarlError(f"rollout_batched: the history of this rollout ({history_bytes(T, B, N, E, D) / 1e9:.1f} GB) is not "
+                                 "stored, and regenerating it needs the fused policy step (embedding_dim = rnn_hidden_dim = 128, "
+                                 "2 GRU layers, depth 1..3, 9 actions)")
+        slot = (lambda i: i % (D + 1)) if replay else (lambda i: i)     # history step i -> index into hist_a / hist_c
+        hist_a, hist_c = (torch.zeros(D + 1 if replay else T + D, B, N, E, **f32) for _ in range(2))
         v = torch.zeros(T + 1, B, N, **f32)
         logp = torch.zeros(T, B, N, **f32)
         act = torch.zeros(T, B, N, dtype=torch.int32, device=dev)
@@ -670,7 +769,7 @@ class MAPPO:
                 own = actor_only or not quirks
                 back = (k + 1) if own else (k // 2 + 1)
                 src = (hist_a if (net == "actor" or actor_only) else hist_c) if own else (hist_c if k % 2 == 0 else hist_a)
-                out.append(src[t - back + D] if t - back >= 0 else zeros_hist)
+                out.append(src[slot(t - back + D)] if t - back >= 0 else zeros_hist)
             return out
 
         def critic_step(t, graph):
@@ -681,15 +780,15 @@ class MAPPO:
             w_eff = w.reshape(E).contiguous()
             return emb_c, feat_c[0]
 
-        if use_fused is None:
-            use_fused = fused_policy.supported(self)
         if use_fused:
             # ONE launch per env step for both networks (csrc/policy_fused.cu); embeddings / values / log-probs / actions
             # land directly in their rollout slabs.  The critic's effective head row is constant while the weights are
-            # (one power iteration on a [1,E] matrix is already converged), so it is computed once.
+            # (one power iteration on a [1,E] matrix is already converged), so it is computed once.  A replay-mode batch keeps the
+            # step (its own copy of the weights) to regenerate the history in training.
             w, _ = self.critic.head_weight()
-            fused = fused_policy.FusedRolloutStep(self, w.reshape(E).contiguous())
-            oxy_i = engine.boundary_xy.contiguous()
+            fused = fused_policy.FusedRolloutStep(self, w.reshape(E).contiguous(), snapshot=replay)
+            oxy_i = engine.boundary_xy.clone() if replay else engine.boundary_xy.contiguous()
+            rep_ = HistoryReplay(fused, oxy_i, o_count, quirks) if replay else None
             none_if_zero = lambda lst: [None if h is zeros_hist else h for h in lst]   # noqa: E731
             def timed(name, fn):
                 if timers is None:
@@ -712,8 +811,8 @@ class MAPPO:
             if pipelines > 1 and (timers is None or not auto) and groups == 1 and not actor_only:
                 # (an explicit pipelines=G together with timers: CUDA events around every launch of the pipelined schedule itself)
                 self._rollout_pipelined(engine, arena, T, seed, deterministic, int(pipelines), fused, oxy_i, o_count, hist_a, hist_c,
-                                        act, logp, v, zeros_hist, timers=timers)
-                return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp)
+                                        act, logp, v, zeros_hist, timers=timers, slot=slot)
+                return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp, rep_)
             # Single pipeline.  The A* replanning due every `difficulty` steps only needs the env state, not the action: it runs
             # on a side stream concurrently with the policy kernel and is joined before the env kernel consumes the paths.
             overlap = timers is None and groups == 1
@@ -735,7 +834,7 @@ class MAPPO:
                 timed("env_observe_kernel", engine.observe)
                 h_t, h_tc = none_if_zero(history(t)), none_if_zero(history(t, "critic"))
                 timed("policy_step_kernel", lambda: fused.step(engine, oxy_i, o_count, t, seed, deterministic, h_t, h_tc,
-                                                               hist_a[t + D], hist_c[t + D], ha, hc, act[t], logp[t], v[t],
+                                                               hist_a[slot(t + D)], hist_c[slot(t + D)], ha, hc, act[t], logp[t], v[t],
                                                                nets=("actor",) if actor_only else ("actor", "critic")))
                 if join is not None:
                     main.wait_event(join)
@@ -744,11 +843,11 @@ class MAPPO:
             if actor_only:
                 return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp)
             engine.observe()
-            h_fin = none_if_zero(([hist_c[T - 1 + D]] + history(T - 1)[:D - 1]) if quirks else history(T, "critic"))
+            h_fin = none_if_zero(([hist_c[slot(T - 1 + D)]] + history(T - 1)[:D - 1]) if quirks else history(T, "critic"))
             scratch = torch.empty(B, N, E, **f32)
             fused.step(engine, oxy_i, o_count, T, seed, deterministic, h_fin, h_fin, scratch, scratch, ha, hc, None, None, v[T],
                        nets=("critic",))
-            return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp)
+            return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp, rep_)
 
         for t in range(T):
             engine.observe()
@@ -787,7 +886,7 @@ class MAPPO:
         return max(1, min(8, (B * N) // 8192))
 
     def _rollout_pipelined(self, engine, arena, T, seed, deterministic, G, fused, oxy_i, o_count, hist_a, hist_c, act, logp, v,
-                           zeros_hist, timers=None):
+                           zeros_hist, timers=None, slot=lambda i: i):
         """G independent env-group pipelines, one stream (+ one A* side stream) each; see rollout_batched.
         timers: dict name -> list of (start, end) CUDA events recorded on the launching stream around every launch.  If it holds a
         "_policy_dbg" int64 tensor [T, G, >= CTAs per launch, 16], every policy launch instead writes its per-CTA record there (slots
@@ -847,14 +946,7 @@ class MAPPO:
                 sl = slice(lo, hi)
 
                 def hist_of(t, net="actor"):
-                    out = []
-                    for k in range(D):
-                        if self.reference_quirks:      # the aliased list: C(t-1), A(t-1), C(t-2), ...
-                            back, src = k // 2 + 1, (hist_c if k % 2 == 0 else hist_a)
-                        else:                          # each network's own embeddings
-                            back, src = k + 1, (hist_a if net == "actor" else hist_c)
-                        out.append(src[t - back + D][sl] if t - back >= 0 else None)
-                    return out
+                    return _history_inputs(hist_a, hist_c, t, D, self.reference_quirks, net, slot, sl)
 
                 def refresh():
                     view.p_state, view.e_state, view.map_id = engine.p_state[sl], engine.e_state[sl], engine.map_id[sl]
@@ -873,7 +965,7 @@ class MAPPO:
                     timed("env_observe_kernel", st, lambda: engine.observe(lo=lo, hi=hi))
                     h_t, h_tc = hist_of(t), hist_of(t, "critic")
                     timed("policy_step_kernel", st, lambda: fused.step(
-                        view, oxy_i, o_count, t, seed, deterministic, h_t, h_tc, hist_a[t + D][sl], hist_c[t + D][sl], ha, hc,
+                        view, oxy_i, o_count, t, seed, deterministic, h_t, h_tc, hist_a[slot(t + D)][sl], hist_c[slot(t + D)][sl], ha, hc,
                         act[t][sl], logp[t][sl], v[t][sl], row_offset=lo * N, tile_rows=full_tile,
                         debug=dbg[t, g] if dbg is not None else None))
                     if stagger > 0 and t == min(stagger, T - 1) - 1 and g + 1 < G:
@@ -883,7 +975,7 @@ class MAPPO:
                         st.wait_event(join)
                     timed("rollout_kernel", st, lambda: engine._closed_chunk(arena, rec_ptrs, lo, hi, t, 1, act[t:t + 1], 0, seed, st))
                 engine.observe(lo=lo, hi=hi)
-                h_fin = ([hist_c[T - 1 + D][sl]] + hist_of(T - 1)[:D - 1]) if self.reference_quirks else hist_of(T, "critic")
+                h_fin = ([hist_c[slot(T - 1 + D)][sl]] + hist_of(T - 1)[:D - 1]) if self.reference_quirks else hist_of(T, "critic")
                 scratch = torch.empty(hi - lo, N, E, dtype=torch.float32, device=dev)
                 fused.step(view, oxy_i, o_count, T, seed, deterministic, h_fin, h_fin, scratch, scratch, ha, hc, None, None, v[T][sl],
                            nets=("critic",), row_offset=lo * N, tile_rows=full_tile)
@@ -891,7 +983,7 @@ class MAPPO:
                 done.record(st)
             main.wait_event(done)
 
-    def explore_batched(self, engine, arena, T=None, seed=0, host_state=None, host_out=None, reset_reward_norm=False):
+    def explore_batched(self, engine, arena, T=None, seed=0, host_state=None, host_out=None, reset_reward_norm=False, history=None):
         """The batched counterpart of `explore_env` (:731-740) - the call a user makes once per training iteration: one whole
         episode of ALL envs of `engine` with both networks in the loop, replayed from a CUDA graph that is captured on the first
         call (per engine / arena / T / seed; the weight images are re-packed inside the graph, so it follows the optimizer).
@@ -901,12 +993,15 @@ class MAPPO:
         episode bookkeeping; `reset_reward_norm` additionally restarts the running reward statistics).
         host_out: optional dict of HOST tensors filled after the episode - `episode_reward` i64 [B] (sum of the raw rewards over
         pursuers and steps, the evaluator's return), `collision` u8 [B]; the call then synchronises the stream.
-        Returns the TrainBatch of the episode (device resident, ready for `train`)."""
+        history: as in `rollout_batched`, chosen when the graph is captured.
+        Returns the TrainBatch of the episode (device resident, ready for `train`).  It lives in the graph's memory: it is valid until
+        the next call with the same engine / arena / T / seed, which overwrites it - for a replay-mode batch this includes the weight
+        snapshot its history is regenerated with (the graph re-packs it in place)."""
         T = T or arena.T
         key = (id(engine), id(arena), int(T), int(seed))
         graphs = self.__dict__.setdefault("_episode_graphs", {})
         if key not in graphs:
-            graphs[key] = RolloutGraph(self, engine, arena, T, seed)
+            graphs[key] = RolloutGraph(self, engine, arena, T, seed, history=history)
         g = graphs[key]
         if host_state is not None:
             engine.load_host_state(reset_reward_norm=reset_reward_norm, **host_state)
@@ -922,8 +1017,10 @@ class MAPPO:
                 raise _lib.MarlError(f"explore_batched: evader status {int(status)} (A* OPEN / path overflow or target tape exhausted)")
         return g.batch
 
-    def _train_batch(self, engine, arena, T, oxy, hist_a, hist_c, v, logp):
+    def _train_batch(self, engine, arena, T, oxy, hist_a, hist_c, v, logp, replay=None):
         B, D, dev = engine.B, self.depth, self.device
+        if replay is not None:         # the ring holds the last D+1 steps only: the history is regenerated per minibatch
+            hist_a = hist_c = None
         oxy_env = oxy[engine.map_id.long()].contiguous()
         if self.reference_quirks:      # the critic's all-ones adjacency spans all O padded slots in training (:65,677): 76 phantom cells at (0,0)
             o_count_train = torch.full((B,), engine.O, dtype=torch.int32, device=dev)
@@ -933,7 +1030,8 @@ class MAPPO:
                           o_count_train=o_count_train,
                           p_adj_bits=arena.p_adj_bits[:T], e_adj=arena.e_adj[:T], o_adj_bits=arena.o_adj_bits[:T],
                           hist_a=hist_a, hist_c=hist_c, v=v, a=arena.a_n[:T], logp=logp, r=arena.r[:T],
-                          active=arena.active[:T], depth=D)
+                          active=arena.active[:T], depth=D, replay=replay,
+                          map_id=None if replay is None else engine.map_id.to(torch.int32).clone())
 
     def explore_env(self, env, num_episode):
         """Reference signature (:731-740) for the single-env facade `Pursuit_Env`: returns

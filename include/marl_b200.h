@@ -408,8 +408,8 @@ typedef struct marl_policy_step {
     int32_t variant;             /* 0 = choose; 1 = one (tile, network) item per CTA (16 worker warps); 2 = two CTAs per SM; 3 = the actor and
                                     the critic chain of a tile interleaved in one CTA (both networks given); 2 and 3 need d_hidden_out */
     uint64_t seed;               /* sampling: same counter RNG as marl_act_head (keyed by seed, row, t) */
-    const double *d_p_state;     /* [B,N,4] */
-    const double *d_e_state;     /* [B,4] */
+    const void *d_p_state;       /* [B,N,4] double (float with MARL_POLICY_STATE_F32) */
+    const void *d_e_state;       /* [B,4] double (float with MARL_POLICY_STATE_F32) */
     const int32_t *d_oxy;        /* [M,O,2] boundary cells per map (marl_raser_map_build) */
     const int32_t *d_map_id;     /* [B] or NULL */
     const int32_t *d_o_count;    /* [M] real boundary cells per map, clamped to O */
@@ -423,8 +423,15 @@ typedef struct marl_policy_step {
     int32_t tile_rows;           /* 0 = choose the rows per work item with the wave model (a lone launch: fill the last wave); > 0 = that
                                     many rows (a multiple of N, <= 128) - launches that run concurrently with others (env-group
                                     pipelines) use full tiles and leave SMs free for their neighbours */
-    int32_t reserved;
+    int32_t flags;               /* MARL_POLICY_* bits; any other bit set is MARL_EINVAL */
 } marl_policy_step;
+/* marl_policy_step.flags.  Both modes are separate kernel instantiations: flags = 0 runs exactly the default kernels.
+ * STATE_F32: d_p_state / d_e_state point to float [B,N,4] / [B,4] (the rollout arena's per-step records, (float) of the fp64
+ *   state - the very values the kernel converts the fp64 state to) instead of double.  Not with variant 2.
+ * EMBED_ONLY: run the encoder and FCRA chain only and write d_emb_out; no GRU, cells or heads.  d_hidden, d_hidden_out,
+ *   d_action, d_logp and d_value may be NULL.  Used to regenerate the history embeddings of a stored episode. */
+#define MARL_POLICY_STATE_F32 1
+#define MARL_POLICY_EMBED_ONLY 2
 /* Pre-splits (two-term fp16: hi = fp16(w), lo = fp16(w - hi)) and pre-swizzles every dense layer of one network into the shared-memory image the fused kernel
  * streams; call once per weight update. */
 int64_t marl_policy_pack_bytes(int32_t depth, int32_t is_actor);
