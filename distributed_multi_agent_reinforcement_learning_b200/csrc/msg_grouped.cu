@@ -190,11 +190,12 @@ msg_fwd_grouped_kernel(MsgArgs a, const float *__restrict__ W0, const float *__r
 
 // ------------------------------------------------------------------------------------------------------------ backward
 // One launch per relation (REL): keeps the per-lane weight slices and gradient accumulators of only that relation in registers.
-// Persistent warps walk samples with a grid stride; CTA reduction through shared memory, then one atomicAdd per element.
-template <int NA, int REL>
+// Persistent warps walk samples with a grid stride; CTA reduction through shared memory, then either one atomicAdd per element
+// (DET false) or the CTA's row of partial sums to ws[blockIdx.x], reduced in a fixed order by launch_msg_partials_reduce (DET true).
+template <int NA, int REL, bool DET>
 __global__ void __launch_bounds__(128)
 msg_bwd_grouped_kernel(MsgArgs a, const float *__restrict__ W, const float *__restrict__ b, const float *__restrict__ d_agg,
-                       float *__restrict__ gW, float *__restrict__ gb)
+                       float *__restrict__ gW, float *__restrict__ gb, float *__restrict__ ws)
 {
     constexpr int KW = REL == 0 ? 8 : 4;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, N = a.N;
@@ -336,9 +337,13 @@ msg_bwd_grouped_kernel(MsgArgs a, const float *__restrict__ W, const float *__re
     __syncthreads();
     for (int idx = threadIdx.x; idx < (KW + 1) * E; idx += 128) {
         const float v = (s_red[0][idx] + s_red[1][idx]) + (s_red[2][idx] + s_red[3][idx]);
-        const int k = idx / E, c = idx - k * E;
-        if (k < KW) atomicAdd(gW + c * KW + k, v);
-        else atomicAdd(gb + c, v);
+        if (DET) {
+            ws[(int64_t)blockIdx.x * (KW + 1) * E + idx] = v;
+        } else {
+            const int k = idx / E, c = idx - k * E;
+            if (k < KW) atomicAdd(gW + c * KW + k, v);
+            else atomicAdd(gb + c, v);
+        }
     }
 }
 
@@ -356,25 +361,41 @@ int launch_msg_fwd_grouped(const MsgArgs &a, const float *W0, const float *b0, c
     return check_launch("msg_fwd_grouped_kernel");
 }
 
+template <int NA, bool DET>
+static int launch_bwd_na(const MsgArgs &a, const float *W0, const float *b0, const float *W1, const float *b1, const float *W2, const float *b2,
+                         const float *d_agg, float *gW0, float *gb0, float *gW1, float *gb1, float *gW2, float *gb2, float *ws,
+                         cudaStream_t stream)
+{
+    const int64_t blocks = msg_bwd_grouped_blocks(a), E = mg::E;
+    float *ws1 = DET ? ws + blocks * 9 * E : nullptr, *ws2 = DET ? ws + blocks * 14 * E : nullptr;
+    mg::msg_bwd_grouped_kernel<NA, 0, DET><<<(unsigned)blocks, 128, 0, stream>>>(a, W0, b0, d_agg, gW0, gb0, ws);
+    mg::msg_bwd_grouped_kernel<NA, 1, DET><<<(unsigned)blocks, 128, 0, stream>>>(a, W1, b1, d_agg, gW1, gb1, ws1);
+    mg::msg_bwd_grouped_kernel<NA, 2, DET><<<(unsigned)blocks, 128, 0, stream>>>(a, W2, b2, d_agg, gW2, gb2, ws2);
+    int rc = check_launch("msg_bwd_grouped_kernel");
+    if (rc || !DET) return rc;
+    MsgPartials p;
+    p.rel_base[0] = ws; p.rel_base[1] = ws1; p.rel_base[2] = ws2;
+    p.rel_stride[0] = 9 * E; p.rel_stride[1] = 5 * E; p.rel_stride[2] = 5 * E;
+    p.blocks = (int)blocks; p.E = (int)E;
+    return launch_msg_partials_reduce(p, gW0, gb0, gW1, gb1, gW2, gb2, stream);
+}
+
 template <int NA>
 static int launch_bwd_na(const MsgArgs &a, const float *W0, const float *b0, const float *W1, const float *b1, const float *W2, const float *b2,
-                         const float *d_agg, float *gW0, float *gb0, float *gW1, float *gb1, float *gW2, float *gb2, cudaStream_t stream)
+                         const float *d_agg, float *gW0, float *gb0, float *gW1, float *gb1, float *gW2, float *gb2, float *ws,
+                         cudaStream_t stream)
 {
-    int64_t blocks = (a.S + 3) / 4;
-    if (blocks > 148 * 8) blocks = 148 * 8;
-    mg::msg_bwd_grouped_kernel<NA, 0><<<(unsigned)blocks, 128, 0, stream>>>(a, W0, b0, d_agg, gW0, gb0);
-    mg::msg_bwd_grouped_kernel<NA, 1><<<(unsigned)blocks, 128, 0, stream>>>(a, W1, b1, d_agg, gW1, gb1);
-    mg::msg_bwd_grouped_kernel<NA, 2><<<(unsigned)blocks, 128, 0, stream>>>(a, W2, b2, d_agg, gW2, gb2);
-    return check_launch("msg_bwd_grouped_kernel");
+    if (ws) return launch_bwd_na<NA, true>(a, W0, b0, W1, b1, W2, b2, d_agg, gW0, gb0, gW1, gb1, gW2, gb2, ws, stream);
+    return launch_bwd_na<NA, false>(a, W0, b0, W1, b1, W2, b2, d_agg, gW0, gb0, gW1, gb1, gW2, gb2, ws, stream);
 }
 
 int launch_msg_bwd_grouped(const MsgArgs &a, const float *W0, const float *b0, const float *W1, const float *b1, const float *W2,
                            const float *b2, const float *d_agg, float *gW0, float *gb0, float *gW1, float *gb1, float *gW2, float *gb2,
-                           cudaStream_t stream)
+                           float *ws, cudaStream_t stream)
 {
-    if (a.N <= 4) return launch_bwd_na<4>(a, W0, b0, W1, b1, W2, b2, d_agg, gW0, gb0, gW1, gb1, gW2, gb2, stream);
-    if (a.N <= 8) return launch_bwd_na<8>(a, W0, b0, W1, b1, W2, b2, d_agg, gW0, gb0, gW1, gb1, gW2, gb2, stream);
-    return launch_bwd_na<16>(a, W0, b0, W1, b1, W2, b2, d_agg, gW0, gb0, gW1, gb1, gW2, gb2, stream);
+    if (a.N <= 4) return launch_bwd_na<4>(a, W0, b0, W1, b1, W2, b2, d_agg, gW0, gb0, gW1, gb1, gW2, gb2, ws, stream);
+    if (a.N <= 8) return launch_bwd_na<8>(a, W0, b0, W1, b1, W2, b2, d_agg, gW0, gb0, gW1, gb1, gW2, gb2, ws, stream);
+    return launch_bwd_na<16>(a, W0, b0, W1, b1, W2, b2, d_agg, gW0, gb0, gW1, gb1, gW2, gb2, ws, stream);
 }
 
 }  // namespace marl

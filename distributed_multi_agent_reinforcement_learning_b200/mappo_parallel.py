@@ -328,6 +328,23 @@ class _FlatAdam:
         self.flat_grad.zero_()
         self._sync_grads()
 
+    def state_dict(self):
+        """Adam state as CPU tensors and plain values: both moments, the step count and the current learning rate."""
+        return dict(exp_avg=self.exp_avg.cpu(), exp_avg_sq=self.exp_avg_sq.cpu(), step_count=int(self.step_count),
+                    lr=float(self.param_groups[0]["lr"]))
+
+    def load_state_dict(self, sd):
+        """Copies a `state_dict()` into the existing arenas in place: the parameters stay views into `flat_param`."""
+        for k in ("exp_avg", "exp_avg_sq"):
+            if tuple(sd[k].shape) != tuple(self.exp_avg.shape) or sd[k].dtype != self.exp_avg.dtype:
+                raise _lib.MarlError(f"Adam state: {k} is {tuple(sd[k].shape)} {sd[k].dtype}, the optimizer's arena is "
+                                     f"{tuple(self.exp_avg.shape)} {self.exp_avg.dtype}")
+        self.exp_avg.copy_(sd["exp_avg"])
+        self.exp_avg_sq.copy_(sd["exp_avg_sq"])
+        self.step_count = int(sd["step_count"])
+        for g in self.param_groups:
+            g["lr"] = float(sd["lr"])
+
     def step(self):
         self._sync_grads()
         self.step_count += 1

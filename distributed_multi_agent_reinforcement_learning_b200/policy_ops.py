@@ -301,10 +301,14 @@ class _MessageAgg(torch.autograd.Function):
     def backward(ctx, d_agg):
         ws = ctx.saved_tensors
         E = ws[0].shape[0]
+        g = ctx.graph
         grads = [torch.zeros_like(t) for t in ws]
-        _lib.check(_L().marl_dhgn_message_bwd(*ctx.graph._args(E, ctx.all_ones), *[_lib.ptr(t) for t in ws],
-                                              _lib.ptr(d_agg.contiguous()), *[_lib.ptr(g) for g in grads],
-                                              _lib.stream_ptr()), "marl_dhgn_message_bwd")
+        # fixed-order reduction (bit-reproducible gradients); the workspace comes from the caching allocator on this stream, so
+        # the actor / critic streams of concurrent minibatches never share one
+        part = torch.empty(int(_L().marl_dhgn_message_bwd_workspace_bytes(g.N, g.O, E)), dtype=torch.uint8, device=d_agg.device)
+        _lib.check(_L().marl_dhgn_message_bwd_det(*g._args(E, ctx.all_ones), *[_lib.ptr(t) for t in ws],
+                                                  _lib.ptr(d_agg.contiguous()), *[_lib.ptr(t) for t in grads], _lib.ptr(part),
+                                                  _lib.stream_ptr()), "marl_dhgn_message_bwd_det")
         return (None, None, *grads)
 
 
@@ -464,9 +468,10 @@ class _PPOHead(torch.autograd.Function):
         dlogits, dvalue, sums = torch.empty(R, A, **f32), torch.empty(R, **f32), torch.zeros(3, **f32)
         args = [None if t is None else t.contiguous()      # v_old None: the unclipped value loss (use_value_clip = False)
                 for t in (feat_a, feat_c, Wa, ba, w_eff, bc, action, old_logp, adv, v_old, v_target, active)]
-        _lib.check(_L().marl_ppo_head(R, E, A, *[_lib.ptr(t) for t in args], ctypes.c_float(eps), ctypes.c_float(ent_coef),
-                                      _lib.ptr(logp), _lib.ptr(ent), _lib.ptr(val), _lib.ptr(dlogits), _lib.ptr(dvalue),
-                                      _lib.ptr(sums), _lib.stream_ptr()), "marl_ppo_head")
+        part = torch.empty(int(_L().marl_ppo_head_workspace_bytes(R)), dtype=torch.uint8, device=dev)   # fixed-order loss sums
+        _lib.check(_L().marl_ppo_head_det(R, E, A, *[_lib.ptr(t) for t in args], ctypes.c_float(eps), ctypes.c_float(ent_coef),
+                                          _lib.ptr(logp), _lib.ptr(ent), _lib.ptr(val), _lib.ptr(dlogits), _lib.ptr(dvalue),
+                                          _lib.ptr(sums), _lib.ptr(part), _lib.stream_ptr()), "marl_ppo_head_det")
         ctx.save_for_backward(args[0], args[1], args[2], w_eff, dlogits, dvalue, sums, sigma, u2, v)
         ctx.mark_non_differentiable(logp, ent, val, u2, v)
         return sums[0] / sums[2], sums[1] / sums[2], logp, ent, val, u2, v

@@ -380,6 +380,36 @@ class BatchedPursuitEnv:
         for n, t in snap.items():
             getattr(self, n).copy_(t)
 
+    # everything that persists from one training iteration to the next: the snapshot (Welford statistics included), the map
+    # assignment, the target tape and the map / sensor tables (a pool installed once with MapPool.install survives a resume)
+    _STATE = ("p_state", "e_state", "target", "path", "path_len", "time_step", "collision", "done", "tape_pos", "evader_status",
+              "wf_n", "wf_mean", "wf_S", "wf_std", "map_id", "target_tape", "grid_bits", "inflated_bits", "boundary_bits",
+              "boundary_count", "boundary_xy", "raser_bits")
+
+    def state_dict(self):
+        """CPU copies of the engine's persistent tensors, plus the target-tape length."""
+        sd = {n: getattr(self, n).cpu() for n in self._STATE}
+        sd["tape_len"] = int(self._tape_len)
+        return sd
+
+    def load_state_dict(self, sd):
+        """Inverse of `state_dict`.  Every tensor is checked against this engine's shapes and dtypes before any is written (the
+        target tape may have another length); raises MarlError naming the first mismatch."""
+        for n in self._STATE:
+            if n not in sd:
+                raise _lib.MarlError(f"engine state: {n} missing")
+            src, dst = sd[n], getattr(self, n)
+            same = tuple(src.shape) == tuple(dst.shape) or (n == "target_tape" and src.dim() == 3 and src.shape[0] == self.B
+                                                             and src.shape[2] == 2)
+            if not same or src.dtype != dst.dtype:
+                raise _lib.MarlError(f"engine state: {n} is {tuple(src.shape)} {src.dtype}, this engine's is {tuple(dst.shape)} {dst.dtype}")
+        for n in self._STATE:
+            if n == "target_tape" and tuple(sd[n].shape) != tuple(self.target_tape.shape):
+                self.target_tape = sd[n].to(self.device).contiguous()
+            else:
+                getattr(self, n).copy_(sd[n])
+        self._tape_len = int(sd["tape_len"])
+
 
 class EpisodeGraph:
     """One whole closed-loop episode (2*ceil(T/difficulty) kernel launches) captured in a CUDA graph, so replaying

@@ -346,6 +346,18 @@ int marl_dhgn_message_bwd(int32_t S, int32_t N, int32_t O, int32_t E, const floa
                           int32_t all_ones, const float *d_W0, const float *d_b0, const float *d_W1, const float *d_b1,
                           const float *d_W2, const float *d_b2, const float *d_grad_agg, float *d_gW0, float *d_gb0,
                           float *d_gW1, float *d_gb1, float *d_gW2, float *d_gb2, void *stream);
+/* The same backward with a deterministic reduction: every CTA writes its partial weight / bias sums to d_workspace, and a
+ * second kernel adds them in a fixed order into the gradients (+=), so two calls on the same inputs give the same bits.
+ * marl_dhgn_message_bwd reduces with fp32 atomics instead, whose order varies from run to run.  d_workspace: at least
+ * marl_dhgn_message_bwd_workspace_bytes(N, O, E) bytes, which does not depend on S (-1 for an unsupported N, O or E).  A
+ * workspace must not be shared by calls that may run at the same time. */
+int64_t marl_dhgn_message_bwd_workspace_bytes(int32_t N, int32_t O, int32_t E);
+int marl_dhgn_message_bwd_det(int32_t S, int32_t N, int32_t O, int32_t E, const float *d_p, const float *d_e,
+                              const float *d_oxy, const int32_t *d_o_index, const int32_t *d_o_count,
+                              const uint32_t *d_p_adj_bits, const uint8_t *d_e_adj, const uint32_t *d_o_adj_bits,
+                              int32_t all_ones, const float *d_W0, const float *d_b0, const float *d_W1, const float *d_b1,
+                              const float *d_W2, const float *d_b2, const float *d_grad_agg, float *d_gW0, float *d_gb0,
+                              float *d_gW1, float *d_gb1, float *d_gW2, float *d_gb2, void *d_workspace, void *stream);
 /* L1norm(adj) @ hist of DHGN.fcra (:204-233): out[s,i,:] = mean over neighbours j of hist[s*sample_stride + j*agent_stride]. */
 int marl_fcra_agg(int32_t S, int32_t N, int32_t E, const float *d_hist, int64_t sample_stride, int64_t agent_stride,
                   const uint32_t *d_p_adj_bits, int32_t all_ones, float *d_out, void *stream);
@@ -364,6 +376,15 @@ int marl_ppo_head(int64_t R, int32_t E, int32_t A, const float *d_feat_a, const 
                   const float *d_old_logp, const float *d_adv, const float *d_v_old, const float *d_v_target,
                   const float *d_active, float eps, float ent_coef, float *d_logp, float *d_entropy, float *d_value,
                   float *d_dlogits, float *d_dvalue, float *d_sums, void *stream);
+/* marl_ppo_head with the three sums reduced in a fixed order (per-CTA partials in d_workspace, then one reduction kernel)
+ * instead of fp32 atomics: bit-identical results from call to call.  d_workspace: at least marl_ppo_head_workspace_bytes(R)
+ * bytes (-1 for R <= 0), not shared by calls that may run at the same time. */
+int64_t marl_ppo_head_workspace_bytes(int64_t R);
+int marl_ppo_head_det(int64_t R, int32_t E, int32_t A, const float *d_feat_a, const float *d_feat_c, const float *d_Wa,
+                      const float *d_ba, const float *d_wc_eff, const float *d_bc, const float *d_action,
+                      const float *d_old_logp, const float *d_adv, const float *d_v_old, const float *d_v_target,
+                      const float *d_active, float eps, float ent_coef, float *d_logp, float *d_entropy, float *d_value,
+                      float *d_dlogits, float *d_dvalue, float *d_sums, void *d_workspace, void *stream);
 /* Rollout-time heads (:440-449, :513): softmax -> sample (counter RNG keyed by seed,row,t) or argmax -> log-prob; value. */
 int marl_act_head(int64_t R, int32_t E, int32_t A, const float *d_feat_a, const float *d_feat_c, const float *d_Wa,
                   const float *d_ba, const float *d_wc_eff, const float *d_bc, uint64_t seed, int32_t t,

@@ -6,7 +6,12 @@ reset -> batched rollout (all envs, networks in the loop) -> MAPPO.train -> all-
     python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 tools/train_loop.py --envs 512
 
 Prints one line per iteration: mean episode reward per env (sum over pursuers and steps, the quantity the reference's
-evaluator tracks), fraction of envs with a collision, losses, rollout / train wall times."""
+evaluator tracks), fraction of envs with a collision, losses, rollout / train wall times, then after "exact" the iteration, the step
+count, and the reward and losses as float.hex.  Training is bit-reproducible, so two runs with the same arguments print the same exact
+columns:  diff <(grep -o 'exact.*' a.log) <(grep -o 'exact.*' b.log)
+
+    python tools/train_loop.py --envs 512 --iters 3 --save-dir ck       # saves ck/training_state_rank0.pt after every iteration
+    python tools/train_loop.py --envs 512 --iters 6 --resume ck         # continues with iteration 3, as if never stopped"""
 import argparse
 import os
 import sys
@@ -18,6 +23,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from distributed_multi_agent_reinforcement_learning_b200 import default_config, parallel  # noqa: E402
+from distributed_multi_agent_reinforcement_learning_b200.checkpoint import load_training_state, save_training_state  # noqa: E402
 from distributed_multi_agent_reinforcement_learning_b200.mappo_parallel import MAPPO  # noqa: E402
 from distributed_multi_agent_reinforcement_learning_b200.pursuit_env import BatchedPursuitEnv, RolloutArena  # noqa: E402
 
@@ -33,7 +39,12 @@ def main():
     ap.add_argument("--allreduce", default=None, choices=[None, "update", "minibatch"],
                     help="gradient exchange: once per update (reference, default) or once per PPO minibatch")
     ap.add_argument("--host-reset", action="store_true", help="generate episodes on the host with the reference's generators (slow)")
+    ap.add_argument("--save-dir", default=None, help="write the training state (one file per rank) to this directory")
+    ap.add_argument("--save-every", type=int, default=1, help="iterations between saves (the last iteration is always saved)")
+    ap.add_argument("--resume", default=None, help="continue from the training state in this directory")
     args = ap.parse_args()
+    if args.save_every < 1:
+        ap.error("--save-every must be >= 1")
     rank, world, local = (int(os.environ.get(k, d)) for k, d in (("RANK", 0), ("WORLD_SIZE", 1), ("LOCAL_RANK", 0)))
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -48,9 +59,13 @@ def main():
     torch.manual_seed(0)
     mappo = MAPPO(cfg, B, max(1, round(B / 10)), "Learner")
     mappo.sync_weights(0)
-    total_steps = 0
+    total_steps, start = 0, 0
+    state_file = lambda d: os.path.join(d, f"training_state_rank{rank}.pt")     # noqa: E731  (env shards and reward statistics are per rank)
+    if args.resume:
+        extra = load_training_state(state_file(args.resume), mappo, env)
+        start, total_steps = int(extra["next_iter"]), int(extra["total_steps"])
     W, H = cfg.map.map_size
-    for it in range(args.iters):
+    for it in range(start, args.iters):
         t0 = time.perf_counter()
         if args.host_reset:
             env.reset(seed=1000 * rank + it)                   # host generation with the reference's placement rules
@@ -78,9 +93,13 @@ def main():
         if world > 1:
             torch.distributed.all_reduce(stats)
             stats /= world
+        if args.save_dir and ((it + 1) % args.save_every == 0 or it + 1 == args.iters):
+            save_training_state(state_file(args.save_dir), mappo, env, extra=dict(next_iter=it + 1, total_steps=total_steps))
         if rank == 0:
-            print(f"iter {it:3d}  steps {total_steps:9d}  ep_reward {stats[0]:9.2f}  collided {stats[1]:5.2f}  objC {stats[2]:8.4f}  "
-                  f"objA {stats[3]:8.4f}  reset {t1 - t0:5.2f}s  rollout {1e3 * (t2 - t1):7.1f}ms  train {1e3 * (t3 - t2):7.1f}ms", flush=True)
+            s = [float(x) for x in stats.cpu()]
+            print(f"iter {it:3d}  steps {total_steps:9d}  ep_reward {s[0]:9.2f}  collided {s[1]:5.2f}  objC {s[2]:8.4f}  "
+                  f"objA {s[3]:8.4f}  reset {t1 - t0:5.2f}s  rollout {1e3 * (t2 - t1):7.1f}ms  train {1e3 * (t3 - t2):7.1f}ms  "
+                  f"exact {it} {total_steps} {s[0].hex()} {s[2].hex()} {s[3].hex()}", flush=True)
     if world > 1:
         torch.distributed.destroy_process_group()
 
