@@ -2,8 +2,9 @@
 // astar.py:26-161, Occupied_Grid_Map.py:119-191).
 //
 // Replanning: one warp (= one CTA) per environment, whole search state in shared memory: the blocked-node bitmap
-// as one 64-bit column per x, g (fp64 — exact tie-breaking needs the reference's summation order), parent (u16)
-// and the OPEN set.  heapq's pop order is the total order of (f, (x, y)) tuples (ties only between identical
+// as CW 64-bit words per x, g (fp64 — exact tie-breaking needs the reference's summation order), parent (u16)
+// and the OPEN set.  The search lattice is [0, W] x [0, H], H + 1 rows: CW = 1 for H <= 63, CW = 2 for 64 <= H <= 127 (so
+// H = 64 already takes the second word); node ids are x * 64 CW + y.  Shifts along y carry across the words.  heapq's pop order is the total order of (f, (x, y)) tuples (ties only between identical
 // items), so ANY correct priority queue pops the same sequence.  The search is one warp walking a dependent chain (about six
 // cycles per instruction), so a pop is built to be SHORT and independent of |OPEN|: OPEN is an unsorted shared-memory array cut
 // into 32 stripes (slot i belongs to stripe i % 32, stored stripe-major); lane l keeps the minimum of stripe l in registers, so
@@ -38,95 +39,147 @@ struct EvaderArgs {
     double *e_tape2;   // optional [2,B,4]: evader state before / after this attacker_step
 };
 
-__device__ __forceinline__ uint64_t col_of(const uint32_t *bits, int HW, int x)
+// Column x of a bit-packed [W,HW] map as CW 64-bit words (words past HW read as zero)
+template <int CW>
+__device__ __forceinline__ void col_of(uint64_t (&v)[CW], const uint32_t *bits, int HW, int x)
 {
-    uint64_t v = bits[x * HW];
-    if (HW > 1) v |= (uint64_t)bits[x * HW + 1] << 32;
-    return v;
+#pragma unroll
+    for (int k = 0; k < CW; ++k) {
+        v[k] = (k == 0 || 2 * k < HW) ? (uint64_t)bits[x * HW + 2 * k] : 0ull;
+        if (2 * k + 1 < HW) v[k] |= (uint64_t)bits[x * HW + 2 * k + 1] << 32;
+    }
 }
 
-// OR of the column shifted by -e..e (Chebyshev inflation along y), clipped to H bits
-__device__ __forceinline__ uint64_t dilate_y(uint64_t c, int e, uint64_t hmask)
+// Mask of the rows [0, n) of word k (n - 64 k >= 0)
+__device__ __forceinline__ uint64_t low_rows(int n) { return n >= 64 ? ~0ull : ((1ull << n) - 1ull); }
+
+// Word k of the column shifted by -e..e (Chebyshev inflation along y; bits carry across the words), clipped to H bits.  e <= 8.
+template <int CW>
+__device__ __forceinline__ uint64_t dilate_y(const uint64_t *c, int k, int e, uint64_t hmask)
 {
-    uint64_t r = c;
-    for (int d = 1; d <= e; ++d) r |= (c << d) | (c >> d);
+    uint64_t r = c[k];
+    for (int d = 1; d <= e; ++d) {
+        r |= (c[k] << d) | (c[k] >> d);
+        if (k > 0) r |= c[k - 1] >> (64 - d);
+        if (k + 1 < CW) r |= c[k + 1] << (64 - d);
+    }
     return r & hmask;
 }
+
+// Word and bit of row y in a column of CW words
+template <int CW> __device__ __forceinline__ int row_word(int y) { return CW == 1 ? 0 : y >> 6; }
+template <int CW> __device__ __forceinline__ int row_bit(int y) { return CW == 1 ? y : y & 63; }
 
 struct SearchSmem {
     double *g;        // [NODES]
     double *of;       // [kOpenCap] f of OPEN entries, stripe-major: slot i at (i % 32) * kStripeCap + i / 32
-    uint64_t *mov;    // [W1]
-    uint64_t *blk;    // [W1]
+    uint64_t *mov;    // [W1 * CW]
+    uint64_t *blk;    // [W1 * CW], followed by the flood fill's reach [W1 * CW]
     uint16_t *par;    // [NODES]
     uint16_t *on;     // [kOpenCap] node of OPEN entries
 };
 
-__device__ __forceinline__ SearchSmem carve(unsigned char *smem, int W1, int NODES)
+__device__ __forceinline__ SearchSmem carve(unsigned char *smem, int CWW1, int NODES)
 {
     SearchSmem s;
     s.g = reinterpret_cast<double *>(smem);
     s.of = s.g + NODES;
     s.mov = reinterpret_cast<uint64_t *>(s.of + kOpenCap);
-    s.blk = s.mov + W1;
-    s.par = reinterpret_cast<uint16_t *>(s.blk + 2 * W1);   // [blk][reach]
+    s.blk = s.mov + CWW1;
+    s.par = reinterpret_cast<uint16_t *>(s.blk + 2 * CWW1);   // [blk][reach]
     s.on = s.par + ((NODES + 3) & ~3);
     return s;
 }
 
-// Node id = x * 64 + y (H <= 63): decoding a popped node is a shift and a mask instead of an integer division on the search's
-// critical path, and the ids keep heapq's (x, y) tuple order.
-static constexpr int kNodeShift = 6, kNodeStride = 1 << kNodeShift;
-static size_t search_smem_bytes(const EnvDev &c)
+// Node id = x * 64 CW + y: decoding a popped node is a shift and a mask instead of an integer division on the search's
+// critical path, and the ids keep heapq's (x, y) tuple order.  Ids stay below (W + 1) * 64 CW <= 65535 (u16 `par` / `on`),
+// and node << 11 | slot fits 32 bits (kOpenCap <= 2048).
+template <int CW> struct NodeId {
+    static constexpr int kShift = 5 + CW, kStride = 1 << kShift;
+};
+static constexpr size_t search_smem_bytes(int CW, int W)
 {
-    const int W1 = c.W + 1, NODES = W1 * kNodeStride;
-    return sizeof(double) * (NODES + kOpenCap) + sizeof(uint64_t) * 3 * W1 + sizeof(uint16_t) * (((NODES + 3) & ~3) + kOpenCap);
+    const size_t W1 = (size_t)W + 1, NODES = W1 * 64 * CW;
+    return sizeof(double) * (NODES + kOpenCap) + sizeof(uint64_t) * 3 * CW * W1 + sizeof(uint16_t) * (((NODES + 3) & ~(size_t)3) + kOpenCap);
 }
+static constexpr size_t kSearchSmemCap = 227 * 1024;   // opt-in shared memory of one block on sm_100
+// Map limits of the search: H <= 63 with one word per column, 64 <= H <= 127 with two, whose search state must fit one block's
+// shared memory (about 1.3 KB per column plus OPEN: one search per SM at 128 x 128).
+static constexpr int kMaxH1 = 63, kMaxW1 = 254, kMaxH2 = 127;
+static constexpr int max_search_width(int CW)
+{
+    int W = 2;
+    while (search_smem_bytes(CW, W + 1) <= kSearchSmemCap) ++W;
+    return W;
+}
+static constexpr int kMaxW2 = max_search_width(2);
+static_assert(kStripeCap <= 64 && kOpenCap <= 2048, "slot ids are 11 bits and a stripe is read by 2 x 32 lanes");
+static_assert(search_smem_bytes(1, kMaxW1) <= kSearchSmemCap, "one-word search must fit at W = kMaxW1");
+static_assert((kMaxW1 + 1) * NodeId<1>::kStride <= 65536 && (kMaxW2 + 1) * NodeId<2>::kStride <= 65536, "node ids are u16");
 
 // Is `goal` reachable from `start` through unblocked nodes of the [0,W]x[0,H] lattice with 8-connected moves?
-// Bit-parallel flood fill on the 64-bit columns (one lane per column, in-place monotone OR until the fixed point).
+// Bit-parallel flood fill on the columns (one lane per column, in-place monotone OR until the fixed point).
 // Used to cut the search short: when the goal is unreachable the reference's A* exhausts the whole component and
 // returns [s_start] (astar.py:67-71) — the same answer this gives after a few thousand cycles.
+template <int CW>
 __device__ bool goal_reachable(const SearchSmem &sm, uint64_t *reach, int W1, int H1, int sx, int sy, int gx, int gy)
 {
     const int lane = threadIdx.x & 31;
-    const uint64_t dom = (H1 >= 64) ? ~0ull : ((1ull << H1) - 1ull);
-    for (int x = lane; x < W1; x += 32) reach[x] = 0ull;
+    uint64_t dom[CW];
+#pragma unroll
+    for (int k = 0; k < CW; ++k) dom[k] = low_rows(H1 - 64 * k);
+    for (int i = lane; i < W1 * CW; i += 32) reach[i] = 0ull;
     __syncwarp();
-    if (lane == 0) reach[sx] = (1ull << sy) & ~sm.blk[sx];
+    if (lane == 0) {
+        const int i = sx * CW + row_word<CW>(sy);
+        reach[i] = (1ull << row_bit<CW>(sy)) & ~sm.blk[i];
+    }
     __syncwarp();
     for (;;) {
         bool changed = false;
         for (int x = lane; x < W1; x += 32) {
-            const uint64_t c = reach[x];
-            uint64_t nb = c;
-            if (x > 0) nb |= reach[x - 1];
-            if (x + 1 < W1) nb |= reach[x + 1];
-            nb |= (nb << 1) | (nb >> 1);
-            const uint64_t nw = (c | nb) & ~sm.blk[x] & dom;
-            if (nw != c) { reach[x] = nw; changed = true; }
+            uint64_t c[CW], nb[CW];
+#pragma unroll
+            for (int k = 0; k < CW; ++k) {
+                c[k] = reach[x * CW + k];
+                nb[k] = c[k];
+                if (x > 0) nb[k] |= reach[(x - 1) * CW + k];
+                if (x + 1 < W1) nb[k] |= reach[(x + 1) * CW + k];
+            }
+#pragma unroll
+            for (int k = 0; k < CW; ++k) {
+                uint64_t sh = (nb[k] << 1) | (nb[k] >> 1);
+                if (k > 0) sh |= nb[k - 1] >> 63;
+                if (k + 1 < CW) sh |= nb[k + 1] << 63;
+                const uint64_t nw = (c[k] | nb[k] | sh) & ~sm.blk[x * CW + k] & dom[k];
+                if (nw != c[k]) { reach[x * CW + k] = nw; changed = true; }
+            }
         }
         __syncwarp();
-        if ((reach[gx] >> gy) & 1ull) return true;
+        if ((reach[gx * CW + row_word<CW>(gy)] >> row_bit<CW>(gy)) & 1ull) return true;
         if (!__any_sync(0xffffffffu, changed)) return false;
     }
 }
 
 // Evader.replan (agent.py:232-259) for one env by one warp.  Returns the new path length (uniform across lanes);
 // path receives [goal, ..., start].
+template <int CW>
 __device__ int replan_warp(const EnvDev &c, const SearchSmem &sm, const uint32_t *__restrict__ grid,
                            const double *__restrict__ p_state, int N, double ex, double ey, int tx, int ty,
                            int16_t *__restrict__ path, int path_cap, int &status)
 {
     const int lane = threadIdx.x & 31;
-    const int W = c.W, H = c.H, W1 = W + 1, H1 = H + 1, NODES = W1 * kNodeStride;
-    const uint64_t hmask = (H >= 64) ? ~0ull : ((1ull << H) - 1ull);
+    constexpr int kNodeShift = NodeId<CW>::kShift, kNodeStride = NodeId<CW>::kStride;
+    const int W = c.W, H = c.H, W1 = W + 1, H1 = H + 1;
+    uint64_t hmask[CW];
+#pragma unroll
+    for (int k = 0; k < CW; ++k) hmask[k] = low_rows(H - 64 * k);
     const int cx = pyround(ex), cy = pyround(ey);
-    for (int x = lane; x < W1; x += 32) sm.mov[x] = 0ull;
+    for (int i = lane; i < W1 * CW; i += 32) sm.mov[i] = 0ull;
     __syncwarp();
     for (int i = lane; i < N; i += 32) {   // set_moving_obstacle (Occupied_Grid_Map.py:119-124)
         const int mx = pyround(p_state[i * 4]), my = pyround(p_state[i * 4 + 1]);
-        atomicOr((unsigned long long *)&sm.mov[mx], 1ull << my);
+        atomicOr((unsigned long long *)&sm.mov[mx * CW + row_word<CW>(my)], 1ull << row_bit<CW>(my));
     }
     __syncwarp();
     const int ux = (lane == 0 || lane == 1 || lane == 7) ? -1 : ((lane >= 3 && lane <= 5) ? 1 : 0);   // astar.py:11-12
@@ -138,14 +191,23 @@ __device__ int replan_warp(const EnvDev &c, const SearchSmem &sm, const uint32_t
     for (int e = c.e_extend_dis; e >= 0; --e) {
         // ---- Evader.rescan (agent.py:202-230) as column algebra ----
         for (int x = lane; x < W1; x += 32) {
-            uint64_t st = 0ull, pr = 0ull;
+            uint64_t st[CW], pr[CW], view[CW];
+#pragma unroll
+            for (int k = 0; k < CW; ++k) st[k] = pr[k] = view[k] = 0ull;
             for (int xx = max(0, x - e); xx <= min(W - 1, x + e); ++xx) {
-                st |= dilate_y(col_of(grid, c.HW, xx), e, hmask);
-                pr |= dilate_y(sm.mov[xx], e, hmask);
+                uint64_t gc[CW];
+                col_of<CW>(gc, grid, c.HW, xx);
+#pragma unroll
+                for (int k = 0; k < CW; ++k) {
+                    st[k] |= dilate_y<CW>(gc, k, e, hmask[k]);
+                    pr[k] |= dilate_y<CW>(sm.mov + xx * CW, k, e, hmask[k]);
+                }
             }
-            if (x >= W) { st = 0ull; pr = 0ull; }
-            // local_observation: half-open window [p-R, p+R) intersected with the disc d2 <= R^2
-            uint64_t view = 0ull;
+            if (x >= W) {
+#pragma unroll
+                for (int k = 0; k < CW; ++k) st[k] = pr[k] = 0ull;
+            }
+            // local_observation: half-open window [p-R, p+R) intersected with the disc d2 <= R^2 (at most 2R <= 64 rows)
             const int R = c.e_sen_range, dx = cx - x;
             if (x < W && x >= cx - R && x < cx + R) {
                 const int rem = c.e_view2_floor - dx * dx;
@@ -153,25 +215,33 @@ __device__ int replan_warp(const EnvDev &c, const SearchSmem &sm, const uint32_t
                     int k = 0;
                     while ((k + 1) * (k + 1) <= rem) ++k;
                     const int y0 = max(max(cy - k, cy - R), 0), y1 = min(min(cy + k, cy + R - 1), H - 1);
-                    if (y1 >= y0) view = ((y1 - y0 + 1 >= 64) ? ~0ull : ((1ull << (y1 - y0 + 1)) - 1ull)) << y0;
+#pragma unroll
+                    for (int w = 0; w < CW; ++w) {   // rows [y0, y1] of word w
+                        const int a = CW == 1 ? y0 : max(y0 - 64 * w, 0), b = CW == 1 ? y1 : min(y1 - 64 * w, 63);
+                        if (b >= a) view[w] = low_rows(b - a + 1) << a;
+                    }
                 }
             }
-            sm.blk[x] = st | (view & pr);
+#pragma unroll
+            for (int k = 0; k < CW; ++k) sm.blk[x * CW + k] = st[k] | (view[k] & pr[k]);
         }
         __syncwarp();
-        // g: +inf on free nodes, -1 on blocked ones (column-wise: lane l writes rows l and l + 32 of every column)
+        // g: +inf on free nodes, -1 on blocked ones (column-wise: lane l writes rows l + 32 j of every column)
         for (int x = 0; x < W1; ++x) {
-            const uint64_t col = sm.blk[x];
-            const unsigned lo = (unsigned)col, hi = (unsigned)(col >> 32);
-            sm.g[(x << kNodeShift) + lane] = ((lo >> lane) & 1u) ? -1.0 : (double)INFINITY;
-            sm.g[(x << kNodeShift) + 32 + lane] = ((hi >> lane) & 1u) ? -1.0 : (double)INFINITY;
+#pragma unroll
+            for (int k = 0; k < CW; ++k) {
+                const uint64_t col = sm.blk[x * CW + k];
+                const unsigned lo = (unsigned)col, hi = (unsigned)(col >> 32);
+                sm.g[(x << kNodeShift) + 64 * k + lane] = ((lo >> lane) & 1u) ? -1.0 : (double)INFINITY;
+                sm.g[(x << kNodeShift) + 64 * k + 32 + lane] = ((hi >> lane) & 1u) ? -1.0 : (double)INFINITY;
+            }
         }
         __syncwarp();
         // ---- AStar_2D.searching (astar.py:26-73) ----
         n_path = 1;
-        const bool goal_blocked = (sm.blk[tx] >> ty) & 1ull;
+        const bool goal_blocked = (sm.blk[tx * CW + row_word<CW>(ty)] >> row_bit<CW>(ty)) & 1ull;
         // a blocked start expands nothing (astar.py:56-60 tests both ends of every move): OPEN runs empty after the first pop
-        const bool start_blocked = (sm.blk[cx] >> cy) & 1ull;
+        const bool start_blocked = (sm.blk[cx * CW + row_word<CW>(cy)] >> row_bit<CW>(cy)) & 1ull;
         if (!goal_blocked && !start_blocked) {
             unsigned long long *const ofb = reinterpret_cast<unsigned long long *>(sm.of);
             unsigned c_hi = 0xffffffffu, c_lo = 0xffffffffu, c_tag = 0xffffffffu;   // minimum of this lane's stripe: f bits, node << 11 | slot
@@ -189,7 +259,7 @@ __device__ int replan_warp(const EnvDev &c, const SearchSmem &sm, const uint32_t
             bool reached = false;
             for (;;) {
                 if (++pops == kPopBudget) {   // long search: make sure it can succeed before spending more on it
-                    if (!goal_reachable(sm, sm.blk + W1, W1, H1, cx, cy, tx, ty)) break;
+                    if (!goal_reachable<CW>(sm, sm.blk + W1 * CW, W1, H1, cx, cy, tx, ty)) break;
                 }
                 // ---- pop: arg-min of (f, node) over the 32 cached stripe minima ----
                 const unsigned mhi = __reduce_min_sync(0xffffffffu, c_hi);
@@ -331,6 +401,7 @@ __device__ int replan_warp(const EnvDev &c, const SearchSmem &sm, const uint32_t
 
 // One attacker_step per env: replan when due, then move.  (Per-step API; the closed-loop rollout uses
 // evader_replan_kernel + the move fused into rollout_kernel instead.)
+template <int CW>
 __global__ void __launch_bounds__(32)
 evader_kernel(EnvDev c, EvaderArgs r, int replan_only)
 {
@@ -349,8 +420,8 @@ evader_kernel(EnvDev c, EvaderArgs r, int replan_only)
     s.status = 0;
     int16_t *path = r.path + (size_t)b * r.path_cap * 2;
     if (due) {
-        const SearchSmem sm = carve(smem, c.W + 1, (c.W + 1) * kNodeStride);
-        s.plen = replan_warp(c, sm, grid, r.p_state + (size_t)b * c.N * 4, c.N, s.x, s.y, s.tx, s.ty, path, r.path_cap, s.status);
+        const SearchSmem sm = carve(smem, (c.W + 1) * CW, (c.W + 1) * NodeId<CW>::kStride);
+        s.plen = replan_warp<CW>(c, sm, grid, r.p_state + (size_t)b * c.N * 4, c.N, s.x, s.y, s.tx, s.ty, path, r.path_cap, s.status);
     }
     if (lane == 0) {
         if (!replan_only) {
@@ -379,16 +450,22 @@ static int launch_evader(const marl_env_params *p, int32_t B, int32_t M, EvaderA
     if (rc) return rc;
     MARL_REQUIRE(B > 0 && M > 0 && r.path_cap >= 2 && r.tape_len >= 0, "marl_evader: B=%d M=%d path_cap=%d", B, M, r.path_cap);
     MARL_REQUIRE(r.map_id || M >= B, "marl_evader: map_id is NULL but M < B");
-    if (c.H > 63 || c.W > 254 || (c.W + 1) * (c.H + 1) > 65535) {
-        set_error("marl_evader: map %dx%d unsupported by the column-bitmap search (H <= 63, W <= 254)", c.W, c.H);
+    const int CW = c.H <= kMaxH1 ? 1 : 2;   // the lattice has H + 1 rows: H = 64 already needs a second word
+    if (c.H > kMaxH2 || c.W > (CW == 1 ? kMaxW1 : kMaxW2)) {
+        set_error("marl_evader: map %dx%d unsupported by the column-bitmap search (H <= %d needs W <= %d, H <= %d needs W <= %d)",
+                  c.W, c.H, kMaxH1, kMaxW1, kMaxH2, kMaxW2);
         return MARL_EUNSUPPORTED;
     }
-    const size_t smem = search_smem_bytes(c);
-    MARL_REQUIRE(smem <= 227 * 1024, "marl_evader: %zu B shared memory needed", smem);
-    cudaError_t e = cudaFuncSetAttribute(evader_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const size_t smem = search_smem_bytes(CW, c.W);
+    MARL_REQUIRE(smem <= kSearchSmemCap, "marl_evader: %zu B shared memory needed", smem);
+    const void *kern = CW == 1 ? (const void *)evader_kernel<1> : (const void *)evader_kernel<2>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) { set_error("evader: smem %zu: %s", smem, cudaGetErrorString(e)); return MARL_ECUDA; }
     r.B = B;
-    evader_kernel<<<B, 32, smem, (cudaStream_t)stream>>>(c, r, replan_only);
+    if (CW == 1)
+        evader_kernel<1><<<B, 32, smem, (cudaStream_t)stream>>>(c, r, replan_only);
+    else
+        evader_kernel<2><<<B, 32, smem, (cudaStream_t)stream>>>(c, r, replan_only);
     return check_launch("evader_kernel");
 }
 

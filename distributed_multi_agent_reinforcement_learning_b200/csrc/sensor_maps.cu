@@ -14,7 +14,7 @@ raser_map_kernel(EnvDev c, const uint32_t *__restrict__ grid_bits, const double 
     extern __shared__ __align__(16) unsigned char smem[];
     const int W = c.W, H = c.H, HW = c.HW, WH = W * H, O = c.O, OW = c.OW;
     int16_t *s_index = reinterpret_cast<int16_t *>(smem);                 // [WH] list index of a boundary cell, -1 else
-    uint32_t *s_grid = reinterpret_cast<uint32_t *>(s_index + ((WH + 1) & ~1));   // [W*HW]
+    uint32_t *s_grid = reinterpret_cast<uint32_t *>(s_index + ((WH + 3) & ~3));   // [W*HW] (both paddings keep s_beam 8-byte aligned)
     double *s_beam = reinterpret_cast<double *>(s_grid + ((W * HW + 1) & ~1));    // [beams*2]
     __shared__ int s_scan[kMapThreads];
     const int m = blockIdx.x, tid = threadIdx.x;
@@ -110,7 +110,7 @@ extern "C" int marl_raser_map_build(const marl_env_params *p, int32_t M, const u
     MARL_REQUIRE(d_grid_bits && d_beam_dir && d_boundary_bits && d_boundary_count && d_boundary_xy && d_raser_bits,
                  "marl_raser_map_build: null pointer");
     const int WH = c.W * c.H;
-    const size_t smem = sizeof(int16_t) * ((WH + 1) & ~1) + sizeof(uint32_t) * ((c.W * c.HW + 1) & ~1) +
+    const size_t smem = sizeof(int16_t) * ((WH + 3) & ~3) + sizeof(uint32_t) * ((c.W * c.HW + 1) & ~1) +
                         sizeof(double) * 2 * c.sensor_beams;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(raser_map_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

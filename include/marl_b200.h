@@ -109,7 +109,9 @@ int marl_raser_map_build(const marl_env_params *p, int32_t M, const uint32_t *d_
  * is NOT the reference's (search heap or path buffer overflow, tape exhausted) and must be treated as an error.
  * d_e_tape2 f64 [2,B,4] (may be NULL) receives the evader state before ([0]) and after ([1]) this step — the
  * 2-slot tape marl_rollout_steps(K=1) consumes, so a closed-loop env step is two launches.
- * Supported maps: H <= 63, W <= 254 (one 64-bit column per x in shared memory). */
+ * Supported maps: H <= 63 with W <= 254 (one 64-bit word per column of the search lattice in shared memory), and
+ * 64 <= H <= 127 with W <= 162 (two words per column; the search state of a 128 x 128 map takes about 183 KB, so one
+ * search runs per SM).  Other maps return MARL_EUNSUPPORTED before any CUDA call. */
 #define MARL_EV_HEAP_OVERFLOW 1
 #define MARL_EV_PATH_OVERFLOW 2
 #define MARL_EV_TAPE_EXHAUSTED 4

@@ -1,14 +1,19 @@
 """One training iteration at configs[4]'s per-GPU shape (conf/*.yaml: 64 pursuers, 32 768 envs, T 250, O 110, 60x60 map, depth 3) on
 one GPU: device reset -> rollout_batched (history replay: the stored history would take 543 GB) -> one train epoch -> update.
 
-    python tools/train_large.py [--envs 32768] [--mini-batch 32] [--out profiles/r3_train_configs4.json]
+    python tools/train_large.py [--envs 32768] [--mini-batch 32] [--map-size 60 60] [--out profiles/r3_train_configs4.json]
+
+--map-size W H changes only the map's size; its blocks stay centred on it (5 blocks, variance 10, O 110).  64 pursuers do not fit
+a 60x60 map under the reference's placement rule (`reset_fail_envs` counts the envs the reset could not complete); 128 128 seats
+them all.
 
 mini_batch_size: the reference's B/10 would be 3 277 envs = 52 M rows per minibatch, ~27 GB per 128-wide activation.  The default
 is 32 envs = 512 K rows (0.26 GB per 128-wide activation; a minibatch keeps a few dozen of them for the backward pass, and
 CONCURRENT_MINIBATCHES = 3 are in flight), next to the 30 GB arena and the D+1-slab history ring.
 
 Prints one JSON line: per-phase wall times (reset, rollout, a replay-only pass over the epoch's minibatches, the epoch, the update),
-torch.cuda.max_memory_allocated, agent-env-steps/s of the rollout, training samples/s of the epoch, and the GPU's name and power
+torch.cuda.max_memory_allocated, agent-env-steps/s of the rollout, training samples/s of the epoch, the event time of one A* replan
+of all envs on the episode's final states (a replan is due there: T is a multiple of `difficulty`), and the GPU's name and power
 limit read in the same run."""
 import argparse
 import json
@@ -63,13 +68,15 @@ def main():
     ap.add_argument("--depth", type=int, default=3)
     ap.add_argument("--maps", type=int, default=64)
     ap.add_argument("--mini-batch", type=int, default=32)
+    ap.add_argument("--map-size", type=int, nargs=2, default=[60, 60], metavar=("W", "H"))
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     dev = torch.device("cuda", 0)
     torch.cuda.set_device(dev)
     B, N, T, D, mbs = args.envs, args.pursuers, args.steps, args.depth, args.mini_batch
-    cfg = default_config(env__num_defender=N, env__max_steps=T, algo__depth=D, map__map_size=[60, 60], map__num_max_obstacle=110,
-                         algo__learner_device=str(dev), algo__worker_device=str(dev))
+    W, H = args.map_size
+    cfg = default_config(env__num_defender=N, env__max_steps=T, algo__depth=D, map__map_size=[W, H], map__center=[W // 2, H // 2],
+                         map__num_max_obstacle=110, algo__learner_device=str(dev), algo__worker_device=str(dev))
     env = BatchedPursuitEnv(cfg, B, device=dev, num_maps=args.maps)
     arena = RolloutArena(env.params, B, T, dev)
     torch.manual_seed(0)
@@ -87,11 +94,22 @@ def main():
     assert int(env.evader_status.max()) == 0, "evader search overflow / target tape exhausted"
     peak_rollout = torch.cuda.max_memory_allocated()
     progress(f"rollout {t2 - t1:.2f} s, peak {peak_rollout / 1e9:.1f} GB")
+    replan_ms = None
+    if T % env.params.difficulty == 0:
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
+        ev[0].record()
+        env.evader_replan(0, B)
+        ev[1].record()
+        torch.cuda.synchronize()
+        replan_ms = ev[0].elapsed_time(ev[1])
+        assert int(env.evader_status.max()) == 0
+        progress(f"replan of all envs {replan_ms:.1f} ms")
     replay_s = None
     if tb.replay is not None:
+        t_rp = time.perf_counter()
         replay_pass(tb, mbs)
         torch.cuda.synchronize()
-        replay_s = time.perf_counter() - t2
+        replay_s = time.perf_counter() - t_rp
         progress(f"replay pass {replay_s:.2f} s")
     t3 = time.perf_counter()
     obj_c, obj_a, _, _ = mappo.train(tb, B * T * N, return_numpy=False)
@@ -103,12 +121,13 @@ def main():
     t5 = time.perf_counter()
     rows = B * N * T
     out = {
-        "shape": {"envs": B, "pursuers": N, "steps": T, "depth": D, "obstacle_slots": env.O, "map": "60x60", "maps": args.maps,
+        "shape": {"envs": B, "pursuers": N, "steps": T, "depth": D, "obstacle_slots": env.O, "map": f"{W}x{H}", "maps": args.maps,
                   "mini_batch_size": mbs, "minibatches": -(-B // mbs), "concurrent_minibatches": mappo_parallel.CONCURRENT_MINIBATCHES},
         "history": mode, "history_bytes_if_stored": history_bytes(T, B, N, mappo.embedding_dim, D),
         "arena_bytes": arena.nbytes(), "reset_fail_envs": int((env.reset_fail != 0).sum()),
         "s": {"reset": t1 - t0, "rollout": t2 - t1, "replay_pass": replay_s, "epoch": t4 - t3, "update": t5 - t4},
         "replay_share_of_epoch": None if replay_s is None else replay_s / (t4 - t3),
+        "replan_all_envs_ms": replan_ms, "replans_per_episode": -(-T // env.params.difficulty),
         "max_memory_allocated": torch.cuda.max_memory_allocated(), "max_memory_allocated_rollout": peak_rollout,
         "agent_env_steps_per_s": rows / (t2 - t1), "train_samples_per_s": rows / (t4 - t3),
         "losses": {"critic": obj_c, "actor": obj_a},
