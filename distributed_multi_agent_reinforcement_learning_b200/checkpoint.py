@@ -9,7 +9,8 @@ state_dict keys, so `torch.load(f).state_dict()` of either side's file loads int
 `weights_only=True` (no pickled classes, no omegaconf).
 
 `save_training_state` / `load_training_state` write and read one more file: everything a run needs to continue exactly where
-it stopped (optimizer moments, schedule position, reward statistics, engine tables, evaluator bookkeeping, RNG streams)."""
+it stopped (optimizer moments, schedule position, reward statistics, engine tables, evaluator bookkeeping, RNG streams, and the
+recurrent state of an episode stopped at a segment boundary)."""
 import collections
 import os
 import random
@@ -99,11 +100,15 @@ def _fingerprint(mappo, engine):
                 world_size=world)
 
 
-def save_training_state(path, mappo, engine=None, evaluator=None, extra=None):
+_CARRY = ("ha", "hc", "emb_a", "emb_c")
+
+
+def save_training_state(path, mappo, engine=None, evaluator=None, extra=None, carry=None):
     """Writes everything a training run carries from one iteration to the next to ONE `torch.save` file of CPU tensors and plain
     values (it loads with weights_only=True): a shape fingerprint, the actor / critic state_dicts (spectral-norm buffers included),
     the Adam state, `total_step`, the reward normaliser, the engine's state (`BatchedPursuitEnv.state_dict`), the evaluator's
-    bookkeeping, the torch CPU / CUDA, Python `random` and numpy RNG states, and `extra` (the caller's loop counters).
+    bookkeeping, the torch CPU / CUDA, Python `random` and numpy RNG states, `extra` (the caller's loop counters) and `carry`, the
+    RolloutCarry the next rollout segment continues from when the run stops inside an episode (None: at an episode boundary).
     Take it between iterations, after `update()`.  Under torch.distributed every rank writes its own file."""
     rn = getattr(mappo, "reward_norm", None)
     np_state = np.random.get_state(legacy=False)
@@ -119,7 +124,8 @@ def save_training_state(path, mappo, engine=None, evaluator=None, extra=None):
         rng=dict(torch_cpu=torch.get_rng_state(), torch_cuda=torch.cuda.get_rng_state(mappo.device), python=random.getstate(),
                  numpy=dict(bit_generator=np_state["bit_generator"], key=[int(k) for k in np_state["state"]["key"]],
                             pos=int(np_state["state"]["pos"]), has_gauss=int(np_state["has_gauss"]), gauss=float(np_state["gauss"]))),
-        extra=dict(extra or {}))
+        extra=dict(extra or {}),
+        carry=None if carry is None else dict(t0=int(carry.t0), **{k: getattr(carry, k).detach().cpu() for k in _CARRY}))
     d = os.path.dirname(os.path.abspath(path))
     os.makedirs(d, exist_ok=True)
     tmp = path + ".tmp"
@@ -127,11 +133,14 @@ def save_training_state(path, mappo, engine=None, evaluator=None, extra=None):
     os.replace(tmp, path)          # a run interrupted while saving keeps the previous file
 
 
-def load_training_state(path, mappo, engine=None, evaluator=None):
+def load_training_state(path, mappo, engine=None, evaluator=None, carry=None):
     """Restores a `save_training_state` file into freshly built objects of the same shape and returns its `extra` dict.  Every
     fingerprint field (N, E, depth, num_layers, action_dim, parameter count, B, number of maps, rank, world size) and every tensor
     shape is checked before anything is modified; a mismatch raises MarlError naming it.  Parameters are copied in place, so they
-    stay views into the optimizer's flat arena."""
+    stay views into the optimizer's flat arena.
+    carry: a RolloutCarry (e.g. `RolloutCarry.zeros`) that receives the file's carry in place; a file without one (every file
+    written without `carry=`) is at an episode boundary and sets it to t0 = 0 with zero tensors.  A file that holds a carry can
+    only be loaded with one."""
     st = torch.load(path, map_location="cpu", weights_only=True)
     if st.get("version") != TRAINING_STATE_VERSION:
         raise MarlError(f"{path}: training-state format {st.get('version')!r}, this build reads {TRAINING_STATE_VERSION}")
@@ -160,6 +169,14 @@ def load_training_state(path, mappo, engine=None, evaluator=None):
     n = mappo.ac_optimizer.flat_param.numel()
     if st["adam"]["exp_avg"].numel() != n or st["adam"]["exp_avg_sq"].numel() != n:
         raise MarlError(f"{path}: Adam state of {st['adam']['exp_avg'].numel()} elements, here {n}")
+    sc = st.get("carry")
+    if sc is not None and carry is None:
+        raise MarlError(f"{path}: stopped inside an episode (next segment at step {sc['t0']}): pass carry= to restore its recurrent state")
+    if sc is not None:
+        for k in _CARRY:
+            if sc[k].dtype != getattr(carry, k).dtype or tuple(sc[k].shape) != tuple(getattr(carry, k).shape):
+                raise MarlError(f"{path}: carry {k} is {tuple(sc[k].shape)} {sc[k].dtype}, here {tuple(getattr(carry, k).shape)} "
+                                f"{getattr(carry, k).dtype}")
     if engine is not None:
         for k in engine._STATE:
             src, dst = st["engine"].get(k), getattr(engine, k)
@@ -176,6 +193,13 @@ def load_training_state(path, mappo, engine=None, evaluator=None):
             getattr(rn.running_ms, k).copy_(v)
     if engine is not None:
         engine.load_state_dict(st["engine"])
+    if carry is not None:
+        carry.t0 = 0 if sc is None else int(sc["t0"])
+        for k in _CARRY:
+            if sc is None:
+                getattr(carry, k).zero_()
+            else:
+                getattr(carry, k).copy_(sc[k])
     if evaluator is not None:
         ev = st["evaluator"]
         evaluator.recorder = [tuple(r) for r in ev["recorder"]]

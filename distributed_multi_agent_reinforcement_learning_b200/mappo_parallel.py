@@ -47,18 +47,71 @@ def history_bytes(T, B, N, E, D):
     return 2 * (T + D) * B * N * E * 4
 
 
-def _history_inputs(hist_a, hist_c, t, D, quirks, net, slot, sl=slice(None)):
+def _history_inputs(hist_a, hist_c, t, D, quirks, net, slot, sl=slice(None), t0=0):
     """The D history inputs of step t for `net` (k = 0 newest; None = zeros, before the episode's first step), read from the
     [*, B, N, E] buffers at index slot(i) for history step i (t + D is what step t writes).  reference_quirks: the ONE list actor and
-    critic alias (:750-752), C(t-1), A(t-1), C(t-2), ...; otherwise each network's own embeddings."""
+    critic alias (:750-752), C(t-1), A(t-1), C(t-2), ...; otherwise each network's own embeddings.  t is local to a segment that
+    starts at the episode's step t0; indices 0..D-1 hold the embeddings carried in from the previous segment."""
     out = []
     for k in range(D):
         if quirks:
             back, src = k // 2 + 1, (hist_c if k % 2 == 0 else hist_a)
         else:
             back, src = k + 1, (hist_a if net == "actor" else hist_c)
-        out.append(src[slot(t - back + D)][sl] if t - back >= 0 else None)
+        out.append(src[slot(t - back + D)][sl] if t0 + t - back >= 0 else None)
     return out
+
+
+class RolloutCarry:
+    """The recurrent state one rollout segment hands to the next segment of the same episode.
+
+    t0: the episode's env step at which the next segment starts.  ha / hc: the actor's and the critic's GRU hidden states
+    [L, B*N, E] after step t0-1.  emb_a / emb_c: the last D embeddings of each network [D, B, N, E], index j = step t0-D+j (zeros
+    for steps before the episode's first).  A carry with t0 = 0 is the start of an episode: zero hidden states and zero history."""
+
+    def __init__(self, t0, ha, hc, emb_a, emb_c):
+        self.t0, self.ha, self.hc, self.emb_a, self.emb_c = int(t0), ha, hc, emb_a, emb_c
+
+    @classmethod
+    def zeros(cls, mappo, B, N, t0=0):
+        """An episode start (t0 = 0) for B envs of N agents, on the networks' device."""
+        f32 = dict(dtype=torch.float32, device=mappo.device)
+        L, E, D = mappo.num_layers, mappo.embedding_dim, mappo.depth
+        return cls(t0, torch.zeros(L, B * N, E, **f32), torch.zeros(L, B * N, E, **f32), torch.zeros(D, B, N, E, **f32),
+                   torch.zeros(D, B, N, E, **f32))
+
+    def shapes(self):
+        return dict(ha=tuple(self.ha.shape), hc=tuple(self.hc.shape), emb_a=tuple(self.emb_a.shape), emb_c=tuple(self.emb_c.shape))
+
+    def copy_(self, other):
+        """Copies `other`'s step and tensors into this carry's tensors (same shapes)."""
+        self.t0 = int(other.t0)
+        for k in ("ha", "hc", "emb_a", "emb_c"):
+            if getattr(self, k).data_ptr() != getattr(other, k).data_ptr():
+                getattr(self, k).copy_(getattr(other, k))
+        return self
+
+
+def check_segment(carry, S, T_ep, B, N, L, E, D, device, actor_only=False):
+    """Host-side checks of a rollout segment of S steps continuing `carry` in an episode of T_ep steps; raises MarlError before any
+    CUDA call.  S must divide T_ep (a segment never crosses an episode boundary) and the segment must end inside the episode."""
+    if actor_only:
+        raise _lib.MarlError("rollout_batched: actor_only (the evaluator's episode) runs whole episodes and takes no carry")
+    if not isinstance(carry, RolloutCarry):
+        raise _lib.MarlError(f"rollout_batched: carry must be a RolloutCarry, not {type(carry).__name__}")
+    if S <= 0 or T_ep % S != 0:
+        raise _lib.MarlError(f"rollout segment of {S} steps: the length must be a positive divisor of the episode length {T_ep}")
+    if carry.t0 < 0 or carry.t0 + S > T_ep:
+        raise _lib.MarlError(f"rollout segment [{carry.t0}, {carry.t0 + S}) does not lie inside the episode of {T_ep} steps")
+    want = dict(ha=(L, B * N, E), hc=(L, B * N, E), emb_a=(D, B, N, E), emb_c=(D, B, N, E))
+    have = carry.shapes()
+    dev = torch.device(device)
+    for k in want:
+        x = getattr(carry, k)
+        if (have[k] != want[k] or x.dtype != torch.float32 or x.device.type != dev.type
+                or (dev.index is not None and x.device.index != dev.index)):
+            raise _lib.MarlError(f"rollout carry: {k} is {have[k]} {x.dtype} on {x.device}, this rollout needs {want[k]} float32 on "
+                                 f"{device}")
 
 
 def orthogonal_init(layer, gain=1.0):
@@ -360,6 +413,12 @@ class TrainBatch:
     KEYS = ("p", "e", "p_adj_bits", "e_adj", "o_adj_bits", "hist_a", "hist_c", "v", "a", "logp", "r", "active")
     replay = None       # HistoryReplay of a batch whose history was not stored (hist_a = hist_c = None); minibatches regenerate it
     map_id = None       # i32 [B] (replay only)
+    # A rollout segment (rollout_batched(carry=...)) starts at the episode's step t0 from the GRU hidden states h0_a / h0_c
+    # [L, B*N, E]; a replay-mode segment also keeps its D history-prefix slabs prefix_a / prefix_c [D, B, N, E] (a store-mode one has
+    # them as slabs 0..D-1 of hist_a / hist_c).  `carry` is the RolloutCarry the next segment continues from.  A whole-episode batch
+    # has t0 = 0 and None for all of them: zero hidden states and zero history.
+    t0 = 0
+    h0_a = h0_c = prefix_a = prefix_c = carry = None
 
     def __init__(self, **kw):
         self.__dict__.update(kw)
@@ -387,6 +446,11 @@ class TrainBatch:
                         o_count_train=self.o_count_train[lo:hi].contiguous(), p_adj_bits=s(self.p_adj_bits),
                         e_adj=s(self.e_adj), o_adj_bits=s(self.o_adj_bits), hist_a=s(self.hist_a), hist_c=s(self.hist_c),
                         v=s(self.v), a=s(self.a), logp=s(self.logp), r=s(self.r), active=s(self.active), depth=self.depth)
+        if self.h0_a is not None:
+            N = self.N
+            mb.t0 = self.t0
+            mb.h0_a, mb.h0_c = self.h0_a[:, lo * N:hi * N].contiguous(), self.h0_c[:, lo * N:hi * N].contiguous()
+            mb.prefix_a, mb.prefix_c = s(self.prefix_a), s(self.prefix_c)
         if self.replay is not None:
             mb.replay, mb.map_id = self.replay, self.map_id[lo:hi].contiguous()
             self.replay.regenerate(mb)
@@ -418,6 +482,11 @@ class TrainBatch:
                          p_adj_bits=g(self.p_adj_bits), e_adj=g(self.e_adj), o_adj_bits=g(self.o_adj_bits), hist_a=gh(self.hist_a),
                          hist_c=gh(self.hist_c), v=g(self.v), a=g(self.a), logp=g(self.logp), r=g(self.r), active=g(self.active),
                          depth=self.depth)
+        if self.h0_a is not None:                   # hidden states: row (layer l, env b) of the [L*B, N*E] view
+            L, N = self.h0_a.shape[0], self.N
+            out.t0 = self.t0
+            out.h0_a, out.h0_c = (g(h.view(L, B, N, -1)).view(L, mb * N, -1) for h in (self.h0_a, self.h0_c))
+            out.prefix_a, out.prefix_c = gh(self.prefix_a), gh(self.prefix_c)
         if self.replay is not None:
             out.replay, out.map_id = self.replay, g(self.map_id, False)
             self.replay.regenerate(out)
@@ -446,22 +515,29 @@ class HistoryReplay:
     minibatch's own slabs.  The fused step's per-row output does not depend on how the batch is split into launches, and the arena
     records are (float) of the fp64 states the rollout's step converted, so the regenerated history is the stored one bit for bit."""
 
-    def __init__(self, fused, oxy_i32, o_count, quirks):
-        self.fused, self.oxy_i32, self.o_count, self.quirks = fused, oxy_i32, o_count, bool(quirks)
+    def __init__(self, fused, oxy_i32, o_count, quirks, t0=0):
+        self.fused, self.oxy_i32, self.o_count, self.quirks, self.t0 = fused, oxy_i32, o_count, bool(quirks), int(t0)
 
     def regenerate(self, mb, embed_only=None):
         """Fills mb.hist_a / mb.hist_c [T+D, mb, N, E] with T fused steps on the current stream (forced actions, history read from the
-        tensors being filled).  embed_only (default REPLAY_EMBED_ONLY) False runs the full step from zero hidden states and returns the
-        replayed (log-prob, value) [T, mb, N] - the same numbers the rollout stored."""
+        tensors being filled; a segment's slabs 0..D-1 are its history prefix).  embed_only (default REPLAY_EMBED_ONLY) False runs the
+        full step from the batch's start hidden states and returns the replayed (log-prob, value) [T, mb, N] - the same numbers the
+        rollout stored."""
         from types import SimpleNamespace
         embed_only = REPLAY_EMBED_ONLY if embed_only is None else embed_only
-        T, B, N, D, E = mb.T, mb.B, mb.N, mb.depth, self.fused.E
+        T, B, N, D, E, t0 = mb.T, mb.B, mb.N, mb.depth, self.fused.E, self.t0
         f32 = dict(dtype=torch.float32, device=mb.p.device)
         mb.hist_a, mb.hist_c = torch.zeros(T + D, B, N, E, **f32), torch.zeros(T + D, B, N, E, **f32)
+        if mb.prefix_a is not None:
+            mb.hist_a[:D].copy_(mb.prefix_a)
+            mb.hist_c[:D].copy_(mb.prefix_c)
         flags = fused_policy.STATE_F32 | (fused_policy.EMBED_ONLY if embed_only else 0)
         ha = hc = act = logp = v = None
         if not embed_only:
-            ha, hc = torch.zeros(2, B * N, E, **f32), torch.zeros(2, B * N, E, **f32)
+            if mb.h0_a is None:
+                ha, hc = torch.zeros(2, B * N, E, **f32), torch.zeros(2, B * N, E, **f32)
+            else:
+                ha, hc = mb.h0_a.clone(), mb.h0_c.clone()
             act = mb.a.to(torch.int32)
             logp, v = torch.empty(T, B, N, **f32), torch.empty(T, B, N, **f32)
         view = SimpleNamespace(B=B, N=N, O=self.oxy_i32.shape[1], map_id=mb.map_id)
@@ -469,9 +545,9 @@ class HistoryReplay:
         for t in range(T):
             view.p_state, view.e_state = mb.p[t], mb.e[t]
             view.p_adj_bits, view.e_adj, view.o_adj_bits = mb.p_adj_bits[t], mb.e_adj[t], mb.o_adj_bits[t]
-            h_a = _history_inputs(mb.hist_a, mb.hist_c, t, D, self.quirks, "actor", ident)
-            h_c = _history_inputs(mb.hist_a, mb.hist_c, t, D, self.quirks, "critic", ident)
-            self.fused.step(view, self.oxy_i32, self.o_count, t, 0, True, h_a, h_c, mb.hist_a[t + D], mb.hist_c[t + D], ha, hc,
+            h_a = _history_inputs(mb.hist_a, mb.hist_c, t, D, self.quirks, "actor", ident, t0=t0)
+            h_c = _history_inputs(mb.hist_a, mb.hist_c, t, D, self.quirks, "critic", ident, t0=t0)
+            self.fused.step(view, self.oxy_i32, self.o_count, t0 + t, 0, True, h_a, h_c, mb.hist_a[t + D], mb.hist_c[t + D], ha, hc,
                             None if act is None else act[t], None if logp is None else logp[t], None if v is None else v[t],
                             force_action=True, flags=flags)
         return None if embed_only else (logp, v)
@@ -482,14 +558,16 @@ class RolloutGraph:
     """`MAPPO.rollout_batched` for all envs of an engine (networks in the loop) captured as ONE CUDA graph: per env step
     observe -> fused policy step (encoder + GRU + heads of both networks, one launch per env group) -> A* replan when due ->
     fused evader-move / step / reward-norm / store kernel; no host involvement on replay.  The engine state the episode starts
-    from is whatever the engine holds at replay time."""
+    from is whatever the engine holds at replay time.  With `carry` (a RolloutCarry whose tensors stay put: the graph reads them on
+    every replay) the graph is one segment of T steps starting at the episode's step carry.t0."""
 
-    def __init__(self, mappo, engine, arena, T, seed, policy_dbg=None, history=None):
+    def __init__(self, mappo, engine, arena, T, seed, policy_dbg=None, history=None, carry=None):
         snap = engine.snapshot()
         kw = {} if policy_dbg is None else dict(timers={"_policy_dbg": policy_dbg}, pipelines=policy_dbg.shape[1])
         # decided once: the warm-up's allocations would otherwise change the free memory the captured rollout sees
         kw["history"] = history or mappo.history_mode(T, engine.B, engine.N)
-        mappo.rollout_batched(engine, arena, T, seed=seed, history=kw["history"])   # eager warm-up (kernel attributes, stream pool)
+        kw["carry"] = self.carry = carry
+        mappo.rollout_batched(engine, arena, T, seed=seed, history=kw["history"], carry=carry)   # eager warm-up (kernel attributes, stream pool)
         torch.cuda.synchronize()
         engine.restore(snap)
         self.graph = torch.cuda.CUDAGraph()
@@ -548,7 +626,10 @@ class MAPPO:
         T, B, N, E = mb.T, mb.B, mb.N, self.embedding_dim
         graph = mb.graph()
         enc = self.actor.shared_net
-        h0 = torch.zeros(self.num_layers, B * N, E, dtype=torch.float32, device=self.device)
+        if mb.h0_a is None:             # a whole episode starts from zero hidden states
+            h0_a = h0_c = torch.zeros(self.num_layers, B * N, E, dtype=torch.float32, device=self.device)
+        else:                           # a segment from the hidden states the rollout carried into it
+            h0_a, h0_c = mb.h0_a, mb.h0_c
         # The two networks are independent until the loss: the critic branch runs on a side stream, concurrently with the actor
         # branch (forward here, and backward too: autograd replays each node on the stream of its forward).  The GRU sequence
         # kernels of a minibatch only fill 50-100 of the 148 SMs, so the pair overlaps almost perfectly.
@@ -561,16 +642,16 @@ class MAPPO:
             side.wait_stream(main)
             with torch.cuda.stream(side):
                 emb_c = enc.encode(graph, True, mb.history("critic"))
-                feat_c, _ = self.critic.features(emb_c.view(T, B * N, E), h0)
+                feat_c, _ = self.critic.features(emb_c.view(T, B * N, E), h0_c)
             emb_a = enc.encode(graph, False, mb.history("actor"))
-            feat_a, _ = self.actor.features(emb_a.view(T, B * N, E), h0)
+            feat_a, _ = self.actor.features(emb_a.view(T, B * N, E), h0_a)
             main.wait_stream(side)
             feat_c.record_stream(main)
         else:
             emb_a = enc.encode(graph, False, mb.history("actor"))
-            feat_a, _ = self.actor.features(emb_a.view(T, B * N, E), h0)
+            feat_a, _ = self.actor.features(emb_a.view(T, B * N, E), h0_a)
             emb_c = enc.encode(graph, True, mb.history("critic"))
-            feat_c, _ = self.critic.features(emb_c.view(T, B * N, E), h0)
+            feat_c, _ = self.critic.features(emb_c.view(T, B * N, E), h0_c)
         cm = self.critic.Mean
         R = T * B * N
         flat = lambda x: x.reshape(R)
@@ -734,7 +815,7 @@ class MAPPO:
 
     @torch.no_grad()
     def rollout_batched(self, engine, arena, T=None, seed=0, deterministic=False, groups=1, use_fused=None, timers=None,
-                        pipelines=None, actor_only=False, history=None):
+                        pipelines=None, actor_only=False, history=None, carry=None):
         """MAPPO.run_episode (:742-827) for all B envs of a BatchedPursuitEnv at once, entirely on the GPU.
         Per step: observe kernel -> fused encoder (actor, then critic with all-ones adjacency) -> GRU cell -> heads ->
         closed-loop env kernel (evader move + pursuer step + reward-norm + store).  Fills `arena` plus the history /
@@ -746,10 +827,22 @@ class MAPPO:
         history: 'store' keeps the full [T+D,B,N,E] history of both networks in the batch; 'replay' keeps only a ring of D+1 slabs
         per network during the episode (step t reads at most D steps back) and returns a batch with hist_a = hist_c = None that
         regenerates each minibatch's history in training (HistoryReplay).  None chooses with `history_mode` (store when it fits
-        comfortably).  Replay needs the fused step; actor_only rollouts always store."""
-        T = T or arena.T
+        comfortably).  Replay needs the fused step; actor_only rollouts always store.
+
+        carry: None (a whole episode from the engine's state at step 0) or a RolloutCarry: one segment of T = S steps of an episode of
+        cfg.env.max_steps steps (S divides it), starting at the episode's step carry.t0 from the carried hidden states and history.
+        The history rule, the sampling RNG key and the A* replan schedule use the episode's step; the engine must be at carry.t0.
+        The batch records its start state (t0, h0_a / h0_c, the history prefix) and its `carry` is where the next segment starts."""
         B, N, E, D, L = engine.B, engine.N, self.embedding_dim, self.depth, self.num_layers
         dev = self.device
+        if carry is not None:
+            T = arena.T if T is None else int(T)
+            check_segment(carry, T, int(self.cfg.env.max_steps), B, N, L, E, D, dev, actor_only)
+            if not torch.cuda.is_current_stream_capturing() and not bool((engine.time_step == carry.t0).all()):
+                raise _lib.MarlError(f"rollout segment from step {carry.t0}: the engine's envs are at steps "
+                                     f"{sorted(set(engine.time_step.tolist()))[:4]}")
+        T = T or arena.T
+        t0 = 0 if carry is None else carry.t0
         f32 = dict(dtype=torch.float32, device=dev)
         if use_fused is None:
             use_fused = fused_policy.supported(self)
@@ -769,7 +862,12 @@ class MAPPO:
         v = torch.zeros(T + 1, B, N, **f32)
         logp = torch.zeros(T, B, N, **f32)
         act = torch.zeros(T, B, N, dtype=torch.int32, device=dev)
-        ha, hc = torch.zeros(L, B * N, E, **f32), torch.zeros(L, B * N, E, **f32)
+        if carry is None:
+            ha, hc = torch.zeros(L, B * N, E, **f32), torch.zeros(L, B * N, E, **f32)
+        else:                                   # history steps 0..D-1 (slot(i) = i in both modes) are the carried embeddings
+            ha, hc = carry.ha.clone(), carry.hc.clone()
+            hist_a[:D].copy_(carry.emb_a)
+            hist_c[:D].copy_(carry.emb_c)
         oxy = engine.boundary_xy.to(torch.float32).contiguous()                 # [M,O,2]
         o_count = torch.clamp(engine.boundary_count, max=engine.O).contiguous()  # rollout: the O_b real cells
         enc = self.actor.shared_net
@@ -786,7 +884,7 @@ class MAPPO:
                 own = actor_only or not quirks
                 back = (k + 1) if own else (k // 2 + 1)
                 src = (hist_a if (net == "actor" or actor_only) else hist_c) if own else (hist_c if k % 2 == 0 else hist_a)
-                out.append(src[slot(t - back + D)] if t - back >= 0 else zeros_hist)
+                out.append(src[slot(t - back + D)] if t0 + t - back >= 0 else zeros_hist)
             return out
 
         def critic_step(t, graph):
@@ -805,7 +903,12 @@ class MAPPO:
             w, _ = self.critic.head_weight()
             fused = fused_policy.FusedRolloutStep(self, w.reshape(E).contiguous(), snapshot=replay)
             oxy_i = engine.boundary_xy.clone() if replay else engine.boundary_xy.contiguous()
-            rep_ = HistoryReplay(fused, oxy_i, o_count, quirks) if replay else None
+            rep_ = HistoryReplay(fused, oxy_i, o_count, quirks, t0) if replay else None
+            # The bootstrap value v[T] is a critic-only step at the episode's end.  A segment that ends inside the episode computes it
+            # with the step of both networks instead (the actor's outputs are discarded): that is the kernel the next segment's first
+            # step runs on the same state, and the critic-only kernel rounds the GRU cell and the value sum differently, so v[T] is
+            # then bit for bit the value the next segment starts with.
+            pair_bootstrap = carry is not None and t0 + T < int(self.cfg.env.max_steps)
             none_if_zero = lambda lst: [None if h is zeros_hist else h for h in lst]   # noqa: E731
             def timed(name, fn):
                 if timers is None:
@@ -827,9 +930,10 @@ class MAPPO:
                     pipelines = int(os.environ["MARL_PIPELINES"])
             if pipelines > 1 and (timers is None or not auto) and groups == 1 and not actor_only:
                 # (an explicit pipelines=G together with timers: CUDA events around every launch of the pipelined schedule itself)
-                self._rollout_pipelined(engine, arena, T, seed, deterministic, int(pipelines), fused, oxy_i, o_count, hist_a, hist_c,
-                                        act, logp, v, zeros_hist, timers=timers, slot=slot)
-                return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp, rep_)
+                nxt = self._rollout_pipelined(engine, arena, T, seed, deterministic, int(pipelines), fused, oxy_i, o_count, hist_a,
+                                              hist_c, act, logp, v, zeros_hist, timers=timers, slot=slot, carry=carry,
+                                              pair_bootstrap=pair_bootstrap)
+                return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp, rep_, carry, nxt)
             # Single pipeline.  The A* replanning due every `difficulty` steps only needs the env state, not the action: it runs
             # on a side stream concurrently with the policy kernel and is joined before the env kernel consumes the paths.
             overlap = timers is None and groups == 1
@@ -841,7 +945,7 @@ class MAPPO:
             diff = int(engine.params.difficulty)
             for t in range(T):
                 join = None
-                if overlap and t % diff == 0:
+                if overlap and (t0 + t) % diff == 0:
                     fork = torch.cuda.Event()
                     fork.record(main)
                     side.wait_event(fork)
@@ -850,21 +954,26 @@ class MAPPO:
                     join.record(side)
                 timed("env_observe_kernel", engine.observe)
                 h_t, h_tc = none_if_zero(history(t)), none_if_zero(history(t, "critic"))
-                timed("policy_step_kernel", lambda: fused.step(engine, oxy_i, o_count, t, seed, deterministic, h_t, h_tc,
+                timed("policy_step_kernel", lambda: fused.step(engine, oxy_i, o_count, t0 + t, seed, deterministic, h_t, h_tc,
                                                                hist_a[slot(t + D)], hist_c[slot(t + D)], ha, hc, act[t], logp[t], v[t],
                                                                nets=("actor",) if actor_only else ("actor", "critic")))
                 if join is not None:
                     main.wait_event(join)
-                engine.rollout_closed(arena, 1, t0=t, action_tape=act[t:t + 1], env_t0=t, groups=groups, timers=timers,
+                engine.rollout_closed(arena, 1, t0=t, action_tape=act[t:t + 1], env_t0=t0 + t, groups=groups, timers=timers,
                                       skip_replan=join is not None)
             if actor_only:
                 return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp)
             engine.observe()
             h_fin = none_if_zero(([hist_c[slot(T - 1 + D)]] + history(T - 1)[:D - 1]) if quirks else history(T, "critic"))
             scratch = torch.empty(B, N, E, **f32)
-            fused.step(engine, oxy_i, o_count, T, seed, deterministic, h_fin, h_fin, scratch, scratch, ha, hc, None, None, v[T],
-                       nets=("critic",))
-            return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp, rep_)
+            nxt = None if carry is None else self._next_carry(carry, T, hist_a, hist_c, slot, ha, hc.clone())
+            if pair_bootstrap:              # (on copies: the bootstrap step updates the hidden states in place)
+                fused.step(engine, oxy_i, o_count, t0 + T, seed, deterministic, none_if_zero(history(T)), h_fin, torch.empty_like(scratch),
+                           scratch, ha.clone(), hc, torch.empty_like(act[0]), torch.empty_like(logp[0]), v[T])
+            else:
+                fused.step(engine, oxy_i, o_count, t0 + T, seed, deterministic, h_fin, h_fin, scratch, scratch, ha, hc, None, None, v[T],
+                           nets=("critic",))
+            return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp, rep_, carry, nxt)
 
         for t in range(T):
             engine.observe()
@@ -873,17 +982,17 @@ class MAPPO:
             emb_a = enc.encode(graph, False, history(t))
             feat_a, ha = self.actor.features(emb_a.view(1, B * N, E), ha)
             if actor_only:
-                a_i, _, lp, _ = ops.act_head(feat_a[0], None, self.actor.Mean.weight, self.actor.Mean.bias, None, None, seed, t,
+                a_i, _, lp, _ = ops.act_head(feat_a[0], None, self.actor.Mean.weight, self.actor.Mean.bias, None, None, seed, t0 + t,
                                              deterministic)
                 hist_a[t + D] = emb_a
             else:
                 emb_c, feat_c = critic_step(t, graph)
                 a_i, _, lp, val = ops.act_head(feat_a[0], feat_c, self.actor.Mean.weight, self.actor.Mean.bias, w_eff,
-                                               self.critic.Mean.bias, seed, t, deterministic)
+                                               self.critic.Mean.bias, seed, t0 + t, deterministic)
                 hist_a[t + D], hist_c[t + D] = emb_a, emb_c
                 v[t] = val.view(B, N)
             logp[t], act[t] = lp.view(B, N), a_i.view(B, N)
-            engine.rollout_closed(arena, 1, t0=t, action_tape=act[t:t + 1], env_t0=t, groups=groups)
+            engine.rollout_closed(arena, 1, t0=t, action_tape=act[t:t + 1], env_t0=t0 + t, groups=groups)
         if actor_only:
             return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp)
         # bootstrap value of the final state (:806-825): only the critic's dataset is updated once more
@@ -891,11 +1000,12 @@ class MAPPO:
         graph = ops.GraphBatch(engine.p_state.to(torch.float32), engine.e_state.to(torch.float32), oxy, engine.map_id,
                                o_count, engine.p_adj_bits, engine.e_adj, engine.o_adj_bits)
         hist_final = ([hist_c[T - 1 + D]] + history(T - 1)[:D - 1]) if quirks else history(T, "critic")
+        nxt = None if carry is None else self._next_carry(carry, T, hist_a, hist_c, slot, ha, hc)
         emb_c = enc.encode(graph, True, hist_final)
-        feat_c, hc = self.critic.features(emb_c.view(1, B * N, E), hc)
+        feat_c, _ = self.critic.features(emb_c.view(1, B * N, E), hc)
         w, _ = self.critic.head_weight()
         v[T] = torch.nn.functional.linear(feat_c[0], w, self.critic.Mean.bias).view(B, N)
-        return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp)
+        return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp, None, carry, nxt)
 
     @staticmethod
     def default_pipelines(B, N):
@@ -903,8 +1013,9 @@ class MAPPO:
         return max(1, min(8, (B * N) // 8192))
 
     def _rollout_pipelined(self, engine, arena, T, seed, deterministic, G, fused, oxy_i, o_count, hist_a, hist_c, act, logp, v,
-                           zeros_hist, timers=None, slot=lambda i: i):
-        """G independent env-group pipelines, one stream (+ one A* side stream) each; see rollout_batched.
+                           zeros_hist, timers=None, slot=lambda i: i, carry=None, pair_bootstrap=False):
+        """G independent env-group pipelines, one stream (+ one A* side stream) each; see rollout_batched.  Each group starts from its
+        rows of `carry` (None: zero hidden states at step 0); returns the RolloutCarry of the segment's end (None without a carry).
         timers: dict name -> list of (start, end) CUDA events recorded on the launching stream around every launch.  If it holds a
         "_policy_dbg" int64 tensor [T, G, >= CTAs per launch, 16], every policy launch instead writes its per-CTA record there (slots
         13 / 14 = %globaltimer at CTA start / end in ns, 15 = SM id; csrc/policy_fused.cu) - usable under CUDA-graph capture, which
@@ -948,6 +1059,9 @@ class MAPPO:
         # policy kernels fill the SMs meanwhile.
         stagger = int(os.environ.get("MARL_STAGGER", PIPELINE_STAGGER))
         stagger_ev = None
+        t0 = 0 if carry is None else carry.t0
+        if carry is not None:           # every group writes its rows of the next carry's hidden states
+            next_ha, next_hc = torch.empty_like(carry.ha), torch.empty_like(carry.hc)
         for g in range(G):
             lo, hi = g * B // G, (g + 1) * B // G
             st, side = engine._pipe_streams[2 * g], engine._pipe_streams[2 * g + 1]
@@ -958,12 +1072,15 @@ class MAPPO:
             with torch.cuda.stream(st):
                 view = _View()
                 view.B, view.N, view.O = hi - lo, N, engine.O
-                ha = torch.zeros(L, (hi - lo) * N, E, dtype=torch.float32, device=dev)
-                hc = torch.zeros(L, (hi - lo) * N, E, dtype=torch.float32, device=dev)
+                if carry is None:
+                    ha = torch.zeros(L, (hi - lo) * N, E, dtype=torch.float32, device=dev)
+                    hc = torch.zeros(L, (hi - lo) * N, E, dtype=torch.float32, device=dev)
+                else:
+                    ha, hc = carry.ha[:, lo * N:hi * N].clone(), carry.hc[:, lo * N:hi * N].clone()
                 sl = slice(lo, hi)
 
                 def hist_of(t, net="actor"):
-                    return _history_inputs(hist_a, hist_c, t, D, self.reference_quirks, net, slot, sl)
+                    return _history_inputs(hist_a, hist_c, t, D, self.reference_quirks, net, slot, sl, t0=t0)
 
                 def refresh():
                     view.p_state, view.e_state, view.map_id = engine.p_state[sl], engine.e_state[sl], engine.map_id[sl]
@@ -972,7 +1089,7 @@ class MAPPO:
                 refresh()
                 for t in range(T):
                     join = None
-                    if t % diff == 0:
+                    if (t0 + t) % diff == 0:
                         ev = torch.cuda.Event()
                         ev.record(st)
                         side.wait_event(ev)
@@ -982,7 +1099,7 @@ class MAPPO:
                     timed("env_observe_kernel", st, lambda: engine.observe(lo=lo, hi=hi))
                     h_t, h_tc = hist_of(t), hist_of(t, "critic")
                     timed("policy_step_kernel", st, lambda: fused.step(
-                        view, oxy_i, o_count, t, seed, deterministic, h_t, h_tc, hist_a[slot(t + D)][sl], hist_c[slot(t + D)][sl], ha, hc,
+                        view, oxy_i, o_count, t0 + t, seed, deterministic, h_t, h_tc, hist_a[slot(t + D)][sl], hist_c[slot(t + D)][sl], ha, hc,
                         act[t][sl], logp[t][sl], v[t][sl], row_offset=lo * N, tile_rows=full_tile,
                         debug=dbg[t, g] if dbg is not None else None))
                     if stagger > 0 and t == min(stagger, T - 1) - 1 and g + 1 < G:
@@ -994,13 +1111,24 @@ class MAPPO:
                 engine.observe(lo=lo, hi=hi)
                 h_fin = ([hist_c[slot(T - 1 + D)][sl]] + hist_of(T - 1)[:D - 1]) if self.reference_quirks else hist_of(T, "critic")
                 scratch = torch.empty(hi - lo, N, E, dtype=torch.float32, device=dev)
-                fused.step(view, oxy_i, o_count, T, seed, deterministic, h_fin, h_fin, scratch, scratch, ha, hc, None, None, v[T][sl],
-                           nets=("critic",), row_offset=lo * N, tile_rows=full_tile)
+                if carry is not None:   # before the bootstrap step, which updates hc in place
+                    next_ha[:, lo * N:hi * N].copy_(ha)
+                    next_hc[:, lo * N:hi * N].copy_(hc)
+                if pair_bootstrap:      # see rollout_batched
+                    fused.step(view, oxy_i, o_count, t0 + T, seed, deterministic, hist_of(T), h_fin, torch.empty_like(scratch), scratch,
+                               ha, hc, torch.empty_like(act[0][sl]), torch.empty_like(logp[0][sl]), v[T][sl], row_offset=lo * N,
+                               tile_rows=full_tile)
+                else:
+                    fused.step(view, oxy_i, o_count, t0 + T, seed, deterministic, h_fin, h_fin, scratch, scratch, ha, hc, None, None,
+                               v[T][sl], nets=("critic",), row_offset=lo * N, tile_rows=full_tile)
                 done = torch.cuda.Event()
                 done.record(st)
             main.wait_event(done)
+        if carry is not None:
+            return self._next_carry(carry, T, hist_a, hist_c, slot, next_ha, next_hc)
 
-    def explore_batched(self, engine, arena, T=None, seed=0, host_state=None, host_out=None, reset_reward_norm=False, history=None):
+    def explore_batched(self, engine, arena, T=None, seed=0, host_state=None, host_out=None, reset_reward_norm=False, history=None,
+                        carry=None):
         """The batched counterpart of `explore_env` (:731-740) - the call a user makes once per training iteration: one whole
         episode of ALL envs of `engine` with both networks in the loop, replayed from a CUDA graph that is captured on the first
         call (per engine / arena / T / seed; the weight images are re-packed inside the graph, so it follows the optimizer).
@@ -1013,15 +1141,32 @@ class MAPPO:
         history: as in `rollout_batched`, chosen when the graph is captured.
         Returns the TrainBatch of the episode (device resident, ready for `train`).  It lives in the graph's memory: it is valid until
         the next call with the same engine / arena / T / seed, which overwrites it - for a replay-mode batch this includes the weight
-        snapshot its history is regenerated with (the graph re-packs it in place)."""
-        T = T or arena.T
-        key = (id(engine), id(arena), int(T), int(seed))
+        snapshot its history is regenerated with (the graph re-packs it in place).
+
+        carry: as in `rollout_batched` - one segment of T steps from carry.t0, usually the previous segment's `batch.carry` (or
+        `RolloutCarry.zeros` at an episode's start).  One graph is captured per segment start; the carry is copied into that graph's
+        own input buffers before the replay, so consecutive segments chain.  The engine must be at step carry.t0 (checked: one
+        synchronisation), and host_state (an episode start) is only accepted with t0 = 0."""
+        T = (T or arena.T) if carry is None else (arena.T if T is None else int(T))
+        if carry is not None:
+            check_segment(carry, T, int(self.cfg.env.max_steps), engine.B, engine.N, self.num_layers, self.embedding_dim,
+                          self.depth, self.device)
+            if host_state is not None and carry.t0 != 0:
+                raise _lib.MarlError(f"explore_batched: host_state starts an episode, the carry continues one at step {carry.t0}")
+        key = (id(engine), id(arena), int(T), int(seed)) + (() if carry is None else (carry.t0,))
         graphs = self.__dict__.setdefault("_episode_graphs", {})
-        if key not in graphs:
-            graphs[key] = RolloutGraph(self, engine, arena, T, seed, history=history)
-        g = graphs[key]
         if host_state is not None:
             engine.load_host_state(reset_reward_norm=reset_reward_norm, **host_state)
+        if carry is not None:
+            at = engine.time_step.tolist()
+            if any(s != carry.t0 for s in at):
+                raise _lib.MarlError(f"explore_batched: segment from step {carry.t0}, the engine's envs are at steps {sorted(set(at))[:4]}")
+        if key not in graphs:
+            graphs[key] = RolloutGraph(self, engine, arena, T, seed, history=history,
+                                       carry=None if carry is None else RolloutCarry.zeros(self, engine.B, engine.N, carry.t0))
+        g = graphs[key]
+        if carry is not None:
+            g.carry.copy_(carry)
         g.replay()
         if host_out is not None:
             if "episode_reward" in host_out:
@@ -1034,8 +1179,18 @@ class MAPPO:
                 raise _lib.MarlError(f"explore_batched: evader status {int(status)} (A* OPEN / path overflow or target tape exhausted)")
         return g.batch
 
-    def _train_batch(self, engine, arena, T, oxy, hist_a, hist_c, v, logp, replay=None):
+    def _next_carry(self, carry, T, hist_a, hist_c, slot, ha, hc):
+        """The carry after a segment of T steps: its hidden states and the embeddings of its history steps T..T+D-1."""
+        last = lambda h: torch.stack([h[slot(T + j)] for j in range(self.depth)])     # noqa: E731
+        return RolloutCarry(carry.t0 + T, ha, hc, last(hist_a), last(hist_c))
+
+    def _train_batch(self, engine, arena, T, oxy, hist_a, hist_c, v, logp, replay=None, carry=None, next_carry=None):
         B, D, dev = engine.B, self.depth, self.device
+        seg = {}
+        if carry is not None:
+            seg = dict(t0=carry.t0, h0_a=carry.ha, h0_c=carry.hc, carry=next_carry)
+            if replay is not None:
+                seg.update(prefix_a=carry.emb_a, prefix_c=carry.emb_c)
         if replay is not None:         # the ring holds the last D+1 steps only: the history is regenerated per minibatch
             hist_a = hist_c = None
         oxy_env = oxy[engine.map_id.long()].contiguous()
@@ -1048,7 +1203,7 @@ class MAPPO:
                           p_adj_bits=arena.p_adj_bits[:T], e_adj=arena.e_adj[:T], o_adj_bits=arena.o_adj_bits[:T],
                           hist_a=hist_a, hist_c=hist_c, v=v, a=arena.a_n[:T], logp=logp, r=arena.r[:T],
                           active=arena.active[:T], depth=D, replay=replay,
-                          map_id=None if replay is None else engine.map_id.to(torch.int32).clone())
+                          map_id=None if replay is None else engine.map_id.to(torch.int32).clone(), **seg)
 
     def explore_env(self, env, num_episode):
         """Reference signature (:731-740) for the single-env facade `Pursuit_Env`: returns

@@ -11,7 +11,14 @@ count, and the reward and losses as float.hex.  Training is bit-reproducible, so
 columns:  diff <(grep -o 'exact.*' a.log) <(grep -o 'exact.*' b.log)
 
     python tools/train_loop.py --envs 512 --iters 3 --save-dir ck       # saves ck/training_state_rank0.pt after every iteration
-    python tools/train_loop.py --envs 512 --iters 6 --resume ck         # continues with iteration 3, as if never stopped"""
+    python tools/train_loop.py --envs 512 --iters 6 --resume ck         # continues with iteration 3, as if never stopped
+
+--segment S (a divisor of --steps; default: the whole episode) makes one iteration one rollout segment of S env steps followed by the
+epoch and update on it; the GRU hidden states and the history embeddings carry over to the next segment of the same episode, and envs
+are reset only at episode starts.  The episode reward is printed on the iteration that ends an episode ("-" on the others), and
+--save-dir / --resume work at any segment boundary.
+
+    python tools/train_loop.py --envs 512 --steps 150 --segment 50 --iters 6      # two episodes, three updates each"""
 import argparse
 import os
 import sys
@@ -24,7 +31,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from distributed_multi_agent_reinforcement_learning_b200 import default_config, parallel  # noqa: E402
 from distributed_multi_agent_reinforcement_learning_b200.checkpoint import load_training_state, save_training_state  # noqa: E402
-from distributed_multi_agent_reinforcement_learning_b200.mappo_parallel import MAPPO  # noqa: E402
+from distributed_multi_agent_reinforcement_learning_b200.mappo_parallel import MAPPO, RolloutCarry  # noqa: E402
 from distributed_multi_agent_reinforcement_learning_b200.pursuit_env import BatchedPursuitEnv, RolloutArena  # noqa: E402
 
 
@@ -34,6 +41,7 @@ def main():
     ap.add_argument("--maps", type=int, default=32)
     ap.add_argument("--pursuers", type=int, default=8)
     ap.add_argument("--steps", type=int, default=150)
+    ap.add_argument("--segment", type=int, default=None, help="env steps per iteration, a divisor of --steps (default: --steps)")
     ap.add_argument("--iters", type=int, default=10)
     ap.add_argument("--depth", type=int, default=1)
     ap.add_argument("--allreduce", default=None, choices=[None, "update", "minibatch"],
@@ -45,6 +53,10 @@ def main():
     args = ap.parse_args()
     if args.save_every < 1:
         ap.error("--save-every must be >= 1")
+    S = args.steps if args.segment is None else args.segment
+    if S < 1 or args.steps % S:
+        ap.error(f"--segment {S} must be a positive divisor of --steps {args.steps}")
+    n_seg = args.steps // S
     rank, world, local = (int(os.environ.get(k, d)) for k, d in (("RANK", 0), ("WORLD_SIZE", 1), ("LOCAL_RANK", 0)))
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -55,35 +67,52 @@ def main():
                          algo__learner_device=str(dev), algo__worker_device=str(dev))
     B, T, N = args.envs, args.steps, args.pursuers
     env = BatchedPursuitEnv(cfg, B, device=dev, num_maps=args.maps)
-    arena = RolloutArena(env.params, B, T, dev)
+    arena = RolloutArena(env.params, B, S, dev)
     torch.manual_seed(0)
     mappo = MAPPO(cfg, B, max(1, round(B / 10)), "Learner")
     mappo.sync_weights(0)
     total_steps, start = 0, 0
+    carry = RolloutCarry.zeros(mappo, B, N) if n_seg > 1 else None     # where the next segment of the current episode starts
+    ep_sum = torch.zeros(B, dtype=torch.int64, device=dev)              # raw reward of the current episode so far, per env
     state_file = lambda d: os.path.join(d, f"training_state_rank{rank}.pt")     # noqa: E731  (env shards and reward statistics are per rank)
     if args.resume:
-        extra = load_training_state(state_file(args.resume), mappo, env)
+        extra = load_training_state(state_file(args.resume), mappo, env, carry=carry)
         start, total_steps = int(extra["next_iter"]), int(extra["total_steps"])
+        if carry is not None:
+            ep_sum = extra["ep_reward_so_far"].to(dev)
+            if carry.t0 != (start % n_seg) * S:
+                raise SystemExit(f"--resume: the file continues at step {carry.t0} of an episode, iteration {start} of --segment {S} "
+                                 f"starts at step {(start % n_seg) * S}")
     W, H = cfg.map.map_size
     for it in range(start, args.iters):
+        ep, seg = divmod(it, n_seg)                    # episode and segment index (one segment per episode by default: ep == it)
         t0 = time.perf_counter()
-        if args.host_reset:
-            env.reset(seed=1000 * rank + it)                   # host generation with the reference's placement rules
-            g = np.random.default_rng(7 + 1000 * rank + it)
-            env.set_target_tape(np.stack([g.integers(0, W, (B, 16)), g.integers(0, H, (B, 16))], -1).astype(np.int32))
-        else:
-            env.reset_device(seed=1000 * rank + it)            # same rules, generated on the GPU (csrc/reset_kernels.cu)
+        if seg == 0:
+            if args.host_reset:
+                env.reset(seed=1000 * rank + ep)                   # host generation with the reference's placement rules
+                g = np.random.default_rng(7 + 1000 * rank + ep)
+                env.set_target_tape(np.stack([g.integers(0, W, (B, 16)), g.integers(0, H, (B, 16))], -1).astype(np.int32))
+            else:
+                env.reset_device(seed=1000 * rank + ep)            # same rules, generated on the GPU (csrc/reset_kernels.cu)
+            if carry is not None:
+                carry = RolloutCarry.zeros(mappo, B, N)
+            ep_sum.zero_()
         torch.cuda.synchronize()
         t1 = time.perf_counter()
-        if not args.host_reset:
+        if not args.host_reset and seg == 0:
             assert int(env.reset_fail.sum()) == 0, "device reset could not place every pursuer / evader"
-        tb = mappo.rollout_batched(env, arena, T, seed=it * world + rank)     # distinct sampling streams per replica and iteration
+        # distinct sampling streams per replica and episode; the segments of an episode share one (keyed by the episode's step)
+        tb = mappo.rollout_batched(env, arena, S, seed=ep * world + rank, carry=carry)
         torch.cuda.synchronize()
         t2 = time.perf_counter()
         assert int(env.evader_status.max()) == 0, "evader search overflow / target tape exhausted"
-        ep_reward = float(arena.raw_reward.sum(dim=(0, 2)).float().mean())
+        ep_sum += arena.raw_reward.sum(dim=(0, 2))
+        ep_end = seg == n_seg - 1
+        ep_reward = float(ep_sum.float().mean())
         collided = float(env.collision.float().mean())
-        total_steps += world * B * T
+        total_steps += world * B * S
+        if carry is not None:
+            carry = tb.carry
         for _ in range(int(cfg.algo.epochs)):                       # main.py:99: K epochs over the same buffers, one Adam step each
             obj_c, obj_a, _, _ = mappo.train(tb, total_steps, return_numpy=False, allreduce=args.allreduce)
             mappo.update(total_steps)
@@ -94,12 +123,16 @@ def main():
             torch.distributed.all_reduce(stats)
             stats /= world
         if args.save_dir and ((it + 1) % args.save_every == 0 or it + 1 == args.iters):
-            save_training_state(state_file(args.save_dir), mappo, env, extra=dict(next_iter=it + 1, total_steps=total_steps))
+            extra = dict(next_iter=it + 1, total_steps=total_steps)
+            if carry is not None:
+                extra["ep_reward_so_far"] = ep_sum.cpu()
+            save_training_state(state_file(args.save_dir), mappo, env, extra=extra, carry=None if ep_end else carry)
         if rank == 0:
             s = [float(x) for x in stats.cpu()]
-            print(f"iter {it:3d}  steps {total_steps:9d}  ep_reward {s[0]:9.2f}  collided {s[1]:5.2f}  objC {s[2]:8.4f}  "
+            rew, rew_hex = (f"{s[0]:9.2f}", s[0].hex()) if ep_end else (f"{'-':>9}", "-")
+            print(f"iter {it:3d}  steps {total_steps:9d}  ep_reward {rew}  collided {s[1]:5.2f}  objC {s[2]:8.4f}  "
                   f"objA {s[3]:8.4f}  reset {t1 - t0:5.2f}s  rollout {1e3 * (t2 - t1):7.1f}ms  train {1e3 * (t3 - t2):7.1f}ms  "
-                  f"exact {it} {total_steps} {s[0].hex()} {s[2].hex()} {s[3].hex()}", flush=True)
+                  f"exact {it} {total_steps} {rew_hex} {s[2].hex()} {s[3].hex()}", flush=True)
     if world > 1:
         torch.distributed.destroy_process_group()
 
