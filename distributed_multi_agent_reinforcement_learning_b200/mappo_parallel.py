@@ -20,6 +20,7 @@ Reference quirks kept on purpose (SURVEY 7.4-5; parity is defined per phase):
 """
 import os
 import time
+from types import SimpleNamespace
 
 import numpy as np
 import torch
@@ -31,7 +32,6 @@ from .normalization import Normalization
 from .replay_buffer import BigBuffer, ReplayBuffer
 
 
-PIPELINE_STAGGER = 0        # env steps by which consecutive env-group pipelines of a rollout are offset (see _rollout_pipelined)
 TWO_STREAM_TRAIN = True     # actor and critic branches of a training minibatch on two CUDA streams
 import os as _os
 CONCURRENT_MINIBATCHES = int(_os.environ.get("MARL_CONCURRENT_MB", "3"))  # minibatches of an epoch in flight at once (their clip-accumulate order is replayed afterwards)
@@ -60,6 +60,15 @@ def _history_inputs(hist_a, hist_c, t, D, quirks, net, slot, sl=slice(None), t0=
             back, src = k + 1, (hist_a if net == "actor" else hist_c)
         out.append(src[slot(t - back + D)][sl] if t0 + t - back >= 0 else None)
     return out
+
+
+def _bootstrap_history(hist_a, hist_c, T, D, quirks, slot, sl=slice(None), t0=0):
+    """The critic's D history inputs of the bootstrap value after a segment's last step T-1 (None = zeros).  reference_quirks: only the
+    critic's dataset is updated once more (:806-825), so the aliased list is C(T-1), then the list of step T-1 without its oldest entry;
+    otherwise the critic's own history of step T."""
+    if quirks:
+        return [hist_c[slot(T - 1 + D)][sl]] + _history_inputs(hist_a, hist_c, T - 1, D, True, "actor", slot, sl, t0)[:D - 1]
+    return _history_inputs(hist_a, hist_c, T, D, False, "critic", slot, sl, t0)
 
 
 class RolloutCarry:
@@ -438,23 +447,26 @@ class TrainBatch:
                    hist_c=tm(d["critic_historical_embedding"]).float(), v=tm(d["v_n"]).float(), a=tm(d["a_n"]).float(),
                    logp=tm(d["a_logprob_n"]).float(), r=tm(d["r"]).float(), active=tm(d["active"]).float(), depth=depth)
 
-    def minibatch(self, lo, hi):
-        """Envs [lo, hi): contiguous copies of the time-major slabs (the reference's sequential `batch[key][index]`).  A replay-mode
-        batch regenerates the minibatch's history from its slabs (on the current stream)."""
-        s = lambda x: None if x is None else x[:, lo:hi].contiguous()     # noqa: E731
-        mb = TrainBatch(p=s(self.p), e=s(self.e), oxy=self.oxy[lo:hi].contiguous(),
-                        o_count_train=self.o_count_train[lo:hi].contiguous(), p_adj_bits=s(self.p_adj_bits),
-                        e_adj=s(self.e_adj), o_adj_bits=s(self.o_adj_bits), hist_a=s(self.hist_a), hist_c=s(self.hist_c),
-                        v=s(self.v), a=s(self.a), logp=s(self.logp), r=s(self.r), active=s(self.active), depth=self.depth)
-        if self.h0_a is not None:
-            N = self.N
+    def _select(self, tm, em):
+        """The minibatch of the envs that `tm` selects from a time-major slab ([X, B, ...] -> [X, mb, ...]) and `em` from an env-major
+        tensor ([B, ...] -> [mb, ...]).  A replay-mode batch regenerates the minibatch's history from its slabs (on the current stream)."""
+        opt = lambda x: None if x is None else tm(x)     # noqa: E731
+        mb = TrainBatch(p=tm(self.p), e=tm(self.e), oxy=em(self.oxy), o_count_train=em(self.o_count_train), p_adj_bits=tm(self.p_adj_bits),
+                        e_adj=tm(self.e_adj), o_adj_bits=tm(self.o_adj_bits), hist_a=opt(self.hist_a), hist_c=opt(self.hist_c),
+                        v=tm(self.v), a=tm(self.a), logp=tm(self.logp), r=tm(self.r), active=tm(self.active), depth=self.depth)
+        if self.h0_a is not None:                   # hidden states [L, B*N, E], selected as the time-major [L, B, N, E]
+            L, E = self.h0_a.shape[0], self.h0_a.shape[-1]
             mb.t0 = self.t0
-            mb.h0_a, mb.h0_c = self.h0_a[:, lo * N:hi * N].contiguous(), self.h0_c[:, lo * N:hi * N].contiguous()
-            mb.prefix_a, mb.prefix_c = s(self.prefix_a), s(self.prefix_c)
+            mb.h0_a, mb.h0_c = (tm(h.view(L, self.B, self.N, E)).view(L, -1, E) for h in (self.h0_a, self.h0_c))
+            mb.prefix_a, mb.prefix_c = opt(self.prefix_a), opt(self.prefix_c)
         if self.replay is not None:
-            mb.replay, mb.map_id = self.replay, self.map_id[lo:hi].contiguous()
+            mb.replay, mb.map_id = self.replay, em(self.map_id)
             self.replay.regenerate(mb)
         return mb
+
+    def minibatch(self, lo, hi):
+        """Envs [lo, hi): contiguous copies of the slabs (the reference's sequential `batch[key][index]`)."""
+        return self._select(lambda x: x[:, lo:hi].contiguous(), lambda x: x[lo:hi].contiguous())
 
     def minibatch_indexed(self, index):
         """Envs `index` (int64 device tensor, any order): the reference's `batch[key][index]` (:665-679) for an arbitrary index list,
@@ -477,20 +489,7 @@ class TrainBatch:
                                                    _lib.stream_ptr()), "marl_gather_rows")
             return out
 
-        gh = lambda x: None if x is None else g(x)      # noqa: E731
-        out = TrainBatch(p=g(self.p), e=g(self.e), oxy=g(self.oxy, False), o_count_train=g(self.o_count_train, False),
-                         p_adj_bits=g(self.p_adj_bits), e_adj=g(self.e_adj), o_adj_bits=g(self.o_adj_bits), hist_a=gh(self.hist_a),
-                         hist_c=gh(self.hist_c), v=g(self.v), a=g(self.a), logp=g(self.logp), r=g(self.r), active=g(self.active),
-                         depth=self.depth)
-        if self.h0_a is not None:                   # hidden states: row (layer l, env b) of the [L*B, N*E] view
-            L, N = self.h0_a.shape[0], self.N
-            out.t0 = self.t0
-            out.h0_a, out.h0_c = (g(h.view(L, B, N, -1)).view(L, mb * N, -1) for h in (self.h0_a, self.h0_c))
-            out.prefix_a, out.prefix_c = gh(self.prefix_a), gh(self.prefix_c)
-        if self.replay is not None:
-            out.replay, out.map_id = self.replay, g(self.map_id, False)
-            self.replay.regenerate(out)
-        return out, g
+        return self._select(g, lambda x: g(x, False)), g
 
     def graph(self):
         T, B, N = self.T, self.B, self.N
@@ -523,7 +522,6 @@ class HistoryReplay:
         tensors being filled; a segment's slabs 0..D-1 are its history prefix).  embed_only (default REPLAY_EMBED_ONLY) False runs the
         full step from the batch's start hidden states and returns the replayed (log-prob, value) [T, mb, N] - the same numbers the
         rollout stored."""
-        from types import SimpleNamespace
         embed_only = REPLAY_EMBED_ONLY if embed_only is None else embed_only
         T, B, N, D, E, t0 = mb.T, mb.B, mb.N, mb.depth, self.fused.E, self.t0
         f32 = dict(dtype=torch.float32, device=mb.p.device)
@@ -554,16 +552,17 @@ class HistoryReplay:
 
 
 class RolloutGraph:
-    # (policy_dbg: see MAPPO._rollout_pipelined - an instrumented capture for measurements, not for production replays)
-    """`MAPPO.rollout_batched` for all envs of an engine (networks in the loop) captured as ONE CUDA graph: per env step
-    observe -> fused policy step (encoder + GRU + heads of both networks, one launch per env group) -> A* replan when due ->
-    fused evader-move / step / reward-norm / store kernel; no host involvement on replay.  The engine state the episode starts
-    from is whatever the engine holds at replay time.  With `carry` (a RolloutCarry whose tensors stay put: the graph reads them on
-    every replay) the graph is one segment of T steps starting at the episode's step carry.t0."""
+    """`MAPPO.rollout_batched` for all envs of an engine (networks in the loop) captured as ONE CUDA graph: the fused schedule of
+    G env-group pipelines, per env step and group observe -> fused policy step (encoder + GRU + heads of both networks, one launch)
+    || A* replan when due -> fused evader-move / step / reward-norm / store kernel; no host involvement on replay.  The engine state
+    the episode starts from is whatever the engine holds at replay time.  With `carry` (a RolloutCarry whose tensors stay put: the
+    graph reads them on every replay) the graph is one segment of T steps starting at the episode's step carry.t0.
+    policy_dbg: an instrumented capture for measurements, not for production replays - an int64 tensor [T, G, >= CTAs per launch,
+    16] that every policy launch of the G pipelines writes its per-CTA record to (see MAPPO.rollout_batched)."""
 
     def __init__(self, mappo, engine, arena, T, seed, policy_dbg=None, history=None, carry=None):
         snap = engine.snapshot()
-        kw = {} if policy_dbg is None else dict(timers={"_policy_dbg": policy_dbg}, pipelines=policy_dbg.shape[1])
+        kw = {} if policy_dbg is None else dict(policy_dbg=policy_dbg, pipelines=policy_dbg.shape[1])
         # decided once: the warm-up's allocations would otherwise change the free memory the captured rollout sees
         kw["history"] = history or mappo.history_mode(T, engine.B, engine.N)
         kw["carry"] = self.carry = carry
@@ -814,12 +813,27 @@ class MAPPO:
         return "store" if history_bytes(T, B, N, self.embedding_dim, self.depth) <= STORE_HISTORY_SHARE * free else "replay"
 
     @torch.no_grad()
-    def rollout_batched(self, engine, arena, T=None, seed=0, deterministic=False, groups=1, use_fused=None, timers=None,
-                        pipelines=None, actor_only=False, history=None, carry=None):
+    def rollout_batched(self, engine, arena, T=None, seed=0, deterministic=False, use_fused=None, timers=None, pipelines=None,
+                        actor_only=False, history=None, carry=None, policy_dbg=None):
         """MAPPO.run_episode (:742-827) for all B envs of a BatchedPursuitEnv at once, entirely on the GPU.
         Per step: observe kernel -> fused encoder (actor, then critic with all-ones adjacency) -> GRU cell -> heads ->
         closed-loop env kernel (evader move + pursuer step + reward-norm + store).  Fills `arena` plus the history /
         value / log-prob slabs and returns a TrainBatch ready for `train`.
+
+        With the fused policy step (use_fused; default: whenever the networks' shape has one) the envs are cut into G contiguous
+        env-group pipelines, each stepping through the episode on its own stream: observe -> ONE policy launch for both networks ->
+        env step, with the A* replan due every `difficulty` steps on the group's side stream beside the policy launch (it needs the
+        env state, not the action) and joined before the env step.  One group's small kernels and the long tail of its replanning
+        (the slowest of its searches gates its env step) then overlap with the other groups' policy kernels instead of idling the
+        GPU.  Results are the same for any G (the envs are independent and the sampling RNG is keyed by the global row).  G is 1 for
+        actor_only, else `pipelines`, else 1 with `timers`, else MARL_PIPELINES or `default_pipelines(B, N)`.  Without the fused
+        step (network shapes it does not cover) the unfused kernels run one after another on the current stream.
+
+        timers: dict name -> list of (start, end) CUDA events around every launch of the T steps (env_observe_kernel,
+        policy_step_kernel, evader_kernel(replan), rollout_kernel(closed)); the replan then runs on the group's own stream, after the
+        policy launch.  The bootstrap step is not timed.  policy_dbg: int64 [T, G, >= CTAs per launch, 16]; every policy launch of
+        the T steps writes its per-CTA record there (slots 13 / 14 = %globaltimer at CTA start / end in ns, 15 = SM id;
+        csrc/policy_fused.cu) - usable under CUDA-graph capture, which is how bench.py times the kernel inside the schedule.
 
         actor_only=True is the EVALUATOR's episode (evaluator.py:118-156): no critic, and the actor's history is its OWN
         embeddings A(t-1), A(t-2), ... (its dataset is not aliased with a critic's there); values / bootstrap stay zero.
@@ -870,138 +884,54 @@ class MAPPO:
             hist_c[:D].copy_(carry.emb_c)
         oxy = engine.boundary_xy.to(torch.float32).contiguous()                 # [M,O,2]
         o_count = torch.clamp(engine.boundary_count, max=engine.O).contiguous()  # rollout: the O_b real cells
-        enc = self.actor.shared_net
-        zeros_hist = torch.zeros(B, N, E, **f32)
-        w_eff = None
-
-        quirks = self.reference_quirks
-
-        def history(t, net="actor"):
-            # reference: one aliased list for both nets (:750-752): newest first = C(t-1), A(t-1), C(t-2), A(t-2), ...
-            # actor_only (the evaluator) / reference_quirks=False: each network's own embeddings, newest first
-            out = []
-            for k in range(D):
-                own = actor_only or not quirks
-                back = (k + 1) if own else (k // 2 + 1)
-                src = (hist_a if (net == "actor" or actor_only) else hist_c) if own else (hist_c if k % 2 == 0 else hist_a)
-                out.append(src[slot(t - back + D)] if t0 + t - back >= 0 else zeros_hist)
-            return out
-
-        def critic_step(t, graph):
-            nonlocal hc, w_eff
-            emb_c = enc.encode(graph, True, history(t, "critic"))
-            feat_c, hc = self.critic.features(emb_c.view(1, B * N, E), hc)
-            w, _ = self.critic.head_weight()
-            w_eff = w.reshape(E).contiguous()
-            return emb_c, feat_c[0]
 
         if use_fused:
-            # ONE launch per env step for both networks (csrc/policy_fused.cu); embeddings / values / log-probs / actions
-            # land directly in their rollout slabs.  The critic's effective head row is constant while the weights are
-            # (one power iteration on a [1,E] matrix is already converged), so it is computed once.  A replay-mode batch keeps the
-            # step (its own copy of the weights) to regenerate the history in training.
+            # ONE launch per env step and group for both networks (csrc/policy_fused.cu); embeddings / values / log-probs / actions
+            # land directly in their rollout slabs.  The critic's effective head row is constant while the weights are (one power
+            # iteration on a [1,E] matrix is already converged), so it is computed once.  A replay-mode batch keeps the step (its own
+            # copy of the weights) to regenerate the history in training.
             w, _ = self.critic.head_weight()
             fused = fused_policy.FusedRolloutStep(self, w.reshape(E).contiguous(), snapshot=replay)
             oxy_i = engine.boundary_xy.clone() if replay else engine.boundary_xy.contiguous()
-            rep_ = HistoryReplay(fused, oxy_i, o_count, quirks, t0) if replay else None
-            # The bootstrap value v[T] is a critic-only step at the episode's end.  A segment that ends inside the episode computes it
-            # with the step of both networks instead (the actor's outputs are discarded): that is the kernel the next segment's first
-            # step runs on the same state, and the critic-only kernel rounds the GRU cell and the value sum differently, so v[T] is
-            # then bit for bit the value the next segment starts with.
-            pair_bootstrap = carry is not None and t0 + T < int(self.cfg.env.max_steps)
-            none_if_zero = lambda lst: [None if h is zeros_hist else h for h in lst]   # noqa: E731
-            def timed(name, fn):
-                if timers is None:
-                    return fn()
-                a_, b_ = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                a_.record()
-                fn()
-                b_.record()
-                timers.setdefault(name, []).append((a_, b_))
-
-            # Env-group pipelines: the envs are independent, so the batch is cut into G contiguous groups, each stepping through
-            # the episode on its own stream (observe -> policy step || A* replan -> env step).  One group's small kernels and the
-            # long tail of its replanning (the slowest of its searches gates its env step) then overlap with the other groups'
-            # policy kernels instead of idling the GPU.  Same results for any G (the sampling RNG is keyed by the global row).
-            auto = pipelines is None
-            if auto:
-                pipelines = self.default_pipelines(B, N) if (timers is None and groups == 1) else 1
-                if os.environ.get("MARL_PIPELINES") and timers is None and groups == 1:      # tuning knob for tools/
-                    pipelines = int(os.environ["MARL_PIPELINES"])
-            if pipelines > 1 and (timers is None or not auto) and groups == 1 and not actor_only:
-                # (an explicit pipelines=G together with timers: CUDA events around every launch of the pipelined schedule itself)
-                nxt = self._rollout_pipelined(engine, arena, T, seed, deterministic, int(pipelines), fused, oxy_i, o_count, hist_a,
-                                              hist_c, act, logp, v, zeros_hist, timers=timers, slot=slot, carry=carry,
-                                              pair_bootstrap=pair_bootstrap)
-                return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp, rep_, carry, nxt)
-            # Single pipeline.  The A* replanning due every `difficulty` steps only needs the env state, not the action: it runs
-            # on a side stream concurrently with the policy kernel and is joined before the env kernel consumes the paths.
-            overlap = timers is None and groups == 1
-            main = torch.cuda.current_stream()
-            if overlap:
-                if getattr(engine, "_replan_stream", None) is None:
-                    engine._replan_stream = torch.cuda.Stream(device=dev)
-                side = engine._replan_stream
-            diff = int(engine.params.difficulty)
-            for t in range(T):
-                join = None
-                if overlap and (t0 + t) % diff == 0:
-                    fork = torch.cuda.Event()
-                    fork.record(main)
-                    side.wait_event(fork)
-                    engine.evader_replan(0, B, side)
-                    join = torch.cuda.Event()
-                    join.record(side)
-                timed("env_observe_kernel", engine.observe)
-                h_t, h_tc = none_if_zero(history(t)), none_if_zero(history(t, "critic"))
-                timed("policy_step_kernel", lambda: fused.step(engine, oxy_i, o_count, t0 + t, seed, deterministic, h_t, h_tc,
-                                                               hist_a[slot(t + D)], hist_c[slot(t + D)], ha, hc, act[t], logp[t], v[t],
-                                                               nets=("actor",) if actor_only else ("actor", "critic")))
-                if join is not None:
-                    main.wait_event(join)
-                engine.rollout_closed(arena, 1, t0=t, action_tape=act[t:t + 1], env_t0=t0 + t, groups=groups, timers=timers,
-                                      skip_replan=join is not None)
-            if actor_only:
-                return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp)
-            engine.observe()
-            h_fin = none_if_zero(([hist_c[slot(T - 1 + D)]] + history(T - 1)[:D - 1]) if quirks else history(T, "critic"))
-            scratch = torch.empty(B, N, E, **f32)
-            nxt = None if carry is None else self._next_carry(carry, T, hist_a, hist_c, slot, ha, hc.clone())
-            if pair_bootstrap:              # (on copies: the bootstrap step updates the hidden states in place)
-                fused.step(engine, oxy_i, o_count, t0 + T, seed, deterministic, none_if_zero(history(T)), h_fin, torch.empty_like(scratch),
-                           scratch, ha.clone(), hc, torch.empty_like(act[0]), torch.empty_like(logp[0]), v[T])
-            else:
-                fused.step(engine, oxy_i, o_count, t0 + T, seed, deterministic, h_fin, h_fin, scratch, scratch, ha, hc, None, None, v[T],
-                           nets=("critic",))
+            rep_ = HistoryReplay(fused, oxy_i, o_count, self.reference_quirks, t0) if replay else None
+            G = (1 if actor_only else int(pipelines) if pipelines is not None else 1 if timers is not None
+                 else int(os.environ.get("MARL_PIPELINES") or self.default_pipelines(B, N)))
+            nxt = self._rollout_fused(engine, arena, T, seed, deterministic, G, fused, oxy_i, o_count, hist_a, hist_c, ha, hc, act, logp,
+                                      v, slot, carry, actor_only, timers, policy_dbg)
             return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp, rep_, carry, nxt)
 
+        enc = self.actor.shared_net
+        quirks = self.reference_quirks and not actor_only
+        zeros_hist = torch.zeros(B, N, E, **f32)
+        zeros_for_none = lambda hs: [zeros_hist if h is None else h for h in hs]     # noqa: E731
+        observed = lambda: ops.GraphBatch(engine.p_state.to(torch.float32), engine.e_state.to(torch.float32), oxy,   # noqa: E731
+                                          engine.map_id, o_count, engine.p_adj_bits, engine.e_adj, engine.o_adj_bits)
         for t in range(T):
             engine.observe()
-            graph = ops.GraphBatch(engine.p_state.to(torch.float32), engine.e_state.to(torch.float32), oxy, engine.map_id,
-                                   o_count, engine.p_adj_bits, engine.e_adj, engine.o_adj_bits)
-            emb_a = enc.encode(graph, False, history(t))
+            graph = observed()
+            emb_a = enc.encode(graph, False, zeros_for_none(_history_inputs(hist_a, hist_c, t, D, quirks, "actor", slot, t0=t0)))
             feat_a, ha = self.actor.features(emb_a.view(1, B * N, E), ha)
             if actor_only:
                 a_i, _, lp, _ = ops.act_head(feat_a[0], None, self.actor.Mean.weight, self.actor.Mean.bias, None, None, seed, t0 + t,
                                              deterministic)
                 hist_a[t + D] = emb_a
             else:
-                emb_c, feat_c = critic_step(t, graph)
-                a_i, _, lp, val = ops.act_head(feat_a[0], feat_c, self.actor.Mean.weight, self.actor.Mean.bias, w_eff,
-                                               self.critic.Mean.bias, seed, t0 + t, deterministic)
+                emb_c = enc.encode(graph, True, zeros_for_none(_history_inputs(hist_a, hist_c, t, D, quirks, "critic", slot, t0=t0)))
+                feat_c, hc = self.critic.features(emb_c.view(1, B * N, E), hc)
+                w, _ = self.critic.head_weight()
+                a_i, _, lp, val = ops.act_head(feat_a[0], feat_c[0], self.actor.Mean.weight, self.actor.Mean.bias,
+                                               w.reshape(E).contiguous(), self.critic.Mean.bias, seed, t0 + t, deterministic)
                 hist_a[t + D], hist_c[t + D] = emb_a, emb_c
                 v[t] = val.view(B, N)
             logp[t], act[t] = lp.view(B, N), a_i.view(B, N)
-            engine.rollout_closed(arena, 1, t0=t, action_tape=act[t:t + 1], env_t0=t0 + t, groups=groups)
+            engine.rollout_closed(arena, 1, t0=t, action_tape=act[t:t + 1], env_t0=t0 + t)
         if actor_only:
             return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp)
-        # bootstrap value of the final state (:806-825): only the critic's dataset is updated once more
+        # bootstrap value of the final state (:806-825)
         engine.observe()
-        graph = ops.GraphBatch(engine.p_state.to(torch.float32), engine.e_state.to(torch.float32), oxy, engine.map_id,
-                               o_count, engine.p_adj_bits, engine.e_adj, engine.o_adj_bits)
-        hist_final = ([hist_c[T - 1 + D]] + history(T - 1)[:D - 1]) if quirks else history(T, "critic")
+        graph = observed()
         nxt = None if carry is None else self._next_carry(carry, T, hist_a, hist_c, slot, ha, hc)
-        emb_c = enc.encode(graph, True, hist_final)
+        emb_c = enc.encode(graph, True, zeros_for_none(_bootstrap_history(hist_a, hist_c, T, D, quirks, slot, t0=t0)))
         feat_c, _ = self.critic.features(emb_c.view(1, B * N, E), hc)
         w, _ = self.critic.head_weight()
         v[T] = torch.nn.functional.linear(feat_c[0], w, self.critic.Mean.bias).view(B, N)
@@ -1012,34 +942,30 @@ class MAPPO:
         """Env-group pipelines of a batched rollout: one per 8192 (env, agent) rows, at most 8."""
         return max(1, min(8, (B * N) // 8192))
 
-    def _rollout_pipelined(self, engine, arena, T, seed, deterministic, G, fused, oxy_i, o_count, hist_a, hist_c, act, logp, v,
-                           zeros_hist, timers=None, slot=lambda i: i, carry=None, pair_bootstrap=False):
-        """G independent env-group pipelines, one stream (+ one A* side stream) each; see rollout_batched.  Each group starts from its
-        rows of `carry` (None: zero hidden states at step 0); returns the RolloutCarry of the segment's end (None without a carry).
-        timers: dict name -> list of (start, end) CUDA events recorded on the launching stream around every launch.  If it holds a
-        "_policy_dbg" int64 tensor [T, G, >= CTAs per launch, 16], every policy launch instead writes its per-CTA record there (slots
-        13 / 14 = %globaltimer at CTA start / end in ns, 15 = SM id; csrc/policy_fused.cu) - usable under CUDA-graph capture, which
-        is how bench.py times the kernel inside the schedule it reports."""
-        dbg = timers.pop("_policy_dbg", None) if timers is not None else None
-        if timers is not None and not timers and dbg is not None:
-            timers = None                                   # only the in-kernel records were asked for: no events (graph capture)
-        B, N, E, D, L = engine.B, engine.N, self.embedding_dim, self.depth, self.num_layers
-        dev = self.device
-        main = torch.cuda.current_stream()
+    def _rollout_fused(self, engine, arena, T, seed, deterministic, G, fused, oxy_i, o_count, hist_a, hist_c, h0_a, h0_c, act, logp, v,
+                       slot, carry, actor_only, timers, policy_dbg):
+        """The fused schedule of `rollout_batched`: G independent env-group pipelines, one stream (+ one A* side stream) each.  Each
+        group starts from its rows of the hidden states h0_a / h0_c [L, B*N, E] (one group steps them in place); returns the
+        RolloutCarry of the segment's end (None without a carry)."""
+        B, N, E, D = engine.B, engine.N, self.embedding_dim, self.depth
+        f32 = dict(dtype=torch.float32, device=self.device)
+        quirks = self.reference_quirks and not actor_only
+        nets = ("actor",) if actor_only else ("actor", "critic")
+        t0 = 0 if carry is None else carry.t0
+        # The bootstrap value v[T] is a critic-only step at the episode's end.  A segment that ends inside the episode computes it with
+        # the step of both networks instead (the actor's outputs are discarded): that is the kernel the next segment's first step runs
+        # on the same state, and the critic-only kernel rounds the GRU cell and the value sum differently, so v[T] is then bit for bit
+        # the value the next segment starts with.
+        pair_bootstrap = carry is not None and t0 + T < int(self.cfg.env.max_steps)
         if len(getattr(engine, "_pipe_streams", [])) < 2 * G:
-            # MARL_PIPE_PRIORITY (measurement knob): "astar" / "policy" gives the A* side streams / the policy streams the high priority
-            prio = os.environ.get("MARL_PIPE_PRIORITY", "")
-            engine._pipe_streams = [torch.cuda.Stream(device=dev, priority=(-1 if (prio == "astar" and i % 2 == 1) or (prio == "policy" and i % 2 == 0) else 0))
-                                    for i in range(2 * G)]
+            engine._pipe_streams = [torch.cuda.Stream(device=self.device) for _ in range(2 * G)]
         rec_ptrs = arena.record_pointers()
         diff = int(engine.params.difficulty)
-        full_tile = (128 // N) * N if N <= 128 else 0      # concurrent launches: full tiles, SMs left over for the neighbours
-        if os.environ.get("MARL_PIPE_TILE_ROWS"):            # tuning knob for tools/
-            full_tile = int(os.environ["MARL_PIPE_TILE_ROWS"])
-        fork = torch.cuda.Event(enable_timing=timers is not None)
-        fork.record(main)
-        if timers is not None:
-            timers["_t0"] = fork
+        # A lone launch takes the kernel's wave model (tile_rows 0: see policy_fused.cu); concurrent launches take full tiles and leave
+        # SMs over for the neighbouring groups' kernels.
+        tile = 0
+        if G > 1:
+            tile = int(os.environ.get("MARL_PIPE_TILE_ROWS") or ((128 // N) * N if N <= 128 else 0))     # (the knob: tools/)
 
         def timed(name, stream, fn):
             if timers is None:
@@ -1050,77 +976,60 @@ class MAPPO:
             b_.record(stream)
             timers.setdefault(name, []).append((a_, b_))
 
-        class _View:                                     # what FusedRolloutStep.step reads from an engine, for envs [lo, hi)
-            pass
-
-        # Stagger: every group replans at the same env steps (t % difficulty == 0), and a replan stalls its group for the length of
-        # its slowest A* search; groups that run in lockstep would all be stalled at once.  Group g therefore starts when group g-1
-        # has launched its policy step number `stagger`: the stalls then fall on different wall-clock times and the other groups'
-        # policy kernels fill the SMs meanwhile.
-        stagger = int(os.environ.get("MARL_STAGGER", PIPELINE_STAGGER))
-        stagger_ev = None
-        t0 = 0 if carry is None else carry.t0
+        main = torch.cuda.current_stream()
+        fork = torch.cuda.Event()
+        fork.record(main)
         if carry is not None:           # every group writes its rows of the next carry's hidden states
             next_ha, next_hc = torch.empty_like(carry.ha), torch.empty_like(carry.hc)
         for g in range(G):
             lo, hi = g * B // G, (g + 1) * B // G
+            sl, rows = slice(lo, hi), slice(lo * N, hi * N)
             st, side = engine._pipe_streams[2 * g], engine._pipe_streams[2 * g + 1]
             st.wait_event(fork)
-            if stagger_ev is not None:
-                st.wait_event(stagger_ev)
-                stagger_ev = None
             with torch.cuda.stream(st):
-                view = _View()
-                view.B, view.N, view.O = hi - lo, N, engine.O
-                if carry is None:
-                    ha = torch.zeros(L, (hi - lo) * N, E, dtype=torch.float32, device=dev)
-                    hc = torch.zeros(L, (hi - lo) * N, E, dtype=torch.float32, device=dev)
-                else:
-                    ha, hc = carry.ha[:, lo * N:hi * N].clone(), carry.hc[:, lo * N:hi * N].clone()
-                sl = slice(lo, hi)
+                # what FusedRolloutStep.step reads from an engine, for envs [lo, hi) (views: the kernels update them in place)
+                view = SimpleNamespace(B=hi - lo, N=N, O=engine.O, p_state=engine.p_state[sl], e_state=engine.e_state[sl],
+                                       map_id=engine.map_id[sl], p_adj_bits=engine.p_adj_bits[sl], e_adj=engine.e_adj[sl],
+                                       o_adj_bits=engine.o_adj_bits[sl])
+                ha, hc = h0_a[:, rows].contiguous(), h0_c[:, rows].contiguous()
 
-                def hist_of(t, net="actor"):
-                    return _history_inputs(hist_a, hist_c, t, D, self.reference_quirks, net, slot, sl, t0=t0)
+                def hist_of(t, net):
+                    return _history_inputs(hist_a, hist_c, t, D, quirks, net, slot, sl, t0=t0)
 
-                def refresh():
-                    view.p_state, view.e_state, view.map_id = engine.p_state[sl], engine.e_state[sl], engine.map_id[sl]
-                    view.p_adj_bits, view.e_adj, view.o_adj_bits = engine.p_adj_bits[sl], engine.e_adj[sl], engine.o_adj_bits[sl]
-
-                refresh()
                 for t in range(T):
-                    join = None
-                    if (t0 + t) % diff == 0:
+                    replan, join = (t0 + t) % diff == 0, None
+                    if replan and timers is None:
                         ev = torch.cuda.Event()
                         ev.record(st)
                         side.wait_event(ev)
-                        timed("evader_kernel", side, lambda: engine.evader_replan(lo, hi, side))
+                        engine.evader_replan(lo, hi, side)
                         join = torch.cuda.Event()
                         join.record(side)
                     timed("env_observe_kernel", st, lambda: engine.observe(lo=lo, hi=hi))
-                    h_t, h_tc = hist_of(t), hist_of(t, "critic")
                     timed("policy_step_kernel", st, lambda: fused.step(
-                        view, oxy_i, o_count, t0 + t, seed, deterministic, h_t, h_tc, hist_a[slot(t + D)][sl], hist_c[slot(t + D)][sl], ha, hc,
-                        act[t][sl], logp[t][sl], v[t][sl], row_offset=lo * N, tile_rows=full_tile,
-                        debug=dbg[t, g] if dbg is not None else None))
-                    if stagger > 0 and t == min(stagger, T - 1) - 1 and g + 1 < G:
-                        stagger_ev = torch.cuda.Event()
-                        stagger_ev.record(st)
+                        view, oxy_i, o_count, t0 + t, seed, deterministic, hist_of(t, "actor"), hist_of(t, "critic"),
+                        hist_a[slot(t + D)][sl], hist_c[slot(t + D)][sl], ha, hc, act[t][sl], logp[t][sl], v[t][sl], nets=nets,
+                        row_offset=lo * N, tile_rows=tile, debug=None if policy_dbg is None else policy_dbg[t, g]))
                     if join is not None:
                         st.wait_event(join)
-                    timed("rollout_kernel", st, lambda: engine._closed_chunk(arena, rec_ptrs, lo, hi, t, 1, act[t:t + 1], 0, seed, st))
-                engine.observe(lo=lo, hi=hi)
-                h_fin = ([hist_c[slot(T - 1 + D)][sl]] + hist_of(T - 1)[:D - 1]) if self.reference_quirks else hist_of(T, "critic")
-                scratch = torch.empty(hi - lo, N, E, dtype=torch.float32, device=dev)
-                if carry is not None:   # before the bootstrap step, which updates hc in place
-                    next_ha[:, lo * N:hi * N].copy_(ha)
-                    next_hc[:, lo * N:hi * N].copy_(hc)
-                if pair_bootstrap:      # see rollout_batched
-                    fused.step(view, oxy_i, o_count, t0 + T, seed, deterministic, hist_of(T), h_fin, torch.empty_like(scratch), scratch,
-                               ha, hc, torch.empty_like(act[0][sl]), torch.empty_like(logp[0][sl]), v[T][sl], row_offset=lo * N,
-                               tile_rows=full_tile)
-                else:
-                    fused.step(view, oxy_i, o_count, t0 + T, seed, deterministic, h_fin, h_fin, scratch, scratch, ha, hc, None, None,
-                               v[T][sl], nets=("critic",), row_offset=lo * N, tile_rows=full_tile)
+                    elif replan:
+                        timed("evader_kernel(replan)", st, lambda: engine.evader_replan(lo, hi, st))
+                    timed("rollout_kernel(closed)", st, lambda: engine._closed_chunk(arena, rec_ptrs, lo, hi, t, 1, act[t:t + 1], 0, seed,
+                                                                                      st))
+                if not actor_only:
+                    engine.observe(lo=lo, hi=hi)
+                    h_fin = _bootstrap_history(hist_a, hist_c, T, D, quirks, slot, sl, t0)
+                    scratch = torch.empty(hi - lo, N, E, **f32)
+                    if carry is not None:   # before the bootstrap step, which updates the hidden states in place
+                        next_ha[:, rows].copy_(ha)
+                        next_hc[:, rows].copy_(hc)
+                    if pair_bootstrap:
+                        fused.step(view, oxy_i, o_count, t0 + T, seed, deterministic, hist_of(T, "actor"), h_fin, torch.empty_like(scratch),
+                                   scratch, ha, hc, torch.empty_like(act[0][sl]), torch.empty_like(logp[0][sl]), v[T][sl],
+                                   row_offset=lo * N, tile_rows=tile)
+                    else:
+                        fused.step(view, oxy_i, o_count, t0 + T, seed, deterministic, h_fin, h_fin, scratch, scratch, ha, hc, None, None,
+                                   v[T][sl], nets=("critic",), row_offset=lo * N, tile_rows=tile)
                 done = torch.cuda.Event()
                 done.record(st)
             main.wait_event(done)

@@ -310,7 +310,7 @@ class BatchedPursuitEnv:
             "marl_rollout_closed")
         self.launches += 1
 
-    def rollout_closed(self, arena, K, t0=0, action_tape=None, seed=0, env_t0=0, timers=None, groups=1, skip_replan=False):
+    def rollout_closed(self, arena, K, t0=0, action_tape=None, seed=0, env_t0=0, groups=1):
         """K closed-loop env iterations with the A* evader on the GPU.  The evader's per-step move is fused into the
         rollout kernel; replanning is one launch per `difficulty` steps, so K steps are 2*ceil(K/difficulty) launches
         per group.  `env_t0` is the (lock-step) env time_step at entry.
@@ -318,10 +318,7 @@ class BatchedPursuitEnv:
         groups > 1 splits the envs into that many contiguous sub-batches, each running its own launch chain on its own
         CUDA stream: a search that takes 100x longer than the median (A* is a long-tailed workload) then only holds
         up its own sub-batch while the other chains keep the SMs busy.  Results are identical for any grouping.
-        Nothing touches the host, so the whole thing can be captured in a CUDA graph (EpisodeGraph).
-        timers: optional dict name -> list of (start_event, end_event) around every launch (groups == 1 only).
-        skip_replan: the caller has already launched evader_replan for this boundary (e.g. on a side stream, overlapped
-        with the policy kernel) and joined it."""
+        Nothing touches the host, so the whole thing can be captured in a CUDA graph (EpisodeGraph)."""
         assert arena.B == self.B
         if action_tape is not None:
             assert tuple(action_tape.shape) == (K, self.B, self.N) and action_tape.dtype == torch.int32
@@ -331,28 +328,14 @@ class BatchedPursuitEnv:
         groups = max(1, min(int(groups), self.B))
         bounds = [(g * self.B // groups, (g + 1) * self.B // groups) for g in range(groups)]
 
-        def mark(name):
-            if timers is None or groups != 1:
-                return None
-            ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
-            timers.setdefault(name, []).append(ev)
-            ev[0].record()
-            return ev
-
         def chain(lo, hi, stream):
             k = 0
             while k < K:
                 ts = env_t0 + k
-                if ts % D == 0 and not skip_replan:
-                    ev = mark("evader_kernel(replan)")
+                if ts % D == 0:
                     self.evader_replan(lo, hi, stream)
-                    if ev:
-                        ev[1].record()
                 chunk = min(D - ts % D, K - k)
-                ev = mark("rollout_kernel(closed)")
                 self._closed_chunk(arena, rec_ptrs, lo, hi, t0 + k, chunk, action_tape, k, seed, stream)
-                if ev:
-                    ev[1].record()
                 k += chunk
 
         if groups == 1:
