@@ -41,8 +41,9 @@ constexpr int WSTAGE = 2 * TILE;          // one k-block of a 128-row weight uni
 constexpr int MISC_BYTES = 3072;           // barriers, fp32 state of the tile
 constexpr int OXY_CAP = 256;               // boundary cells of one map staged per worker warp (fast message path: O <= 256)
 constexpr int OXY_BYTES = 16 * OXY_CAP * 8; // up to 16 worker warps x 256 float2
-constexpr int SMEM_BYTES = X_BYTES + NSTAGE * WSTAGE + MISC_BYTES + OXY_BYTES;   // 227 KB
-constexpr bool kDualByDefault = false;     // measured: the two-CTA-per-SM kernel is 10 % slower than 16 worker warps in one CTA (see Mem<DUAL>)
+// shared memory of the one-chain kernel: X | weight ring | barriers + fp32 state | boundary-cell staging
+constexpr int RING_OFF = X_BYTES, MISC_OFF = RING_OFF + NSTAGE * WSTAGE, OXY_OFF = MISC_OFF + MISC_BYTES;
+constexpr int SMEM_BYTES = OXY_OFF + OXY_BYTES;   // 227 KB
 // Worker-warp count WW is a template parameter of the kernel: 16 worker warps (8 rows each in the SIMT phases, 32 columns each in
 // the epilogues) when an env fits in 8 rows - the SIMT phases are latency-bound, twice the warps hide twice the latency - and 8
 // worker warps (16 rows / 64 columns each) for N = 16, whose env-grouped message path needs a whole env per warp.
@@ -52,27 +53,6 @@ struct Lay {
     static constexpr int RPW = ROWS / WW;            // rows per warp in the SIMT phases
     static constexpr int CPT = 128 / (WW / 4);       // accumulator columns per thread in the epilogues
     static constexpr int WORKERS = WW * 32, THREADS = (WW + 2) * 32;
-};
-// DUAL = two CTAs per SM (8 worker warps, 96 registers, 110 KB shared memory, 256 TMEM columns each): while one CTA waits for its
-// MMAs the other runs its SIMT phases / epilogues, which hides the hand-over and tensor time that a single resident CTA spends idle.
-// What it costs: the weight ring shrinks to two 16 KB stages (one operand plane of a k-block each), and the GRU - whose four gate
-// accumulators of 128 columns need all 512 TMEM columns for one tile - runs in two 64-column halves, each half re-staging x and
-// h_prev in X (they come back from L2), with the new state written straight from registers to a second hidden buffer.
-// MEASURED (bench shape, tools/fused_phase_profile.py with MARL_VARIANT=2): correct (same parity tests), but 0.44 ms per launch
-// against 0.40 ms for one CTA with 16 worker warps.  With 16 warps the SIMT phases are instruction-ISSUE-bound (stall samples are
-// "selected / not selected"; 319 K warp instructions per item over 4 schedulers = 80 K of the ~110 K SIMT cycles), so a co-resident
-// CTA cannot speed them up, and this variant's own SIMT work is larger (8-row-per-warp code does not fit 96 registers at 16 rows per
-// warp: spills; six extra X fills per item).  Kept selectable (marl_policy_step.variant = 2) and tested; not the default.
-template <bool DUAL>
-struct Mem {
-    static constexpr int NST = DUAL ? 2 : NSTAGE;
-    static constexpr int STAGE = DUAL ? TILE : WSTAGE;                 // bytes per ring stage
-    static constexpr int OXY = DUAL ? 176 : OXY_CAP;                   // boundary cells staged per worker warp
-    static constexpr int OXY_WARPS = DUAL ? 8 : 16;
-    static constexpr int RING_OFF = X_BYTES, MISC_OFF = X_BYTES + NST * STAGE, OXY_OFF = MISC_OFF + MISC_BYTES;
-    static constexpr int BYTES = OXY_OFF + OXY_WARPS * OXY * 8;        // 227 KB / 110 KB
-    static constexpr int TMEM_COLS = DUAL ? 256 : 512;
-    static constexpr int BAR_READY = 2 * NST, BAR_DONE = 2 * NST + 1;
 };
 
 struct Unit {
@@ -99,7 +79,7 @@ struct NetArgs {
     const float *hist[MAXD];   // [B,N,E] history embeddings, k = 0 most recent; null = zeros
     float *emb_out;            // [B,N,E]
     const float *hidden_in;    // [2, R, E] previous hidden state
-    float *hidden_out;         // [2, R, E] new hidden state (may alias hidden_in in the one-CTA-per-SM kernel)
+    float *hidden_out;         // [2, R, E] new hidden state (may alias hidden_in)
     int all_ones;              // critic
 };
 
@@ -148,25 +128,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
             : "r"(bar), "r"(parity)
             : "memory");
     } while (!done);
-}
-// same, but the polling warp sleeps between attempts: a waiting warp that spins takes issue slots from the warps that work (the
-// other CTA of the SM in the two-CTA variant, the worker warps for the loader / issuer lanes)
-__device__ __forceinline__ void mbar_wait_sleep(uint32_t bar, uint32_t parity, unsigned ns)
-{
-    uint32_t done;
-    for (;;) {
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-            "selp.u32 %0, 1, 0, p;\n"
-            "}\n"
-            : "=r"(done)
-            : "r"(bar), "r"(parity)
-            : "memory");
-        if (done) break;
-        __nanosleep(ns);
-    }
 }
 __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar)
 {
@@ -299,13 +260,11 @@ struct Ctx {
     int64_t row0;        // first global row of the tile
     int warp, lane;
     uint32_t tmem, bar_a_ready, bar_mma_done;
-    unsigned wait_sleep_ns;   // 0: spin while waiting for the MMAs; > 0: sleep between polls (two-CTA variant)
     int group;           // groups completed so far (parity of mma_done)
     float4 *s_p;         // [128] fp32 pursuer state of the tile's rows (converted once)
     float4 *s_e;         // [32] fp32 evader state of the tile's envs (when the tile has <= 32 envs)
     float *s_val;        // [WW/4][128] scratch for the critic value (aliases s_p, which is dead by then)
-    float2 *s_oxy;       // [worker warps][oxy_cap] boundary cells of the env a warp is working on (obstacle relation)
-    int oxy_cap;
+    float2 *s_oxy;       // [worker warps][OXY_CAP] boundary cells of the env a warp is working on (obstacle relation)
 };
 
 __device__ __forceinline__ bool row_info(const Ctx &c, int r, int64_t &gr, int &env, int &i)
@@ -354,8 +313,7 @@ __device__ __forceinline__ void signal_ready(Ctx &c)
 }
 __device__ __forceinline__ void wait_done(Ctx &c)
 {
-    if (c.wait_sleep_ns) mbar_wait_sleep(c.bar_mma_done, (uint32_t)(c.group & 1), c.wait_sleep_ns);
-    else mbar_wait(c.bar_mma_done, (uint32_t)(c.group & 1));
+    mbar_wait(c.bar_mma_done, (uint32_t)(c.group & 1));
     tc_fence_after();
     ++c.group;
 }
@@ -550,7 +508,7 @@ __device__ void phase_msg_fast(const Ctx &c, int rel, const float (&w)[4][8], co
             const int2 *oxy = reinterpret_cast<const int2 *>(a->oxy) + (int64_t)m * a->O;
             // the map's boundary cells -> this warp's shared-memory staging (one broadcast LDS.64 per cell in the loops below;
             // the loops are unrolled so that several cells are in flight)
-            float2 *so = c.s_oxy + c.warp * c.oxy_cap;
+            float2 *so = c.s_oxy + c.warp * OXY_CAP;
             __syncwarp();                                      // the previous env's readers are done
 #pragma unroll
             for (int t = 0; t < 8; ++t) {
@@ -667,7 +625,7 @@ template <int WW>
 __device__ __forceinline__ bool fast_env_path(const Ctx &c)
 {
     const StepArgs *a = c.a;
-    return (a->N == 4 || a->N == 8 || a->N == 16) && a->N <= Lay<WW>::RPW && a->O <= c.oxy_cap;
+    return (a->N == 4 || a->N == 8 || a->N == 16) && a->N <= Lay<WW>::RPW && a->O <= OXY_CAP;
 }
 
 template <int WW, bool F32>
@@ -794,7 +752,8 @@ __device__ __forceinline__ void hidden_store(const Ctx &c, const float4 (&v)[Lay
     for (int rr = 0; rr < RPW; ++rr) x_store4(c.X, RPW * c.warp + rr, c.lane, v[rr]);
 }
 
-// global rows [R,E] -> X in two chunks of 8 rows per warp (the two-CTA variant runs at 96 registers: 8 x float4 in flight)
+// global rows [R,E] -> X in chunks of 8 rows per warp.  The pair kernel issues the loads of all its chunks before it waits for the
+// running MMA group and stores them to X after the wait.
 template <int WW>
 __device__ __forceinline__ void rows_prefetch8(const Ctx &c, const float *src, int chunk, float4 (&v)[8])
 {
@@ -956,63 +915,6 @@ __device__ void epi_cell(const Ctx &c, int l, bool want_value)
     }
 }
 
-// ---- epilogue (two-CTA variant): one 64-column half of the GRU cell.  Accumulators r @0, z @64, n_i @128, n_h @192 (64 columns
-// each, column j of the half = output column 64*half + j); h_prev is read back from X; the new state goes straight from registers
-// to the OUTPUT hidden buffer (X must keep h_prev for the other half, the input buffer must keep it for the reload).
-// thread <-> row 32*(warp&3)+lane, columns [32*(warp>>2), +32) of the half (8 worker warps).
-__device__ void epi_cell_half(const Ctx &c, int l, int half, bool want_value, float &vdot)
-{
-    const NetArgs *na = c.na;
-    const int row = 32 * (c.warp & 3) + c.lane, hh = c.warp >> 2;
-    const float *bi = na->b_ih[l], *bh = na->b_hh[l];
-    const uint32_t taddr = c.tmem + ((uint32_t)(32 * (c.warp & 3)) << 16);
-    int64_t gr;
-    int env, i;
-    const bool ok = row_info(c, row, gr, env, i);
-    float *dst = na->hidden_out + ((int64_t)l * c.a->R + gr) * E;
-#pragma unroll 1
-    for (int j0 = 32 * hh; j0 < 32 * hh + 32; j0 += 8) {
-        uint32_t ar[8], az[8], an[8], ahn[8];
-        asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                     : "=r"(ar[0]), "=r"(ar[1]), "=r"(ar[2]), "=r"(ar[3]), "=r"(ar[4]), "=r"(ar[5]), "=r"(ar[6]), "=r"(ar[7]) : "r"(taddr + (uint32_t)j0));
-        asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                     : "=r"(az[0]), "=r"(az[1]), "=r"(az[2]), "=r"(az[3]), "=r"(az[4]), "=r"(az[5]), "=r"(az[6]), "=r"(az[7]) : "r"(taddr + (uint32_t)(64 + j0)));
-        asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                     : "=r"(an[0]), "=r"(an[1]), "=r"(an[2]), "=r"(an[3]), "=r"(an[4]), "=r"(an[5]), "=r"(an[6]), "=r"(an[7]) : "r"(taddr + (uint32_t)(128 + j0)));
-        asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                     : "=r"(ahn[0]), "=r"(ahn[1]), "=r"(ahn[2]), "=r"(ahn[3]), "=r"(ahn[4]), "=r"(ahn[5]), "=r"(ahn[6]), "=r"(ahn[7]) : "r"(taddr + (uint32_t)(192 + j0)));
-        const int col = 64 * half + j0;
-        float hp[8];
-        x_load8(c.X, row, col >> 3, hp);
-        tmem_wait_ld();
-        float hn[8];
-#pragma unroll
-        for (int q4 = 0; q4 < 8; q4 += 4) {
-            const float4 bir = __ldg(reinterpret_cast<const float4 *>(bi + col + q4)), bhr = __ldg(reinterpret_cast<const float4 *>(bh + col + q4));
-            const float4 biz = __ldg(reinterpret_cast<const float4 *>(bi + E + col + q4)), bhz = __ldg(reinterpret_cast<const float4 *>(bh + E + col + q4));
-            const float4 bin = __ldg(reinterpret_cast<const float4 *>(bi + 2 * E + col + q4)), bhn = __ldg(reinterpret_cast<const float4 *>(bh + 2 * E + col + q4));
-            float4 wv = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (want_value) wv = __ldg(reinterpret_cast<const float4 *>(na->head_w_eff + col + q4));
-            const float f_bir[4] = {bir.x, bir.y, bir.z, bir.w}, f_bhr[4] = {bhr.x, bhr.y, bhr.z, bhr.w};
-            const float f_biz[4] = {biz.x, biz.y, biz.z, biz.w}, f_bhz[4] = {bhz.x, bhz.y, bhz.z, bhz.w};
-            const float f_bin[4] = {bin.x, bin.y, bin.z, bin.w}, f_bhn[4] = {bhn.x, bhn.y, bhn.z, bhn.w};
-            const float f_w[4] = {wv.x, wv.y, wv.z, wv.w};
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const float r = fast_sigmoid((__uint_as_float(ar[q4 + q]) + f_bir[q]) + f_bhr[q]);
-                const float z = fast_sigmoid((__uint_as_float(az[q4 + q]) + f_biz[q]) + f_bhz[q]);
-                const float n = fast_tanh((__uint_as_float(an[q4 + q]) + f_bin[q]) + r * (__uint_as_float(ahn[q4 + q]) + f_bhn[q]));
-                hn[q4 + q] = (1.f - z) * n + z * hp[q4 + q];
-                vdot = fmaf(f_w[q], hn[q4 + q], vdot);
-            }
-        }
-        if (ok) {
-            *reinterpret_cast<float4 *>(dst + col) = make_float4(hn[0], hn[1], hn[2], hn[3]);
-            *reinterpret_cast<float4 *>(dst + col + 4) = make_float4(hn[4], hn[5], hn[6], hn[7]);
-        }
-    }
-}
-
 // ---- epilogue: actor head (softmax -> sample / argmax -> log-prob), same arithmetic and RNG as act_head_kernel -----------
 template <int A>
 __device__ void epi_head(const Ctx &c)
@@ -1059,25 +961,22 @@ __device__ void epi_head(const Ctx &c)
 }
 
 // FL: marl_policy_step.flags (MARL_POLICY_STATE_F32 / MARL_POLICY_EMBED_ONLY), one instantiation per combination
-template <int WW, bool DUAL, int FL>
-__global__ void __launch_bounds__(Lay<WW>::THREADS, DUAL ? 2 : 1)
+template <int WW, int FL>
+__global__ void __launch_bounds__(Lay<WW>::THREADS, 1)
 policy_step_kernel(const __grid_constant__ StepArgs a)
 {
-    static_assert(!DUAL || WW == 8, "the two-CTA variant runs 8 worker warps");
-    static_assert(!DUAL || FL == 0, "the two-CTA variant has no flag instantiations");
     constexpr bool F32 = (FL & MARL_POLICY_STATE_F32) != 0, EMB = (FL & MARL_POLICY_EMBED_ONLY) != 0;
-    using M = Mem<DUAL>;
-    constexpr int RPW = Lay<WW>::RPW, NST = M::NST;
+    constexpr int RPW = Lay<WW>::RPW;
     extern __shared__ __align__(1024) unsigned char smem[];
     if ((smem_u32(smem) & 1023u) != 0u) __trap();          // SWIZZLE_128B atoms need 1024-byte alignment
     unsigned char *X = smem;
-    unsigned char *Wst = smem + M::RING_OFF;
-    uint64_t *bars = reinterpret_cast<uint64_t *>(smem + M::MISC_OFF);   // full[NST], empty[NST], a_ready, mma_done
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 2 * NST + 2);
-    static_assert(2 * NST + 3 <= 16, "barrier block");
+    unsigned char *Wst = smem + RING_OFF;
+    uint64_t *bars = reinterpret_cast<uint64_t *>(smem + MISC_OFF);   // full[NSTAGE], empty[NSTAGE], a_ready, mma_done
+    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 2 * NSTAGE + 2);
+    static_assert(2 * NSTAGE + 3 <= 16, "barrier block");
     float4 *s_p = reinterpret_cast<float4 *>(bars + 16);                                  // 128 x float4 (later: s_val)
     float4 *s_e = s_p + ROWS;                                                               // 32 x float4
-    float2 *s_oxy = reinterpret_cast<float2 *>(smem + M::OXY_OFF);
+    float2 *s_oxy = reinterpret_cast<float2 *>(smem + OXY_OFF);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     int net, tile;
     if (a.net_count == 2) { net = (int)blockIdx.x < a.n_tiles ? 1 : 0; tile = (int)blockIdx.x % a.n_tiles; }   // critic items first
@@ -1085,16 +984,16 @@ policy_step_kernel(const __grid_constant__ StepArgs a)
     const NetArgs *na = &a.net[net];
 
     if (threadIdx.x == 0) {
-        for (int s = 0; s < NST; ++s) {
+        for (int s = 0; s < NSTAGE; ++s) {
             mbar_init(smem_u32(&bars[s]), 1);            // full: one arrive.expect_tx + the bulk copy's bytes
-            mbar_init(smem_u32(&bars[NST + s]), 1);      // empty: one tcgen05.commit
+            mbar_init(smem_u32(&bars[NSTAGE + s]), 1);      // empty: one tcgen05.commit
         }
-        mbar_init(smem_u32(&bars[M::BAR_READY]), Lay<WW>::WORKERS);   // a_ready
-        mbar_init(smem_u32(&bars[M::BAR_DONE]), 1);        // mma_done
+        mbar_init(smem_u32(&bars[BAR_A_READY]), Lay<WW>::WORKERS);   // a_ready
+        mbar_init(smem_u32(&bars[BAR_MMA_DONE]), 1);        // mma_done
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == WW + 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(M::TMEM_COLS) : "memory");
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(512) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     tc_fence_before();
@@ -1106,7 +1005,7 @@ policy_step_kernel(const __grid_constant__ StepArgs a)
         // ================================================================================= workers
         Ctx c;
         c.a = &a; c.na = na; c.X = X; c.row0 = (int64_t)tile * a.rows_per_tile; c.warp = warp; c.lane = lane;
-        c.tmem = tmem_base; c.bar_a_ready = smem_u32(&bars[M::BAR_READY]); c.bar_mma_done = smem_u32(&bars[M::BAR_DONE]); c.group = 0; c.s_p = s_p; c.s_e = s_e; c.s_val = reinterpret_cast<float *>(s_p); c.s_oxy = s_oxy; c.oxy_cap = M::OXY; c.wait_sleep_ns = DUAL ? 100u : 0u;
+        c.tmem = tmem_base; c.bar_a_ready = smem_u32(&bars[BAR_A_READY]); c.bar_mma_done = smem_u32(&bars[BAR_MMA_DONE]); c.group = 0; c.s_p = s_p; c.s_e = s_e; c.s_val = reinterpret_cast<float *>(s_p); c.s_oxy = s_oxy;
         {   // fp32 copies of the tile's pursuer / evader states (converted once; every SIMT phase reads them from smem)
             const int t = threadIdx.x;
             if (t < ROWS) {
@@ -1165,7 +1064,7 @@ policy_step_kernel(const __grid_constant__ StepArgs a)
         }
         if constexpr (EMB) {
             // embeddings only: the unit program ends with the FCRA chain (fill_net), nothing is left to hand over
-        } else if constexpr (!DUAL) {
+        } else {
             for (int l = 0; l < 2; ++l) {
                 signal_ready(c);                                           // W_ih: r @0, z @128, n @256
                 hidden_prefetch<WW>(c, l, pre);                                //   ... while it runs: h_prev of this layer
@@ -1177,48 +1076,6 @@ policy_step_kernel(const __grid_constant__ StepArgs a)
                 PF_TICK(11);
                 epi_cell<WW>(c, l, l == 1 && na->head_w_eff != nullptr);
                 PF_TICK(9);
-            }
-        } else {
-            // GRU in two 64-column halves per layer (256 TMEM columns: r @0, z @64, n_i @128, n_h @192).  X holds x, then h_prev,
-            // for each half; x comes back from where it was stored (the embedding / the new state of layer 0), h_prev from the
-            // INPUT hidden buffer, the new state goes to the OUTPUT hidden buffer.
-            for (int l = 0; l < 2; ++l) {
-                const float *x_src = l == 0 ? na->emb_out : na->hidden_out;                  // layer 1's input = layer 0's new state
-                const float *h_src = na->hidden_in + (int64_t)l * a.R * E;
-                const bool want_value = l == 1 && na->head_w_eff != nullptr;
-                float vdot = 0.f;
-                float4 v8[8];
-                for (int half = 0; half < 2; ++half) {
-                    if (half == 1 || l == 1) {                                               // (l = 0, half 0: X still holds the embedding)
-                        fill_x<WW>(c, x_src);
-                        PF_TICK(8);
-                    }
-                    signal_ready(c);                                       // W_ih rows of this half: r @0, z @64, n_i @128
-                    rows_prefetch8<WW>(c, h_src, 0, v8);                   //   ... while it runs: the first chunk of h_prev
-                    wait_done(c);
-                    PF_TICK(11);
-                    rows_store8<WW>(c, 0, v8);
-                    rows_prefetch8<WW>(c, h_src, 1, v8);
-                    rows_store8<WW>(c, 1, v8);
-                    PF_TICK(8);
-                    hand_over(c);                                          // W_hh rows of this half: r +=, z +=, n_h @192
-                    PF_TICK(11);
-                    epi_cell_half(c, l, half, want_value, vdot);
-                    worker_sync<WW>();                                     // every reader of h_prev in X is done; the half's new state is in memory
-                    PF_TICK(9);
-                }
-                if (want_value) {
-                    const int row = 32 * (warp & 3) + lane, hh = warp >> 2;
-                    c.s_val[hh * ROWS + row] = vdot;
-                    worker_sync<WW>();
-                    int64_t gr;
-                    int env, i;
-                    if (hh == 0 && a.value && row_info(c, row, gr, env, i)) a.value[gr] = (c.s_val[row] + c.s_val[ROWS + row]) + __ldg(na->head_b);
-                }
-            }
-            if (net == 0) {                                                // the actor head reads the new state of layer 1
-                fill_x<WW>(c, na->hidden_out + a.R * E);
-                PF_TICK(8);
             }
         }
         if (!EMB && net == 0) {
@@ -1240,17 +1097,14 @@ policy_step_kernel(const __grid_constant__ StepArgs a)
             int it = 0;
             for (int u = 0; u < na->n_units; ++u) {
                 const Unit un = na->u[u];
-                // one stage = a k-block of both operand planes (32 KB), or - two-CTA variant - of one plane (16 KB); the packed unit is
-                // [kb0: hi plane, lo plane][kb1: hi plane, lo plane], so either way the stages are consecutive slices of it
-                const uint32_t bytes = (DUAL ? 1u : 2u) * un.n_out * 128u;
-                for (int st = 0; st < (DUAL ? 2 * NKB : NKB); ++st, ++it) {
-                    const int s = it % NST, round = it / NST;
-                    if (round > 0) {
-                        if (DUAL) mbar_wait_sleep(smem_u32(&bars[NST + s]), (uint32_t)((round - 1) & 1), 100u);
-                        else mbar_wait(smem_u32(&bars[NST + s]), (uint32_t)((round - 1) & 1));
-                    }
+                // one stage = a k-block of both operand planes (32 KB); the packed unit is [kb0: hi plane, lo plane][kb1: hi plane,
+                // lo plane], so the stages are consecutive slices of it
+                const uint32_t bytes = 2u * un.n_out * 128u;
+                for (int st = 0; st < NKB; ++st, ++it) {
+                    const int s = it % NSTAGE, round = it / NSTAGE;
+                    if (round > 0) mbar_wait(smem_u32(&bars[NSTAGE + s]), (uint32_t)((round - 1) & 1));
                     mbar_expect_tx(smem_u32(&bars[s]), bytes);
-                    bulk_g2s(smem_u32(Wst + s * M::STAGE), na->packed + un.off + (size_t)st * bytes, bytes, smem_u32(&bars[s]));
+                    bulk_g2s(smem_u32(Wst + s * WSTAGE), na->packed + un.off + (size_t)st * bytes, bytes, smem_u32(&bars[s]));
                 }
             }
         }
@@ -1263,59 +1117,34 @@ policy_step_kernel(const __grid_constant__ StepArgs a)
             for (int u = 0; u < na->n_units; ++u) {
                 const Unit un = na->u[u];
                 if (fresh_group) {
-                    if (DUAL) mbar_wait_sleep(smem_u32(&bars[M::BAR_READY]), (uint32_t)(group & 1), 50u);
-                    else mbar_wait(smem_u32(&bars[M::BAR_READY]), (uint32_t)(group & 1));
+                    mbar_wait(smem_u32(&bars[BAR_A_READY]), (uint32_t)(group & 1));
                     tc_fence_after();
                     fresh_group = false;
                 }
                 const uint32_t idesc = idesc_f16(un.n_out);
                 const uint32_t acc = tmem_base + un.acc_col;
                 const uint32_t lo_off = (uint32_t)un.n_out * 128u;
-                if constexpr (!DUAL) {
-                    for (int kb = 0; kb < NKB; ++kb, ++it) {
-                        const int s = it % NST, round = it / NST;
-                        mbar_wait(smem_u32(&bars[s]), (uint32_t)(round & 1));
-                        tc_fence_after();
-                        const uint32_t xa = smem_u32(X + kb * XKB), wb = smem_u32(Wst + s * M::STAGE);
-                        // descriptors of the first K=16 slice; the next slices are +32 bytes = +2 in the (addr >> 4) field
-                        const uint64_t a_hi0 = make_desc(xa), a_lo0 = make_desc(xa + TILE), b_hi0 = make_desc(wb), b_lo0 = make_desc(wb + lo_off);
-                        if (elect_one()) {
+                for (int kb = 0; kb < NKB; ++kb, ++it) {
+                    const int s = it % NSTAGE, round = it / NSTAGE;
+                    mbar_wait(smem_u32(&bars[s]), (uint32_t)(round & 1));
+                    tc_fence_after();
+                    const uint32_t xa = smem_u32(X + kb * XKB), wb = smem_u32(Wst + s * WSTAGE);
+                    // descriptors of the first K=16 slice; the next slices are +32 bytes = +2 in the (addr >> 4) field
+                    const uint64_t a_hi0 = make_desc(xa), a_lo0 = make_desc(xa + TILE), b_hi0 = make_desc(wb), b_lo0 = make_desc(wb + lo_off);
+                    if (elect_one()) {
 #pragma unroll
-                            for (int kk = 0; kk < 4; ++kk) {
-                                const uint64_t a_hi = a_hi0 + 2 * kk, a_lo = a_lo0 + 2 * kk, b_hi = b_hi0 + 2 * kk, b_lo = b_lo0 + 2 * kk;
-                                umma_f16(acc, a_hi, b_hi, idesc, (un.accumulate || kb || kk) ? 1u : 0u);
-                                umma_f16(acc, a_lo, b_hi, idesc, 1u);
-                                umma_f16(acc, a_hi, b_lo, idesc, 1u);
-                            }
-                            umma_commit(smem_u32(&bars[NST + s]));
+                        for (int kk = 0; kk < 4; ++kk) {
+                            const uint64_t a_hi = a_hi0 + 2 * kk, a_lo = a_lo0 + 2 * kk, b_hi = b_hi0 + 2 * kk, b_lo = b_lo0 + 2 * kk;
+                            umma_f16(acc, a_hi, b_hi, idesc, (un.accumulate || kb || kk) ? 1u : 0u);
+                            umma_f16(acc, a_lo, b_hi, idesc, 1u);
+                            umma_f16(acc, a_hi, b_lo, idesc, 1u);
                         }
-                        __syncwarp();
+                        umma_commit(smem_u32(&bars[NSTAGE + s]));
                     }
-                } else {
-                    for (int st = 0; st < 2 * NKB; ++st, ++it) {          // stage = one plane of the weights: hi (pairs with A_hi and A_lo), then lo
-                        const int s = it % NST, round = it / NST, kb = st >> 1;
-                        mbar_wait(smem_u32(&bars[s]), (uint32_t)(round & 1));
-                        tc_fence_after();
-                        const uint32_t xa = smem_u32(X + kb * XKB);
-                        const uint64_t a_hi0 = make_desc(xa), a_lo0 = make_desc(xa + TILE), b0 = make_desc(smem_u32(Wst + s * M::STAGE));
-                        if (elect_one()) {
-                            if ((st & 1) == 0) {
-#pragma unroll
-                                for (int kk = 0; kk < 4; ++kk) {
-                                    umma_f16(acc, a_hi0 + 2 * kk, b0 + 2 * kk, idesc, (un.accumulate || kb || kk) ? 1u : 0u);
-                                    umma_f16(acc, a_lo0 + 2 * kk, b0 + 2 * kk, idesc, 1u);
-                                }
-                            } else {
-#pragma unroll
-                                for (int kk = 0; kk < 4; ++kk) umma_f16(acc, a_hi0 + 2 * kk, b0 + 2 * kk, idesc, 1u);
-                            }
-                            umma_commit(smem_u32(&bars[NST + s]));
-                        }
-                        __syncwarp();
-                    }
+                    __syncwarp();
                 }
                 if (un.last) {
-                    if (elect_one()) umma_commit(smem_u32(&bars[M::BAR_DONE]));
+                    if (elect_one()) umma_commit(smem_u32(&bars[BAR_MMA_DONE]));
                     __syncwarp();
                     ++group;
                     fresh_group = true;
@@ -1325,7 +1154,7 @@ policy_step_kernel(const __grid_constant__ StepArgs a)
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == WW + 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(M::TMEM_COLS) : "memory");
+    if (warp == WW + 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(512) : "memory");
 }
 
 
@@ -1564,7 +1393,7 @@ policy_pair_kernel(const __grid_constant__ StepArgs a)
         Ctx c;
         c.a = &a; c.row0 = (int64_t)tile * a.rows_per_tile; c.warp = warp; c.lane = lane; c.group = 0; c.s_p = s_p; c.s_e = s_e;
         c.s_val = reinterpret_cast<float *>(s_oxy);      // value partials: the boundary-cell staging is dead once the GRU starts
-        c.s_oxy = s_oxy; c.oxy_cap = OXY_CAP; c.wait_sleep_ns = 0u;
+        c.s_oxy = s_oxy;
         c.na = &a.net[0]; c.X = smem; c.tmem = tmem_base; c.bar_a_ready = 0; c.bar_mma_done = 0;
         {
             const int t = threadIdx.x;
@@ -1884,7 +1713,7 @@ struct UnitSrc {
     int split = 1 << 30, jump = 0;      // see pack_unit_kernel
 };
 
-static int build_units(const marl_dhgn_weights *w, int depth, int is_actor, int A, UnitSrc *us, int mode /* 0 one chain per CTA, 1 two CTAs per SM, 2 pair */)
+static int build_units(const marl_dhgn_weights *w, int depth, int is_actor, int A, UnitSrc *us, bool pair /* else one chain per CTA */)
 {
     int n = 0;
     auto add = [&](const float *W, int64_t ld, int rows, int n_out, int k0, int acc, int accu, int last) {
@@ -1906,7 +1735,7 @@ static int build_units(const marl_dhgn_weights *w, int depth, int is_actor, int 
         add(w->fcra_w[k], 2 * E, E, E, 0, 128, 1, 1);
     }
     for (int l = 0; l < 2; ++l) {
-        if (mode == 2) {
+        if (pair) {
             // pair kernel: 64-column halves, accumulators r @0, z @64, n_i @128, n_h @192, in the order
             // W_ih(half 0) | W_hh(half 0) | W_hh(half 1) | W_ih(half 1): X holds x, h_prev, h_prev, x (one re-staging of each)
             const float *wi = w->gru_w_ih[l], *wh = w->gru_w_hh[l];
@@ -1917,20 +1746,11 @@ static int build_units(const marl_dhgn_weights *w, int depth, int is_actor, int 
             add_rz(wh, 0, 1); add(wh + g2, E, 64, 64, 0, 192, 0, 1);
             add_rz(wh + ro, 0, 0); add(wh + g2 + ro, E, 64, 64, 0, 192, 0, 1);
             add_rz(wi + ro, 0, 1); add(wi + g2 + ro, E, 64, 64, 0, 128, 0, 1);
-        } else if (mode == 0) {
+        } else {
             for (int g = 0; g < 3; ++g) add(w->gru_w_ih[l] + (int64_t)g * E * E, E, E, E, 0, 128 * g, 0, g == 2);
             add(w->gru_w_hh[l], E, E, E, 0, 0, 1, 0);
             add(w->gru_w_hh[l] + (int64_t)E * E, E, E, E, 0, 128, 1, 0);
             add(w->gru_w_hh[l] + (int64_t)2 * E * E, E, E, E, 0, 384, 0, 1);
-        } else {
-            // two-CTA variant: output columns [64*half, +64) of every gate, accumulators r @0, z @64, n_i @128, n_h @192
-            for (int half = 0; half < 2; ++half) {
-                const int64_t ro = (int64_t)64 * half * E;
-                for (int g = 0; g < 3; ++g) add(w->gru_w_ih[l] + (int64_t)g * E * E + ro, E, 64, 64, 0, 64 * g, 0, g == 2);
-                add(w->gru_w_hh[l] + ro, E, 64, 64, 0, 0, 1, 0);
-                add(w->gru_w_hh[l] + (int64_t)E * E + ro, E, 64, 64, 0, 64, 1, 0);
-                add(w->gru_w_hh[l] + (int64_t)2 * E * E + ro, E, 64, 64, 0, 192, 0, 1);
-            }
         }
     }
     if (is_actor) add(w->head_w, E, A, 16, 0, 0, 0, 1);
@@ -1944,7 +1764,7 @@ static int build_units(const marl_dhgn_weights *w, int depth, int is_actor, int 
 // ceil(items / SMs) waves; a slightly smaller tile that fills the last wave beats a full tile that leaves most SMs idle in it
 // (32768 rows x 2 networks: 512 items of 128 rows = 3.46 -> 4 waves, 586 items of 112 rows = 3.96 waves).  Cost model of one item:
 // SIMT phases proportional to the rows, MMA phases constant (M = 128 regardless) - measured ~3 : 1 at 128 rows.
-static int choose_rows_per_tile(int64_t R, int N, int nets, int ctas_per_sm, int requested)
+static int choose_rows_per_tile(int64_t R, int N, int nets, int requested)
 {
     static int sms = 0;
     if (sms == 0) {
@@ -1953,16 +1773,11 @@ static int choose_rows_per_tile(int64_t R, int N, int nets, int ctas_per_sm, int
     }
     const int full = (ROWS / N) * N;
     if (requested > 0 && requested <= full && requested % N == 0) return requested;
-    if (const char *force = getenv("MARL_POLICY_ROWS_PER_TILE")) {            // tuning knob for tools/: a multiple of N in [N, full]
-        const int v = atoi(force);
-        if (v >= N && v <= full && v % N == 0) return v;
-    }
     int best = full;
     double best_cost = 0.0;
     for (int rpt = full; rpt >= N && rpt * 4 >= full * 3; rpt -= N) {
         const int64_t items = ((R + rpt - 1) / rpt) * nets;
-        const int64_t slots = (int64_t)sms * ctas_per_sm;
-        const double waves = (double)((items + slots - 1) / slots);
+        const double waves = (double)((items + sms - 1) / sms);
         const double cost = waves * (0.75 * rpt / full + 0.25);
         if (best_cost == 0.0 || cost < best_cost - 1e-12) { best_cost = cost; best = rpt; }
     }
@@ -1993,7 +1808,7 @@ using namespace marl;
 extern "C" int64_t marl_policy_pack_bytes(int32_t depth, int32_t is_actor)
 {
     if (depth < 1 || depth > pf::MAXD) return -1;
-    return 3 * pf::layout_bytes(depth, is_actor) + 2 * 4 * pf::E * (int64_t)sizeof(float);   // [one chain per CTA][two CTAs per SM][pair][combined GRU biases]
+    return 2 * pf::layout_bytes(depth, is_actor) + 2 * 4 * pf::E * (int64_t)sizeof(float);   // [one chain per CTA][pair][combined GRU biases]
 }
 
 extern "C" int marl_policy_pack(const marl_dhgn_weights *w, int32_t depth, int32_t is_actor, int32_t action_dim, void *d_packed,
@@ -2004,9 +1819,9 @@ extern "C" int marl_policy_pack(const marl_dhgn_weights *w, int32_t depth, int32
     MARL_REQUIRE(d_packed && ((uintptr_t)d_packed & 1023) == 0, "marl_policy_pack: workspace must be 1024-byte aligned");
     MARL_REQUIRE(!is_actor || (action_dim >= 1 && action_dim <= 16), "marl_policy_pack: action_dim=%d (1..16)", action_dim);
     unsigned char *out = static_cast<unsigned char *>(d_packed);
-    for (int mode = 0; mode < 3; ++mode) {
+    for (const bool pair : {false, true}) {
         pf::UnitSrc us[pf::MAX_UNITS];
-        const int n = pf::build_units(w, depth, is_actor, action_dim, us, mode);
+        const int n = pf::build_units(w, depth, is_actor, action_dim, us, pair);
         for (int u = 0; u < n; ++u) {
             const int total = us[u].n_out * 128;
             pf::pack_unit_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(us[u].W, us[u].ld, us[u].rows, us[u].n_out, us[u].k0, us[u].split, us[u].jump, out);
@@ -2023,7 +1838,7 @@ extern "C" int marl_policy_pack(const marl_dhgn_weights *w, int32_t depth, int32
     return MARL_OK;
 }
 
-static int fill_net(pf::NetArgs &na, const marl_dhgn_weights *w, const marl_policy_net_io *io, int depth, int is_actor, int A, int mode,
+static int fill_net(pf::NetArgs &na, const marl_dhgn_weights *w, const marl_policy_net_io *io, int depth, int is_actor, int A, bool pair,
                     bool embed_only)
 {
     int rc = pf::check_weights(w, depth, is_actor);
@@ -2031,9 +1846,9 @@ static int fill_net(pf::NetArgs &na, const marl_dhgn_weights *w, const marl_poli
     MARL_REQUIRE(io->d_packed && (embed_only || io->d_hidden) && io->d_emb_out, "marl_policy_rollout_step: null packed / hidden / emb_out (%s)",
                  is_actor ? "actor" : "critic");
     pf::UnitSrc us[pf::MAX_UNITS];
-    na.n_units = pf::build_units(w, depth, is_actor, A, us, mode);
+    na.n_units = pf::build_units(w, depth, is_actor, A, us, pair);
     if (embed_only) na.n_units = 6 + 3 * depth;           // the encoder and FCRA units lead the program (build_units)
-    uint32_t off = (uint32_t)(mode * pf::layout_bytes(depth, is_actor));
+    uint32_t off = (uint32_t)(pair ? pf::layout_bytes(depth, is_actor) : 0);
     for (int u = 0; u < na.n_units; ++u) {
         na.u[u] = pf::Unit{off, (uint16_t)us[u].n_out, (uint16_t)us[u].acc_col, (uint8_t)us[u].accumulate, (uint8_t)us[u].last, 0};
         off += (uint32_t)pf::unit_bytes(us[u].n_out);
@@ -2048,7 +1863,7 @@ static int fill_net(pf::NetArgs &na, const marl_dhgn_weights *w, const marl_poli
     }
     for (int l = 0; l < 2; ++l) {
         na.b_ih[l] = w->gru_b_ih[l]; na.b_hh[l] = w->gru_b_hh[l];
-        na.b_comb[l] = reinterpret_cast<const float *>(static_cast<const unsigned char *>(io->d_packed) + 3 * pf::layout_bytes(depth, is_actor)) + l * 4 * pf::E;
+        na.b_comb[l] = reinterpret_cast<const float *>(static_cast<const unsigned char *>(io->d_packed) + 2 * pf::layout_bytes(depth, is_actor)) + l * 4 * pf::E;
     }
     na.head_b = w->head_b;
     na.head_w_eff = is_actor ? nullptr : w->head_w;
@@ -2072,24 +1887,18 @@ extern "C" int marl_policy_rollout_step(const marl_policy_step *s, const marl_dh
     MARL_REQUIRE((actor_w && actor_io) || (critic_w && critic_io), "marl_policy_rollout_step: no network given");
     MARL_REQUIRE((s->flags & ~(MARL_POLICY_STATE_F32 | MARL_POLICY_EMBED_ONLY)) == 0, "marl_policy_rollout_step: unknown flags 0x%x",
                  (unsigned)s->flags);
-    MARL_REQUIRE(s->variant != 2 || s->flags == 0, "marl_policy_rollout_step: variant 2 runs without flags (flags=0x%x)", (unsigned)s->flags);
+    MARL_REQUIRE(s->variant != 2, "marl_policy_rollout_step: variant 2 (two CTAs per SM) was removed; use 0, 1 or 3");
+    MARL_REQUIRE(s->variant == 0 || s->variant == 1 || s->variant == 3, "marl_policy_rollout_step: variant=%d (0, 1 or 3)", s->variant);
     const bool embed_only = (s->flags & MARL_POLICY_EMBED_ONLY) != 0;
     pf::StepArgs a{};
     a.B = s->B; a.N = s->N; a.O = s->O; a.NW = (s->N + 31) / 32; a.OW = (s->O + 31) / 32; a.depth = s->depth; a.A = s->action_dim;
     a.R = (int64_t)s->B * s->N;
     const bool has_a = actor_w && actor_io, has_c = critic_w && critic_io;
     const int nets = (has_a ? 1 : 0) + (has_c ? 1 : 0);
-    // kernel variant: two CTAs per SM need a separate output hidden buffer (the GRU re-reads the previous state), <= 176 boundary
-    // cells for the shared-memory staging of the env-grouped message path and envs of <= 16 agents-per-warp rows as usual
-    const bool pingpong = (!has_a || (actor_io->d_hidden_out && actor_io->d_hidden_out != actor_io->d_hidden)) &&
-                          (!has_c || (critic_io->d_hidden_out && critic_io->d_hidden_out != critic_io->d_hidden));
-    MARL_REQUIRE(s->variant >= 0 && s->variant <= 3, "marl_policy_rollout_step: variant=%d (0..3)", s->variant);
-    MARL_REQUIRE(s->variant != 2 || pingpong, "marl_policy_rollout_step: variant 2 needs d_hidden_out != d_hidden");
     MARL_REQUIRE(s->variant != 3 || (has_a && has_c), "marl_policy_rollout_step: variant 3 (actor + critic chains in one CTA) needs both networks");
-    const bool pair = s->variant == 3;
-    const bool dual = !pair && (s->variant == 2 || (s->variant == 0 && s->flags == 0 && pingpong && pf::kDualByDefault && s->O <= pf::Mem<true>::OXY));
-    const int mode = pair ? 2 : (dual ? 1 : 0);
-    a.rows_per_tile = pf::choose_rows_per_tile(a.R, s->N, pair ? 1 : nets, dual ? 2 : 1, s->tile_rows);
+    // variant 0: the pair kernel whenever both networks are stepped, one chain per CTA for a single network
+    const bool pair = s->variant == 3 || (s->variant == 0 && has_a && has_c);
+    a.rows_per_tile = pf::choose_rows_per_tile(a.R, s->N, pair ? 1 : nets, s->tile_rows);
     a.n_tiles = (int)((a.R + a.rows_per_tile - 1) / a.rows_per_tile);
     a.p_state = s->d_p_state; a.e_state = s->d_e_state; a.oxy = s->d_oxy; a.map_id = s->d_map_id; a.o_count = s->d_o_count;
     a.p_adj = s->d_p_adj_bits; a.e_adj = s->d_e_adj; a.o_adj = s->d_o_adj_bits;
@@ -2097,14 +1906,13 @@ extern "C" int marl_policy_rollout_step(const marl_policy_step *s, const marl_dh
     a.row_offset = s->row_offset;
     a.dbg = static_cast<long long *>(s->d_debug);
     int rc;
-    if (has_a) { rc = fill_net(a.net[0], actor_w, actor_io, s->depth, 1, s->action_dim, mode, embed_only); if (rc) return rc; }
-    if (has_c) { rc = fill_net(a.net[1], critic_w, critic_io, s->depth, 0, s->action_dim, mode, embed_only); if (rc) return rc; }
+    if (has_a) { rc = fill_net(a.net[0], actor_w, actor_io, s->depth, 1, s->action_dim, pair, embed_only); if (rc) return rc; }
+    if (has_c) { rc = fill_net(a.net[1], critic_w, critic_io, s->depth, 0, s->action_dim, pair, embed_only); if (rc) return rc; }
     a.net_count = nets;
     a.net_first = has_a ? 0 : 1;
     const unsigned grid = (unsigned)(a.n_tiles * (pair ? 1 : a.net_count));
-    auto launch = [&](auto kernel, int threads, int smem_bytes, bool max_carveout) -> int {
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-        if (e == cudaSuccess && max_carveout) e = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    auto launch = [&](auto kernel, int threads, int smem_bytes) -> int {
+        const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
         if (e != cudaSuccess) { set_error("policy_step_kernel: smem %d: %s", smem_bytes, cudaGetErrorString(e)); return MARL_ECUDA; }
         kernel<<<grid, threads, smem_bytes, (cudaStream_t)stream>>>(a);
         return MARL_OK;
@@ -2115,14 +1923,13 @@ extern "C" int marl_policy_rollout_step(const marl_policy_step *s, const marl_dh
     // the flags select a kernel instantiation (no runtime branch in the phases); flags = 0 is the default kernels
     auto dispatch = [&](auto fl) -> int {
         constexpr int FL = decltype(fl)::value;
-        if (pair8) return launch(pf::policy_pair_kernel<8, false, FL>, (8 + 4) * 32, pf::MemPair::BYTES, false);
+        if (pair8) return launch(pf::policy_pair_kernel<8, false, FL>, (8 + 4) * 32, pf::MemPair::BYTES);
         if constexpr (FL == 0) {
-            if (pair && getenv("MARL_POLICY_PROFILE")) return launch(pf::policy_pair_kernel<16, true, 0>, (16 + 4) * 32, pf::MemPair::BYTES, false);
-            if (dual) return launch(pf::policy_step_kernel<8, true, 0>, pf::Lay<8>::THREADS, pf::Mem<true>::BYTES, true);
+            if (pair && getenv("MARL_POLICY_PROFILE")) return launch(pf::policy_pair_kernel<16, true, 0>, (16 + 4) * 32, pf::MemPair::BYTES);
         }
-        if (pair) return launch(pf::policy_pair_kernel<16, false, FL>, (16 + 4) * 32, pf::MemPair::BYTES, false);
-        if (!step8) return launch(pf::policy_step_kernel<16, false, FL>, pf::Lay<16>::THREADS, pf::Mem<false>::BYTES, false);
-        return launch(pf::policy_step_kernel<8, false, FL>, pf::Lay<8>::THREADS, pf::Mem<false>::BYTES, false);
+        if (pair) return launch(pf::policy_pair_kernel<16, false, FL>, (16 + 4) * 32, pf::MemPair::BYTES);
+        if (!step8) return launch(pf::policy_step_kernel<16, FL>, pf::Lay<16>::THREADS, pf::SMEM_BYTES);
+        return launch(pf::policy_step_kernel<8, FL>, pf::Lay<8>::THREADS, pf::SMEM_BYTES);
     };
     switch (s->flags) {
     case 0: rc = dispatch(std::integral_constant<int, 0>{}); break;

@@ -6,7 +6,6 @@ whenever the weights change, i.e. once per rollout.  Built with `snapshot=True` 
 kernel reads unpacked (message layers, biases, head rows), so it keeps computing the rollout-time networks after the optimizer
 has stepped the live parameters - what a replay of the episode's history embeddings needs."""
 import ctypes as C
-import os
 
 import torch
 
@@ -40,11 +39,6 @@ STATE_F32 = 1       # d_p_state / d_e_state are float [B,N,4] / [B,4] (the rollo
 EMBED_ONLY = 2      # encoder + FCRA chain only: write the embeddings; hidden states, actions, log-probs and values untouched
 
 
-# Kernel variant used when the caller does not ask for one (marl_policy_step.variant): 3 = the actor and the critic chain of a row
-# tile interleaved in ONE CTA (policy_pair_kernel) whenever both networks are stepped, 1 = one (tile, network) item per CTA.
-DEFAULT_VARIANT = int(os.environ.get("MARL_POLICY_VARIANT", "3"))
-
-
 def supported(mappo):
     return (mappo.embedding_dim == 128 and mappo.num_layers == 2 and 1 <= mappo.depth <= 3 and mappo.action_dim == 9
             and mappo.rnn_hidden_dim == 128)
@@ -66,7 +60,6 @@ class FusedRolloutStep:
         self.depth, self.E, self.A = int(mappo.depth), 128, int(mappo.action_dim)
         dev = mappo.device
         self._keep = []
-        self._next_hidden = {}
         enc = mappo.actor.shared_net
         self.w = {}
         self.packed = {}
@@ -109,14 +102,8 @@ class FusedRolloutStep:
         action i32 [B,N], logp / value f32 [B,N] outputs.
         flags: STATE_F32 (engine.p_state / e_state are the fp32 records [B,N,4] / [B,4]) | EMBED_ONLY (ha / hc / action / logp /
         value may be None and are not touched).
-        variant: 0 = DEFAULT_VARIANT, 1 = one (tile, network) item per CTA (hidden state updated in place), 2 = two such CTAs per
-        SM, 3 = both networks' chains of a tile interleaved in one CTA.  Variant 2 reads the previous hidden state from one
-        buffer and writes the new one to another; afterwards the two tensors trade their storage, so for the caller `ha` / `hc`
-        are still updated "in place" (views taken before the call keep the old state)."""
-        if int(variant) == 0 and DEFAULT_VARIANT == 3 and "actor" in nets and "critic" in nets:
-            variant = 3          # (16-agent envs run the pair kernel with 8 worker warps: their message path needs a whole env per warp)
-        if int(variant) == 3 and not ("actor" in nets and "critic" in nets):
-            variant = 1          # a single network (the critic-only bootstrap step): nothing to interleave
+        variant: 0 = choose (3 when both networks are stepped, else 1), 1 = one (tile, network) item per CTA, 3 = both
+        networks' chains of a tile interleaved in one CTA (needs both networks).  The hidden states are updated in place."""
         s = PolicyStep()
         s.B, s.N, s.O, s.E, s.depth, s.action_dim = engine.B, engine.N, engine.O, self.E, self.depth, self.A
         s.t, s.deterministic, s.seed = int(t), 1 if deterministic else 0, int(seed) & 0xFFFFFFFFFFFFFFFF
@@ -131,7 +118,7 @@ class FusedRolloutStep:
                                                                         P(engine.map_id), P(o_count))
         s.d_p_adj_bits, s.d_e_adj, s.d_o_adj_bits = P(engine.p_adj_bits), P(engine.e_adj), P(engine.o_adj_bits)
         s.d_action, s.d_logp, s.d_value = P(action), P(logp), P(value)
-        ios, swaps = {}, []
+        ios = {}
         for name, hist, emb, hid in (("actor", hist_a, emb_a, ha), ("critic", hist_c, emb_c, hc)):
             if name not in nets:
                 continue
@@ -141,18 +128,8 @@ class FusedRolloutStep:
                 io.d_hist[k] = P(hist[k]) if hist[k] is not None else None
             assert hid is None or hid.is_contiguous()
             io.d_emb_out, io.d_hidden, io.d_hidden_out = P(emb), P(hid), None
-            if int(variant) == 2:                            # the two-CTA-per-SM kernel re-reads the previous state: separate output buffer
-                # the partner buffer belongs to THIS hidden-state tensor (env-group pipelines step their own states concurrently)
-                nxt = getattr(hid, "_marl_next", None)
-                if nxt is None or nxt.shape != hid.shape or nxt.device != hid.device:
-                    nxt = torch.empty_like(hid)
-                    hid._marl_next = nxt
-                io.d_hidden_out = P(nxt)
-                swaps.append((hid, nxt))
             ios[name] = io
         a_w, a_io = (C.byref(self.w["actor"]), C.byref(ios["actor"])) if "actor" in ios else (None, None)
         c_w, c_io = (C.byref(self.w["critic"]), C.byref(ios["critic"])) if "critic" in ios else (None, None)
         _lib.check(self.lib.marl_policy_rollout_step(C.byref(s), a_w, a_io, c_w, c_io, _lib.stream_ptr()),
                    "marl_policy_rollout_step")
-        for hid, nxt in swaps:                               # the caller's tensor now holds the new state, its partner the old buffer
-            hid.data, nxt.data = nxt.data, hid.data

@@ -421,15 +421,14 @@ typedef struct marl_policy_net_io {
     const float *d_hist[3];      /* history embeddings [B,N,E], k = 0 the most recent; NULL = zeros (:750-752) */
     float *d_emb_out;            /* [B,N,E] this step's embedding (stored at t+D of the history buffer) */
     float *d_hidden;             /* [2, B*N, E] GRU hidden state (input; also the output when d_hidden_out is NULL) */
-    float *d_hidden_out;         /* NULL (update d_hidden in place) or a distinct [2, B*N, E] buffer for the new state: the caller
-                                    ping-pongs the two.  Required by the two-CTA-per-SM kernel variant (its GRU runs in two
-                                    column halves and re-reads the previous state) */
+    float *d_hidden_out;         /* NULL (update d_hidden in place) or a distinct [2, B*N, E] buffer for the new state */
 } marl_policy_net_io;
 typedef struct marl_policy_step {
     int32_t B, N, O, E, depth, action_dim, t, deterministic;
     int32_t force_action;        /* != 0: d_action is an INPUT (teacher forcing); d_logp is the log-prob of that action */
-    int32_t variant;             /* 0 = choose; 1 = one (tile, network) item per CTA (16 worker warps); 2 = two CTAs per SM; 3 = the actor and
-                                    the critic chain of a tile interleaved in one CTA (both networks given); 2 and 3 need d_hidden_out */
+    int32_t variant;             /* 0 = choose: 3 when both networks are given, else 1; 1 = one (tile, network) item per CTA; 3 = the
+                                    actor and the critic chain of a tile interleaved in one CTA (both networks given); 2 (two CTAs
+                                    per SM) was removed: MARL_EINVAL */
     uint64_t seed;               /* sampling: same counter RNG as marl_act_head (keyed by seed, row, t) */
     const void *d_p_state;       /* [B,N,4] double (float with MARL_POLICY_STATE_F32) */
     const void *d_e_state;       /* [B,4] double (float with MARL_POLICY_STATE_F32) */
@@ -450,7 +449,7 @@ typedef struct marl_policy_step {
 } marl_policy_step;
 /* marl_policy_step.flags.  Both modes are separate kernel instantiations: flags = 0 runs exactly the default kernels.
  * STATE_F32: d_p_state / d_e_state point to float [B,N,4] / [B,4] (the rollout arena's per-step records, (float) of the fp64
- *   state - the very values the kernel converts the fp64 state to) instead of double.  Not with variant 2.
+ *   state - the very values the kernel converts the fp64 state to) instead of double.
  * EMBED_ONLY: run the encoder and FCRA chain only and write d_emb_out; no GRU, cells or heads.  d_hidden, d_hidden_out,
  *   d_action, d_logp and d_value may be NULL.  Used to regenerate the history embeddings of a stored episode. */
 #define MARL_POLICY_STATE_F32 1

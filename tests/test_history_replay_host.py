@@ -44,7 +44,7 @@ def _step_args(flags, variant):
 def test_bad_flags_fail_without_a_gpu():
     from distributed_multi_agent_reinforcement_learning_b200 import _lib, fused_policy
     L = _lib.lib()
-    for flags, variant, what in ((4, 0, b"unknown flags"), (1 << 30, 3, b"unknown flags"),
+    for flags, variant, what in ((4, 0, b"unknown flags"), (1 << 30, 3, b"unknown flags"), (0, 2, b"variant 2"),
                                  (fused_policy.STATE_F32, 2, b"variant 2"), (fused_policy.EMBED_ONLY, 2, b"variant 2")):
         s, w, io = _step_args(flags, variant)
         rc = L.marl_policy_rollout_step(ctypes.byref(s), ctypes.byref(w), ctypes.byref(io), ctypes.byref(w), ctypes.byref(io), None)

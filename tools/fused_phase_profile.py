@@ -1,4 +1,5 @@
-"""Profiling aid: per-phase cycle counters of the fused policy step kernel (marl_policy_step.d_debug) at the bench shape."""
+"""Profiling aid: per-phase cycle counters of the fused policy step kernel (marl_policy_step.d_debug) at the bench shape.
+MARL_VARIANT=3 (default: the pair kernel the bench runs) or 1 (one (tile, network) chain per CTA)."""
 import os
 import sys
 
@@ -12,7 +13,10 @@ from distributed_multi_agent_reinforcement_learning_b200.fused_policy import Fus
 from distributed_multi_agent_reinforcement_learning_b200.mappo_parallel import MAPPO  # noqa: E402
 from distributed_multi_agent_reinforcement_learning_b200.pursuit_env import BatchedPursuitEnv  # noqa: E402
 
-if int(os.environ.get("MARL_VARIANT", "0")) == 3:
+VARIANT = {"1": 1, "3": 3}.get(os.environ.get("MARL_VARIANT", "3"))
+if VARIANT is None:
+    sys.exit(f"MARL_VARIANT={os.environ['MARL_VARIANT']!r}: 1 (one chain per CTA) or 3 (pair kernel)")
+if VARIANT == 3:
     os.environ["MARL_POLICY_PROFILE"] = "1"
 cfg = bench.make_cfg()
 B, M, N, E = bench.B_PER_GPU, 32, bench.N_AGENTS, 128
@@ -40,12 +44,12 @@ for it in range(3):
     s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     torch.cuda.synchronize()
     s.record()
-    fused.step(env, oxy_i, o_count, it, 1, False, hist, hist, emb_a, emb_c, ha, hc, act, logp, val, debug=dbg, variant=int(os.environ.get("MARL_VARIANT", "0")))
+    fused.step(env, oxy_i, o_count, it, 1, False, hist, hist, emb_a, emb_c, ha, hc, act, logp, val, debug=dbg, variant=VARIANT)
     e.record()
     e.synchronize()
     print("launch ms", s.elapsed_time(e))
 d = dbg.cpu().numpy().astype(np.float64)
-if int(os.environ.get("MARL_VARIANT", "0")) == 3:
+if VARIANT == 3:
     d_all = d
     d = d[: int((d[:, 13] > 1e15).sum())]
 # wall-clock schedule of the launch: effective SM clock, gaps between consecutive CTAs of one SM
@@ -60,7 +64,7 @@ for s_ in np.unique(sm[ok]):
     if s_ == 0:
         print("SM 0 schedule (start us, dur us):", [(round((g0[i] - g0[ok].min()) / 1e3, 1), round((g1[i] - g0[i]) / 1e3, 1)) for i in idx])
 print(f"gap between consecutive CTAs on an SM: median {np.median(gaps) / 1e3:.2f} us, max {np.max(gaps) / 1e3:.2f} us; CTAs per SM: {ok.sum() / len(np.unique(sm[ok])):.2f}")
-if int(os.environ.get("MARL_VARIANT", "0")) == 3:
+if VARIANT == 3:
     grid = len(d)                                 # CTA rows carry a %globaltimer stamp; the per-step rows follow them
     d = d[:grid]
     tot = d[:, 12]
