@@ -73,13 +73,11 @@ _PROTOTYPES = {
                                       _VP, _VP, _VP, _U64, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP,
                                       C.POINTER(RolloutRecords), _VP]),
     "marl_dhgn_message_fwd": (C.c_int, [_I32] * 4 + [_VP] * 8 + [_I32] + [_VP] * 8),
-    "marl_dhgn_message_bwd": (C.c_int, [_I32] * 4 + [_VP] * 8 + [_I32] + [_VP] * 14),
     "marl_dhgn_message_bwd_workspace_bytes": (_I64, [_I32, _I32, _I32]),
     "marl_dhgn_message_bwd_det": (C.c_int, [_I32] * 4 + [_VP] * 8 + [_I32] + [_VP] * 15),
     "marl_fcra_agg": (C.c_int, [_I32, _I32, _I32, _VP, _I64, _I64, _VP, _I32, _VP, _VP]),
     "marl_gru_cell_fwd": (C.c_int, [_I64, _I32] + [_VP] * 9),
     "marl_gru_cell_bwd": (C.c_int, [_I64, _I32] + [_VP] * 10),
-    "marl_ppo_head": (C.c_int, [_I64, _I32, _I32] + [_VP] * 12 + [_F32, _F32] + [_VP] * 7),
     "marl_ppo_head_workspace_bytes": (_I64, [_I64]),
     "marl_ppo_head_det": (C.c_int, [_I64, _I32, _I32] + [_VP] * 12 + [_F32, _F32] + [_VP] * 8),
     "marl_act_head": (C.c_int, [_I64, _I32, _I32] + [_VP] * 6 + [_U64, _I32, _I32] + [_VP] * 5),

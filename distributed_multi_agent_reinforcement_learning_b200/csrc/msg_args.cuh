@@ -20,9 +20,8 @@ struct MsgArgs {
 // sample-grouped kernels (msg_grouped.cu): E = 128, N <= 16, O <= 256; return MARL_EUNSUPPORTED otherwise
 int launch_msg_fwd_grouped(const MsgArgs &a, const float *W0, const float *b0, const float *W1, const float *b1, const float *W2,
                            const float *b2, float *agg, cudaStream_t stream);
-// ws == nullptr: every CTA adds its sums into gW / gb with atomics.  Otherwise CTA b of the launch of relation r writes its
-// (KW_r + 1) x E sums (KW = 8, 4, 4) to ws + blocks * E * {0, 9, 14}[r] + b * (KW_r + 1) * E and nothing else;
-// launch_msg_partials_reduce adds them.
+// ws is required: CTA b of the launch of relation r writes its (KW_r + 1) x E sums (KW = 8, 4, 4) to
+// ws + blocks * E * {0, 9, 14}[r] + b * (KW_r + 1) * E and nothing else; launch_msg_partials_reduce adds them into gW / gb.
 int launch_msg_bwd_grouped(const MsgArgs &a, const float *W0, const float *b0, const float *W1, const float *b1, const float *W2,
                            const float *b2, const float *d_agg, float *gW0, float *gb0, float *gW1, float *gb1, float *gW2, float *gb2,
                            float *ws, cudaStream_t stream);

@@ -123,15 +123,13 @@ msg_agg_fwd_kernel(MsgArgs a, const float *__restrict__ W0, const float *__restr
 
 // ---- backward w.r.t. the three message layers (inputs are data: no input gradient) ---------------------------
 // Pre-activations are recomputed; each warp walks many rows and keeps its dW slices in registers, then the CTA
-// reduces through shared memory and either issues one atomicAdd per weight element (DET false) or writes its 19 x E row of
-// partial sums to ws[blockIdx.x], reduced in a fixed order by msg_partials_reduce_kernel (DET true).
-template <int CPL, bool DET>
+// reduces through shared memory and writes its 19 x E row of partial sums to ws[blockIdx.x], reduced in a fixed order by
+// msg_partials_reduce_kernel.
+template <int CPL>
 __global__ void __launch_bounds__(kPolThreads)
 msg_agg_bwd_kernel(MsgArgs a, const float *__restrict__ W0, const float *__restrict__ b0, const float *__restrict__ W1,
                    const float *__restrict__ b1, const float *__restrict__ W2, const float *__restrict__ b2,
-                   const float *__restrict__ d_agg, float *__restrict__ gW0, float *__restrict__ gb0,
-                   float *__restrict__ gW1, float *__restrict__ gb1, float *__restrict__ gW2, float *__restrict__ gb2,
-                   float *__restrict__ ws)
+                   const float *__restrict__ d_agg, float *__restrict__ ws)
 {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, E = 32 * CPL;
     MsgWeights<CPL> w;
@@ -213,7 +211,7 @@ msg_agg_bwd_kernel(MsgArgs a, const float *__restrict__ W0, const float *__restr
             }
         }
     }
-    // CTA reduction: [warps][19*E] in shared memory, then one atomic or one partial per element
+    // CTA reduction: [warps][19*E] in shared memory, then one partial per element
     extern __shared__ float s_red[];
     float *mine = s_red + warp * 19 * E;
 #pragma unroll
@@ -228,17 +226,7 @@ msg_agg_bwd_kernel(MsgArgs a, const float *__restrict__ W0, const float *__restr
     for (int idx = threadIdx.x; idx < 19 * E; idx += kPolThreads) {
         float v = 0.f;
         for (int wv = 0; wv < kPolThreads / 32; ++wv) v += s_red[wv * 19 * E + idx];
-        if (DET) {
-            ws[(int64_t)blockIdx.x * 19 * E + idx] = v;
-            continue;
-        }
-        const int k = idx / E, c = idx - k * E;
-        if (k < 8) atomicAdd(gW0 + c * 8 + k, v);
-        else if (k == 8) atomicAdd(gb0 + c, v);
-        else if (k < 13) atomicAdd(gW1 + c * 4 + (k - 9), v);
-        else if (k == 13) atomicAdd(gb1 + c, v);
-        else if (k < 18) atomicAdd(gW2 + c * 4 + (k - 14), v);
-        else atomicAdd(gb2 + c, v);
+        ws[(int64_t)blockIdx.x * 19 * E + idx] = v;
     }
 }
 
@@ -369,11 +357,11 @@ struct HeadArgs {
     float *d_logits;             // [R,A]  d(actor_loss_sum)/d logits   (divide by sum(active) afterwards)
     float *d_value;              // [R]    d(critic_loss_sum)/d value
     float *sums;                 // [3] += {sum actor_term*active, sum critic_term*active, sum active}
-    float *partials;             // [gridDim.x][3] per-CTA sums of the deterministic epilogue (DET), reduced by ppo_sums_reduce_kernel
+    float *partials;             // [gridDim.x][3] per-CTA sums, reduced into sums by ppo_sums_reduce_kernel
 };
 
-// DET false: each CTA adds its three sums to h.sums with atomics; true: it writes them to h.partials[blockIdx.x].
-template <int CPL, int A, bool DET>
+// Each CTA writes its three sums to h.partials[blockIdx.x].
+template <int CPL, int A>
 __global__ void __launch_bounds__(kPolThreads)
 ppo_head_kernel(HeadArgs h)
 {
@@ -478,8 +466,7 @@ ppo_head_kernel(HeadArgs h)
     if (threadIdx.x < 3) {
         float v = 0.f;
         for (int wv = 0; wv < kPolThreads / 32; ++wv) v += s_part[wv][threadIdx.x];
-        if (DET) h.partials[blockIdx.x * 3 + threadIdx.x] = v;
-        else atomicAdd(h.sums + threadIdx.x, v);
+        h.partials[blockIdx.x * 3 + threadIdx.x] = v;
     }
 }
 
@@ -672,44 +659,6 @@ extern "C" int marl_dhgn_message_fwd(MSG_ARGS_DECL, const float *d_W0, const flo
     MSG_ARGS_DECL, const float *d_W0, const float *d_b0, const float *d_W1, const float *d_b1, const float *d_W2, const float *d_b2, \
         const float *d_grad_agg, float *d_gW0, float *d_gb0, float *d_gW1, float *d_gb1, float *d_gW2, float *d_gb2
 
-// d_ws == nullptr: atomic epilogue (marl_dhgn_message_bwd); otherwise per-CTA partials + fixed-order reduction
-static int message_bwd(const char *name, MSG_BWD_DECL, float *d_ws, void *stream)
-{
-    MsgArgs a;
-    int rc = fill_msg_args(a, S, N, O, E, d_p, d_e, d_oxy, d_o_index, d_o_count, d_p_adj_bits, d_e_adj, d_o_adj_bits, all_ones);
-    if (rc) return rc;
-    MARL_REQUIRE(d_W0 && d_b0 && d_W1 && d_b1 && d_W2 && d_b2 && d_grad_agg && d_gW0 && d_gb0 && d_gW1 && d_gb1 && d_gW2 && d_gb2,
-                 "%s: null pointer", name);
-    if (msg_grouped_supported(a, E))
-        return launch_msg_bwd_grouped(a, d_W0, d_b0, d_W1, d_b1, d_W2, d_b2, d_grad_agg, d_gW0, d_gb0, d_gW1, d_gb1, d_gW2, d_gb2, d_ws,
-                                      (cudaStream_t)stream);
-    return dispatch_cpl(E, [&](auto C_) -> int {
-        constexpr int CPL = decltype(C_)::value;
-        int blocks = grid_for_rows((int64_t)S * N);
-        if (blocks > kMsgBwdRowMaxCTAs) blocks = kMsgBwdRowMaxCTAs;   // persistent: fewer, longer warps -> fewer atomics / partials
-        const size_t smem = sizeof(float) * (kPolThreads / 32) * 19 * E;
-        if (!d_ws) {
-            msg_agg_bwd_kernel<CPL, false><<<blocks, kPolThreads, smem, (cudaStream_t)stream>>>(
-                a, d_W0, d_b0, d_W1, d_b1, d_W2, d_b2, d_grad_agg, d_gW0, d_gb0, d_gW1, d_gb1, d_gW2, d_gb2, nullptr);
-            return check_launch("msg_agg_bwd_kernel");
-        }
-        msg_agg_bwd_kernel<CPL, true><<<blocks, kPolThreads, smem, (cudaStream_t)stream>>>(
-            a, d_W0, d_b0, d_W1, d_b1, d_W2, d_b2, d_grad_agg, d_gW0, d_gb0, d_gW1, d_gb1, d_gW2, d_gb2, d_ws);
-        int rc2 = check_launch("msg_agg_bwd_kernel");
-        if (rc2) return rc2;
-        MsgPartials p;
-        for (int r = 0; r < 3; ++r) { p.rel_base[r] = d_ws + (r == 0 ? 0 : (r == 1 ? 9 : 14)) * E; p.rel_stride[r] = 19 * E; }
-        p.blocks = blocks; p.E = E;
-        return launch_msg_partials_reduce(p, d_gW0, d_gb0, d_gW1, d_gb1, d_gW2, d_gb2, (cudaStream_t)stream);
-    });
-}
-
-extern "C" int marl_dhgn_message_bwd(MSG_BWD_DECL, void *stream)
-{
-    return message_bwd("marl_dhgn_message_bwd", S, N, O, E, d_p, d_e, d_oxy, d_o_index, d_o_count, d_p_adj_bits, d_e_adj, d_o_adj_bits,
-                       all_ones, d_W0, d_b0, d_W1, d_b1, d_W2, d_b2, d_grad_agg, d_gW0, d_gb0, d_gW1, d_gb1, d_gW2, d_gb2, nullptr, stream);
-}
-
 static bool supported_width(int E) { return E == 32 || E == 64 || E == 128; }
 
 extern "C" int64_t marl_dhgn_message_bwd_workspace_bytes(int32_t N, int32_t O, int32_t E)
@@ -725,9 +674,29 @@ extern "C" int marl_dhgn_message_bwd_det(MSG_BWD_DECL, void *d_workspace, void *
 {
     MARL_REQUIRE(supported_width(E), "marl_dhgn_message_bwd_det: E=%d (32, 64 or 128)", E);
     MARL_REQUIRE(d_workspace, "marl_dhgn_message_bwd_det: null workspace");
-    return message_bwd("marl_dhgn_message_bwd_det", S, N, O, E, d_p, d_e, d_oxy, d_o_index, d_o_count, d_p_adj_bits, d_e_adj,
-                       d_o_adj_bits, all_ones, d_W0, d_b0, d_W1, d_b1, d_W2, d_b2, d_grad_agg, d_gW0, d_gb0, d_gW1, d_gb1, d_gW2, d_gb2,
-                       static_cast<float *>(d_workspace), stream);
+    MsgArgs a;
+    int rc = fill_msg_args(a, S, N, O, E, d_p, d_e, d_oxy, d_o_index, d_o_count, d_p_adj_bits, d_e_adj, d_o_adj_bits, all_ones);
+    if (rc) return rc;
+    MARL_REQUIRE(d_W0 && d_b0 && d_W1 && d_b1 && d_W2 && d_b2 && d_grad_agg && d_gW0 && d_gb0 && d_gW1 && d_gb1 && d_gW2 && d_gb2,
+                 "marl_dhgn_message_bwd_det: null pointer");
+    float *d_ws = static_cast<float *>(d_workspace);
+    if (msg_grouped_supported(a, E))
+        return launch_msg_bwd_grouped(a, d_W0, d_b0, d_W1, d_b1, d_W2, d_b2, d_grad_agg, d_gW0, d_gb0, d_gW1, d_gb1, d_gW2, d_gb2, d_ws,
+                                      (cudaStream_t)stream);
+    return dispatch_cpl(E, [&](auto C_) -> int {
+        constexpr int CPL = decltype(C_)::value;
+        int blocks = grid_for_rows((int64_t)S * N);
+        if (blocks > kMsgBwdRowMaxCTAs) blocks = kMsgBwdRowMaxCTAs;   // persistent: fewer, longer warps -> fewer partials
+        const size_t smem = sizeof(float) * (kPolThreads / 32) * 19 * E;
+        msg_agg_bwd_kernel<CPL><<<blocks, kPolThreads, smem, (cudaStream_t)stream>>>(a, d_W0, d_b0, d_W1, d_b1, d_W2, d_b2,
+                                                                                     d_grad_agg, d_ws);
+        int rc2 = check_launch("msg_agg_bwd_kernel");
+        if (rc2) return rc2;
+        MsgPartials p;
+        for (int r = 0; r < 3; ++r) { p.rel_base[r] = d_ws + (r == 0 ? 0 : (r == 1 ? 9 : 14)) * E; p.rel_stride[r] = 19 * E; }
+        p.blocks = blocks; p.E = E;
+        return launch_msg_partials_reduce(p, d_gW0, d_gb0, d_gW1, d_gb1, d_gW2, d_gb2, (cudaStream_t)stream);
+    });
 }
 
 extern "C" int marl_fcra_agg(int32_t S, int32_t N, int32_t E, const float *d_hist, int64_t sample_stride,
@@ -783,39 +752,6 @@ static inline int ppo_head_blocks(int64_t R)
     return (int)(blocks > 148 * 8 ? 148 * 8 : blocks);
 }
 
-// d_ws == nullptr: atomic epilogue (marl_ppo_head); otherwise per-CTA partials + fixed-order reduction
-static int ppo_head(const char *name, PPO_HEAD_DECL, float *d_ws, void *stream)
-{
-    MARL_REQUIRE(R > 0 && A == MARL_NUM_ACTIONS, "%s: R=%lld A=%d (action_dim must be %d)", name, (long long)R, A, MARL_NUM_ACTIONS);
-    MARL_REQUIRE(d_feat_a && d_feat_c && d_Wa && d_ba && d_wc_eff && d_bc && d_action && d_old_logp && d_adv &&
-                     d_v_target && d_active && d_logp && d_entropy && d_value && d_dlogits && d_dvalue && d_sums,
-                 "%s: null pointer", name);
-    HeadArgs h;
-    h.R = R; h.E = E; h.A = A; h.feat_a = d_feat_a; h.feat_c = d_feat_c; h.Wa = d_Wa; h.ba = d_ba; h.wc_eff = d_wc_eff;
-    h.bc = d_bc; h.action = d_action; h.old_logp = d_old_logp; h.adv = d_adv; h.v_old = d_v_old; h.v_target = d_v_target;
-    h.active = d_active; h.eps = eps; h.ent_coef = ent_coef; h.logp = d_logp; h.entropy = d_entropy; h.value = d_value;
-    h.d_logits = d_dlogits; h.d_value = d_dvalue; h.sums = d_sums; h.partials = d_ws;
-    return dispatch_cpl(E, [&](auto C_) -> int {
-        constexpr int CPL = decltype(C_)::value;
-        const int blocks = ppo_head_blocks(R);
-        if (!d_ws) {
-            ppo_head_kernel<CPL, MARL_NUM_ACTIONS, false><<<blocks, kPolThreads, 0, (cudaStream_t)stream>>>(h);
-            return check_launch("ppo_head_kernel");
-        }
-        ppo_head_kernel<CPL, MARL_NUM_ACTIONS, true><<<blocks, kPolThreads, 0, (cudaStream_t)stream>>>(h);
-        int rc = check_launch("ppo_head_kernel");
-        if (rc) return rc;
-        ppo_sums_reduce_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(blocks, d_ws, d_sums);
-        return check_launch("ppo_sums_reduce_kernel");
-    });
-}
-
-extern "C" int marl_ppo_head(PPO_HEAD_DECL, void *stream)
-{
-    return ppo_head("marl_ppo_head", R, E, A, d_feat_a, d_feat_c, d_Wa, d_ba, d_wc_eff, d_bc, d_action, d_old_logp, d_adv, d_v_old,
-                    d_v_target, d_active, eps, ent_coef, d_logp, d_entropy, d_value, d_dlogits, d_dvalue, d_sums, nullptr, stream);
-}
-
 extern "C" int64_t marl_ppo_head_workspace_bytes(int64_t R)
 {
     return R > 0 ? (int64_t)ppo_head_blocks(R) * 3 * (int64_t)sizeof(float) : -1;
@@ -825,9 +761,26 @@ extern "C" int marl_ppo_head_det(PPO_HEAD_DECL, void *d_workspace, void *stream)
 {
     MARL_REQUIRE(supported_width(E), "marl_ppo_head_det: E=%d (32, 64 or 128)", E);
     MARL_REQUIRE(d_workspace, "marl_ppo_head_det: null workspace");
-    return ppo_head("marl_ppo_head_det", R, E, A, d_feat_a, d_feat_c, d_Wa, d_ba, d_wc_eff, d_bc, d_action, d_old_logp, d_adv, d_v_old,
-                    d_v_target, d_active, eps, ent_coef, d_logp, d_entropy, d_value, d_dlogits, d_dvalue, d_sums,
-                    static_cast<float *>(d_workspace), stream);
+    MARL_REQUIRE(R > 0 && A == MARL_NUM_ACTIONS, "marl_ppo_head_det: R=%lld A=%d (action_dim must be %d)", (long long)R, A,
+                 MARL_NUM_ACTIONS);
+    MARL_REQUIRE(d_feat_a && d_feat_c && d_Wa && d_ba && d_wc_eff && d_bc && d_action && d_old_logp && d_adv &&
+                     d_v_target && d_active && d_logp && d_entropy && d_value && d_dlogits && d_dvalue && d_sums,
+                 "marl_ppo_head_det: null pointer");
+    float *d_ws = static_cast<float *>(d_workspace);
+    HeadArgs h;
+    h.R = R; h.E = E; h.A = A; h.feat_a = d_feat_a; h.feat_c = d_feat_c; h.Wa = d_Wa; h.ba = d_ba; h.wc_eff = d_wc_eff;
+    h.bc = d_bc; h.action = d_action; h.old_logp = d_old_logp; h.adv = d_adv; h.v_old = d_v_old; h.v_target = d_v_target;
+    h.active = d_active; h.eps = eps; h.ent_coef = ent_coef; h.logp = d_logp; h.entropy = d_entropy; h.value = d_value;
+    h.d_logits = d_dlogits; h.d_value = d_dvalue; h.sums = d_sums; h.partials = d_ws;
+    return dispatch_cpl(E, [&](auto C_) -> int {
+        constexpr int CPL = decltype(C_)::value;
+        const int blocks = ppo_head_blocks(R);
+        ppo_head_kernel<CPL, MARL_NUM_ACTIONS><<<blocks, kPolThreads, 0, (cudaStream_t)stream>>>(h);
+        int rc = check_launch("ppo_head_kernel");
+        if (rc) return rc;
+        ppo_sums_reduce_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(blocks, d_ws, d_sums);
+        return check_launch("ppo_sums_reduce_kernel");
+    });
 }
 
 extern "C" int marl_act_head(int64_t R, int32_t E, int32_t A, const float *d_feat_a, const float *d_feat_c,

@@ -331,28 +331,22 @@ int marl_envn2n_rollout(const marl_envn2n_params *p, int32_t B, int32_t T, int32
  * library GEMMs on the host side; these entry points fuse everything pairwise / sparse / pointwise around them so that
  * no [.,N,N,8], [.,N,O,4] or dense 0/1 adjacency tensor is materialised.  E = embedding_dim in {32, 64, 128}.
  *
- * marl_dhgn_message_{fwd,bwd}: DHGN.message + L1-normalised mean aggregation of the three relations
+ * marl_dhgn_message_fwd / marl_dhgn_message_bwd_det: DHGN.message + L1-normalised mean aggregation of the three relations
  * (DHGN/mappo_parallel.py:256-281,323-348) from bit-packed adjacency.  S samples x N agents;
  * p f32 [S,N,4], e f32 [S,4], oxy f32 [Bo,O,2] + o_index i32 [S] + o_count i32 [Bo] (obstacle cells per map; the count
  * is what "all ones" spans for the critic: O_b during rollout, O in training — :64-65, SURVEY 7.4-5);
- * W0 [E,8], W1 [E,4], W2 [E,4] = MSG_layers.{0,1,2}.weight.  Out: agg f32 [S,N,3,E] (input of AGG_vertex_0).
- * bwd accumulates (+=) the weight/bias gradients; inputs are data, so there is no input gradient. */
+ * W0 [E,8], W1 [E,4], W2 [E,4] = MSG_layers.{0,1,2}.weight.  Out: agg f32 [S,N,3,E] (input of AGG_vertex_0). */
 int marl_dhgn_message_fwd(int32_t S, int32_t N, int32_t O, int32_t E, const float *d_p, const float *d_e,
                           const float *d_oxy, const int32_t *d_o_index, const int32_t *d_o_count,
                           const uint32_t *d_p_adj_bits, const uint8_t *d_e_adj, const uint32_t *d_o_adj_bits,
                           int32_t all_ones, const float *d_W0, const float *d_b0, const float *d_W1, const float *d_b1,
                           const float *d_W2, const float *d_b2, float *d_agg, void *stream);
-int marl_dhgn_message_bwd(int32_t S, int32_t N, int32_t O, int32_t E, const float *d_p, const float *d_e,
-                          const float *d_oxy, const int32_t *d_o_index, const int32_t *d_o_count,
-                          const uint32_t *d_p_adj_bits, const uint8_t *d_e_adj, const uint32_t *d_o_adj_bits,
-                          int32_t all_ones, const float *d_W0, const float *d_b0, const float *d_W1, const float *d_b1,
-                          const float *d_W2, const float *d_b2, const float *d_grad_agg, float *d_gW0, float *d_gb0,
-                          float *d_gW1, float *d_gb1, float *d_gW2, float *d_gb2, void *stream);
-/* The same backward with a deterministic reduction: every CTA writes its partial weight / bias sums to d_workspace, and a
- * second kernel adds them in a fixed order into the gradients (+=), so two calls on the same inputs give the same bits.
- * marl_dhgn_message_bwd reduces with fp32 atomics instead, whose order varies from run to run.  d_workspace: at least
- * marl_dhgn_message_bwd_workspace_bytes(N, O, E) bytes, which does not depend on S (-1 for an unsupported N, O or E).  A
- * workspace must not be shared by calls that may run at the same time. */
+/* The backward accumulates (+=) the weight / bias gradients gW0 [E,8], gb0 [E], gW1 / gW2 [E,4], gb1 / gb2 [E] from
+ * d_grad_agg [S,N,3,E]; inputs are data, so there is no input gradient.  The reduction is deterministic: every CTA writes its
+ * partial weight / bias sums to d_workspace, and a second kernel adds them in a fixed order into the gradients, so two calls
+ * on the same inputs give the same bits.  d_workspace: at least marl_dhgn_message_bwd_workspace_bytes(N, O, E) bytes, which
+ * does not depend on S (-1 for an unsupported N, O or E).  A workspace must not be shared by calls that may run at the same
+ * time. */
 int64_t marl_dhgn_message_bwd_workspace_bytes(int32_t N, int32_t O, int32_t E);
 int marl_dhgn_message_bwd_det(int32_t S, int32_t N, int32_t O, int32_t E, const float *d_p, const float *d_e,
                               const float *d_oxy, const int32_t *d_o_index, const int32_t *d_o_count,
@@ -372,15 +366,9 @@ int marl_gru_cell_bwd(int64_t R, int32_t E, const float *d_dh_new, const float *
 /* Actor softmax/Categorical + critic head + PPO-clip / clipped value losses, forward AND backward in one pass
  * (:437,446-456,526,692-706).  Adds {sum actor_term*active, sum critic_term*active, sum active} to d_sums[3] and
  * writes d(sum)/d logits [R,A], d(sum)/d value [R]; the caller divides by sum(active).  d_v_old == NULL selects the unclipped
- * value loss (values_now - v_target)^2 of use_value_clip = False (:703-704). */
-int marl_ppo_head(int64_t R, int32_t E, int32_t A, const float *d_feat_a, const float *d_feat_c, const float *d_Wa,
-                  const float *d_ba, const float *d_wc_eff, const float *d_bc, const float *d_action,
-                  const float *d_old_logp, const float *d_adv, const float *d_v_old, const float *d_v_target,
-                  const float *d_active, float eps, float ent_coef, float *d_logp, float *d_entropy, float *d_value,
-                  float *d_dlogits, float *d_dvalue, float *d_sums, void *stream);
-/* marl_ppo_head with the three sums reduced in a fixed order (per-CTA partials in d_workspace, then one reduction kernel)
- * instead of fp32 atomics: bit-identical results from call to call.  d_workspace: at least marl_ppo_head_workspace_bytes(R)
- * bytes (-1 for R <= 0), not shared by calls that may run at the same time. */
+ * value loss (values_now - v_target)^2 of use_value_clip = False (:703-704).  The three sums are reduced in a fixed order
+ * (per-CTA partials in d_workspace, then one reduction kernel): bit-identical results from call to call.  d_workspace: at
+ * least marl_ppo_head_workspace_bytes(R) bytes (-1 for R <= 0), not shared by calls that may run at the same time. */
 int64_t marl_ppo_head_workspace_bytes(int64_t R);
 int marl_ppo_head_det(int64_t R, int32_t E, int32_t A, const float *d_feat_a, const float *d_feat_c, const float *d_Wa,
                       const float *d_ba, const float *d_wc_eff, const float *d_bc, const float *d_action,

@@ -534,8 +534,8 @@ def test_shuffled_minibatches_through_the_gather_kernel():
     assert torch.equal(tr["permutation"].cpu(), torch.arange(episodes))
     for a_, b_ in zip(tr_seq["mb"], tr["mb"]):            # identity permutation: the forward passes are bit-identical ...
         assert torch.equal(a_["logp"], b_["logp"]) and torch.equal(a_["ent"], b_["ent"]) and torch.equal(a_["val"], b_["val"])
-    # ... and so are the gradients up to the summation order of the message layers' atomic weight-gradient reduction
-    torch.testing.assert_close(g_id, g_seq, rtol=1e-5, atol=1e-7)
+    # ... and so are the gradients: both epochs feed the same minibatches to kernels that reduce in a fixed order
+    assert torch.equal(g_id, g_seq)
     perm = [3, 0, 4, 2, 1]
     reset_sn()
     g_perm, _ = _train_grads(m, buf, steps, permutation=perm)
