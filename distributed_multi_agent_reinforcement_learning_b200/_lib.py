@@ -111,6 +111,7 @@ _PROTOTYPES = {
     "marl_welford_update_f64": (C.c_int, [_I32, _I32, _VP, _VP, _VP, _VP, _VP, _VP, _I32, _VP]),
     "marl_gae_workspace_bytes": (_I64, [_I32, _I32, _I32]),
     "marl_gae": (C.c_int, [_I32, _I32, _I32, _VP, _VP, _VP, _I32, _F32, _F32, _I32, _VP, _VP, _VP, _VP]),
+    "marl_gae_boundary": (C.c_int, [_I32, _I32, _I32, _I32, _VP, _VP, _VP, _VP, _F32, _F32, _I32, _VP, _VP, _VP, _VP]),
     "marl_gather_rows": (C.c_int, [_VP, _VP, _VP, _I32, _I64, _I64, _VP]),
     "marl_env3d_step": (C.c_int, [_VP, _I32] + [_VP] * 10),
     "marl_env3d_evader_step": (C.c_int, [_VP, _I32] + [_VP] * 4),

@@ -108,7 +108,8 @@ def save_training_state(path, mappo, engine=None, evaluator=None, extra=None, ca
     values (it loads with weights_only=True): a shape fingerprint, the actor / critic state_dicts (spectral-norm buffers included),
     the Adam state, `total_step`, the reward normaliser, the engine's state (`BatchedPursuitEnv.state_dict`), the evaluator's
     bookkeeping, the torch CPU / CUDA, Python `random` and numpy RNG states, `extra` (the caller's loop counters) and `carry`, the
-    RolloutCarry the next rollout segment continues from when the run stops inside an episode (None: at an episode boundary).
+    RolloutCarry the next rollout segment continues from when the run stops inside an episode (None: at an episode boundary), with
+    its episode index (the count an auto-reset rollout stream keeps).
     Take it between iterations, after `update()`.  Under torch.distributed every rank writes its own file."""
     rn = getattr(mappo, "reward_norm", None)
     np_state = np.random.get_state(legacy=False)
@@ -125,7 +126,8 @@ def save_training_state(path, mappo, engine=None, evaluator=None, extra=None, ca
                  numpy=dict(bit_generator=np_state["bit_generator"], key=[int(k) for k in np_state["state"]["key"]],
                             pos=int(np_state["state"]["pos"]), has_gauss=int(np_state["has_gauss"]), gauss=float(np_state["gauss"]))),
         extra=dict(extra or {}),
-        carry=None if carry is None else dict(t0=int(carry.t0), **{k: getattr(carry, k).detach().cpu() for k in _CARRY}))
+        carry=None if carry is None else dict(t0=int(carry.t0), episode=int(getattr(carry, "episode", 0)),
+                                              **{k: getattr(carry, k).detach().cpu() for k in _CARRY}))
     d = os.path.dirname(os.path.abspath(path))
     os.makedirs(d, exist_ok=True)
     tmp = path + ".tmp"
@@ -140,7 +142,7 @@ def load_training_state(path, mappo, engine=None, evaluator=None, carry=None):
     stay views into the optimizer's flat arena.
     carry: a RolloutCarry (e.g. `RolloutCarry.zeros`) that receives the file's carry in place; a file without one (every file
     written without `carry=`) is at an episode boundary and sets it to t0 = 0 with zero tensors.  A file that holds a carry can
-    only be loaded with one."""
+    only be loaded with one.  The carry's episode index is the file's (0 for a file without one)."""
     st = torch.load(path, map_location="cpu", weights_only=True)
     if st.get("version") != TRAINING_STATE_VERSION:
         raise MarlError(f"{path}: training-state format {st.get('version')!r}, this build reads {TRAINING_STATE_VERSION}")
@@ -195,6 +197,7 @@ def load_training_state(path, mappo, engine=None, evaluator=None, carry=None):
         engine.load_state_dict(st["engine"])
     if carry is not None:
         carry.t0 = 0 if sc is None else int(sc["t0"])
+        carry.episode = 0 if sc is None else int(sc.get("episode", 0))
         for k in _CARRY:
             if sc is None:
                 getattr(carry, k).zero_()

@@ -91,6 +91,57 @@ gae_scan_kernel(int B, int T, int N, const float *__restrict__ r, const float *_
     }
 }
 
+// GAE of a time-major rollout segment [T,B,N] whose episode ends after step k-1 (0 < k < T): steps k..T-1 are the next episode's
+// start and bootstrap from v[T]; steps 0..k-1 end the previous episode and bootstrap from v_boot [B,N] (its value after its last
+// step) instead of v[k].  Each piece is exactly gae_scan_kernel's recursion on its own steps: the recursion does not cross k.
+// Partials as in gae_scan_kernel, over all T steps, for adv_norm_kernel.  The block reduction below repeats gae_scan_kernel's (kept
+// apart so that kernel's code stays as it is): the two must stay in step, adv_norm_kernel reads one (sum, sum of squares) per block.
+__global__ void __launch_bounds__(kGaeThreads)
+gae_scan_boundary_kernel(int B, int T, int N, int k, const float *__restrict__ r, const float *__restrict__ v,
+                         const float *__restrict__ v_boot, const float *__restrict__ active, float gamma, float gl,
+                         float *__restrict__ adv, float *__restrict__ v_target, double *__restrict__ partial)
+{
+    const int64_t chain = (int64_t)blockIdx.x * kGaeThreads + threadIdx.x;
+    const int64_t st = (int64_t)B * N;
+    double sum = 0.0, sq = 0.0;
+    if (chain < st) {
+        float gae = 0.0f;
+        float v_next = v[chain + (int64_t)T * st];
+        for (int t = T - 1; t >= 0; --t) {
+            if (t == k - 1) {                       // the previous episode's last step: its own bootstrap, a fresh recursion
+                gae = 0.0f;
+                v_next = v_boot[chain];
+            }
+            const int64_t i = chain + (int64_t)t * st;
+            const float v_t = v[i];
+            const float delta = __fmul_rn(__fsub_rn(__fadd_rn(r[i], __fmul_rn(gamma, v_next)), v_t), active[i]);
+            gae = __fadd_rn(delta, __fmul_rn(gl, gae));
+            adv[i] = gae;
+            v_target[i] = __fadd_rn(gae, v_t);
+            sum += (double)gae;
+            sq += (double)gae * (double)gae;
+            v_next = v_t;
+        }
+    }
+    __shared__ double s_sum[kGaeThreads / 32], s_sq[kGaeThreads / 32];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        sum += __shfl_down_sync(0xffffffffu, sum, o);
+        sq += __shfl_down_sync(0xffffffffu, sq, o);
+    }
+    if ((threadIdx.x & 31) == 0) {
+        s_sum[threadIdx.x >> 5] = sum;
+        s_sq[threadIdx.x >> 5] = sq;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double a = 0, q = 0;
+        for (int w = 0; w < kGaeThreads / 32; ++w) { a += s_sum[w]; q += s_sq[w]; }
+        partial[2 * blockIdx.x] = a;
+        partial[2 * blockIdx.x + 1] = q;
+    }
+}
+
 // adv = (adv - mean) / (std_unbiased + 1e-5) * active over the whole tensor (mappo_parallel.py:655-658).
 // Every block re-reduces the (few thousand) partials in the same order -> deterministic mean/std.
 __global__ void __launch_bounds__(256)
@@ -183,6 +234,29 @@ extern "C" int marl_gae(int32_t B, int32_t T, int32_t N, const float *d_r, const
     if (use_adv_norm) {
         const int64_t total = chains * T;
         MARL_REQUIRE(total > 1, "marl_gae: adv-norm needs more than one sample");
+        int nb = (int)((total + 255) / 256);
+        if (nb > 148 * 8) nb = 148 * 8;
+        adv_norm_kernel<<<nb, 256, 0, s>>>(total, blocks, (const double *)d_workspace, d_active, d_adv);
+        rc = check_launch("adv_norm_kernel");
+    }
+    return rc;
+}
+
+extern "C" int marl_gae_boundary(int32_t B, int32_t T, int32_t N, int32_t k, const float *d_r, const float *d_v, const float *d_v_boot,
+                                 const float *d_active, float gamma, float gamma_lamda, int32_t use_adv_norm, float *d_adv,
+                                 float *d_v_target, void *d_workspace, void *stream)
+{
+    MARL_REQUIRE(B > 0 && T > 1 && N > 0 && k > 0 && k < T, "marl_gae_boundary: B=%d T=%d N=%d k=%d", B, T, N, k);
+    MARL_REQUIRE(d_r && d_v && d_v_boot && d_active && d_adv && d_v_target && d_workspace, "marl_gae_boundary: null pointer");
+    const int64_t chains = (int64_t)B * N;
+    const int blocks = (int)((chains + kGaeThreads - 1) / kGaeThreads);
+    cudaStream_t s = (cudaStream_t)stream;
+    gae_scan_boundary_kernel<<<blocks, kGaeThreads, 0, s>>>(B, T, N, k, d_r, d_v, d_v_boot, d_active, gamma, gamma_lamda, d_adv,
+                                                            d_v_target, (double *)d_workspace);
+    int rc = check_launch("gae_scan_boundary_kernel");
+    if (rc) return rc;
+    if (use_adv_norm) {
+        const int64_t total = chains * T;
         int nb = (int)((total + 255) / 256);
         if (nb > 148 * 8) nb = 148 * 8;
         adv_norm_kernel<<<nb, 256, 0, s>>>(total, blocks, (const double *)d_workspace, d_active, d_adv);

@@ -78,23 +78,24 @@ class RolloutCarry:
     [L, B*N, E] after step t0-1.  emb_a / emb_c: the last D embeddings of each network [D, B, N, E], index j = step t0-D+j (zeros
     for steps before the episode's first).  A carry with t0 = 0 is the start of an episode: zero hidden states and zero history."""
 
-    def __init__(self, t0, ha, hc, emb_a, emb_c):
+    def __init__(self, t0, ha, hc, emb_a, emb_c, episode=0):
         self.t0, self.ha, self.hc, self.emb_a, self.emb_c = int(t0), ha, hc, emb_a, emb_c
+        self.episode = int(episode)     # index of the episode that step t0 belongs to (counted by an auto-reset rollout stream)
 
     @classmethod
-    def zeros(cls, mappo, B, N, t0=0):
+    def zeros(cls, mappo, B, N, t0=0, episode=0):
         """An episode start (t0 = 0) for B envs of N agents, on the networks' device."""
         f32 = dict(dtype=torch.float32, device=mappo.device)
         L, E, D = mappo.num_layers, mappo.embedding_dim, mappo.depth
         return cls(t0, torch.zeros(L, B * N, E, **f32), torch.zeros(L, B * N, E, **f32), torch.zeros(D, B, N, E, **f32),
-                   torch.zeros(D, B, N, E, **f32))
+                   torch.zeros(D, B, N, E, **f32), episode=episode)
 
     def shapes(self):
         return dict(ha=tuple(self.ha.shape), hc=tuple(self.hc.shape), emb_a=tuple(self.emb_a.shape), emb_c=tuple(self.emb_c.shape))
 
     def copy_(self, other):
-        """Copies `other`'s step and tensors into this carry's tensors (same shapes)."""
-        self.t0 = int(other.t0)
+        """Copies `other`'s step, episode and tensors into this carry's tensors (same shapes)."""
+        self.t0, self.episode = int(other.t0), int(other.episode)
         for k in ("ha", "hc", "emb_a", "emb_c"):
             if getattr(self, k).data_ptr() != getattr(other, k).data_ptr():
                 getattr(self, k).copy_(getattr(other, k))
@@ -112,6 +113,10 @@ def check_segment(carry, S, T_ep, B, N, L, E, D, device, actor_only=False):
         raise _lib.MarlError(f"rollout segment of {S} steps: the length must be a positive divisor of the episode length {T_ep}")
     if carry.t0 < 0 or carry.t0 + S > T_ep:
         raise _lib.MarlError(f"rollout segment [{carry.t0}, {carry.t0 + S}) does not lie inside the episode of {T_ep} steps")
+    _check_carry_tensors(carry, B, N, L, E, D, device)
+
+
+def _check_carry_tensors(carry, B, N, L, E, D, device):
     want = dict(ha=(L, B * N, E), hc=(L, B * N, E), emb_a=(D, B, N, E), emb_c=(D, B, N, E))
     have = carry.shapes()
     dev = torch.device(device)
@@ -121,6 +126,45 @@ def check_segment(carry, S, T_ep, B, N, L, E, D, device, actor_only=False):
                 or (dev.index is not None and x.device.index != dev.index)):
             raise _lib.MarlError(f"rollout carry: {k} is {have[k]} {x.dtype} on {x.device}, this rollout needs {want[k]} float32 on "
                                  f"{device}")
+
+
+class AutoReset:
+    """Lets a rollout segment run across an episode boundary (`rollout_batched(carry=..., auto_reset=AutoReset(...))`).
+
+    All envs of a batch step in lock-step and an episode ends only at cfg.env.max_steps, so the boundary falls at the same step of the
+    segment for every env.  There the rollout bootstraps the finished episode e, resets every env on the device with
+    `engine.reset_device(seed=reset_seed(e + 1), tape_len=tape_len)`, zeroes both networks' hidden states and history, and continues
+    with episode e + 1.  The actions of episode e are sampled with seed `sample_seed(e)` (keyed by row and the episode's step, as in a
+    whole-episode rollout), so a stream of segments collects the episodes that `reset_device(reset_seed(e))` followed by
+    `rollout_batched(max_steps, seed=sample_seed(e))` collects, bit for bit.  reset_seed / sample_seed: host callables, episode
+    index -> int."""
+
+    def __init__(self, reset_seed, sample_seed, tape_len=16):
+        self.reset_seed, self.sample_seed, self.tape_len = reset_seed, sample_seed, int(tape_len)
+
+
+def check_auto_reset(auto_reset, carry, S, T_ep, B, N, L, E, D, device, actor_only=False, use_fused=True, seed=0):
+    """Host-side checks of an auto-reset rollout segment (any 1 <= S <= T_ep from any step 0 <= carry.t0 < T_ep); raises MarlError
+    before any CUDA call."""
+    if not isinstance(auto_reset, AutoReset):
+        raise _lib.MarlError(f"rollout_batched: auto_reset must be an AutoReset, not {type(auto_reset).__name__}")
+    if carry is None:
+        raise _lib.MarlError("rollout_batched: auto_reset continues a stream of segments and needs a carry (RolloutCarry.zeros at the "
+                             "start)")
+    if actor_only:
+        raise _lib.MarlError("rollout_batched: actor_only (the evaluator's episode) runs whole episodes and takes no auto_reset")
+    if not use_fused:
+        raise _lib.MarlError("rollout_batched: auto_reset needs the fused policy step (embedding_dim = rnn_hidden_dim = 128, "
+                             "2 GRU layers, depth 1..3, 9 actions)")
+    if seed != 0:
+        raise _lib.MarlError(f"rollout_batched: seed={seed} with auto_reset: the sampling seeds come from auto_reset.sample_seed")
+    if not isinstance(carry, RolloutCarry):
+        raise _lib.MarlError(f"rollout_batched: carry must be a RolloutCarry, not {type(carry).__name__}")
+    if S <= 0 or S > T_ep:
+        raise _lib.MarlError(f"auto-reset rollout segment of {S} steps: the length must lie in [1, {T_ep}], the episode length")
+    if carry.t0 < 0 or carry.t0 >= T_ep:
+        raise _lib.MarlError(f"auto-reset rollout segment from step {carry.t0}: the start must lie in [0, {T_ep})")
+    _check_carry_tensors(carry, B, N, L, E, D, device)
 
 
 def orthogonal_init(layer, gain=1.0):
@@ -428,6 +472,14 @@ class TrainBatch:
     # has t0 = 0 and None for all of them: zero hidden states and zero history.
     t0 = 0
     h0_a = h0_c = prefix_a = prefix_c = carry = None
+    # A segment that crossed an episode boundary (rollout_batched(auto_reset=...)) has boundary = k: steps [0, k) end one episode and
+    # [k, T) start the next, which trains from zero hidden states and zero history, on its own maps oxy2 / o_count_train2 (replay2:
+    # its HistoryReplay).  v_boot [B,N] is the bootstrap value after step k-1.  `pieces()` views it as those two ordinary batches; a
+    # minibatch of it holds the minibatches of both pieces in `parts`.  ended_collision / ended_evader_status [B]: the flags of the
+    # episode that ended during the segment (the reset cleared the engine's).
+    boundary = v_boot = oxy2 = o_count_train2 = replay2 = parts = None
+    ended_collision = ended_evader_status = None
+    zero_prefix = False     # a store-mode piece whose history slabs 0..D-1 belong to the previous episode: they read as zeros
 
     def __init__(self, **kw):
         self.__dict__.update(kw)
@@ -450,7 +502,17 @@ class TrainBatch:
     def _select(self, tm, em):
         """The minibatch of the envs that `tm` selects from a time-major slab ([X, B, ...] -> [X, mb, ...]) and `em` from an env-major
         tensor ([B, ...] -> [mb, ...]).  A replay-mode batch regenerates the minibatch's history from its slabs (on the current stream)."""
-        opt = lambda x: None if x is None else tm(x)     # noqa: E731
+        if self.boundary is not None:
+            parts = [pc._select(tm, em) for pc in self.pieces()]
+            cat = lambda k: torch.cat([getattr(x, k) for x in parts])     # noqa: E731
+            return TrainBatch(p=cat("p"), a=cat("a"), logp=cat("logp"), r=cat("r"), active=cat("active"), v=tm(self.v), depth=self.depth,
+                              boundary=self.boundary, parts=parts)
+
+        def opt(x):
+            if x is None or not self.zero_prefix:
+                return None if x is None else tm(x)
+            h = tm(x[self.depth:])                      # the minibatch's own copy, with D zero slabs in front
+            return torch.cat([h.new_zeros((self.depth,) + tuple(h.shape[1:])), h])
         mb = TrainBatch(p=tm(self.p), e=tm(self.e), oxy=em(self.oxy), o_count_train=em(self.o_count_train), p_adj_bits=tm(self.p_adj_bits),
                         e_adj=tm(self.e_adj), o_adj_bits=tm(self.o_adj_bits), hist_a=opt(self.hist_a), hist_c=opt(self.hist_c),
                         v=tm(self.v), a=tm(self.a), logp=tm(self.logp), r=tm(self.r), active=tm(self.active), depth=self.depth)
@@ -463,6 +525,23 @@ class TrainBatch:
             mb.replay, mb.map_id = self.replay, em(self.map_id)
             self.replay.regenerate(mb)
         return mb
+
+    def pieces(self):
+        """A batch that crossed an episode boundary at step k as two ordinary batches sharing its slabs: steps [0, k) (the segment's
+        start state, the ended episode's maps, bootstrapped with v_boot) and steps [k, T) (an episode start on the new maps)."""
+        k, D = self.boundary, self.depth
+        first = lambda x, n=k: None if x is None else x[:n]     # noqa: E731
+        last = lambda x: None if x is None else x[k:]           # noqa: E731
+        keys = ("p", "e", "p_adj_bits", "e_adj", "o_adj_bits", "a", "logp", "r", "active")
+        common = lambda f: {n: f(getattr(self, n)) for n in keys}     # noqa: E731
+        one = TrainBatch(**common(first), oxy=self.oxy, o_count_train=self.o_count_train, hist_a=first(self.hist_a, k + D),
+                         hist_c=first(self.hist_c, k + D), v=torch.cat([self.v[:k], self.v_boot.unsqueeze(0)]), depth=D, t0=self.t0,
+                         h0_a=self.h0_a, h0_c=self.h0_c, prefix_a=self.prefix_a, prefix_c=self.prefix_c, replay=self.replay,
+                         map_id=self.map_id)
+        two = TrainBatch(**common(last), oxy=self.oxy2, o_count_train=self.o_count_train2, hist_a=last(self.hist_a),
+                         hist_c=last(self.hist_c), v=self.v[k:], depth=D, replay=self.replay2, map_id=self.map_id,
+                         zero_prefix=self.hist_a is not None)
+        return one, two
 
     def minibatch(self, lo, hi):
         """Envs [lo, hi): contiguous copies of the slabs (the reference's sequential `batch[key][index]`)."""
@@ -623,6 +702,28 @@ class MAPPO:
     # ------------------------------------------------------------------------------------------------ training
     def _forward_losses(self, mb, adv, v_target, side=None):
         T, B, N, E = mb.T, mb.B, mb.N, self.embedding_dim
+        if mb.parts is None:
+            feat_a, feat_c = self._features(mb, side)
+        else:                           # a segment that crossed an episode boundary: the GRU and the history restart with each piece
+            feats = [self._features(part, side) for part in mb.parts]
+            feat_a, feat_c = (torch.cat([f[i] for f in feats]) for i in (0, 1))
+        cm = self.critic.Mean
+        R = T * B * N
+        flat = lambda x: x.reshape(R)
+        la, lc, logp, ent, val, u2, v2 = ops.ppo_head(
+            feat_a.reshape(R, E), feat_c.reshape(R, E), self.actor.Mean.weight, self.actor.Mean.bias,
+            cm.weight_orig if self.sn else cm.weight, cm.bias, cm.weight_u if self.sn else torch.ones(1, device=self.device),
+            flat(mb.a), flat(mb.logp), flat(adv), flat(mb.v[:-1]) if self.use_value_clip else None, flat(v_target), flat(mb.active), self.epsilon,
+            self.entropy_coef)
+        if self.sn:
+            with torch.no_grad():
+                cm.weight_u.copy_(u2)
+                cm.weight_v.copy_(v2)
+        return la, lc, logp.view(T, B, N), ent.view(T, B, N), val.view(T, B, N)
+
+    def _features(self, mb, side=None):
+        """The GRU outputs [T, B*N, E] of the actor and the critic over a minibatch's steps, from its start state."""
+        T, B, N, E = mb.T, mb.B, mb.N, self.embedding_dim
         graph = mb.graph()
         enc = self.actor.shared_net
         if mb.h0_a is None:             # a whole episode starts from zero hidden states
@@ -651,27 +752,22 @@ class MAPPO:
             feat_a, _ = self.actor.features(emb_a.view(T, B * N, E), h0_a)
             emb_c = enc.encode(graph, True, mb.history("critic"))
             feat_c, _ = self.critic.features(emb_c.view(T, B * N, E), h0_c)
-        cm = self.critic.Mean
-        R = T * B * N
-        flat = lambda x: x.reshape(R)
-        la, lc, logp, ent, val, u2, v2 = ops.ppo_head(
-            feat_a.reshape(R, E), feat_c.reshape(R, E), self.actor.Mean.weight, self.actor.Mean.bias,
-            cm.weight_orig if self.sn else cm.weight, cm.bias, cm.weight_u if self.sn else torch.ones(1, device=self.device),
-            flat(mb.a), flat(mb.logp), flat(adv), flat(mb.v[:-1]) if self.use_value_clip else None, flat(v_target), flat(mb.active), self.epsilon,
-            self.entropy_coef)
-        if self.sn:
-            with torch.no_grad():
-                cm.weight_u.copy_(u2)
-                cm.weight_v.copy_(v2)
-        return la, lc, logp.view(T, B, N), ent.view(T, B, N), val.view(T, B, N)
+        return feat_a, feat_c
 
     def gae(self, tb):
-        """GAE + advantage normalisation on a time-major TrainBatch (kernel 3b)."""
+        """GAE + advantage normalisation on a time-major TrainBatch (kernel 3b; marl_gae_boundary for a batch that crossed an
+        episode boundary)."""
         L = _lib.lib()
         import ctypes
         T, B, N = tb.T, tb.B, tb.N
         adv, vt = torch.empty_like(tb.r), torch.empty_like(tb.r)
         ws = torch.zeros(int(L.marl_gae_workspace_bytes(B, T, N)), dtype=torch.uint8, device=tb.r.device)
+        if tb.boundary is not None:     # a segment that crossed an episode boundary: the recursion restarts there
+            _lib.check(L.marl_gae_boundary(B, T, N, int(tb.boundary), _lib.ptr(tb.r), _lib.ptr(tb.v), _lib.ptr(tb.v_boot),
+                                           _lib.ptr(tb.active), ctypes.c_float(self.gamma), ctypes.c_float(self.gamma * self.lamda),
+                                           1 if self.use_adv_norm else 0, _lib.ptr(adv), _lib.ptr(vt), _lib.ptr(ws), _lib.stream_ptr()),
+                       "marl_gae_boundary")
+            return adv, vt
         _lib.check(L.marl_gae(B, T, N, _lib.ptr(tb.r), _lib.ptr(tb.v), _lib.ptr(tb.active), 1, ctypes.c_float(self.gamma),
                               ctypes.c_float(self.gamma * self.lamda), 1 if self.use_adv_norm else 0, _lib.ptr(adv),
                               _lib.ptr(vt), _lib.ptr(ws), _lib.stream_ptr()), "marl_gae")
@@ -814,7 +910,7 @@ class MAPPO:
 
     @torch.no_grad()
     def rollout_batched(self, engine, arena, T=None, seed=0, deterministic=False, use_fused=None, timers=None, pipelines=None,
-                        actor_only=False, history=None, carry=None, policy_dbg=None):
+                        actor_only=False, history=None, carry=None, policy_dbg=None, auto_reset=None):
         """MAPPO.run_episode (:742-827) for all B envs of a BatchedPursuitEnv at once, entirely on the GPU.
         Per step: observe kernel -> fused encoder (actor, then critic with all-ones adjacency) -> GRU cell -> heads ->
         closed-loop env kernel (evader move + pursuer step + reward-norm + store).  Fills `arena` plus the history /
@@ -846,10 +942,26 @@ class MAPPO:
         carry: None (a whole episode from the engine's state at step 0) or a RolloutCarry: one segment of T = S steps of an episode of
         cfg.env.max_steps steps (S divides it), starting at the episode's step carry.t0 from the carried hidden states and history.
         The history rule, the sampling RNG key and the A* replan schedule use the episode's step; the engine must be at carry.t0.
-        The batch records its start state (t0, h0_a / h0_c, the history prefix) and its `carry` is where the next segment starts."""
+        The batch records its start state (t0, h0_a / h0_c, the history prefix) and its `carry` is where the next segment starts.
+
+        auto_reset: None, or an AutoReset with a carry: the segment may be any 1 <= S <= cfg.env.max_steps steps from any step carry.t0 of
+        episode carry.episode, and when the episode ends inside it (at the segment's step k) the rollout bootstraps that episode, resets
+        the envs on the device and continues with the next episode (see AutoReset; the fused step only, seeds from the AutoReset).  A
+        batch that crosses the boundary has `boundary` = k, `v_boot` [B,N] (the finished episode's bootstrap value) and the two episodes'
+        map data, and trains as two pieces with their own start states (`TrainBatch.pieces`).  A segment that ends exactly at the
+        episode's end resets at its end.  Whenever the envs were reset, `ended_collision` / `ended_evader_status` [B] keep the finished
+        episode's flags that the reset clears, and the next carry starts episode carry.episode + 1."""
         B, N, E, D, L = engine.B, engine.N, self.embedding_dim, self.depth, self.num_layers
         dev = self.device
-        if carry is not None:
+        if auto_reset is not None:
+            T = arena.T if T is None else int(T)
+            fused_ok = use_fused is not False and fused_policy.supported(self)
+            check_auto_reset(auto_reset, carry, T, int(self.cfg.env.max_steps), B, N, L, E, D, dev, actor_only, fused_ok, seed)
+            if not bool((engine.time_step == carry.t0).all()):
+                raise _lib.MarlError(f"rollout segment from step {carry.t0}: the engine's envs are at steps "
+                                     f"{sorted(set(engine.time_step.tolist()))[:4]}")
+            seed = auto_reset.sample_seed(carry.episode)
+        elif carry is not None:
             T = arena.T if T is None else int(T)
             check_segment(carry, T, int(self.cfg.env.max_steps), B, N, L, E, D, dev, actor_only)
             if not torch.cuda.is_current_stream_capturing() and not bool((engine.time_step == carry.t0).all()):
@@ -896,9 +1008,9 @@ class MAPPO:
             rep_ = HistoryReplay(fused, oxy_i, o_count, self.reference_quirks, t0) if replay else None
             G = (1 if actor_only else int(pipelines) if pipelines is not None else 1 if timers is not None
                  else int(os.environ.get("MARL_PIPELINES") or self.default_pipelines(B, N)))
-            nxt = self._rollout_fused(engine, arena, T, seed, deterministic, G, fused, oxy_i, o_count, hist_a, hist_c, ha, hc, act, logp,
-                                      v, slot, carry, actor_only, timers, policy_dbg)
-            return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp, rep_, carry, nxt)
+            nxt, ended = self._rollout_fused(engine, arena, T, seed, deterministic, G, fused, oxy_i, o_count, hist_a, hist_c, ha, hc, act,
+                                             logp, v, slot, carry, actor_only, timers, policy_dbg, auto_reset, oxy, replay)
+            return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp, rep_, carry, nxt, ended)
 
         enc = self.actor.shared_net
         quirks = self.reference_quirks and not actor_only
@@ -943,20 +1055,24 @@ class MAPPO:
         return max(1, min(8, (B * N) // 8192))
 
     def _rollout_fused(self, engine, arena, T, seed, deterministic, G, fused, oxy_i, o_count, hist_a, hist_c, h0_a, h0_c, act, logp, v,
-                       slot, carry, actor_only, timers, policy_dbg):
+                       slot, carry, actor_only, timers, policy_dbg, auto_reset=None, oxy=None, replay=False):
         """The fused schedule of `rollout_batched`: G independent env-group pipelines, one stream (+ one A* side stream) each.  Each
-        group starts from its rows of the hidden states h0_a / h0_c [L, B*N, E] (one group steps them in place); returns the
-        RolloutCarry of the segment's end (None without a carry)."""
-        B, N, E, D = engine.B, engine.N, self.embedding_dim, self.depth
+        group starts from its rows of the hidden states h0_a / h0_c [L, B*N, E] (one group steps them in place).  Returns the
+        RolloutCarry of the segment's end (None without a carry) and, when auto_reset reset the envs during the segment, a namespace of
+        what the batch needs about the episode that ended (else None)."""
+        B, N, E, D, L = engine.B, engine.N, self.embedding_dim, self.depth, self.num_layers
         f32 = dict(dtype=torch.float32, device=self.device)
         quirks = self.reference_quirks and not actor_only
         nets = ("actor",) if actor_only else ("actor", "critic")
         t0 = 0 if carry is None else carry.t0
+        T_ep = int(self.cfg.env.max_steps)
+        # auto_reset: the episode ends after the segment's step k-1 when k = T_ep - t0 <= T; k < T crosses the boundary
+        k = T_ep - t0 if auto_reset is not None and t0 + T >= T_ep else None
         # The bootstrap value v[T] is a critic-only step at the episode's end.  A segment that ends inside the episode computes it with
         # the step of both networks instead (the actor's outputs are discarded): that is the kernel the next segment's first step runs
         # on the same state, and the critic-only kernel rounds the GRU cell and the value sum differently, so v[T] is then bit for bit
         # the value the next segment starts with.
-        pair_bootstrap = carry is not None and t0 + T < int(self.cfg.env.max_steps)
+        pair_bootstrap = carry is not None and t0 + T < T_ep
         if len(getattr(engine, "_pipe_streams", [])) < 2 * G:
             engine._pipe_streams = [torch.cuda.Stream(device=self.device) for _ in range(2 * G)]
         rec_ptrs = arena.record_pointers()
@@ -977,64 +1093,94 @@ class MAPPO:
             timers.setdefault(name, []).append((a_, b_))
 
         main = torch.cuda.current_stream()
-        fork = torch.cuda.Event()
-        fork.record(main)
         if carry is not None:           # every group writes its rows of the next carry's hidden states
             next_ha, next_hc = torch.empty_like(carry.ha), torch.empty_like(carry.hc)
-        for g in range(G):
-            lo, hi = g * B // G, (g + 1) * B // G
-            sl, rows = slice(lo, hi), slice(lo * N, hi * N)
-            st, side = engine._pipe_streams[2 * g], engine._pipe_streams[2 * g + 1]
-            st.wait_event(fork)
-            with torch.cuda.stream(st):
-                # what FusedRolloutStep.step reads from an engine, for envs [lo, hi) (views: the kernels update them in place)
-                view = SimpleNamespace(B=hi - lo, N=N, O=engine.O, p_state=engine.p_state[sl], e_state=engine.e_state[sl],
-                                       map_id=engine.map_id[sl], p_adj_bits=engine.p_adj_bits[sl], e_adj=engine.e_adj[sl],
-                                       o_adj_bits=engine.o_adj_bits[sl])
-                ha, hc = h0_a[:, rows].contiguous(), h0_c[:, rows].contiguous()
 
-                def hist_of(t, net):
-                    return _history_inputs(hist_a, hist_c, t, D, quirks, net, slot, sl, t0=t0)
-
-                for t in range(T):
-                    replan, join = (t0 + t) % diff == 0, None
-                    if replan and timers is None:
-                        ev = torch.cuda.Event()
-                        ev.record(st)
-                        side.wait_event(ev)
-                        engine.evader_replan(lo, hi, side)
-                        join = torch.cuda.Event()
-                        join.record(side)
-                    timed("env_observe_kernel", st, lambda: engine.observe(lo=lo, hi=hi))
-                    timed("policy_step_kernel", st, lambda: fused.step(
-                        view, oxy_i, o_count, t0 + t, seed, deterministic, hist_of(t, "actor"), hist_of(t, "critic"),
-                        hist_a[slot(t + D)][sl], hist_c[slot(t + D)][sl], ha, hc, act[t][sl], logp[t][sl], v[t][sl], nets=nets,
-                        row_offset=lo * N, tile_rows=tile, debug=None if policy_dbg is None else policy_dbg[t, g]))
-                    if join is not None:
-                        st.wait_event(join)
-                    elif replan:
-                        timed("evader_kernel(replan)", st, lambda: engine.evader_replan(lo, hi, st))
-                    timed("rollout_kernel(closed)", st, lambda: engine._closed_chunk(arena, rec_ptrs, lo, hi, t, 1, act[t:t + 1], 0, seed,
-                                                                                      st))
-                if not actor_only:
-                    engine.observe(lo=lo, hi=hi)
-                    h_fin = _bootstrap_history(hist_a, hist_c, T, D, quirks, slot, sl, t0)
-                    scratch = torch.empty(hi - lo, N, E, **f32)
-                    if carry is not None:   # before the bootstrap step, which updates the hidden states in place
-                        next_ha[:, rows].copy_(ha)
-                        next_hc[:, rows].copy_(hc)
-                    if pair_bootstrap:
-                        fused.step(view, oxy_i, o_count, t0 + T, seed, deterministic, hist_of(T, "actor"), h_fin, torch.empty_like(scratch),
-                                   scratch, ha, hc, torch.empty_like(act[0][sl]), torch.empty_like(logp[0][sl]), v[T][sl],
-                                   row_offset=lo * N, tile_rows=tile)
+        def pipelines(t_lo, t_hi, off, seed, oxy_i, o_count, v_end, pair, h0_a, h0_c, last):
+            """Segment steps [t_lo, t_hi) of one episode, at its steps t + off, then the bootstrap value after step t_hi - 1 into v_end;
+            forked from and joined back into the current stream.  h0_a / h0_c: the hidden states at t_lo (None: zeros).  last: the
+            piece that ends the segment (it writes the next carry's hidden states)."""
+            fork = torch.cuda.Event()
+            fork.record(main)
+            for g in range(G):
+                lo, hi = g * B // G, (g + 1) * B // G
+                sl, rows = slice(lo, hi), slice(lo * N, hi * N)
+                st, side = engine._pipe_streams[2 * g], engine._pipe_streams[2 * g + 1]
+                st.wait_event(fork)
+                with torch.cuda.stream(st):
+                    # what FusedRolloutStep.step reads from an engine, for envs [lo, hi) (views: the kernels update them in place)
+                    view = SimpleNamespace(B=hi - lo, N=N, O=engine.O, p_state=engine.p_state[sl], e_state=engine.e_state[sl],
+                                           map_id=engine.map_id[sl], p_adj_bits=engine.p_adj_bits[sl], e_adj=engine.e_adj[sl],
+                                           o_adj_bits=engine.o_adj_bits[sl])
+                    if h0_a is None:
+                        ha, hc = torch.zeros(L, (hi - lo) * N, E, **f32), torch.zeros(L, (hi - lo) * N, E, **f32)
                     else:
-                        fused.step(view, oxy_i, o_count, t0 + T, seed, deterministic, h_fin, h_fin, scratch, scratch, ha, hc, None, None,
-                                   v[T][sl], nets=("critic",), row_offset=lo * N, tile_rows=tile)
-                done = torch.cuda.Event()
-                done.record(st)
-            main.wait_event(done)
-        if carry is not None:
-            return self._next_carry(carry, T, hist_a, hist_c, slot, next_ha, next_hc)
+                        ha, hc = h0_a[:, rows].contiguous(), h0_c[:, rows].contiguous()
+
+                    def hist_of(t, net):
+                        return _history_inputs(hist_a, hist_c, t, D, quirks, net, slot, sl, t0=off)
+
+                    for t in range(t_lo, t_hi):
+                        replan, join = (off + t) % diff == 0, None
+                        if replan and timers is None:
+                            ev = torch.cuda.Event()
+                            ev.record(st)
+                            side.wait_event(ev)
+                            engine.evader_replan(lo, hi, side)
+                            join = torch.cuda.Event()
+                            join.record(side)
+                        timed("env_observe_kernel", st, lambda: engine.observe(lo=lo, hi=hi))
+                        timed("policy_step_kernel", st, lambda: fused.step(
+                            view, oxy_i, o_count, off + t, seed, deterministic, hist_of(t, "actor"), hist_of(t, "critic"),
+                            hist_a[slot(t + D)][sl], hist_c[slot(t + D)][sl], ha, hc, act[t][sl], logp[t][sl], v[t][sl], nets=nets,
+                            row_offset=lo * N, tile_rows=tile, debug=None if policy_dbg is None else policy_dbg[t, g]))
+                        if join is not None:
+                            st.wait_event(join)
+                        elif replan:
+                            timed("evader_kernel(replan)", st, lambda: engine.evader_replan(lo, hi, st))
+                        timed("rollout_kernel(closed)", st, lambda: engine._closed_chunk(arena, rec_ptrs, lo, hi, t, 1, act[t:t + 1], 0,
+                                                                                          seed, st))
+                    if not actor_only:
+                        engine.observe(lo=lo, hi=hi)
+                        h_fin = _bootstrap_history(hist_a, hist_c, t_hi, D, quirks, slot, sl, off)
+                        scratch = torch.empty(hi - lo, N, E, **f32)
+                        if carry is not None and last:  # before the bootstrap step, which updates the hidden states in place
+                            next_ha[:, rows].copy_(ha)
+                            next_hc[:, rows].copy_(hc)
+                        if pair:
+                            fused.step(view, oxy_i, o_count, off + t_hi, seed, deterministic, hist_of(t_hi, "actor"), h_fin,
+                                       torch.empty_like(scratch), scratch, ha, hc, torch.empty_like(act[0][sl]),
+                                       torch.empty_like(logp[0][sl]), v_end[sl], row_offset=lo * N, tile_rows=tile)
+                        else:
+                            fused.step(view, oxy_i, o_count, off + t_hi, seed, deterministic, h_fin, h_fin, scratch, scratch, ha, hc,
+                                       None, None, v_end[sl], nets=("critic",), row_offset=lo * N, tile_rows=tile)
+                    done = torch.cuda.Event()
+                    done.record(st)
+                main.wait_event(done)
+
+        if k is None:
+            pipelines(0, T, t0, seed, oxy_i, o_count, v[T], pair_bootstrap, h0_a, h0_c, True)
+            if carry is not None:
+                return self._next_carry(carry, T, hist_a, hist_c, slot, next_ha, next_hc), None
+            return None, None
+        # auto-reset: episode e ends after step k-1.  Its pipelines end with the whole-episode rollout's critic-only bootstrap step.
+        e = carry.episode
+        v_boot = v[T] if k == T else torch.empty(B, N, **f32)
+        pipelines(0, k, t0, seed, oxy_i, o_count, v_boot, False, h0_a, h0_c, k == T)
+        # All groups are joined: the maps and their sensor tables are shared by envs of different groups, and the reset regenerates
+        # them in place.  Keep what the reset clears or the batch's first piece still needs.
+        oxy_env, o_count_train = self._train_map_data(engine, oxy)
+        ended = SimpleNamespace(k=k, collision=engine.collision.clone(), evader_status=engine.evader_status.clone(), oxy=oxy_env,
+                                o_count_train=o_count_train)
+        engine.reset_device(seed=auto_reset.reset_seed(e + 1), tape_len=auto_reset.tape_len)
+        if k == T:
+            return RolloutCarry.zeros(self, B, N, episode=e + 1), ended
+        ended.v_boot = v_boot
+        oxy_i = engine.boundary_xy.clone() if replay else engine.boundary_xy.contiguous()
+        o_count = torch.clamp(engine.boundary_count, max=engine.O).contiguous()
+        ended.oxy_i, ended.o_count = oxy_i, o_count
+        pipelines(k, T, -k, auto_reset.sample_seed(e + 1), oxy_i, o_count, v[T], True, None, None, True)
+        return self._next_carry(carry, T, hist_a, hist_c, slot, next_ha, next_hc, start=k), ended
 
     def explore_batched(self, engine, arena, T=None, seed=0, host_state=None, host_out=None, reset_reward_norm=False, history=None,
                         carry=None):
@@ -1088,13 +1234,27 @@ class MAPPO:
                 raise _lib.MarlError(f"explore_batched: evader status {int(status)} (A* OPEN / path overflow or target tape exhausted)")
         return g.batch
 
-    def _next_carry(self, carry, T, hist_a, hist_c, slot, ha, hc):
-        """The carry after a segment of T steps: its hidden states and the embeddings of its history steps T..T+D-1."""
-        last = lambda h: torch.stack([h[slot(T + j)] for j in range(self.depth)])     # noqa: E731
-        return RolloutCarry(carry.t0 + T, ha, hc, last(hist_a), last(hist_c))
+    def _next_carry(self, carry, T, hist_a, hist_c, slot, ha, hc, start=None):
+        """The carry after a segment of T steps: its hidden states and the embeddings of its history steps T..T+D-1.  start: the
+        segment's step at which a new episode began (auto-reset); history steps before it are zeros in the carry."""
+        D = self.depth
+        if start is None:
+            last = lambda h: torch.stack([h[slot(T + j)] for j in range(D)])     # noqa: E731
+            return RolloutCarry(carry.t0 + T, ha, hc, last(hist_a), last(hist_c), episode=carry.episode)
+        last = lambda h: torch.stack([h[slot(T + j)] if T + j - D >= start else torch.zeros_like(h[0]) for j in range(D)])  # noqa: E731
+        return RolloutCarry(T - start, ha, hc, last(hist_a), last(hist_c), episode=carry.episode + 1)
 
-    def _train_batch(self, engine, arena, T, oxy, hist_a, hist_c, v, logp, replay=None, carry=None, next_carry=None):
-        B, D, dev = engine.B, self.depth, self.device
+    def _train_map_data(self, engine, oxy):
+        """Per-env obstacle cells [B,O,2] and the cell counts the training forward's critic uses, from the maps `oxy` [M,O,2] (f32)."""
+        oxy_env = oxy[engine.map_id.long()].contiguous()
+        if self.reference_quirks:      # the critic's all-ones adjacency spans all O padded slots in training (:65,677): 76 phantom cells at (0,0)
+            o_count_train = torch.full((engine.B,), engine.O, dtype=torch.int32, device=self.device)
+        else:                          # ... or the map's real boundary cells, as in the rollout
+            o_count_train = torch.clamp(engine.boundary_count, max=engine.O)[engine.map_id.long()].to(torch.int32).contiguous()
+        return oxy_env, o_count_train
+
+    def _train_batch(self, engine, arena, T, oxy, hist_a, hist_c, v, logp, replay=None, carry=None, next_carry=None, ended=None):
+        D = self.depth
         seg = {}
         if carry is not None:
             seg = dict(t0=carry.t0, h0_a=carry.ha, h0_c=carry.hc, carry=next_carry)
@@ -1102,11 +1262,16 @@ class MAPPO:
                 seg.update(prefix_a=carry.emb_a, prefix_c=carry.emb_c)
         if replay is not None:         # the ring holds the last D+1 steps only: the history is regenerated per minibatch
             hist_a = hist_c = None
-        oxy_env = oxy[engine.map_id.long()].contiguous()
-        if self.reference_quirks:      # the critic's all-ones adjacency spans all O padded slots in training (:65,677): 76 phantom cells at (0,0)
-            o_count_train = torch.full((B,), engine.O, dtype=torch.int32, device=dev)
-        else:                          # ... or the map's real boundary cells, as in the rollout
-            o_count_train = torch.clamp(engine.boundary_count, max=engine.O)[engine.map_id.long()].to(torch.int32).contiguous()
+        if ended is None:
+            oxy_env, o_count_train = self._train_map_data(engine, oxy)
+        else:                          # the envs were reset during the segment: the maps of the episode that ended
+            oxy_env, o_count_train = ended.oxy, ended.o_count_train
+            seg.update(ended_collision=ended.collision, ended_evader_status=ended.evader_status)
+            if ended.k < T:            # the segment's second piece: the next episode's start, on the new maps
+                oxy2, o_count_train2 = self._train_map_data(engine, engine.boundary_xy.to(torch.float32).contiguous())
+                seg.update(boundary=ended.k, v_boot=ended.v_boot, oxy2=oxy2, o_count_train2=o_count_train2)
+                if replay is not None:
+                    seg["replay2"] = HistoryReplay(replay.fused, ended.oxy_i, ended.o_count, replay.quirks)
         return TrainBatch(p=arena.p_state_f32[:T], e=arena.e_state_f32[:T, :, 0].contiguous(), oxy=oxy_env,
                           o_count_train=o_count_train,
                           p_adj_bits=arena.p_adj_bits[:T], e_adj=arena.e_adj[:T], o_adj_bits=arena.o_adj_bits[:T],

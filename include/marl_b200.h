@@ -169,6 +169,14 @@ int64_t marl_gae_workspace_bytes(int32_t B, int32_t T, int32_t N);
 int marl_gae(int32_t B, int32_t T, int32_t N, const float *d_r, const float *d_v, const float *d_active,
              int32_t time_major, float gamma, float gamma_lamda, int32_t use_adv_norm, float *d_adv,
              float *d_v_target, void *d_workspace, void *stream);
+/* GAE of a time-major rollout segment that crosses an episode boundary: r, active, adv, v_target [T,B,N], v [T+1,B,N],
+ * v_boot [B,N], 0 < k < T.  Steps k..T-1 (the next episode's start) are marl_gae on those steps with v[k..T]; steps 0..k-1 (the
+ * previous episode's end) are marl_gae on those steps bootstrapped with v_boot, that episode's value after its last step, in place of
+ * v[k]: the recursion does not cross k.  Advantage normalisation (use_adv_norm) runs over all T*B*N samples with marl_gae's
+ * fixed-order reduction.  d_workspace: >= marl_gae_workspace_bytes(B,T,N) bytes. */
+int marl_gae_boundary(int32_t B, int32_t T, int32_t N, int32_t k, const float *d_r, const float *d_v, const float *d_v_boot,
+                      const float *d_active, float gamma, float gamma_lamda, int32_t use_adv_norm, float *d_adv,
+                      float *d_v_target, void *d_workspace, void *stream);
 
 /* ---- kernel 4: minibatch gather ------------------------------------------------------------------
  * Replaces `batch[key][index]` (DHGN/mappo_parallel.py:665-679): copies rows d_index[i] (i < n_index) of a

@@ -18,7 +18,14 @@ epoch and update on it; the GRU hidden states and the history embeddings carry o
 are reset only at episode starts.  The episode reward is printed on the iteration that ends an episode ("-" on the others), and
 --save-dir / --resume work at any segment boundary.
 
-    python tools/train_loop.py --envs 512 --steps 150 --segment 50 --iters 6      # two episodes, three updates each"""
+    python tools/train_loop.py --envs 512 --steps 150 --segment 50 --iters 6      # two episodes, three updates each
+
+--auto-reset lets the segments run across episode boundaries (MAPPO.rollout_batched(auto_reset=...)): --segment may then be any
+1 <= S <= --steps, and the rollout resets the envs on the device itself when an episode ends inside a segment.  The episodes and their
+seeds are the ones the loop uses without it, so for an S that divides --steps both print the same exact columns.  The iteration that
+finishes an episode prints its reward.
+
+    python tools/train_loop.py --envs 512 --steps 150 --segment 64 --auto-reset --iters 7"""
 import argparse
 import os
 import sys
@@ -31,7 +38,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from distributed_multi_agent_reinforcement_learning_b200 import default_config, parallel  # noqa: E402
 from distributed_multi_agent_reinforcement_learning_b200.checkpoint import load_training_state, save_training_state  # noqa: E402
-from distributed_multi_agent_reinforcement_learning_b200.mappo_parallel import MAPPO, RolloutCarry  # noqa: E402
+from distributed_multi_agent_reinforcement_learning_b200.mappo_parallel import MAPPO, AutoReset, RolloutCarry  # noqa: E402
 from distributed_multi_agent_reinforcement_learning_b200.pursuit_env import BatchedPursuitEnv, RolloutArena  # noqa: E402
 
 
@@ -42,6 +49,8 @@ def main():
     ap.add_argument("--pursuers", type=int, default=8)
     ap.add_argument("--steps", type=int, default=150)
     ap.add_argument("--segment", type=int, default=None, help="env steps per iteration, a divisor of --steps (default: --steps)")
+    ap.add_argument("--auto-reset", action="store_true",
+                    help="segments may cross episode boundaries: any --segment in [1, --steps], envs reset inside the rollout")
     ap.add_argument("--iters", type=int, default=10)
     ap.add_argument("--depth", type=int, default=1)
     ap.add_argument("--allreduce", default=None, choices=[None, "update", "minibatch"],
@@ -54,7 +63,12 @@ def main():
     if args.save_every < 1:
         ap.error("--save-every must be >= 1")
     S = args.steps if args.segment is None else args.segment
-    if S < 1 or args.steps % S:
+    if args.auto_reset:
+        if args.host_reset:
+            ap.error("--auto-reset resets the envs on the device; it does not combine with --host-reset")
+        if S < 1 or S > args.steps:
+            ap.error(f"--segment {S} must lie in [1, --steps {args.steps}] with --auto-reset")
+    elif S < 1 or args.steps % S:
         ap.error(f"--segment {S} must be a positive divisor of --steps {args.steps}")
     n_seg = args.steps // S
     rank, world, local = (int(os.environ.get(k, d)) for k, d in (("RANK", 0), ("WORLD_SIZE", 1), ("LOCAL_RANK", 0)))
@@ -75,6 +89,8 @@ def main():
     carry = RolloutCarry.zeros(mappo, B, N) if n_seg > 1 else None     # where the next segment of the current episode starts
     ep_sum = torch.zeros(B, dtype=torch.int64, device=dev)              # raw reward of the current episode so far, per env
     state_file = lambda d: os.path.join(d, f"training_state_rank{rank}.pt")     # noqa: E731  (env shards and reward statistics are per rank)
+    if args.auto_reset:
+        return auto_reset_loop(args, rank, world, dev, cfg, env, arena, mappo, state_file)
     if args.resume:
         extra = load_training_state(state_file(args.resume), mappo, env, carry=carry)
         start, total_steps = int(extra["next_iter"]), int(extra["total_steps"])
@@ -132,6 +148,66 @@ def main():
             rew, rew_hex = (f"{s[0]:9.2f}", s[0].hex()) if ep_end else (f"{'-':>9}", "-")
             print(f"iter {it:3d}  steps {total_steps:9d}  ep_reward {rew}  collided {s[1]:5.2f}  objC {s[2]:8.4f}  "
                   f"objA {s[3]:8.4f}  reset {t1 - t0:5.2f}s  rollout {1e3 * (t2 - t1):7.1f}ms  train {1e3 * (t3 - t2):7.1f}ms  "
+                  f"exact {it} {total_steps} {rew_hex} {s[2].hex()} {s[3].hex()}", flush=True)
+    if world > 1:
+        torch.distributed.destroy_process_group()
+
+
+def auto_reset_loop(args, rank, world, dev, cfg, env, arena, mappo, state_file):
+    """The loop of --auto-reset: one segment of S steps per iteration, episode e reset on the device with seed 1000*rank + e and sampled
+    with seed e*world + rank (the seeds of the loop without --auto-reset), the resets inside the rollout."""
+    B, N, S, T_ep = args.envs, args.pursuers, args.segment or args.steps, args.steps
+    auto = AutoReset(reset_seed=lambda e: 1000 * rank + e, sample_seed=lambda e: e * world + rank)
+    carry = RolloutCarry.zeros(mappo, B, N)
+    ep_sum = torch.zeros(B, dtype=torch.int64, device=dev)
+    total_steps, start = 0, 0
+    if args.resume:
+        extra = load_training_state(state_file(args.resume), mappo, env, carry=carry)
+        start, total_steps = int(extra["next_iter"]), int(extra["total_steps"])
+        ep_sum = extra["ep_reward_so_far"].to(dev)
+        if divmod(start * S, T_ep) != (carry.episode, carry.t0):
+            raise SystemExit(f"--resume: the file continues at step {carry.t0} of episode {carry.episode}, iteration {start} of "
+                             f"--segment {S} starts at step {start * S % T_ep} of episode {start * S // T_ep}")
+    else:
+        env.reset_device(seed=auto.reset_seed(0), tape_len=auto.tape_len)
+        torch.cuda.synchronize()
+        assert int(env.reset_fail.sum()) == 0, "device reset could not place every pursuer / evader"
+    for it in range(start, args.iters):
+        t1 = time.perf_counter()
+        tb = mappo.rollout_batched(env, arena, S, carry=carry, auto_reset=auto)
+        torch.cuda.synchronize()
+        t2 = time.perf_counter()
+        assert int(env.evader_status.max()) == 0, "evader search overflow / target tape exhausted"
+        ep_end = tb.ended_collision is not None     # an episode ended inside or at the end of this segment and the envs were reset
+        k = S if tb.boundary is None else tb.boundary
+        ep_sum += arena.raw_reward[:k].sum(dim=(0, 2))
+        ep_reward = float(ep_sum.float().mean())
+        if ep_end:
+            assert int(tb.ended_evader_status.max()) == 0, "evader search overflow / target tape exhausted"
+            assert int(env.reset_fail.sum()) == 0, "device reset could not place every pursuer / evader"
+            collided = float(tb.ended_collision.float().mean())
+            ep_sum = arena.raw_reward[k:S].sum(dim=(0, 2))
+        else:
+            collided = float(env.collision.float().mean())
+        total_steps += world * B * S
+        carry = tb.carry
+        for _ in range(int(cfg.algo.epochs)):
+            obj_c, obj_a, _, _ = mappo.train(tb, total_steps, return_numpy=False, allreduce=args.allreduce)
+            mappo.update(total_steps)
+        torch.cuda.synchronize()
+        t3 = time.perf_counter()
+        stats = torch.tensor([ep_reward, collided, obj_c, obj_a], device=dev, dtype=torch.float64)
+        if world > 1:
+            torch.distributed.all_reduce(stats)
+            stats /= world
+        if args.save_dir and ((it + 1) % args.save_every == 0 or it + 1 == args.iters):
+            save_training_state(state_file(args.save_dir), mappo, env, extra=dict(next_iter=it + 1, total_steps=total_steps,
+                                                                                  ep_reward_so_far=ep_sum.cpu()), carry=carry)
+        if rank == 0:
+            s = [float(x) for x in stats.cpu()]
+            rew, rew_hex = (f"{s[0]:9.2f}", s[0].hex()) if ep_end else (f"{'-':>9}", "-")
+            print(f"iter {it:3d}  steps {total_steps:9d}  ep_reward {rew}  collided {s[1]:5.2f}  objC {s[2]:8.4f}  "
+                  f"objA {s[3]:8.4f}  reset {0.0:5.2f}s  rollout {1e3 * (t2 - t1):7.1f}ms  train {1e3 * (t3 - t2):7.1f}ms  "
                   f"exact {it} {total_steps} {rew_hex} {s[2].hex()} {s[3].hex()}", flush=True)
     if world > 1:
         torch.distributed.destroy_process_group()
