@@ -88,6 +88,7 @@ _PROTOTYPES = {
     "marl_policy_pack_bytes": (_I64, [_I32, _I32]),
     "marl_policy_pack": (C.c_int, [_VP, _I32, _I32, _I32, _VP, _VP]),
     "marl_policy_rollout_step": (C.c_int, [_VP] * 6),
+    "marl_policy_rollout_step_dseed": (C.c_int, [_VP] * 7),
     "marl_entity_agg_fwd": (C.c_int, [_I64, _I32, _I32, _I32, _I32, _VP, _I32, _VP, _I64, _I64, _I64, _VP, _VP]),
     "marl_entity_agg_bwd": (C.c_int, [_I64, _I32, _I32, _VP, _I32, _VP, _VP, _VP]),
     "marl_gru_pack_bytes": (_I64, []),
@@ -104,6 +105,9 @@ _PROTOTYPES = {
     "marl_rowgemm_tf32x3": (C.c_int, [_I64, _I32, _I32, _I32, _VP, _I64, _VP, _I64, _VP, _VP, _VP, _I64, _VP, _I64, _I32, _VP]),
     "marl_map_generate": (C.c_int, [_PP, _I32, _I32, C.c_double, C.c_double, C.c_double, _U64, _VP, _VP, _VP]),
     "marl_env_reset_place": (C.c_int, [_PP, _I32, _I32, _VP, _VP, _U64, C.c_double, _I32, _I32, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "marl_map_generate_dseed": (C.c_int, [_PP, _I32, _I32, C.c_double, C.c_double, C.c_double, _VP, _VP, _VP, _VP]),
+    "marl_env_reset_place_dseed": (C.c_int, [_PP, _I32, _I32, _VP, _VP, _VP, C.c_double, _I32, _I32, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "marl_target_tape_generate": (C.c_int, [_PP, _I32, _I32, _VP, _VP, _VP]),
     "marl_clip_workspace_bytes": (_I64, [_I64]),
     "marl_clip_grad_norm": (C.c_int, [_I64, _VP, _F32, _VP, _VP, _VP]),
     "marl_adam_step": (C.c_int, [_I64, _VP, _VP, _VP, _VP, _F32, _F32, _F32, _F32, _I64, _VP]),
@@ -180,6 +184,13 @@ def stream_ptr(stream=None):
     import torch
     s = stream if stream is not None else torch.cuda.current_stream()
     return s.cuda_stream
+
+
+def u64_bits(v):
+    """The int64 whose bit pattern is the u64 `int(v) & (2**64 - 1)`: what an int64 device word holds for a seed the kernels read as
+    uint64_t (the value a by-value call passes through ctypes.c_uint64)."""
+    v = int(v) & 0xFFFFFFFFFFFFFFFF
+    return v - (1 << 64) if v >= (1 << 63) else v
 
 
 def ptr_or_int(v):

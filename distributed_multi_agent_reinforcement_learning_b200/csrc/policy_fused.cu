@@ -94,6 +94,7 @@ struct StepArgs {
     int32_t *action;
     float *logp, *value;
     uint64_t seed;
+    const uint64_t *d_seed;   // non-null: the sampling seed is read from this device word when the kernel runs (seed is ignored)
     int t, deterministic, force_action, net_first, net_count;
     int64_t row_offset;   // RNG key offset of row 0 (sub-batch launches)
     long long *dbg;   // optional [grid,16] per-CTA phase cycle counters (profiling aid)
@@ -945,7 +946,8 @@ __device__ void epi_head(const Ctx &c)
 #pragma unroll
         for (int k = 0; k < A; ++k) if (sm[k] > best) { best = sm[k]; act = k; }
     } else {
-        const uint64_t hsh = splitmix64(c.a->seed ^ splitmix64((uint64_t)(gr + c.a->row_offset) * 0x100000001B3ull + (uint64_t)c.a->t));
+        const uint64_t seed = c.a->d_seed ? *c.a->d_seed : c.a->seed;
+        const uint64_t hsh = splitmix64(seed ^ splitmix64((uint64_t)(gr + c.a->row_offset) * 0x100000001B3ull + (uint64_t)c.a->t));
         const float u = (float)(hsh >> 40) * (1.0f / 16777216.0f) * psum;
         float cs = 0.f;
         act = A - 1;
@@ -1874,8 +1876,8 @@ static int fill_net(pf::NetArgs &na, const marl_dhgn_weights *w, const marl_poli
     return MARL_OK;
 }
 
-extern "C" int marl_policy_rollout_step(const marl_policy_step *s, const marl_dhgn_weights *actor_w, const marl_policy_net_io *actor_io,
-                                        const marl_dhgn_weights *critic_w, const marl_policy_net_io *critic_io, void *stream)
+static int policy_rollout_step(const marl_policy_step *s, const marl_dhgn_weights *actor_w, const marl_policy_net_io *actor_io,
+                               const marl_dhgn_weights *critic_w, const marl_policy_net_io *critic_io, const uint64_t *d_seed, void *stream)
 {
     MARL_REQUIRE(s != nullptr, "marl_policy_rollout_step: step struct is NULL");
     MARL_REQUIRE(s->E == pf::E, "marl_policy_rollout_step: embedding_dim=%d (the fused kernel is built for 128)", s->E);
@@ -1902,7 +1904,7 @@ extern "C" int marl_policy_rollout_step(const marl_policy_step *s, const marl_dh
     a.n_tiles = (int)((a.R + a.rows_per_tile - 1) / a.rows_per_tile);
     a.p_state = s->d_p_state; a.e_state = s->d_e_state; a.oxy = s->d_oxy; a.map_id = s->d_map_id; a.o_count = s->d_o_count;
     a.p_adj = s->d_p_adj_bits; a.e_adj = s->d_e_adj; a.o_adj = s->d_o_adj_bits;
-    a.action = s->d_action; a.logp = s->d_logp; a.value = s->d_value; a.seed = s->seed; a.t = s->t; a.deterministic = s->deterministic; a.force_action = s->force_action;
+    a.action = s->d_action; a.logp = s->d_logp; a.value = s->d_value; a.seed = s->seed; a.d_seed = d_seed; a.t = s->t; a.deterministic = s->deterministic; a.force_action = s->force_action;
     a.row_offset = s->row_offset;
     a.dbg = static_cast<long long *>(s->d_debug);
     int rc;
@@ -1939,4 +1941,18 @@ extern "C" int marl_policy_rollout_step(const marl_policy_step *s, const marl_dh
     }
     if (rc) return rc;
     return check_launch("policy_step_kernel");
+}
+
+extern "C" int marl_policy_rollout_step(const marl_policy_step *s, const marl_dhgn_weights *actor_w, const marl_policy_net_io *actor_io,
+                                        const marl_dhgn_weights *critic_w, const marl_policy_net_io *critic_io, void *stream)
+{
+    return policy_rollout_step(s, actor_w, actor_io, critic_w, critic_io, nullptr, stream);
+}
+
+extern "C" int marl_policy_rollout_step_dseed(const marl_policy_step *s, const marl_dhgn_weights *actor_w, const marl_policy_net_io *actor_io,
+                                              const marl_dhgn_weights *critic_w, const marl_policy_net_io *critic_io, const uint64_t *d_seed,
+                                              void *stream)
+{
+    MARL_REQUIRE(d_seed != nullptr, "marl_policy_rollout_step_dseed: d_seed is NULL");
+    return policy_rollout_step(s, actor_w, actor_io, critic_w, critic_io, d_seed, stream);
 }

@@ -5,7 +5,8 @@
 // own counter-based stream (splitmix64 of (seed, env, draw index)), so results are rule-equivalent and distribution-equivalent to
 // the reference, not stream-equivalent (the reference's interpreter-global Mersenne-Twister streams are inherently serial).
 // Rejection sampling is sequential per env and cheap: one thread per env / per map; the work bitmap lives in a global scratch
-// row.  The per-map sensor tables are then built by marl_raser_map_build.
+// row.  The per-map sensor tables are then built by marl_raser_map_build.  The *_dseed entry points and the target-tape draw read the
+// seed from a device word when the kernel runs, so a CUDA graph that captures a reset follows that word.
 #include "common.cuh"
 
 namespace marl {
@@ -30,11 +31,12 @@ __device__ __forceinline__ void bit_set(uint32_t *bits, int HW, int x, int y) { 
 
 // base_env.py:37-50 + Occupied_Grid_Map.py:46-62: blocks of x,y in [-3,3) around N(center, variance); then the 2-cell inflation
 __global__ void __launch_bounds__(64)
-map_generate_kernel(EnvDev c, int M, int num_blocks, double cx, double cy, double sigma, uint64_t seed, uint32_t *__restrict__ grid_bits,
-                    uint32_t *__restrict__ inflated_bits)
+map_generate_kernel(EnvDev c, int M, int num_blocks, double cx, double cy, double sigma, uint64_t seed, const uint64_t *__restrict__ d_seed,
+                    uint32_t *__restrict__ grid_bits, uint32_t *__restrict__ inflated_bits)
 {
     const int m = blockIdx.x * 64 + threadIdx.x;
     if (m >= M) return;
+    if (d_seed) seed = *d_seed;      // device-seeded launch (graph-capturable: the seed is read when the kernel runs)
     uint32_t *g = grid_bits + (size_t)m * c.W * c.HW, *inf = inflated_bits + (size_t)m * c.W * c.HW;
     for (int i = 0; i < c.W * c.HW; ++i) { g[i] = 0u; inf[i] = 0u; }
     Stream64 rng{splitmix64(seed ^ 0x6d61707300000000ull) ^ splitmix64((uint64_t)m), 0};
@@ -59,11 +61,12 @@ map_generate_kernel(EnvDev c, int M, int num_blocks, double cx, double cy, doubl
 // base_env.py:52-152 for one env per thread
 __global__ void __launch_bounds__(64)
 reset_place_kernel(EnvDev c, int B, const uint32_t *__restrict__ inflated_bits, const int32_t *__restrict__ map_id, uint64_t seed,
-                   double min_dist, int extend, double comm_range, double sen_range, int max_draws, double *__restrict__ p_state,
+                   const uint64_t *__restrict__ d_seed, double min_dist, int extend, double comm_range, double sen_range, int max_draws, double *__restrict__ p_state,
                    double *__restrict__ e_state, int32_t *__restrict__ target, uint32_t *__restrict__ scratch, int32_t *__restrict__ fail)
 {
     const int b = blockIdx.x * 64 + threadIdx.x;
     if (b >= B) return;
+    if (d_seed) seed = *d_seed;
     const int m = map_id ? map_id[b] : b;
     const uint32_t *inf = inflated_bits + (size_t)m * c.W * c.HW;
     uint32_t *work = scratch + (size_t)b * c.W * c.HW;
@@ -118,31 +121,89 @@ reset_place_kernel(EnvDev c, int B, const uint32_t *__restrict__ inflated_bits, 
     if (fail) fail[b] = failed;
 }
 
+// candidate-target tape of the mid-episode init_target (base_env.py:52-70): tape[b, l] = (randint(0, W-1), randint(0, H-1)), the
+// distribution of the torch draw in BatchedPursuitEnv.reset_device, from env b's own stream of (seed, b)
+__global__ void __launch_bounds__(64)
+target_tape_kernel(int B, int L, int W, int H, const uint64_t *__restrict__ d_seed, int32_t *__restrict__ tape)
+{
+    const int b = blockIdx.x * 64 + threadIdx.x;
+    if (b >= B) return;
+    Stream64 rng{splitmix64(*d_seed ^ 0x7461706500000000ull) ^ splitmix64((uint64_t)b), 0};
+    int32_t *row = tape + (size_t)b * L * 2;
+    for (int l = 0; l < L; ++l) {
+        row[2 * l] = rng.randint(0, W - 1);
+        row[2 * l + 1] = rng.randint(0, H - 1);
+    }
+}
+
 }  // namespace marl
 
 using namespace marl;
 
-extern "C" int marl_map_generate(const marl_env_params *p, int32_t M, int32_t num_blocks, double center_x, double center_y, double variance,
-                                 uint64_t seed, uint32_t *d_grid_bits, uint32_t *d_inflated_bits, void *stream)
+static int map_generate(const marl_env_params *p, int32_t M, int32_t num_blocks, double center_x, double center_y, double variance,
+                        uint64_t seed, const uint64_t *d_seed, uint32_t *d_grid_bits, uint32_t *d_inflated_bits, void *stream)
 {
     EnvDev c;
     int rc = make_env_dev(p, &c);
     if (rc) return rc;
     MARL_REQUIRE(M > 0 && num_blocks >= 0 && variance >= 0 && d_grid_bits && d_inflated_bits, "marl_map_generate: bad arguments");
-    map_generate_kernel<<<(M + 63) / 64, 64, 0, (cudaStream_t)stream>>>(c, M, num_blocks, center_x, center_y, variance, seed, d_grid_bits, d_inflated_bits);
+    map_generate_kernel<<<(M + 63) / 64, 64, 0, (cudaStream_t)stream>>>(c, M, num_blocks, center_x, center_y, variance, seed, d_seed, d_grid_bits,
+                                                                      d_inflated_bits);
     return check_launch("map_generate_kernel");
 }
 
-extern "C" int marl_env_reset_place(const marl_env_params *p, int32_t B, int32_t M, const uint32_t *d_inflated_bits, const int32_t *d_map_id,
-                                    uint64_t seed, double min_dist, int32_t extend, int32_t max_draws, double *d_p_state, double *d_e_state,
-                                    int32_t *d_target, uint32_t *d_scratch, int32_t *d_fail, void *stream)
+static int env_reset_place(const marl_env_params *p, int32_t B, int32_t M, const uint32_t *d_inflated_bits, const int32_t *d_map_id,
+                           uint64_t seed, const uint64_t *d_seed, double min_dist, int32_t extend, int32_t max_draws, double *d_p_state,
+                           double *d_e_state, int32_t *d_target, uint32_t *d_scratch, int32_t *d_fail, void *stream)
 {
     EnvDev c;
     int rc = make_env_dev(p, &c);
     if (rc) return rc;
     MARL_REQUIRE(B > 0 && M > 0 && d_inflated_bits && d_p_state && d_e_state && d_target && d_scratch && max_draws > 0 && extend >= 0 && min_dist >= 0,
                  "marl_env_reset_place: bad arguments");
-    reset_place_kernel<<<(B + 63) / 64, 64, 0, (cudaStream_t)stream>>>(c, B, d_inflated_bits, d_map_id, seed, min_dist, extend, p->d_comm_range,
-                                                                      p->d_sen_range, max_draws, d_p_state, d_e_state, d_target, d_scratch, d_fail);
+    reset_place_kernel<<<(B + 63) / 64, 64, 0, (cudaStream_t)stream>>>(c, B, d_inflated_bits, d_map_id, seed, d_seed, min_dist, extend,
+                                                                      p->d_comm_range, p->d_sen_range, max_draws, d_p_state, d_e_state, d_target,
+                                                                      d_scratch, d_fail);
     return check_launch("reset_place_kernel");
+}
+
+extern "C" int marl_map_generate(const marl_env_params *p, int32_t M, int32_t num_blocks, double center_x, double center_y, double variance,
+                                 uint64_t seed, uint32_t *d_grid_bits, uint32_t *d_inflated_bits, void *stream)
+{
+    return map_generate(p, M, num_blocks, center_x, center_y, variance, seed, nullptr, d_grid_bits, d_inflated_bits, stream);
+}
+
+extern "C" int marl_map_generate_dseed(const marl_env_params *p, int32_t M, int32_t num_blocks, double center_x, double center_y,
+                                       double variance, const uint64_t *d_seed, uint32_t *d_grid_bits, uint32_t *d_inflated_bits, void *stream)
+{
+    MARL_REQUIRE(d_seed != nullptr, "marl_map_generate_dseed: d_seed is NULL");
+    return map_generate(p, M, num_blocks, center_x, center_y, variance, 0, d_seed, d_grid_bits, d_inflated_bits, stream);
+}
+
+extern "C" int marl_env_reset_place(const marl_env_params *p, int32_t B, int32_t M, const uint32_t *d_inflated_bits, const int32_t *d_map_id,
+                                    uint64_t seed, double min_dist, int32_t extend, int32_t max_draws, double *d_p_state, double *d_e_state,
+                                    int32_t *d_target, uint32_t *d_scratch, int32_t *d_fail, void *stream)
+{
+    return env_reset_place(p, B, M, d_inflated_bits, d_map_id, seed, nullptr, min_dist, extend, max_draws, d_p_state, d_e_state, d_target,
+                           d_scratch, d_fail, stream);
+}
+
+extern "C" int marl_env_reset_place_dseed(const marl_env_params *p, int32_t B, int32_t M, const uint32_t *d_inflated_bits,
+                                          const int32_t *d_map_id, const uint64_t *d_seed, double min_dist, int32_t extend, int32_t max_draws,
+                                          double *d_p_state, double *d_e_state, int32_t *d_target, uint32_t *d_scratch, int32_t *d_fail,
+                                          void *stream)
+{
+    MARL_REQUIRE(d_seed != nullptr, "marl_env_reset_place_dseed: d_seed is NULL");
+    return env_reset_place(p, B, M, d_inflated_bits, d_map_id, 0, d_seed, min_dist, extend, max_draws, d_p_state, d_e_state, d_target,
+                           d_scratch, d_fail, stream);
+}
+
+extern "C" int marl_target_tape_generate(const marl_env_params *p, int32_t B, int32_t L, const uint64_t *d_seed, int32_t *d_tape, void *stream)
+{
+    EnvDev c;
+    int rc = make_env_dev(p, &c);
+    if (rc) return rc;
+    MARL_REQUIRE(B > 0 && L > 0 && d_seed && d_tape, "marl_target_tape_generate: bad arguments (B=%d L=%d)", B, L);
+    target_tape_kernel<<<(B + 63) / 64, 64, 0, (cudaStream_t)stream>>>(B, L, c.W, c.H, d_seed, d_tape);
+    return check_launch("target_tape_kernel");
 }

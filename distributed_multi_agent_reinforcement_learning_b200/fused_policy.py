@@ -97,11 +97,13 @@ class FusedRolloutStep:
             keep.append(buf)
 
     def step(self, engine, oxy_i32, o_count, t, seed, deterministic, hist_a, hist_c, emb_a, emb_c, ha, hc, action, logp, value,
-             nets=("actor", "critic"), force_action=False, debug=None, variant=0, row_offset=0, tile_rows=0, flags=0):
+             nets=("actor", "critic"), force_action=False, debug=None, variant=0, row_offset=0, tile_rows=0, flags=0, d_seed=None):
         """hist_*: list (k = 0 newest) of [B,N,E] tensors or None (zeros); emb_*: [B,N,E] outputs; ha/hc: [2,B*N,E] in/out;
         action i32 [B,N], logp / value f32 [B,N] outputs.
         flags: STATE_F32 (engine.p_state / e_state are the fp32 records [B,N,4] / [B,4]) | EMBED_ONLY (ha / hc / action / logp /
         value may be None and are not touched).
+        d_seed: None, or a one-element int64 device tensor holding the sampling seed's u64 bit pattern, read when the kernel runs
+        (marl_policy_rollout_step_dseed: a captured step follows the word; `seed` is then ignored).
         variant: 0 = choose (3 when both networks are stepped, else 1), 1 = one (tile, network) item per CTA, 3 = both
         networks' chains of a tile interleaved in one CTA (needs both networks).  The hidden states are updated in place."""
         s = PolicyStep()
@@ -131,5 +133,9 @@ class FusedRolloutStep:
             ios[name] = io
         a_w, a_io = (C.byref(self.w["actor"]), C.byref(ios["actor"])) if "actor" in ios else (None, None)
         c_w, c_io = (C.byref(self.w["critic"]), C.byref(ios["critic"])) if "critic" in ios else (None, None)
-        _lib.check(self.lib.marl_policy_rollout_step(C.byref(s), a_w, a_io, c_w, c_io, _lib.stream_ptr()),
-                   "marl_policy_rollout_step")
+        if d_seed is None:
+            _lib.check(self.lib.marl_policy_rollout_step(C.byref(s), a_w, a_io, c_w, c_io, _lib.stream_ptr()),
+                       "marl_policy_rollout_step")
+        else:
+            _lib.check(self.lib.marl_policy_rollout_step_dseed(C.byref(s), a_w, a_io, c_w, c_io, _lib.ptr(d_seed), _lib.stream_ptr()),
+                       "marl_policy_rollout_step_dseed")

@@ -137,10 +137,13 @@ class AutoReset:
     with episode e + 1.  The actions of episode e are sampled with seed `sample_seed(e)` (keyed by row and the episode's step, as in a
     whole-episode rollout), so a stream of segments collects the episodes that `reset_device(reset_seed(e))` followed by
     `rollout_batched(max_steps, seed=sample_seed(e))` collects, bit for bit.  reset_seed / sample_seed: host callables, episode
-    index -> int."""
+    index -> int.  tape: the target tape's draw, as in `reset_device` - "torch" (a torch.Generator) or "device"
+    (marl_target_tape_generate), which `explore_batched` needs to replay the reset from a CUDA graph."""
 
-    def __init__(self, reset_seed, sample_seed, tape_len=16):
-        self.reset_seed, self.sample_seed, self.tape_len = reset_seed, sample_seed, int(tape_len)
+    def __init__(self, reset_seed, sample_seed, tape_len=16, tape="torch"):
+        if tape not in ("torch", "device"):
+            raise ValueError(f"AutoReset: tape={tape!r}, 'torch' or 'device'")
+        self.reset_seed, self.sample_seed, self.tape_len, self.tape = reset_seed, sample_seed, int(tape_len), tape
 
 
 def check_auto_reset(auto_reset, carry, S, T_ep, B, N, L, E, D, device, actor_only=False, use_fused=True, seed=0):
@@ -664,6 +667,65 @@ class RolloutGraph:
         self.graph.replay()
 
 
+class AutoResetStream:
+    """The CUDA graphs of one auto-reset segment stream of `explore_batched`: one graph per segment start t0 (a stream of S-step
+    segments visits T_ep / gcd(S, T_ep) of them), all sharing the stream's memory.
+
+    * Inputs: one RolloutCarry (the segment's start state, copied in before each replay) and one int64 [3] seed word (sample_seed(e),
+      reset_seed(e + 1), sample_seed(e + 1), filled from the host before each replay).  The policy launches and the reset read the seeds
+      through the device-seeded entry points, so a graph is not tied to the episode it was captured in.
+    * Outputs: the batch's S-sized slabs (history or ring, values, log-probs, actions) and the next carry, owned by the stream, not by a
+      graph.  Everything else a graph allocates comes from one memory pool shared by the stream's graphs, which is safe because a
+      stream's replays never overlap.  So a batch is valid until the next call of the same stream, whatever that call's start is.
+    * Capture: an eager warm-up of the segment (kernel attributes, stream pool), then the engine is put back from device clones of
+      every tensor it keeps across episodes (BatchedPursuitEnv._STATE and reset_fail; the warm-up may have reset the maps) and the
+      critic's spectral-norm vectors, then the capture."""
+
+    def __init__(self, mappo, engine, arena, S, tape_len, history):
+        B, N, E, D, L = engine.B, engine.N, mappo.embedding_dim, mappo.depth, mappo.num_layers
+        f32 = dict(dtype=torch.float32, device=mappo.device)
+        self.engine, self.arena = engine, arena      # the stream is keyed by their ids: keeping them alive keeps the ids unique
+        self.S, self.history = S, history or mappo.history_mode(S, B, N)
+        rows = D + 1 if self.history == "replay" else S + D
+        self.carry = RolloutCarry.zeros(mappo, B, N)
+        self.seeds = torch.zeros(3, dtype=torch.int64, device=mappo.device)
+        self.out = SimpleNamespace(hist_a=torch.zeros(rows, B, N, E, **f32), hist_c=torch.zeros(rows, B, N, E, **f32),
+                                   v=torch.zeros(S + 1, B, N, **f32), logp=torch.zeros(S, B, N, **f32),
+                                   act=torch.zeros(S, B, N, dtype=torch.int32, device=mappo.device),
+                                   carry=RolloutCarry.zeros(mappo, B, N))
+        self.pool = torch.cuda.graph_pool_handle()
+        self.graphs = {}                # t0 -> (CUDAGraph, TrainBatch, next (t0, episode increment))
+        self.tape_ptr = engine.target_tape.data_ptr()
+
+    def capture(self, mappo, engine, arena, t0, auto_reset):
+        carry = RolloutCarry(t0, self.carry.ha, self.carry.hc, self.carry.emb_a, self.carry.emb_c)
+        kw = dict(history=self.history, carry=carry, auto_reset=auto_reset, out=self.out, device_seeds=self.seeds)
+        engine._reset_buffers()
+        names = engine._STATE + ("reset_fail",)
+        saved = {n: getattr(engine, n).clone() for n in names}
+        cm = mappo.critic.Mean
+        sn = (cm.weight_u.clone(), cm.weight_v.clone()) if mappo.sn else None
+        mappo.rollout_batched(engine, arena, self.S, **kw)        # eager warm-up
+        torch.cuda.synchronize()
+        for n in names:
+            getattr(engine, n).copy_(saved[n])
+        if sn is not None:
+            cm.weight_u.copy_(sn[0])
+            cm.weight_v.copy_(sn[1])
+        del saved
+        graph = torch.cuda.CUDAGraph()
+        side = torch.cuda.Stream()
+        side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(side):
+            with torch.cuda.graph(graph, stream=side, pool=self.pool):
+                batch = mappo.rollout_batched(engine, arena, self.S, **kw)
+        torch.cuda.current_stream().wait_stream(side)
+        torch.cuda.synchronize()
+        nxt = (batch.carry.t0, 0 if batch.ended_collision is None else 1)
+        self.graphs[t0] = (graph, batch, nxt)
+        return self.graphs[t0]
+
+
 class MAPPO:
     def __init__(self, cfg, batch_size, mini_batch_size, agent_type, reference_quirks=None):
         """reference_quirks (default True, or `cfg.algo.reference_quirks`): keep the two reference behaviours that make its rollout
@@ -910,7 +972,7 @@ class MAPPO:
 
     @torch.no_grad()
     def rollout_batched(self, engine, arena, T=None, seed=0, deterministic=False, use_fused=None, timers=None, pipelines=None,
-                        actor_only=False, history=None, carry=None, policy_dbg=None, auto_reset=None):
+                        actor_only=False, history=None, carry=None, policy_dbg=None, auto_reset=None, out=None, device_seeds=None):
         """MAPPO.run_episode (:742-827) for all B envs of a BatchedPursuitEnv at once, entirely on the GPU.
         Per step: observe kernel -> fused encoder (actor, then critic with all-ones adjacency) -> GRU cell -> heads ->
         closed-loop env kernel (evader move + pursuer step + reward-norm + store).  Fills `arena` plus the history /
@@ -950,14 +1012,19 @@ class MAPPO:
         batch that crosses the boundary has `boundary` = k, `v_boot` [B,N] (the finished episode's bootstrap value) and the two episodes'
         map data, and trains as two pieces with their own start states (`TrainBatch.pieces`).  A segment that ends exactly at the
         episode's end resets at its end.  Whenever the envs were reset, `ended_collision` / `ended_evader_status` [B] keep the finished
-        episode's flags that the reset clears, and the next carry starts episode carry.episode + 1."""
+        episode's flags that the reset clears, and the next carry starts episode carry.episode + 1.
+
+        out / device_seeds (internal, for `explore_batched`'s auto-reset graphs): `out` is a SimpleNamespace of preallocated slabs
+        (hist_a, hist_c, v, logp, act) and a RolloutCarry `carry` that the batch and its next carry are written into instead of fresh
+        tensors; `device_seeds` an int64 [3] device tensor (sample_seed(e), reset_seed(e + 1), sample_seed(e + 1) as u64 bit patterns)
+        that the policy launches and the reset read when they run, in place of the AutoReset's host seeds."""
         B, N, E, D, L = engine.B, engine.N, self.embedding_dim, self.depth, self.num_layers
         dev = self.device
         if auto_reset is not None:
             T = arena.T if T is None else int(T)
             fused_ok = use_fused is not False and fused_policy.supported(self)
             check_auto_reset(auto_reset, carry, T, int(self.cfg.env.max_steps), B, N, L, E, D, dev, actor_only, fused_ok, seed)
-            if not bool((engine.time_step == carry.t0).all()):
+            if not torch.cuda.is_current_stream_capturing() and not bool((engine.time_step == carry.t0).all()):
                 raise _lib.MarlError(f"rollout segment from step {carry.t0}: the engine's envs are at steps "
                                      f"{sorted(set(engine.time_step.tolist()))[:4]}")
             seed = auto_reset.sample_seed(carry.episode)
@@ -984,10 +1051,13 @@ class MAPPO:
                                  "stored, and regenerating it needs the fused policy step (embedding_dim = rnn_hidden_dim = 128, "
                                  "2 GRU layers, depth 1..3, 9 actions)")
         slot = (lambda i: i % (D + 1)) if replay else (lambda i: i)     # history step i -> index into hist_a / hist_c
-        hist_a, hist_c = (torch.zeros(D + 1 if replay else T + D, B, N, E, **f32) for _ in range(2))
-        v = torch.zeros(T + 1, B, N, **f32)
-        logp = torch.zeros(T, B, N, **f32)
-        act = torch.zeros(T, B, N, dtype=torch.int32, device=dev)
+        if out is None:
+            hist_a, hist_c = (torch.zeros(D + 1 if replay else T + D, B, N, E, **f32) for _ in range(2))
+            v = torch.zeros(T + 1, B, N, **f32)
+            logp = torch.zeros(T, B, N, **f32)
+            act = torch.zeros(T, B, N, dtype=torch.int32, device=dev)
+        else:
+            hist_a, hist_c, v, logp, act = (getattr(out, k).zero_() for k in ("hist_a", "hist_c", "v", "logp", "act"))
         if carry is None:
             ha, hc = torch.zeros(L, B * N, E, **f32), torch.zeros(L, B * N, E, **f32)
         else:                                   # history steps 0..D-1 (slot(i) = i in both modes) are the carried embeddings
@@ -1009,7 +1079,8 @@ class MAPPO:
             G = (1 if actor_only else int(pipelines) if pipelines is not None else 1 if timers is not None
                  else int(os.environ.get("MARL_PIPELINES") or self.default_pipelines(B, N)))
             nxt, ended = self._rollout_fused(engine, arena, T, seed, deterministic, G, fused, oxy_i, o_count, hist_a, hist_c, ha, hc, act,
-                                             logp, v, slot, carry, actor_only, timers, policy_dbg, auto_reset, oxy, replay)
+                                             logp, v, slot, carry, actor_only, timers, policy_dbg, auto_reset, oxy, replay,
+                                             None if out is None else out.carry, device_seeds)
             return self._train_batch(engine, arena, T, oxy, hist_a, hist_c, v, logp, rep_, carry, nxt, ended)
 
         enc = self.actor.shared_net
@@ -1055,11 +1126,12 @@ class MAPPO:
         return max(1, min(8, (B * N) // 8192))
 
     def _rollout_fused(self, engine, arena, T, seed, deterministic, G, fused, oxy_i, o_count, hist_a, hist_c, h0_a, h0_c, act, logp, v,
-                       slot, carry, actor_only, timers, policy_dbg, auto_reset=None, oxy=None, replay=False):
+                       slot, carry, actor_only, timers, policy_dbg, auto_reset=None, oxy=None, replay=False, out_carry=None, device_seeds=None):
         """The fused schedule of `rollout_batched`: G independent env-group pipelines, one stream (+ one A* side stream) each.  Each
         group starts from its rows of the hidden states h0_a / h0_c [L, B*N, E] (one group steps them in place).  Returns the
         RolloutCarry of the segment's end (None without a carry) and, when auto_reset reset the envs during the segment, a namespace of
-        what the batch needs about the episode that ended (else None)."""
+        what the batch needs about the episode that ended (else None).  out_carry: the RolloutCarry the next carry is written into (else
+        fresh tensors); device_seeds: see `rollout_batched`."""
         B, N, E, D, L = engine.B, engine.N, self.embedding_dim, self.depth, self.num_layers
         f32 = dict(dtype=torch.float32, device=self.device)
         quirks = self.reference_quirks and not actor_only
@@ -1093,10 +1165,16 @@ class MAPPO:
             timers.setdefault(name, []).append((a_, b_))
 
         main = torch.cuda.current_stream()
-        if carry is not None:           # every group writes its rows of the next carry's hidden states
+        if out_carry is not None:
+            next_ha, next_hc = out_carry.ha, out_carry.hc
+        elif carry is not None:         # every group writes its rows of the next carry's hidden states
             next_ha, next_hc = torch.empty_like(carry.ha), torch.empty_like(carry.hc)
+        dseed = (lambda i: None) if device_seeds is None else (lambda i: device_seeds[i:i + 1])     # noqa: E731
 
-        def pipelines(t_lo, t_hi, off, seed, oxy_i, o_count, v_end, pair, h0_a, h0_c, last):
+        def into(nc):
+            return nc if out_carry is None else out_carry.copy_(nc)
+
+        def pipelines(t_lo, t_hi, off, seed, oxy_i, o_count, v_end, pair, h0_a, h0_c, last, d_seed=None):
             """Segment steps [t_lo, t_hi) of one episode, at its steps t + off, then the bootstrap value after step t_hi - 1 into v_end;
             forked from and joined back into the current stream.  h0_a / h0_c: the hidden states at t_lo (None: zeros).  last: the
             piece that ends the segment (it writes the next carry's hidden states)."""
@@ -1133,7 +1211,7 @@ class MAPPO:
                         timed("policy_step_kernel", st, lambda: fused.step(
                             view, oxy_i, o_count, off + t, seed, deterministic, hist_of(t, "actor"), hist_of(t, "critic"),
                             hist_a[slot(t + D)][sl], hist_c[slot(t + D)][sl], ha, hc, act[t][sl], logp[t][sl], v[t][sl], nets=nets,
-                            row_offset=lo * N, tile_rows=tile, debug=None if policy_dbg is None else policy_dbg[t, g]))
+                            row_offset=lo * N, tile_rows=tile, debug=None if policy_dbg is None else policy_dbg[t, g], d_seed=d_seed))
                         if join is not None:
                             st.wait_event(join)
                         elif replan:
@@ -1150,40 +1228,41 @@ class MAPPO:
                         if pair:
                             fused.step(view, oxy_i, o_count, off + t_hi, seed, deterministic, hist_of(t_hi, "actor"), h_fin,
                                        torch.empty_like(scratch), scratch, ha, hc, torch.empty_like(act[0][sl]),
-                                       torch.empty_like(logp[0][sl]), v_end[sl], row_offset=lo * N, tile_rows=tile)
+                                       torch.empty_like(logp[0][sl]), v_end[sl], row_offset=lo * N, tile_rows=tile, d_seed=d_seed)
                         else:
                             fused.step(view, oxy_i, o_count, off + t_hi, seed, deterministic, h_fin, h_fin, scratch, scratch, ha, hc,
-                                       None, None, v_end[sl], nets=("critic",), row_offset=lo * N, tile_rows=tile)
+                                       None, None, v_end[sl], nets=("critic",), row_offset=lo * N, tile_rows=tile, d_seed=d_seed)
                     done = torch.cuda.Event()
                     done.record(st)
                 main.wait_event(done)
 
         if k is None:
-            pipelines(0, T, t0, seed, oxy_i, o_count, v[T], pair_bootstrap, h0_a, h0_c, True)
+            pipelines(0, T, t0, seed, oxy_i, o_count, v[T], pair_bootstrap, h0_a, h0_c, True, dseed(0))
             if carry is not None:
-                return self._next_carry(carry, T, hist_a, hist_c, slot, next_ha, next_hc), None
+                return into(self._next_carry(carry, T, hist_a, hist_c, slot, next_ha, next_hc)), None
             return None, None
         # auto-reset: episode e ends after step k-1.  Its pipelines end with the whole-episode rollout's critic-only bootstrap step.
         e = carry.episode
         v_boot = v[T] if k == T else torch.empty(B, N, **f32)
-        pipelines(0, k, t0, seed, oxy_i, o_count, v_boot, False, h0_a, h0_c, k == T)
+        pipelines(0, k, t0, seed, oxy_i, o_count, v_boot, False, h0_a, h0_c, k == T, dseed(0))
         # All groups are joined: the maps and their sensor tables are shared by envs of different groups, and the reset regenerates
         # them in place.  Keep what the reset clears or the batch's first piece still needs.
         oxy_env, o_count_train = self._train_map_data(engine, oxy)
         ended = SimpleNamespace(k=k, collision=engine.collision.clone(), evader_status=engine.evader_status.clone(), oxy=oxy_env,
                                 o_count_train=o_count_train)
-        engine.reset_device(seed=auto_reset.reset_seed(e + 1), tape_len=auto_reset.tape_len)
+        reset_seed = auto_reset.reset_seed(e + 1) if device_seeds is None else dseed(1)
+        engine.reset_device(seed=reset_seed, tape_len=auto_reset.tape_len, tape=auto_reset.tape)
         if k == T:
-            return RolloutCarry.zeros(self, B, N, episode=e + 1), ended
+            return into(RolloutCarry.zeros(self, B, N, episode=e + 1)), ended
         ended.v_boot = v_boot
         oxy_i = engine.boundary_xy.clone() if replay else engine.boundary_xy.contiguous()
         o_count = torch.clamp(engine.boundary_count, max=engine.O).contiguous()
         ended.oxy_i, ended.o_count = oxy_i, o_count
-        pipelines(k, T, -k, auto_reset.sample_seed(e + 1), oxy_i, o_count, v[T], True, None, None, True)
-        return self._next_carry(carry, T, hist_a, hist_c, slot, next_ha, next_hc, start=k), ended
+        pipelines(k, T, -k, auto_reset.sample_seed(e + 1), oxy_i, o_count, v[T], True, None, None, True, dseed(2))
+        return into(self._next_carry(carry, T, hist_a, hist_c, slot, next_ha, next_hc, start=k)), ended
 
     def explore_batched(self, engine, arena, T=None, seed=0, host_state=None, host_out=None, reset_reward_norm=False, history=None,
-                        carry=None):
+                        carry=None, auto_reset=None):
         """The batched counterpart of `explore_env` (:731-740) - the call a user makes once per training iteration: one whole
         episode of ALL envs of `engine` with both networks in the loop, replayed from a CUDA graph that is captured on the first
         call (per engine / arena / T / seed; the weight images are re-packed inside the graph, so it follows the optimizer).
@@ -1201,7 +1280,18 @@ class MAPPO:
         carry: as in `rollout_batched` - one segment of T steps from carry.t0, usually the previous segment's `batch.carry` (or
         `RolloutCarry.zeros` at an episode's start).  One graph is captured per segment start; the carry is copied into that graph's
         own input buffers before the replay, so consecutive segments chain.  The engine must be at step carry.t0 (checked: one
-        synchronisation), and host_state (an episode start) is only accepted with t0 = 0."""
+        synchronisation), and host_state (an episode start) is only accepted with t0 = 0.
+
+        auto_reset: an AutoReset with tape="device" (TypeError otherwise) and a carry: one auto-reset segment of T = S steps, with the
+        semantics and the TrainBatch fields of `rollout_batched(carry=carry, auto_reset=auto_reset)` (boundary, v_boot, ended_*, the
+        pieces, and `carry` with its episode index), replayed from a CUDA graph.  The stream of such calls with the same engine / arena
+        / S / tape_len / history keeps one graph per segment start, its input buffers (carry, seeds), the batch's S-sized slabs and the
+        next carry, and one memory pool for the graphs (`AutoResetStream`): the returned batch is valid until the next call of the same
+        stream, whatever its start.  The seeds of the segment's episodes are written to a device word before the replay, so the graphs
+        serve every episode.  The engine's target tape must have auto_reset.tape_len entries.  seed must be 0 (the seeds come from
+        auto_reset), and host_state / host_out are not accepted: the stream resets itself, and the batch holds the per-episode data."""
+        if auto_reset is not None:
+            return MAPPO._explore_auto_reset(self, engine, arena, T, seed, host_state, host_out, history, carry, auto_reset)
         T = (T or arena.T) if carry is None else (arena.T if T is None else int(T))
         if carry is not None:
             check_segment(carry, T, int(self.cfg.env.max_steps), engine.B, engine.N, self.num_layers, self.embedding_dim,
@@ -1233,6 +1323,45 @@ class MAPPO:
             if int(status):                                  # the evader's search overflowed or its target tape ran out: not an episode
                 raise _lib.MarlError(f"explore_batched: evader status {int(status)} (A* OPEN / path overflow or target tape exhausted)")
         return g.batch
+
+    def _explore_auto_reset(self, engine, arena, T, seed, host_state, host_out, history, carry, auto_reset):
+        """explore_batched(auto_reset=...): every refusal before any CUDA call, then one replay of the stream's graph for carry.t0."""
+        if not isinstance(auto_reset, AutoReset) or auto_reset.tape != "device":
+            raise TypeError("explore_batched: auto_reset must be an AutoReset(..., tape='device'): the graph replays the reset, and the "
+                            "torch tape's generator is not graph-safe")
+        if seed != 0:
+            raise _lib.MarlError(f"explore_batched: seed={seed} with auto_reset: the sampling seeds come from auto_reset.sample_seed")
+        if carry is None:
+            raise _lib.MarlError("explore_batched: auto_reset continues a stream of segments and needs a carry (RolloutCarry.zeros at the "
+                                 "start)")
+        if host_state is not None or host_out is not None:
+            raise _lib.MarlError("explore_batched: host_state / host_out do not combine with auto_reset (the stream resets the envs "
+                                 "itself; per-episode returns are in the batch)")
+        S = arena.T if T is None else int(T)
+        check_auto_reset(auto_reset, carry, S, int(self.cfg.env.max_steps), engine.B, engine.N, self.num_layers, self.embedding_dim,
+                         self.depth, self.device, use_fused=fused_policy.supported(self))
+        if engine._tape_len != auto_reset.tape_len or tuple(engine.target_tape.shape) != (engine.B, auto_reset.tape_len, 2):
+            raise _lib.MarlError(f"explore_batched: the engine's target tape has {engine._tape_len} entries, auto_reset.tape_len is "
+                                 f"{auto_reset.tape_len} (reset the envs with reset_device(..., tape_len={auto_reset.tape_len}))")
+        at = engine.time_step.tolist()
+        if any(x != carry.t0 for x in at):
+            raise _lib.MarlError(f"explore_batched: segment from step {carry.t0}, the engine's envs are at steps {sorted(set(at))[:4]}")
+        key = (id(engine), id(arena), S, auto_reset.tape_len, history)
+        streams = self.__dict__.setdefault("_auto_reset_streams", {})
+        st = streams.get(key)
+        if st is None:
+            st = streams[key] = AutoResetStream(self, engine, arena, S, auto_reset.tape_len, history)
+        if st.tape_ptr != engine.target_tape.data_ptr():    # the tape was reallocated: the graphs read the old one
+            st.graphs.clear()
+            st.tape_ptr = engine.target_tape.data_ptr()
+        e = carry.episode
+        st.seeds.copy_(torch.tensor([_lib.u64_bits(x) for x in (auto_reset.sample_seed(e), auto_reset.reset_seed(e + 1),
+                                                                 auto_reset.sample_seed(e + 1))], dtype=torch.int64))
+        st.carry.copy_(carry)
+        graph, batch, (t_next, de) = st.graphs.get(carry.t0) or st.capture(self, engine, arena, carry.t0, auto_reset)
+        graph.replay()
+        batch.carry.t0, batch.carry.episode = t_next, e + de
+        return batch
 
     def _next_carry(self, carry, T, hist_a, hist_c, slot, ha, hc, start=None):
         """The carry after a segment of T steps: its hidden states and the embeddings of its history steps T..T+D-1.  start: the

@@ -170,31 +170,66 @@ class BatchedPursuitEnv:
         self.set_state(ps, es, tg, mid, time_step=0)
         self.start_episode()
 
-    def reset_device(self, seed=0, tape_len=16):
+    def reset_device(self, seed=0, tape_len=16, tape="torch"):
         """Fresh episode for every env, generated ON THE GPU (csrc/reset_kernels.cu): maps, sensor tables, targets, pursuers,
-        evaders and the candidate-target tape.  Same placement rules as `reset` / the reference, per-env counter RNG streams."""
+        evaders and the candidate-target tape.  Same placement rules as `reset` / the reference, per-env counter RNG streams.
+
+        tape: "torch" draws the tape [B, tape_len, 2] with a torch.Generator seeded from `seed`; "device" draws it with
+        marl_target_tape_generate (env b's own counter stream of (seed, b), the same distribution).  Everything else is the same in
+        both modes.  When tape_len is unchanged the tape is written into the existing `target_tape` storage, so a CUDA graph that
+        reads it keeps reading the current episode's tape.
+        seed: a host int, or (tape="device" only) a one-element int64 device tensor holding the seed's u64 bit pattern, read when the
+        kernels run: then every launch is graph-capturable (no generator, no host read, no allocation after the first call)."""
         import ctypes
+        if tape not in ("torch", "device"):
+            raise ValueError(f"tape={tape!r}: 'torch' or 'device'")
+        on_device = isinstance(seed, torch.Tensor)
+        if on_device and tape != "device":
+            raise _lib.MarlError("reset_device: a device-resident seed needs tape='device' (the torch tape is drawn from a host seed)")
+        if tape == "device" and int(tape_len) < 1:
+            raise _lib.MarlError(f"reset_device: tape_len={tape_len}; the device tape has at least one entry")
         p, mc = self.params, self.cfg.map
-        _lib.check(self.lib.marl_map_generate(self._pp(), self.M, int(mc.num_obstacle_block), ctypes.c_double(float(mc.center[0])),
-                                              ctypes.c_double(float(mc.center[1])), ctypes.c_double(float(mc.variance)),
-                                              ctypes.c_uint64(int(seed) & 0xFFFFFFFFFFFFFFFF), _lib.ptr(self.grid_bits),
-                                              _lib.ptr(self.inflated_bits), _lib.stream_ptr()), "marl_map_generate")
+        self._reset_buffers()
+        if on_device:
+            if seed.dtype != torch.int64 or seed.numel() != 1 or not seed.is_cuda:
+                raise _lib.MarlError("reset_device: a device seed is one int64 element on the engine's device")
+            seed_arg, gen, place, sfx = _lib.ptr(seed), self.lib.marl_map_generate_dseed, self.lib.marl_env_reset_place_dseed, "_dseed"
+        else:
+            seed_arg = ctypes.c_uint64(int(seed) & 0xFFFFFFFFFFFFFFFF)
+            gen, place, sfx = self.lib.marl_map_generate, self.lib.marl_env_reset_place, ""
+        _lib.check(gen(self._pp(), self.M, int(mc.num_obstacle_block), ctypes.c_double(float(mc.center[0])),
+                       ctypes.c_double(float(mc.center[1])), ctypes.c_double(float(mc.variance)), seed_arg, _lib.ptr(self.grid_bits),
+                       _lib.ptr(self.inflated_bits), _lib.stream_ptr()), "marl_map_generate" + sfx)
         self.build_sensor_tables()
-        if getattr(self, "_reset_scratch", None) is None:
-            self._reset_scratch = torch.empty(self.B, p.W, p.HW, dtype=torch.int32, device=self.device)
-            self.reset_fail = torch.zeros(self.B, dtype=torch.int32, device=self.device)
-        _lib.check(self.lib.marl_env_reset_place(self._pp(), self.B, self.M, _lib.ptr(self.inflated_bits), _lib.ptr(self.map_id),
-                                                 ctypes.c_uint64(int(seed) & 0xFFFFFFFFFFFFFFFF), ctypes.c_double(4.0), 2, 200000,
-                                                 _lib.ptr(self.p_state), _lib.ptr(self.e_state), _lib.ptr(self.target),
-                                                 _lib.ptr(self._reset_scratch), _lib.ptr(self.reset_fail), _lib.stream_ptr()),
-                   "marl_env_reset_place")
+        _lib.check(place(self._pp(), self.B, self.M, _lib.ptr(self.inflated_bits), _lib.ptr(self.map_id), seed_arg, ctypes.c_double(4.0),
+                         2, 200000, _lib.ptr(self.p_state), _lib.ptr(self.e_state), _lib.ptr(self.target), _lib.ptr(self._reset_scratch),
+                         _lib.ptr(self.reset_fail), _lib.stream_ptr()), "marl_env_reset_place" + sfx)
         self.launches += 2
-        g = torch.Generator(device=self.device).manual_seed(int(seed) & 0x7FFFFFFFFFFFFFFF)
-        tape = torch.stack([torch.randint(0, p.W, (self.B, tape_len), generator=g, device=self.device),
-                            torch.randint(0, p.H, (self.B, tape_len), generator=g, device=self.device)], dim=-1).to(torch.int32)
-        self.target_tape, self._tape_len = tape.contiguous(), tape_len
+        shape = (self.B, int(tape_len), 2)
+        if tuple(self.target_tape.shape) != shape or not self.target_tape.is_contiguous():
+            self.target_tape = torch.empty(shape, dtype=torch.int32, device=self.device)
+        if tape == "device":
+            if not on_device:
+                self._seed_word.fill_(_lib.u64_bits(seed))
+                seed = self._seed_word
+            _lib.check(self.lib.marl_target_tape_generate(self._pp(), self.B, int(tape_len), _lib.ptr(seed), _lib.ptr(self.target_tape),
+                                                          _lib.stream_ptr()), "marl_target_tape_generate")
+            self.launches += 1
+        else:
+            g = torch.Generator(device=self.device).manual_seed(int(seed) & 0x7FFFFFFFFFFFFFFF)
+            self.target_tape.copy_(torch.stack([torch.randint(0, p.W, (self.B, tape_len), generator=g, device=self.device),
+                                                torch.randint(0, p.H, (self.B, tape_len), generator=g, device=self.device)], dim=-1))
+        self._tape_len = int(tape_len)
         self.tape_pos.zero_()
         self.start_episode()
+
+    def _reset_buffers(self):
+        """The device reset's scratch rows, failure flags and seed word (allocated once)."""
+        if getattr(self, "_reset_scratch", None) is None:
+            p = self.params
+            self._reset_scratch = torch.empty(self.B, p.W, p.HW, dtype=torch.int32, device=self.device)
+            self.reset_fail = torch.zeros(self.B, dtype=torch.int32, device=self.device)
+            self._seed_word = torch.zeros(1, dtype=torch.int64, device=self.device)
 
     def start_episode(self):
         self.time_step.zero_()

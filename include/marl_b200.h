@@ -147,6 +147,16 @@ int marl_map_generate(const marl_env_params *p, int32_t M, int32_t num_blocks, d
 int marl_env_reset_place(const marl_env_params *p, int32_t B, int32_t M, const uint32_t *d_inflated_bits, const int32_t *d_map_id,
                          uint64_t seed, double min_dist, int32_t extend, int32_t max_draws, double *d_p_state, double *d_e_state,
                          int32_t *d_target, uint32_t *d_scratch, int32_t *d_fail, void *stream);
+/* Device-seeded twins: the same kernels and the same bits as the by-value calls with seed = *d_seed, read when the kernel runs (a
+ * CUDA graph that captures them follows the seed word instead of freezing the seed it was captured with).  d_seed must not be NULL. */
+int marl_map_generate_dseed(const marl_env_params *p, int32_t M, int32_t num_blocks, double center_x, double center_y, double variance,
+                            const uint64_t *d_seed, uint32_t *d_grid_bits, uint32_t *d_inflated_bits, void *stream);
+int marl_env_reset_place_dseed(const marl_env_params *p, int32_t B, int32_t M, const uint32_t *d_inflated_bits, const int32_t *d_map_id,
+                               const uint64_t *d_seed, double min_dist, int32_t extend, int32_t max_draws, double *d_p_state,
+                               double *d_e_state, int32_t *d_target, uint32_t *d_scratch, int32_t *d_fail, void *stream);
+/* Candidate-target tape of the mid-episode init_target (base_env.py:52-70), filled in place: d_tape i32 [B,L,2], entry (b, l) =
+ * (randint(0, W-1), randint(0, H-1)) from env b's own counter stream keyed by (*d_seed, b).  Row b does not depend on B. */
+int marl_target_tape_generate(const marl_env_params *p, int32_t B, int32_t L, const uint64_t *d_seed, int32_t *d_tape, void *stream);
 
 /* ---- kernel 3a: Welford reward normalisation -----------------------------------------------------
  * Replaces Normalization.__call__ / RunningMeanStd.update (DHGN/normalization.py:4-35) applied per env:
@@ -457,6 +467,10 @@ int marl_policy_pack(const marl_dhgn_weights *w, int32_t depth, int32_t is_actor
 /* One env step of both networks (either pair may be NULL to run only the other, e.g. the critic-only bootstrap :806-825). */
 int marl_policy_rollout_step(const marl_policy_step *s, const marl_dhgn_weights *actor_w, const marl_policy_net_io *actor_io,
                              const marl_dhgn_weights *critic_w, const marl_policy_net_io *critic_io, void *stream);
+/* The same step with the sampling seed read from the device word d_seed (not NULL) when the kernel runs; s->seed is ignored. */
+int marl_policy_rollout_step_dseed(const marl_policy_step *s, const marl_dhgn_weights *actor_w, const marl_policy_net_io *actor_io,
+                                   const marl_dhgn_weights *critic_w, const marl_policy_net_io *critic_io, const uint64_t *d_seed,
+                                   void *stream);
 
 /* ---- second network family: GnnExtractor (obstacle_differ_3hop/mappo_parallel.py:34-70) -------------------------------------
  * L1-normalised adjacency-weighted mean over entities (F.normalize(adj, p=1) then adj @ x, :55-66).  rows = S*N (sample, agent)

@@ -25,7 +25,13 @@ are reset only at episode starts.  The episode reward is printed on the iteratio
 seeds are the ones the loop uses without it, so for an S that divides --steps both print the same exact columns.  The iteration that
 finishes an episode prints its reward.
 
-    python tools/train_loop.py --envs 512 --steps 150 --segment 64 --auto-reset --iters 7"""
+    python tools/train_loop.py --envs 512 --steps 150 --segment 64 --auto-reset --iters 7
+
+--device-tape draws the evader's candidate-target tape on the device (reset_device(tape="device")) instead of with a torch.Generator.
+--graph (needs --auto-reset, implies --device-tape) replays each segment from the CUDA graphs of MAPPO.explore_batched; it prints the same
+exact columns as --device-tape without it.
+
+    python tools/train_loop.py --envs 512 --steps 150 --segment 64 --auto-reset --graph --iters 7"""
 import argparse
 import os
 import sys
@@ -51,6 +57,8 @@ def main():
     ap.add_argument("--segment", type=int, default=None, help="env steps per iteration, a divisor of --steps (default: --steps)")
     ap.add_argument("--auto-reset", action="store_true",
                     help="segments may cross episode boundaries: any --segment in [1, --steps], envs reset inside the rollout")
+    ap.add_argument("--device-tape", action="store_true", help="--auto-reset: draw the target tape on the device")
+    ap.add_argument("--graph", action="store_true", help="--auto-reset: replay the segments from CUDA graphs (implies --device-tape)")
     ap.add_argument("--iters", type=int, default=10)
     ap.add_argument("--depth", type=int, default=1)
     ap.add_argument("--allreduce", default=None, choices=[None, "update", "minibatch"],
@@ -63,6 +71,8 @@ def main():
     if args.save_every < 1:
         ap.error("--save-every must be >= 1")
     S = args.steps if args.segment is None else args.segment
+    if (args.graph or args.device_tape) and not args.auto_reset:
+        ap.error("--graph / --device-tape need --auto-reset")
     if args.auto_reset:
         if args.host_reset:
             ap.error("--auto-reset resets the envs on the device; it does not combine with --host-reset")
@@ -157,7 +167,8 @@ def auto_reset_loop(args, rank, world, dev, cfg, env, arena, mappo, state_file):
     """The loop of --auto-reset: one segment of S steps per iteration, episode e reset on the device with seed 1000*rank + e and sampled
     with seed e*world + rank (the seeds of the loop without --auto-reset), the resets inside the rollout."""
     B, N, S, T_ep = args.envs, args.pursuers, args.segment or args.steps, args.steps
-    auto = AutoReset(reset_seed=lambda e: 1000 * rank + e, sample_seed=lambda e: e * world + rank)
+    auto = AutoReset(reset_seed=lambda e: 1000 * rank + e, sample_seed=lambda e: e * world + rank,
+                     tape="device" if args.device_tape or args.graph else "torch")
     carry = RolloutCarry.zeros(mappo, B, N)
     ep_sum = torch.zeros(B, dtype=torch.int64, device=dev)
     total_steps, start = 0, 0
@@ -169,12 +180,15 @@ def auto_reset_loop(args, rank, world, dev, cfg, env, arena, mappo, state_file):
             raise SystemExit(f"--resume: the file continues at step {carry.t0} of episode {carry.episode}, iteration {start} of "
                              f"--segment {S} starts at step {start * S % T_ep} of episode {start * S // T_ep}")
     else:
-        env.reset_device(seed=auto.reset_seed(0), tape_len=auto.tape_len)
+        env.reset_device(seed=auto.reset_seed(0), tape_len=auto.tape_len, tape=auto.tape)
         torch.cuda.synchronize()
         assert int(env.reset_fail.sum()) == 0, "device reset could not place every pursuer / evader"
     for it in range(start, args.iters):
         t1 = time.perf_counter()
-        tb = mappo.rollout_batched(env, arena, S, carry=carry, auto_reset=auto)
+        if args.graph:
+            tb = mappo.explore_batched(env, arena, S, carry=carry, auto_reset=auto)
+        else:
+            tb = mappo.rollout_batched(env, arena, S, carry=carry, auto_reset=auto)
         torch.cuda.synchronize()
         t2 = time.perf_counter()
         assert int(env.evader_status.max()) == 0, "evader search overflow / target tape exhausted"
