@@ -108,6 +108,8 @@ _PROTOTYPES = {
     "marl_map_generate_dseed": (C.c_int, [_PP, _I32, _I32, C.c_double, C.c_double, C.c_double, _VP, _VP, _VP, _VP]),
     "marl_env_reset_place_dseed": (C.c_int, [_PP, _I32, _I32, _VP, _VP, _VP, C.c_double, _I32, _I32, _VP, _VP, _VP, _VP, _VP, _VP]),
     "marl_target_tape_generate": (C.c_int, [_PP, _I32, _I32, _VP, _VP, _VP]),
+    "marl_map_draw": (C.c_int, [_PP, _I32, _I32, _U64, _VP, _VP]),
+    "marl_map_draw_dseed": (C.c_int, [_PP, _I32, _I32, _VP, _VP, _VP]),
     "marl_clip_workspace_bytes": (_I64, [_I64]),
     "marl_clip_grad_norm": (C.c_int, [_I64, _VP, _F32, _VP, _VP, _VP]),
     "marl_adam_step": (C.c_int, [_I64, _VP, _VP, _VP, _VP, _F32, _F32, _F32, _F32, _I64, _VP]),

@@ -6,7 +6,8 @@
 // the reference, not stream-equivalent (the reference's interpreter-global Mersenne-Twister streams are inherently serial).
 // Rejection sampling is sequential per env and cheap: one thread per env / per map; the work bitmap lives in a global scratch
 // row.  The per-map sensor tables are then built by marl_raser_map_build.  The *_dseed entry points and the target-tape draw read the
-// seed from a device word when the kernel runs, so a CUDA graph that captures a reset follows that word.
+// seed from a device word when the kernel runs, so a CUDA graph that captures a reset follows that word.  A reset that keeps the maps
+// (an installed pool) skips the map and table build and may draw each env's map from the M installed ones (marl_map_draw).
 #include "common.cuh"
 
 namespace marl {
@@ -136,6 +137,17 @@ target_tape_kernel(int B, int L, int W, int H, const uint64_t *__restrict__ d_se
     }
 }
 
+// per-env map draw of a reset that keeps the installed maps: map_id[b] = randint(0, M-1) from env b's own stream of (seed, b)
+__global__ void __launch_bounds__(64)
+map_draw_kernel(int B, int M, uint64_t seed, const uint64_t *__restrict__ d_seed, int32_t *__restrict__ map_id)
+{
+    const int b = blockIdx.x * 64 + threadIdx.x;
+    if (b >= B) return;
+    if (d_seed) seed = *d_seed;
+    Stream64 rng{splitmix64(seed ^ 0x6472617700000000ull) ^ splitmix64((uint64_t)b), 0};
+    map_id[b] = rng.randint(0, M - 1);
+}
+
 }  // namespace marl
 
 using namespace marl;
@@ -206,4 +218,25 @@ extern "C" int marl_target_tape_generate(const marl_env_params *p, int32_t B, in
     MARL_REQUIRE(B > 0 && L > 0 && d_seed && d_tape, "marl_target_tape_generate: bad arguments (B=%d L=%d)", B, L);
     target_tape_kernel<<<(B + 63) / 64, 64, 0, (cudaStream_t)stream>>>(B, L, c.W, c.H, d_seed, d_tape);
     return check_launch("target_tape_kernel");
+}
+
+static int map_draw(const marl_env_params *p, int32_t B, int32_t M, uint64_t seed, const uint64_t *d_seed, int32_t *d_map_id, void *stream)
+{
+    EnvDev c;
+    int rc = make_env_dev(p, &c);
+    if (rc) return rc;
+    MARL_REQUIRE(B > 0 && M > 0 && d_map_id, "marl_map_draw: bad arguments (B=%d M=%d d_map_id=%p)", B, M, (void *)d_map_id);
+    map_draw_kernel<<<(B + 63) / 64, 64, 0, (cudaStream_t)stream>>>(B, M, seed, d_seed, d_map_id);
+    return check_launch("map_draw_kernel");
+}
+
+extern "C" int marl_map_draw(const marl_env_params *p, int32_t B, int32_t M, uint64_t seed, int32_t *d_map_id, void *stream)
+{
+    return map_draw(p, B, M, seed, nullptr, d_map_id, stream);
+}
+
+extern "C" int marl_map_draw_dseed(const marl_env_params *p, int32_t B, int32_t M, const uint64_t *d_seed, int32_t *d_map_id, void *stream)
+{
+    MARL_REQUIRE(d_seed != nullptr, "marl_map_draw_dseed: d_seed is NULL");
+    return map_draw(p, B, M, 0, d_seed, d_map_id, stream);
 }

@@ -7,7 +7,8 @@
   `(total_step, avg_r, std_r, exp_r, *logging_tuple)`, "save when the average return does not get worse".  Its episodes are
   ONE batched arg-max rollout of `num_cpus_eval` independent environments on the GPU (`MAPPO.rollout_batched(deterministic=
   True, actor_only=True)`: the actor alone, fed with its own previous embeddings exactly as `evaluate` does) instead of
-  `num_cpus_eval` Ray tasks.
+  `num_cpus_eval` Ray tasks.  With a map pool (`Evaluator(..., pool=, pool_indices=)`) the episodes are played on a fixed
+  held-out set of maps, so successive evaluations are comparable.
 """
 import time
 
@@ -53,8 +54,21 @@ def evaluate(env, actor, cfg):
 class Evaluator:
     """EvaluatorProc (evaluator.py:20-103) as a plain object.  `agent` is a MAPPO built with agent_type "Evaluator"."""
 
-    def __init__(self, cfg, num_cpus_eval, agent, device=None, seed=0):
+    def __init__(self, cfg, num_cpus_eval, agent, device=None, seed=0, pool=None, pool_indices=None):
+        """pool / pool_indices: evaluate on a fixed held-out set of maps, maps `pool_indices` of a MapPool (default: all of it).  The
+        engine then holds exactly those M maps, installed once (verify=True) on first use, and every evaluation keeps them: env b plays
+        map b % M, and only the placements and the target tape come from the evaluation's seed.  Without a pool, every evaluation
+        generates new maps."""
         self.cfg, self.agent, self.num_cpus_eval = cfg, agent, int(num_cpus_eval)
+        self.pool = pool
+        self.pool_indices = None
+        if pool is not None:
+            idx = np.arange(len(pool)) if pool_indices is None else np.asarray(pool_indices, dtype=np.int64).reshape(-1)
+            if idx.size == 0:
+                raise ValueError("Evaluator: pool_indices selects no map")
+            self.pool_indices = idx
+        elif pool_indices is not None:
+            raise ValueError("Evaluator: pool_indices without a pool")
         self.device = torch.device(device) if device is not None else agent.device
         self.total_step = 0
         self.start_time = time.time()
@@ -91,11 +105,15 @@ class Evaluator:
         all of them in one batched rollout on the device."""
         cfg, B = self.cfg, self.num_cpus_eval
         if self._engine is None:
-            self._engine = BatchedPursuitEnv(cfg, B, device=self.device, num_maps=B)
+            M = B if self.pool is None else len(self.pool_indices)
+            eng = BatchedPursuitEnv(cfg, B, device=self.device, num_maps=M)
+            if self.pool is not None:        # env b plays held-out map b % M (the engine's initial map_id), in every evaluation
+                self.pool.install(eng, self.pool_indices, verify=True)
+            self._engine = eng
             self._arena = RolloutArena(self._engine.params, B, int(cfg.env.max_steps), self._engine.device)
         eng, T = self._engine, int(cfg.env.max_steps)
         self._seed += 1
-        eng.reset_device(seed=self._seed, tape_len=64)
+        eng.reset_device(seed=self._seed, tape_len=64, maps="generate" if self.pool is None else "keep")
         self.agent.rollout_batched(eng, self._arena, T, seed=self._seed, deterministic=True, actor_only=True)
         ret = self._arena.raw_reward[:T].sum(dim=(0, 2)).to(torch.float32)
         steps = torch.full((B,), float(T - 1), dtype=torch.float32, device=ret.device)   # `done` fires at step index T-1

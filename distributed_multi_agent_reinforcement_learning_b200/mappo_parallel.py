@@ -138,19 +138,29 @@ class AutoReset:
     whole-episode rollout), so a stream of segments collects the episodes that `reset_device(reset_seed(e))` followed by
     `rollout_batched(max_steps, seed=sample_seed(e))` collects, bit for bit.  reset_seed / sample_seed: host callables, episode
     index -> int.  tape: the target tape's draw, as in `reset_device` - "torch" (a torch.Generator) or "device"
-    (marl_target_tape_generate), which `explore_batched` needs to replay the reset from a CUDA graph."""
+    (marl_target_tape_generate), which `explore_batched` needs to replay the reset from a CUDA graph.  maps: the reset's map mode, as in
+    `reset_device` - "generate" (new maps every episode), "keep" (the engine's maps and map assignment) or "draw" (every env draws one
+    of the engine's M maps, e.g. an installed pool, per episode)."""
 
-    def __init__(self, reset_seed, sample_seed, tape_len=16, tape="torch"):
+    def __init__(self, reset_seed, sample_seed, tape_len=16, tape="torch", maps="generate"):
         if tape not in ("torch", "device"):
             raise ValueError(f"AutoReset: tape={tape!r}, 'torch' or 'device'")
+        if maps not in ("generate", "keep", "draw"):
+            raise ValueError(f"AutoReset: maps={maps!r}, 'generate', 'keep' or 'draw'")
         self.reset_seed, self.sample_seed, self.tape_len, self.tape = reset_seed, sample_seed, int(tape_len), tape
+        self.maps = maps
 
 
-def check_auto_reset(auto_reset, carry, S, T_ep, B, N, L, E, D, device, actor_only=False, use_fused=True, seed=0):
+def check_auto_reset(auto_reset, carry, S, T_ep, B, N, L, E, D, device, actor_only=False, use_fused=True, seed=0, maps_set=True):
     """Host-side checks of an auto-reset rollout segment (any 1 <= S <= T_ep from any step 0 <= carry.t0 < T_ep); raises MarlError
-    before any CUDA call."""
+    before any CUDA call.  maps_set: whether the engine's maps were ever set (a reset that keeps them needs them)."""
     if not isinstance(auto_reset, AutoReset):
         raise _lib.MarlError(f"rollout_batched: auto_reset must be an AutoReset, not {type(auto_reset).__name__}")
+    if auto_reset.maps not in ("generate", "keep", "draw"):
+        raise _lib.MarlError(f"rollout_batched: auto_reset.maps={auto_reset.maps!r}, 'generate', 'keep' or 'draw'")
+    if auto_reset.maps != "generate" and not maps_set:
+        raise _lib.MarlError(f"rollout_batched: AutoReset(maps={auto_reset.maps!r}) keeps the engine's maps, but they were never set "
+                             "(MapPool.install, set_maps or a reset_device(maps='generate') first)")
     if carry is None:
         raise _lib.MarlError("rollout_batched: auto_reset continues a stream of segments and needs a carry (RolloutCarry.zeros at the "
                              "start)")
@@ -468,7 +478,7 @@ class TrainBatch:
 
     KEYS = ("p", "e", "p_adj_bits", "e_adj", "o_adj_bits", "hist_a", "hist_c", "v", "a", "logp", "r", "active")
     replay = None       # HistoryReplay of a batch whose history was not stored (hist_a = hist_c = None); minibatches regenerate it
-    map_id = None       # i32 [B] (replay only)
+    map_id = None       # i32 [B] (replay only; a batch that crossed an episode boundary: the ids of the episode that ended)
     # A rollout segment (rollout_batched(carry=...)) starts at the episode's step t0 from the GRU hidden states h0_a / h0_c
     # [L, B*N, E]; a replay-mode segment also keeps its D history-prefix slabs prefix_a / prefix_c [D, B, N, E] (a store-mode one has
     # them as slabs 0..D-1 of hist_a / hist_c).  `carry` is the RolloutCarry the next segment continues from.  A whole-episode batch
@@ -477,10 +487,10 @@ class TrainBatch:
     h0_a = h0_c = prefix_a = prefix_c = carry = None
     # A segment that crossed an episode boundary (rollout_batched(auto_reset=...)) has boundary = k: steps [0, k) end one episode and
     # [k, T) start the next, which trains from zero hidden states and zero history, on its own maps oxy2 / o_count_train2 (replay2:
-    # its HistoryReplay).  v_boot [B,N] is the bootstrap value after step k-1.  `pieces()` views it as those two ordinary batches; a
-    # minibatch of it holds the minibatches of both pieces in `parts`.  ended_collision / ended_evader_status [B]: the flags of the
-    # episode that ended during the segment (the reset cleared the engine's).
-    boundary = v_boot = oxy2 = o_count_train2 = replay2 = parts = None
+    # its HistoryReplay; map_id2: its map ids, which a reset that draws the maps changes).  v_boot [B,N] is the bootstrap value after
+    # step k-1.  `pieces()` views it as those two ordinary batches; a minibatch of it holds the minibatches of both pieces in `parts`.
+    # ended_collision / ended_evader_status [B]: the flags of the episode that ended during the segment (the reset cleared the engine's).
+    boundary = v_boot = oxy2 = o_count_train2 = replay2 = map_id2 = parts = None
     ended_collision = ended_evader_status = None
     zero_prefix = False     # a store-mode piece whose history slabs 0..D-1 belong to the previous episode: they read as zeros
 
@@ -542,7 +552,7 @@ class TrainBatch:
                          h0_a=self.h0_a, h0_c=self.h0_c, prefix_a=self.prefix_a, prefix_c=self.prefix_c, replay=self.replay,
                          map_id=self.map_id)
         two = TrainBatch(**common(last), oxy=self.oxy2, o_count_train=self.o_count_train2, hist_a=last(self.hist_a),
-                         hist_c=last(self.hist_c), v=self.v[k:], depth=D, replay=self.replay2, map_id=self.map_id,
+                         hist_c=last(self.hist_c), v=self.v[k:], depth=D, replay=self.replay2, map_id=self.map_id2,
                          zero_prefix=self.hist_a is not None)
         return one, two
 
@@ -1023,7 +1033,8 @@ class MAPPO:
         if auto_reset is not None:
             T = arena.T if T is None else int(T)
             fused_ok = use_fused is not False and fused_policy.supported(self)
-            check_auto_reset(auto_reset, carry, T, int(self.cfg.env.max_steps), B, N, L, E, D, dev, actor_only, fused_ok, seed)
+            check_auto_reset(auto_reset, carry, T, int(self.cfg.env.max_steps), B, N, L, E, D, dev, actor_only, fused_ok, seed,
+                             getattr(engine, "maps_set", False))
             if not torch.cuda.is_current_stream_capturing() and not bool((engine.time_step == carry.t0).all()):
                 raise _lib.MarlError(f"rollout segment from step {carry.t0}: the engine's envs are at steps "
                                      f"{sorted(set(engine.time_step.tolist()))[:4]}")
@@ -1249,9 +1260,9 @@ class MAPPO:
         # them in place.  Keep what the reset clears or the batch's first piece still needs.
         oxy_env, o_count_train = self._train_map_data(engine, oxy)
         ended = SimpleNamespace(k=k, collision=engine.collision.clone(), evader_status=engine.evader_status.clone(), oxy=oxy_env,
-                                o_count_train=o_count_train)
+                                o_count_train=o_count_train, map_id=engine.map_id.clone() if replay else None)
         reset_seed = auto_reset.reset_seed(e + 1) if device_seeds is None else dseed(1)
-        engine.reset_device(seed=reset_seed, tape_len=auto_reset.tape_len, tape=auto_reset.tape)
+        engine.reset_device(seed=reset_seed, tape_len=auto_reset.tape_len, tape=auto_reset.tape, maps=auto_reset.maps)
         if k == T:
             return into(RolloutCarry.zeros(self, B, N, episode=e + 1)), ended
         ended.v_boot = v_boot
@@ -1339,14 +1350,14 @@ class MAPPO:
                                  "itself; per-episode returns are in the batch)")
         S = arena.T if T is None else int(T)
         check_auto_reset(auto_reset, carry, S, int(self.cfg.env.max_steps), engine.B, engine.N, self.num_layers, self.embedding_dim,
-                         self.depth, self.device, use_fused=fused_policy.supported(self))
+                         self.depth, self.device, use_fused=fused_policy.supported(self), maps_set=getattr(engine, "maps_set", False))
         if engine._tape_len != auto_reset.tape_len or tuple(engine.target_tape.shape) != (engine.B, auto_reset.tape_len, 2):
             raise _lib.MarlError(f"explore_batched: the engine's target tape has {engine._tape_len} entries, auto_reset.tape_len is "
                                  f"{auto_reset.tape_len} (reset the envs with reset_device(..., tape_len={auto_reset.tape_len}))")
         at = engine.time_step.tolist()
         if any(x != carry.t0 for x in at):
             raise _lib.MarlError(f"explore_batched: segment from step {carry.t0}, the engine's envs are at steps {sorted(set(at))[:4]}")
-        key = (id(engine), id(arena), S, auto_reset.tape_len, history)
+        key = (id(engine), id(arena), S, auto_reset.tape_len, history, auto_reset.maps)
         streams = self.__dict__.setdefault("_auto_reset_streams", {})
         st = streams.get(key)
         if st is None:
@@ -1400,13 +1411,16 @@ class MAPPO:
                 oxy2, o_count_train2 = self._train_map_data(engine, engine.boundary_xy.to(torch.float32).contiguous())
                 seg.update(boundary=ended.k, v_boot=ended.v_boot, oxy2=oxy2, o_count_train2=o_count_train2)
                 if replay is not None:
-                    seg["replay2"] = HistoryReplay(replay.fused, ended.oxy_i, ended.o_count, replay.quirks)
+                    seg.update(replay2=HistoryReplay(replay.fused, ended.oxy_i, ended.o_count, replay.quirks),
+                               map_id2=engine.map_id.to(torch.int32).clone())
+        map_id = None
+        if replay is not None:         # the map ids of the steps the batch (its first piece) ran: taken before any reset
+            map_id = engine.map_id.to(torch.int32).clone() if ended is None else ended.map_id
         return TrainBatch(p=arena.p_state_f32[:T], e=arena.e_state_f32[:T, :, 0].contiguous(), oxy=oxy_env,
                           o_count_train=o_count_train,
                           p_adj_bits=arena.p_adj_bits[:T], e_adj=arena.e_adj[:T], o_adj_bits=arena.o_adj_bits[:T],
                           hist_a=hist_a, hist_c=hist_c, v=v, a=arena.a_n[:T], logp=logp, r=arena.r[:T],
-                          active=arena.active[:T], depth=D, replay=replay,
-                          map_id=None if replay is None else engine.map_id.to(torch.int32).clone(), **seg)
+                          active=arena.active[:T], depth=D, replay=replay, map_id=map_id, **seg)
 
     def explore_env(self, env, num_episode):
         """Reference signature (:731-740) for the single-env facade `Pursuit_Env`: returns

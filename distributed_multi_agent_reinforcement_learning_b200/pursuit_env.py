@@ -95,6 +95,7 @@ class BatchedPursuitEnv:
         self.grid_bits.copy_(torch.from_numpy(maps.pack_grid(grids)))
         self.inflated_bits.copy_(torch.from_numpy(maps.pack_grid(inflated)))
         self.build_sensor_tables()
+        self.maps_set = True
 
     def build_sensor_tables(self):
         _lib.check(self.lib.marl_raser_map_build(
@@ -143,6 +144,8 @@ class BatchedPursuitEnv:
         self.tape_pos.zero_()
 
     _tape_len = 0
+    maps_set = False    # whether the maps were ever set (set_maps / MapPool.install, a "generate" reset, reset, load_state_dict)
+    MAP_MODES = ("generate", "keep", "draw")
 
     def reset(self, seed=0):
         """Fresh episode for every env (host generation, reference rules; one map per pool slot)."""
@@ -170,7 +173,7 @@ class BatchedPursuitEnv:
         self.set_state(ps, es, tg, mid, time_step=0)
         self.start_episode()
 
-    def reset_device(self, seed=0, tape_len=16, tape="torch"):
+    def reset_device(self, seed=0, tape_len=16, tape="torch", maps="generate"):
         """Fresh episode for every env, generated ON THE GPU (csrc/reset_kernels.cu): maps, sensor tables, targets, pursuers,
         evaders and the candidate-target tape.  Same placement rules as `reset` / the reference, per-env counter RNG streams.
 
@@ -179,8 +182,18 @@ class BatchedPursuitEnv:
         both modes.  When tape_len is unchanged the tape is written into the existing `target_tape` storage, so a CUDA graph that
         reads it keeps reading the current episode's tape.
         seed: a host int, or (tape="device" only) a one-element int64 device tensor holding the seed's u64 bit pattern, read when the
-        kernels run: then every launch is graph-capturable (no generator, no host read, no allocation after the first call)."""
+        kernels run: then every launch is graph-capturable (no generator, no host read, no allocation after the first call).
+        maps: "generate" generates all M maps and builds their sensor tables; "keep" keeps the M maps the engine holds (e.g. a pool
+        installed with MapPool.install) and the map assignment `map_id`, and draws the placements and the tape only; "draw" is "keep"
+        after marl_map_draw gives every env a map drawn uniformly from the M held ones (env b's own stream of (seed, b), written into
+        `map_id` in place).  "keep" / "draw" need maps that were set (set_maps, MapPool.install, a "generate" reset, reset or
+        load_state_dict): MarlError otherwise, before any CUDA call."""
         import ctypes
+        if maps not in self.MAP_MODES:
+            raise ValueError(f"reset_device: maps={maps!r}: 'generate', 'keep' or 'draw'")
+        if maps != "generate" and not self.maps_set:
+            raise _lib.MarlError(f"reset_device(maps={maps!r}) keeps the engine's maps, but they were never set (install a pool with "
+                                 "MapPool.install, call set_maps, or reset with maps='generate' first)")
         if tape not in ("torch", "device"):
             raise ValueError(f"tape={tape!r}: 'torch' or 'device'")
         on_device = isinstance(seed, torch.Tensor)
@@ -194,17 +207,23 @@ class BatchedPursuitEnv:
             if seed.dtype != torch.int64 or seed.numel() != 1 or not seed.is_cuda:
                 raise _lib.MarlError("reset_device: a device seed is one int64 element on the engine's device")
             seed_arg, gen, place, sfx = _lib.ptr(seed), self.lib.marl_map_generate_dseed, self.lib.marl_env_reset_place_dseed, "_dseed"
+            draw = self.lib.marl_map_draw_dseed
         else:
             seed_arg = ctypes.c_uint64(int(seed) & 0xFFFFFFFFFFFFFFFF)
             gen, place, sfx = self.lib.marl_map_generate, self.lib.marl_env_reset_place, ""
-        _lib.check(gen(self._pp(), self.M, int(mc.num_obstacle_block), ctypes.c_double(float(mc.center[0])),
-                       ctypes.c_double(float(mc.center[1])), ctypes.c_double(float(mc.variance)), seed_arg, _lib.ptr(self.grid_bits),
-                       _lib.ptr(self.inflated_bits), _lib.stream_ptr()), "marl_map_generate" + sfx)
-        self.build_sensor_tables()
+            draw = self.lib.marl_map_draw
+        if maps == "generate":
+            _lib.check(gen(self._pp(), self.M, int(mc.num_obstacle_block), ctypes.c_double(float(mc.center[0])),
+                           ctypes.c_double(float(mc.center[1])), ctypes.c_double(float(mc.variance)), seed_arg, _lib.ptr(self.grid_bits),
+                           _lib.ptr(self.inflated_bits), _lib.stream_ptr()), "marl_map_generate" + sfx)
+            self.build_sensor_tables()
+            self.maps_set = True
+        elif maps == "draw":
+            _lib.check(draw(self._pp(), self.B, self.M, seed_arg, _lib.ptr(self.map_id), _lib.stream_ptr()), "marl_map_draw" + sfx)
         _lib.check(place(self._pp(), self.B, self.M, _lib.ptr(self.inflated_bits), _lib.ptr(self.map_id), seed_arg, ctypes.c_double(4.0),
                          2, 200000, _lib.ptr(self.p_state), _lib.ptr(self.e_state), _lib.ptr(self.target), _lib.ptr(self._reset_scratch),
                          _lib.ptr(self.reset_fail), _lib.stream_ptr()), "marl_env_reset_place" + sfx)
-        self.launches += 2
+        self.launches += 1 + (maps != "keep")      # the map generation or draw, and the placement (the table build counts itself)
         shape = (self.B, int(tape_len), 2)
         if tuple(self.target_tape.shape) != shape or not self.target_tape.is_contiguous():
             self.target_tape = torch.empty(shape, dtype=torch.int32, device=self.device)
@@ -427,6 +446,7 @@ class BatchedPursuitEnv:
             else:
                 getattr(self, n).copy_(sd[n])
         self._tape_len = int(sd["tape_len"])
+        self.maps_set = True
 
 
 class EpisodeGraph:

@@ -157,6 +157,11 @@ int marl_env_reset_place_dseed(const marl_env_params *p, int32_t B, int32_t M, c
 /* Candidate-target tape of the mid-episode init_target (base_env.py:52-70), filled in place: d_tape i32 [B,L,2], entry (b, l) =
  * (randint(0, W-1), randint(0, H-1)) from env b's own counter stream keyed by (*d_seed, b).  Row b does not depend on B. */
 int marl_target_tape_generate(const marl_env_params *p, int32_t B, int32_t L, const uint64_t *d_seed, int32_t *d_tape, void *stream);
+/* Per-env map draw of a reset that keeps the M installed maps (a map pool): d_map_id i32 [B], entry b = randint(0, M-1) from env b's
+ * own counter stream keyed by (seed, b) under a tag of its own (not the map, placement or tape streams').  Entry b does not depend on
+ * B.  The _dseed twin reads the seed from the device word d_seed (not NULL) when the kernel runs, with the same bits. */
+int marl_map_draw(const marl_env_params *p, int32_t B, int32_t M, uint64_t seed, int32_t *d_map_id, void *stream);
+int marl_map_draw_dseed(const marl_env_params *p, int32_t B, int32_t M, const uint64_t *d_seed, int32_t *d_map_id, void *stream);
 
 /* ---- kernel 3a: Welford reward normalisation -----------------------------------------------------
  * Replaces Normalization.__call__ / RunningMeanStd.update (DHGN/normalization.py:4-35) applied per env:

@@ -31,7 +31,18 @@ finishes an episode prints its reward.
 --graph (needs --auto-reset, implies --device-tape) replays each segment from the CUDA graphs of MAPPO.explore_batched; it prints the same
 exact columns as --device-tape without it.
 
-    python tools/train_loop.py --envs 512 --steps 150 --segment 64 --auto-reset --graph --iters 7"""
+    python tools/train_loop.py --envs 512 --steps 150 --segment 64 --auto-reset --graph --iters 7
+
+--map-pool DIR trains on the maps of a map pool (MapPool files, e.g. the authors' or one written by tools/make_map_pool.py) instead of
+generated ones: the pool's first M - K maps are installed into the engine once (verified against the files), and every reset of the
+plain, --auto-reset and --graph loops keeps them and draws each env's map from them (reset_device(maps="draw")).  --held-out K keeps
+the pool's last K maps out of training and evaluates the policy on them every --eval-every iterations (an Evaluator with the held-out
+maps: --eval-envs arg-max episodes, env b on held-out map b % K, the same maps every time); rank 0 prints the result on an "eval" line,
+whose float.hex columns follow "hex".  The evaluation does not change the training: the exact columns are those of a run on a pool of
+the first M - K maps alone.
+
+    python tools/make_map_pool.py --maps 2000 --seed 0 --out pool
+    python tools/train_loop.py --envs 512 --steps 150 --segment 64 --auto-reset --map-pool pool --held-out 100 --eval-every 5"""
 import argparse
 import os
 import sys
@@ -44,6 +55,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from distributed_multi_agent_reinforcement_learning_b200 import default_config, parallel  # noqa: E402
 from distributed_multi_agent_reinforcement_learning_b200.checkpoint import load_training_state, save_training_state  # noqa: E402
+from distributed_multi_agent_reinforcement_learning_b200.evaluator import Evaluator  # noqa: E402
+from distributed_multi_agent_reinforcement_learning_b200.map_pool import MapPool, MapPoolError  # noqa: E402
 from distributed_multi_agent_reinforcement_learning_b200.mappo_parallel import MAPPO, AutoReset, RolloutCarry  # noqa: E402
 from distributed_multi_agent_reinforcement_learning_b200.pursuit_env import BatchedPursuitEnv, RolloutArena  # noqa: E402
 
@@ -51,7 +64,11 @@ from distributed_multi_agent_reinforcement_learning_b200.pursuit_env import Batc
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--envs", type=int, default=512)
-    ap.add_argument("--maps", type=int, default=32)
+    ap.add_argument("--maps", type=int, default=None, help="maps generated per reset (default 32); not with --map-pool")
+    ap.add_argument("--map-pool", default=None, help="train on the maps of the MapPool in this directory (resets draw from them)")
+    ap.add_argument("--held-out", type=int, default=0, help="--map-pool: keep the pool's last K maps for evaluation")
+    ap.add_argument("--eval-every", type=int, default=1, help="--held-out: iterations between evaluations")
+    ap.add_argument("--eval-envs", type=int, default=None, help="--held-out: episodes per evaluation (default: K)")
     ap.add_argument("--pursuers", type=int, default=8)
     ap.add_argument("--steps", type=int, default=150)
     ap.add_argument("--segment", type=int, default=None, help="env steps per iteration, a divisor of --steps (default: --steps)")
@@ -70,6 +87,25 @@ def main():
     args = ap.parse_args()
     if args.save_every < 1:
         ap.error("--save-every must be >= 1")
+    pool = None
+    if args.map_pool is None:
+        if args.held_out:
+            ap.error("--held-out needs --map-pool")
+        args.maps = 32 if args.maps is None else args.maps
+    else:
+        if args.host_reset:
+            ap.error("--map-pool draws the envs' maps on the device; it does not combine with --host-reset")
+        if args.maps is not None:
+            ap.error("--map-pool sets the maps (the pool's size less --held-out); it does not combine with --maps")
+        if args.held_out < 0 or args.eval_every < 1 or (args.eval_envs is not None and args.eval_envs < 1):
+            ap.error("--held-out must be >= 0, --eval-every and --eval-envs >= 1")
+        try:
+            pool = MapPool.load(args.map_pool, mmap=True)
+        except MapPoolError as e:
+            ap.error(f"--map-pool: {e}")
+        if args.held_out >= len(pool):
+            ap.error(f"--held-out {args.held_out} leaves no training map of the pool's {len(pool)}")
+        args.maps = len(pool) - args.held_out
     S = args.steps if args.segment is None else args.segment
     if (args.graph or args.device_tape) and not args.auto_reset:
         ap.error("--graph / --device-tape need --auto-reset")
@@ -91,10 +127,21 @@ def main():
                          algo__learner_device=str(dev), algo__worker_device=str(dev))
     B, T, N = args.envs, args.steps, args.pursuers
     env = BatchedPursuitEnv(cfg, B, device=dev, num_maps=args.maps)
+    if pool is not None:
+        pool.install(env, np.arange(args.maps), verify=True)
     arena = RolloutArena(env.params, B, S, dev)
     torch.manual_seed(0)
     mappo = MAPPO(cfg, B, max(1, round(B / 10)), "Learner")
     mappo.sync_weights(0)
+    args.reset_maps = "generate" if pool is None else "draw"
+    args.evaluator = None
+    if pool is not None and args.held_out and rank == 0:
+        with torch.random.fork_rng(devices=[dev]):      # the evaluator's networks do not draw from the training's RNG streams
+            agent = MAPPO(cfg, None, None, "Evaluator")
+        # its seed and recorder are part of the training state, so a resumed run evaluates as if never stopped
+        args.evaluator = Evaluator(cfg, args.eval_envs or args.held_out, agent, device=dev, pool=pool,
+                                   pool_indices=np.arange(args.maps, len(pool)))
+    args.mappo = mappo
     total_steps, start = 0, 0
     carry = RolloutCarry.zeros(mappo, B, N) if n_seg > 1 else None     # where the next segment of the current episode starts
     ep_sum = torch.zeros(B, dtype=torch.int64, device=dev)              # raw reward of the current episode so far, per env
@@ -102,7 +149,7 @@ def main():
     if args.auto_reset:
         return auto_reset_loop(args, rank, world, dev, cfg, env, arena, mappo, state_file)
     if args.resume:
-        extra = load_training_state(state_file(args.resume), mappo, env, carry=carry)
+        extra = load_training_state(state_file(args.resume), mappo, env, evaluator=args.evaluator, carry=carry)
         start, total_steps = int(extra["next_iter"]), int(extra["total_steps"])
         if carry is not None:
             ep_sum = extra["ep_reward_so_far"].to(dev)
@@ -118,8 +165,8 @@ def main():
                 env.reset(seed=1000 * rank + ep)                   # host generation with the reference's placement rules
                 g = np.random.default_rng(7 + 1000 * rank + ep)
                 env.set_target_tape(np.stack([g.integers(0, W, (B, 16)), g.integers(0, H, (B, 16))], -1).astype(np.int32))
-            else:
-                env.reset_device(seed=1000 * rank + ep)            # same rules, generated on the GPU (csrc/reset_kernels.cu)
+            else:                                              # same rules, generated on the GPU (csrc/reset_kernels.cu)
+                env.reset_device(seed=1000 * rank + ep, maps=args.reset_maps)
             if carry is not None:
                 carry = RolloutCarry.zeros(mappo, B, N)
             ep_sum.zero_()
@@ -148,19 +195,38 @@ def main():
         if world > 1:
             torch.distributed.all_reduce(stats)
             stats /= world
+        s = [float(x) for x in stats.cpu()]
+        evaluation = evaluate(args, it, total_steps, s)
         if args.save_dir and ((it + 1) % args.save_every == 0 or it + 1 == args.iters):
             extra = dict(next_iter=it + 1, total_steps=total_steps)
             if carry is not None:
                 extra["ep_reward_so_far"] = ep_sum.cpu()
-            save_training_state(state_file(args.save_dir), mappo, env, extra=extra, carry=None if ep_end else carry)
+            save_training_state(state_file(args.save_dir), mappo, env, evaluator=args.evaluator, extra=extra,
+                                carry=None if ep_end else carry)
         if rank == 0:
-            s = [float(x) for x in stats.cpu()]
             rew, rew_hex = (f"{s[0]:9.2f}", s[0].hex()) if ep_end else (f"{'-':>9}", "-")
             print(f"iter {it:3d}  steps {total_steps:9d}  ep_reward {rew}  collided {s[1]:5.2f}  objC {s[2]:8.4f}  "
                   f"objA {s[3]:8.4f}  reset {t1 - t0:5.2f}s  rollout {1e3 * (t2 - t1):7.1f}ms  train {1e3 * (t3 - t2):7.1f}ms  "
                   f"exact {it} {total_steps} {rew_hex} {s[2].hex()} {s[3].hex()}", flush=True)
+            if evaluation:
+                print(evaluation, flush=True)
     if world > 1:
         torch.distributed.destroy_process_group()
+
+
+def evaluate(args, it, total_steps, s):
+    """--held-out, every --eval-every iterations: arg-max episodes of the current policy on the held-out maps (rank 0 only).  Returns
+    the "eval" line, or None.  It runs before the iteration's save, so the saved evaluator continues where a resumed run expects it."""
+    ev = args.evaluator
+    if ev is None or (it + 1) % args.eval_every:
+        return None
+    t0 = time.perf_counter()
+    weights = lambda net: {k: v.detach().clone() for k, v in net.state_dict().items()}     # noqa: E731
+    with torch.random.fork_rng(devices=[args.mappo.device]):        # leaves the training's RNG streams as they were
+        ev.run(weights(args.mappo.actor), weights(args.mappo.critic), total_steps, s[0], (s[2], s[3]))
+    r = ev.last
+    return (f"eval {it:3d}  steps {total_steps:9d}  held-out maps {args.held_out}  episodes {ev.num_cpus_eval}  avg_r {r['avg_r']:9.2f}  "
+            f"std_r {r['std_r']:8.2f}  time {time.perf_counter() - t0:5.2f}s  hex {it} {float(r['avg_r']).hex()} {float(r['std_r']).hex()}")
 
 
 def auto_reset_loop(args, rank, world, dev, cfg, env, arena, mappo, state_file):
@@ -168,19 +234,19 @@ def auto_reset_loop(args, rank, world, dev, cfg, env, arena, mappo, state_file):
     with seed e*world + rank (the seeds of the loop without --auto-reset), the resets inside the rollout."""
     B, N, S, T_ep = args.envs, args.pursuers, args.segment or args.steps, args.steps
     auto = AutoReset(reset_seed=lambda e: 1000 * rank + e, sample_seed=lambda e: e * world + rank,
-                     tape="device" if args.device_tape or args.graph else "torch")
+                     tape="device" if args.device_tape or args.graph else "torch", maps=args.reset_maps)
     carry = RolloutCarry.zeros(mappo, B, N)
     ep_sum = torch.zeros(B, dtype=torch.int64, device=dev)
     total_steps, start = 0, 0
     if args.resume:
-        extra = load_training_state(state_file(args.resume), mappo, env, carry=carry)
+        extra = load_training_state(state_file(args.resume), mappo, env, evaluator=args.evaluator, carry=carry)
         start, total_steps = int(extra["next_iter"]), int(extra["total_steps"])
         ep_sum = extra["ep_reward_so_far"].to(dev)
         if divmod(start * S, T_ep) != (carry.episode, carry.t0):
             raise SystemExit(f"--resume: the file continues at step {carry.t0} of episode {carry.episode}, iteration {start} of "
                              f"--segment {S} starts at step {start * S % T_ep} of episode {start * S // T_ep}")
     else:
-        env.reset_device(seed=auto.reset_seed(0), tape_len=auto.tape_len, tape=auto.tape)
+        env.reset_device(seed=auto.reset_seed(0), tape_len=auto.tape_len, tape=auto.tape, maps=auto.maps)
         torch.cuda.synchronize()
         assert int(env.reset_fail.sum()) == 0, "device reset could not place every pursuer / evader"
     for it in range(start, args.iters):
@@ -214,15 +280,18 @@ def auto_reset_loop(args, rank, world, dev, cfg, env, arena, mappo, state_file):
         if world > 1:
             torch.distributed.all_reduce(stats)
             stats /= world
+        s = [float(x) for x in stats.cpu()]
+        evaluation = evaluate(args, it, total_steps, s)
         if args.save_dir and ((it + 1) % args.save_every == 0 or it + 1 == args.iters):
-            save_training_state(state_file(args.save_dir), mappo, env, extra=dict(next_iter=it + 1, total_steps=total_steps,
-                                                                                  ep_reward_so_far=ep_sum.cpu()), carry=carry)
+            save_training_state(state_file(args.save_dir), mappo, env, evaluator=args.evaluator,
+                                extra=dict(next_iter=it + 1, total_steps=total_steps, ep_reward_so_far=ep_sum.cpu()), carry=carry)
         if rank == 0:
-            s = [float(x) for x in stats.cpu()]
             rew, rew_hex = (f"{s[0]:9.2f}", s[0].hex()) if ep_end else (f"{'-':>9}", "-")
             print(f"iter {it:3d}  steps {total_steps:9d}  ep_reward {rew}  collided {s[1]:5.2f}  objC {s[2]:8.4f}  "
                   f"objA {s[3]:8.4f}  reset {0.0:5.2f}s  rollout {1e3 * (t2 - t1):7.1f}ms  train {1e3 * (t3 - t2):7.1f}ms  "
                   f"exact {it} {total_steps} {rew_hex} {s[2].hex()} {s[3].hex()}", flush=True)
+            if evaluation:
+                print(evaluation, flush=True)
     if world > 1:
         torch.distributed.destroy_process_group()
 
