@@ -80,6 +80,9 @@ _PROTOTYPES = {
     "marl_gru_cell_bwd": (C.c_int, [_I64, _I32] + [_VP] * 10),
     "marl_ppo_head_workspace_bytes": (_I64, [_I64]),
     "marl_ppo_head_det": (C.c_int, [_I64, _I32, _I32] + [_VP] * 12 + [_F32, _F32] + [_VP] * 8),
+    "marl_ppo_stats_workspace_bytes": (_I64, [_I64]),
+    "marl_ppo_stats": (C.c_int, [_I64] + [_VP] * 7 + [_F32, _VP, _VP, _VP]),
+    "marl_ppo_stats_combine": (C.c_int, [_I32, _VP, _VP, _F32, _VP, _VP]),
     "marl_act_head": (C.c_int, [_I64, _I32, _I32] + [_VP] * 6 + [_U64, _I32, _I32] + [_VP] * 5),
     "marl_gemm_tf32x3": (C.c_int, [_I32, _I32, _I32, _I32, _VP, _I64, _VP, _I64, _VP, _I64, _VP, _VP, _I64, _VP, _I64, _I32, _VP]),
     "marl_policy_pack_bytes": (_I64, [_I32, _I32]),

@@ -19,6 +19,7 @@ from torch.nn.utils import spectral_norm
 
 from . import _lib, policy_ops as ops
 from .mappo_parallel import _FlatAdam, orthogonal_init
+from .train_stats import TrainStats
 
 
 def preproc_layer(input_size, output_size, is_sn=False):
@@ -201,6 +202,7 @@ class MAPPO:
             self.actor.load_state_dict(torch.load(pretrain_dir + "/actor.pth", map_location="cpu").state_dict())
             self.critic.load_state_dict(torch.load(pretrain_dir + "/critic.pth", map_location="cpu").state_dict())
         self.sn, self.args, self.minibuffer = sn, args, None
+        self.last_train_stats = None     # TrainStats of the last train(stats=True)
         self.finalize()
 
     def finalize(self):
@@ -223,7 +225,9 @@ class MAPPO:
                               _lib.ptr(ws), _lib.stream_ptr()), "marl_gae")
         return adv, vt
 
-    def train(self, replay_buffer, total_steps):
+    def train(self, replay_buffer, total_steps, stats=False):
+        """stats=True: PPO diagnostics of the update, one `marl_ppo_stats` row per team-size minibatch, left in
+        `self.last_train_stats` (a TrainStats, see mappo_parallel.MAPPO.train); training and the return value are unchanged."""
         per_team = []
         for num in self.args.pursuer_num:
             batch, T = replay_buffer.get_training_data(num, self.device)
@@ -234,6 +238,10 @@ class MAPPO:
         self.ac_optimizer.zero_grad()
         E, L = self.rnn_hidden_dim, self.num_layers
         cm = self.critic.Mean
+        if stats:
+            n_mb = len(per_team) * len(range(0, self.batch_size, self.mini_batch_size))
+            mb_sums = torch.empty(n_mb, ops.PPO_STATS_SUMS, dtype=torch.float64, device=self.device)
+            norms = torch.empty(n_mb, dtype=torch.float32, device=self.device) if self.use_grad_clip else None
         with torch.enable_grad(), ops.pack_scope():
             for num, batch, T, adv, v_target in per_team:
                 for lo in range(0, self.batch_size, self.mini_batch_size):
@@ -256,12 +264,20 @@ class MAPPO:
                         with torch.no_grad():
                             cm.weight_u.copy_(u2)
                             cm.weight_v.copy_(v2)
+                    if stats:
+                        ops.ppo_stats(logp, batch["a_logprob_n"][idx, :T], ent, val,
+                                      batch["v_n"][idx, :T] if self.use_value_clip else None, v_target[idx],
+                                      batch["active"][idx, :T], self.epsilon, out=mb_sums[update_time])
                     (la + lc).backward()
                     if self.use_grad_clip:
-                        ops.clip_grad_norm_(self.ac_optimizer.flat_grad, 10.0)                    # (:405)
+                        ops.clip_grad_norm_(self.ac_optimizer.flat_grad, 10.0,                    # (:405)
+                                            out=norms[update_time:update_time + 1] if stats else None)
                     object_critics += float(lc.detach())
                     object_actors += float(la.detach())
                     update_time += 1
+        if stats:
+            self.last_train_stats = TrainStats.from_sums(ops.ppo_stats_combine(mb_sums, norms, 10.0), self.epsilon,
+                                                         10.0 if self.use_grad_clip else None)
         if self.use_lr_decay:
             self.lr_decay(total_steps)
         return object_critics / update_time, object_actors / update_time, self.actor.get_gradients(), self.critic.get_gradients()

@@ -30,6 +30,7 @@ from torch.nn.utils import spectral_norm
 from . import _lib, fused_policy, policy_ops as ops
 from .normalization import Normalization
 from .replay_buffer import BigBuffer, ReplayBuffer
+from .train_stats import TrainStats
 
 
 TWO_STREAM_TRAIN = True     # actor and critic branches of a training minibatch on two CUDA streams
@@ -770,6 +771,7 @@ class MAPPO:
                               list(self.actor.Mean.parameters()))
         self.ac_optimizer = _FlatAdam(self.ac_parameters, lr=self.lr, eps=1e-5)
         self.minibuffer, self.total_step, self.cfg = None, 0, cfg
+        self.last_train_stats = None     # TrainStats of the last train(stats=True)
 
     # ------------------------------------------------------------------------------------------------ training
     def _forward_losses(self, mb, adv, v_target, side=None):
@@ -846,7 +848,7 @@ class MAPPO:
         return adv, vt
 
     def train(self, replay_buffer, total_steps, return_numpy=True, trace=None, allreduce=None, mean=False, shuffle=None,
-              shuffle_seed=None, permutation=None):
+              shuffle_seed=None, permutation=None, stats=False):
         """MAPPO.train (:638-723): GAE, then for each sequential minibatch forward / PPO losses / backward with gradients
         accumulating and the global-norm clip applied to the running accumulation; no optimizer step here.
 
@@ -855,7 +857,11 @@ class MAPPO:
         is summed over the replicas (`mean=True`: averaged) before it enters the running, clipped accumulation, so the clip acts on
         the global gradient and all replicas leave `train` with identical gradients; `update()` then only steps).
         shuffle (default `cfg.algo.shuffle_minibatches`, false = the reference's SequentialSampler :665): minibatches are drawn from a
-        device permutation of the envs (seeded by `shuffle_seed`, or given as `permutation`) and gathered by `marl_gather_rows`."""
+        device permutation of the envs (seeded by `shuffle_seed`, or given as `permutation`) and gathered by `marl_gather_rows`.
+        stats=True: PPO diagnostics of the update (entropy, KL, clip fractions, explained variance, gradient norms) are reduced on the
+        device - one `marl_ppo_stats` row per minibatch, on that minibatch's stream, then one `marl_ppo_stats_combine` - and left in
+        `self.last_train_stats` (a TrainStats; this replica's rows: `allreduce_()` makes them global).  Training is unchanged, and the
+        return value too."""
         if allreduce not in (None, "update", "minibatch"):
             raise ValueError(f"allreduce={allreduce!r}: None / 'update' (one all-reduce per update) or 'minibatch'")
         per_mb = allreduce == "minibatch"
@@ -894,6 +900,9 @@ class MAPPO:
         views = self.ac_optimizer._views
         gbuf = torch.zeros(n_mb, flat.numel(), dtype=torch.float32, device=self.device)
         losses = torch.zeros(n_mb, 2, dtype=torch.float32, device=self.device)
+        if stats:       # row m belongs to minibatch m alone, so the result does not depend on which minibatch finishes first
+            mb_sums = torch.empty(n_mb, ops.PPO_STATS_SUMS, dtype=torch.float64, device=self.device)
+            norms = torch.empty(n_mb, dtype=torch.float32, device=self.device) if self.use_grad_clip else None
         main = torch.cuda.current_stream()
         P = max(1, min(CONCURRENT_MINIBATCHES, n_mb))
         if getattr(self, "_mb_streams", None) is None or len(self._mb_streams) < P:
@@ -916,6 +925,9 @@ class MAPPO:
                         if g is not None:
                             gbuf[m, off:off + k].copy_(g.reshape(-1))
                     losses[m, 0], losses[m, 1] = la.detach(), lc.detach()
+                    if stats:
+                        ops.ppo_stats(logp, mb.logp, ent, val, mb.v[:-1] if self.use_value_clip else None, vt_mb, mb.active,
+                                      self.epsilon, out=mb_sums[m])
                     if trace is not None:
                         trace.setdefault("mb", []).append(dict(logp=logp.detach(), ent=ent.detach(), val=val.detach()))
                     del grads, la, lc, logp, ent, val, mb
@@ -929,11 +941,17 @@ class MAPPO:
                     parallel.allreduce_sum_(gbuf[m], mean=mean)
                 flat.add_(gbuf[m])
                 if self.use_grad_clip:
-                    ops.clip_grad_norm_(flat, 5.0)
+                    norm = ops.clip_grad_norm_(flat, 5.0, out=norms[m:m + 1] if stats else None)
+                    if trace is not None:
+                        trace.setdefault("grad_norms", []).append(norm.clone())
+            if stats:
+                stats_sums = ops.ppo_stats_combine(mb_sums, norms, 5.0)
         self.ac_optimizer._sync_grads()
         self._grads_reduced = per_mb
         self.last_train_issue_s = time.perf_counter() - t_issue     # host time to ISSUE the epoch (the device may still be running)
         lh = losses.cpu()
+        if stats:
+            self.last_train_stats = TrainStats.from_sums(stats_sums, self.epsilon, 5.0 if self.use_grad_clip else None)
         if trace is not None:
             for m, rec in enumerate(trace["mb"]):
                 rec["actor_loss"], rec["critic_loss"] = float(lh[m, 0]), float(lh[m, 1])

@@ -36,6 +36,14 @@ def allreduce_sum_(flat, mean=False):
     return flat
 
 
+def allreduce_max_(t):
+    """In-place element-wise maximum of one tensor over the ranks."""
+    rank, ws = world()
+    if ws > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    return t
+
+
 def broadcast_(flat, src=0):
     rank, ws = world()
     if ws > 1:

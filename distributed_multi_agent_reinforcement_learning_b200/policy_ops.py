@@ -515,11 +515,41 @@ def act_head(feat_a, feat_c, Wa, ba, w_eff, bc, seed, t, deterministic):
     return action, action_f, logp, value
 
 
-def clip_grad_norm_(flat_grad, max_norm):
-    """In-place global-norm clip of a flat fp32 gradient arena; returns the pre-clip norm (0-dim tensor)."""
+PPO_STATS_SUMS, PPO_STATS_OUT = 16, 24      # MARL_PPO_STATS_SUMS / MARL_PPO_STATS_OUT (include/marl_b200.h)
+
+
+def ppo_stats(logp, old_logp, entropy, value, v_old, v_target, active, eps, out=None):
+    """PPO diagnostics of one minibatch (marl_ppo_stats): the f64 sums [PPO_STATS_SUMS] of the per-row values, written to `out`
+    (a contiguous f64 tensor of PPO_STATS_SUMS elements, e.g. one row of a [n_mb, PPO_STATS_SUMS] buffer) or a new tensor.
+    All inputs are fp32 tensors of R elements; v_old = None: no value clip."""
+    flat = [None if t is None else t.reshape(-1).contiguous() for t in (logp, old_logp, entropy, value, v_old, v_target, active)]
+    R = flat[0].numel()
+    dev = flat[0].device
+    if out is None:
+        out = torch.empty(PPO_STATS_SUMS, dtype=torch.float64, device=dev)
+    ws = torch.empty(max(int(_L().marl_ppo_stats_workspace_bytes(R)), 0), dtype=torch.uint8, device=dev)
+    _lib.check(_L().marl_ppo_stats(R, *[_lib.ptr(t) for t in flat], ctypes.c_float(eps), _lib.ptr(out), _lib.ptr(ws),
+                                   _lib.stream_ptr()), "marl_ppo_stats")
+    return out
+
+
+def ppo_stats_combine(mb_sums, grad_norms=None, max_norm=0.0, out=None):
+    """The update's statistics vector [PPO_STATS_OUT] (marl_ppo_stats_combine) from the minibatch rows [n_mb, PPO_STATS_SUMS] and
+    the pre-clip gradient norms [n_mb] (None without a gradient clip)."""
+    mb_sums = mb_sums.contiguous()
+    if out is None:
+        out = torch.empty(PPO_STATS_OUT, dtype=torch.float64, device=mb_sums.device)
+    _lib.check(_L().marl_ppo_stats_combine(mb_sums.shape[0] if mb_sums.dim() == 2 else 0, _lib.ptr(mb_sums), _lib.ptr(grad_norms),
+                                           ctypes.c_float(max_norm), _lib.ptr(out), _lib.stream_ptr()), "marl_ppo_stats_combine")
+    return out
+
+
+def clip_grad_norm_(flat_grad, max_norm, out=None):
+    """In-place global-norm clip of a flat fp32 gradient arena; returns the pre-clip norm (0-dim tensor).  `out`: a one-element
+    fp32 device tensor (e.g. `norms[m:m + 1]`) that receives the norm instead of a new tensor."""
     n = flat_grad.numel()
     ws = torch.empty(int(_L().marl_clip_workspace_bytes(n)), dtype=torch.uint8, device=flat_grad.device)
-    total = torch.empty(1, dtype=torch.float32, device=flat_grad.device)
+    total = torch.empty(1, dtype=torch.float32, device=flat_grad.device) if out is None else out
     _lib.check(_L().marl_clip_grad_norm(n, _lib.ptr(flat_grad), ctypes.c_float(max_norm), _lib.ptr(ws), _lib.ptr(total),
                                         _lib.stream_ptr()), "marl_clip_grad_norm")
     return total[0]

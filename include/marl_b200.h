@@ -398,6 +398,36 @@ int marl_ppo_head_det(int64_t R, int32_t E, int32_t A, const float *d_feat_a, co
                       const float *d_old_logp, const float *d_adv, const float *d_v_old, const float *d_v_target,
                       const float *d_active, float eps, float ent_coef, float *d_logp, float *d_entropy, float *d_value,
                       float *d_dlogits, float *d_dvalue, float *d_sums, void *d_workspace, void *stream);
+/* PPO diagnostics of one minibatch of R rows (csrc/train_stats.cu), from marl_ppo_head_det's per-row outputs.  With a = active,
+ * lr = logp - old_logp (in f64), r = exp(lr) and x = v_target - v_old (the raw advantage), d_sums[MARL_PPO_STATS_SUMS] receives
+ * (rows with a == 0 are skipped):
+ *    0 sum a                          6 min lr over active rows (+inf if none)   12 sum a*x            (0 without d_v_old)
+ *    1 sum a*entropy                  7 sum a*[|value - v_old| > eps]            13 sum a*x^2          (0 without d_v_old)
+ *    2 sum a*(-lr)         (k1 KL)      (0 without d_v_old)                      14 1 if d_v_old was given, else 0
+ *    3 sum a*((r-1) - lr)  (k3 KL)    8 sum a*v_target                           15 R (all rows, active or not)
+ *    4 sum a*[|r - 1| > eps]          9 sum a*v_target^2
+ *    5 max lr over active rows       10 sum a*(v_target - value)
+ *      (-inf if none)                11 sum a*(v_target - value)^2
+ * The extreme ratios are kept as log-ratios (r = exp(lr) is monotone), so they are exact.  Accumulated in f64 from the fp32
+ * inputs in a fixed order (grid a function of R only, per-CTA partials in d_workspace, one ordered reduction block): bit-identical
+ * from call to call, no atomics, no allocation, graph-capturable.  d_v_old == NULL: no value clip (slots 7, 12, 13 are 0).
+ * d_workspace: marl_ppo_stats_workspace_bytes(R) bytes (-1 for R <= 0), not shared by calls that may run at the same time.
+ * MARL_EINVAL for R <= 0, a NULL required pointer, or eps < 0 / not finite. */
+#define MARL_PPO_STATS_SUMS 16
+/* marl_ppo_stats_combine writes d_out[MARL_PPO_STATS_OUT]: slots 0..15 are the n_mb minibatch rows added in index order (slot 5 the
+ * maximum, slot 6 the minimum, slot 14 the number of rows given d_v_old), then
+ *   16 n_mb    17 number of gradient norms (n_mb, or 0 if d_grad_norms is NULL)    18 largest norm    19 last norm (the norm of
+ *   the final accumulated gradient)    20 number of norms > max_norm    21..23 zero.
+ * Raw sums and counts, never ratios, so that the vectors of several ranks can be summed (max / min slots reduced with max / min).
+ * d_grad_norms: the pre-clip norms of the n_mb minibatches in accumulation order, or NULL (then max_norm is ignored; otherwise it
+ * must be finite and > 0).  MARL_EINVAL for n_mb < 1 or a NULL d_mb_sums / d_out. */
+#define MARL_PPO_STATS_OUT 24
+int64_t marl_ppo_stats_workspace_bytes(int64_t R);
+int marl_ppo_stats(int64_t R, const float *d_logp, const float *d_old_logp, const float *d_entropy, const float *d_value,
+                   const float *d_v_old, const float *d_v_target, const float *d_active, float eps, double *d_sums,
+                   void *d_workspace, void *stream);
+int marl_ppo_stats_combine(int32_t n_mb, const double *d_mb_sums, const float *d_grad_norms, float max_norm, double *d_out,
+                           void *stream);
 /* Rollout-time heads (:440-449, :513): softmax -> sample (counter RNG keyed by seed,row,t) or argmax -> log-prob; value. */
 int marl_act_head(int64_t R, int32_t E, int32_t A, const float *d_feat_a, const float *d_feat_c, const float *d_Wa,
                   const float *d_ba, const float *d_wc_eff, const float *d_bc, uint64_t seed, int32_t t,

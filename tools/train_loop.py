@@ -42,8 +42,22 @@ whose float.hex columns follow "hex".  The evaluation does not change the traini
 the first M - K maps alone.
 
     python tools/make_map_pool.py --maps 2000 --seed 0 --out pool
-    python tools/train_loop.py --envs 512 --steps 150 --segment 64 --auto-reset --map-pool pool --held-out 100 --eval-every 5"""
+    python tools/train_loop.py --envs 512 --steps 150 --segment 64 --auto-reset --map-pool pool --held-out 100 --eval-every 5
+
+--stats has every epoch reduce the PPO diagnostics of MAPPO.train(stats=True) on the device (a TrainStats, all-reduced over the ranks);
+rank 0 prints them on a "stats" line after the iteration's line: the epoch they belong to (the last one trained), the epoch at which
+--target-kl stopped the update ("-" if it did not), entropy, approx_kl (k3), approx_kl_k1, clip_frac, ratio_min / ratio_max,
+value_clip_frac, explained_variance, rollout_explained_variance, adv_mean / adv_std (raw advantage), return_mean, grad_norm_max /
+grad_norm_last (pre-clip), clipped_minibatches, rows, then their float.hex after "hex" ("-" for a value the configuration does not
+have).  The statistics change nothing in the training: the exact columns are those of a run without --stats.
+--epochs K overrides algo.epochs (K epochs per update, one Adam step each).  --target-kl X (needs K >= 2) stops an update early: when
+the approx_kl of epoch k >= 2 exceeds X, that epoch's gradient is dropped (no Adam step) and the update's remaining epochs are skipped.
+The losses on the iteration's line are then those of the last epoch that stepped.  The decision comes from bit-reproducible statistics, so such runs stay reproducible and resumable; without --stats a "kl_stop" line
+reports each stop.
+
+    python tools/train_loop.py --envs 512 --iters 5 --stats --epochs 4 --target-kl 0.02"""
 import argparse
+import math
 import os
 import sys
 import time
@@ -84,7 +98,20 @@ def main():
     ap.add_argument("--save-dir", default=None, help="write the training state (one file per rank) to this directory")
     ap.add_argument("--save-every", type=int, default=1, help="iterations between saves (the last iteration is always saved)")
     ap.add_argument("--resume", default=None, help="continue from the training state in this directory")
+    ap.add_argument("--stats", action="store_true", help="print the PPO diagnostics of every update on a 'stats' line")
+    ap.add_argument("--epochs", type=int, default=None, help="PPO epochs per update (default: algo.epochs)")
+    ap.add_argument("--target-kl", type=float, default=None,
+                    help="stop an update after epoch k >= 2 whose approx_kl exceeds this, dropping that epoch's gradient")
     args = ap.parse_args()
+    if args.epochs is None:
+        args.epochs = int(default_config().algo.epochs)
+    if args.epochs < 1:
+        ap.error("--epochs must be >= 1")
+    if args.target_kl is not None:
+        if args.epochs < 2:
+            ap.error(f"--target-kl needs at least 2 epochs per update (--epochs; now {args.epochs}): the first epoch always steps")
+        if not math.isfinite(args.target_kl) or args.target_kl < 0:
+            ap.error("--target-kl must be a finite number >= 0")
     if args.save_every < 1:
         ap.error("--save-every must be >= 1")
     pool = None
@@ -123,7 +150,7 @@ def main():
     if world > 1:
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         torch.distributed.init_process_group("nccl", device_id=dev)
-    cfg = default_config(env__num_defender=args.pursuers, env__max_steps=args.steps, algo__depth=args.depth,
+    cfg = default_config(env__num_defender=args.pursuers, env__max_steps=args.steps, algo__depth=args.depth, algo__epochs=args.epochs,
                          algo__learner_device=str(dev), algo__worker_device=str(dev))
     B, T, N = args.envs, args.steps, args.pursuers
     env = BatchedPursuitEnv(cfg, B, device=dev, num_maps=args.maps)
@@ -186,9 +213,7 @@ def main():
         total_steps += world * B * S
         if carry is not None:
             carry = tb.carry
-        for _ in range(int(cfg.algo.epochs)):                       # main.py:99: K epochs over the same buffers, one Adam step each
-            obj_c, obj_a, _, _ = mappo.train(tb, total_steps, return_numpy=False, allreduce=args.allreduce)
-            mappo.update(total_steps)
+        obj_c, obj_a, stats_line = run_epochs(args, mappo, tb, total_steps, it)     # main.py:99: K epochs, one Adam step each
         torch.cuda.synchronize()
         t3 = time.perf_counter()
         stats = torch.tensor([ep_reward, collided, obj_c, obj_a], device=dev, dtype=torch.float64)
@@ -208,10 +233,41 @@ def main():
             print(f"iter {it:3d}  steps {total_steps:9d}  ep_reward {rew}  collided {s[1]:5.2f}  objC {s[2]:8.4f}  "
                   f"objA {s[3]:8.4f}  reset {t1 - t0:5.2f}s  rollout {1e3 * (t2 - t1):7.1f}ms  train {1e3 * (t3 - t2):7.1f}ms  "
                   f"exact {it} {total_steps} {rew_hex} {s[2].hex()} {s[3].hex()}", flush=True)
+            if stats_line:
+                print(stats_line, flush=True)
             if evaluation:
                 print(evaluation, flush=True)
     if world > 1:
         torch.distributed.destroy_process_group()
+
+
+def run_epochs(args, mappo, tb, total_steps, it):
+    """The update on one batch: --epochs epochs of MAPPO.train, each followed by one Adam step (main.py:99), with the statistics of
+    every epoch reduced on the device when --stats or --target-kl needs them.  --target-kl: an epoch k >= 2 whose all-reduced approx_kl
+    exceeds the target gets no Adam step, and the update ends there (every rank takes the same decision from the same global numbers).
+    Returns the losses of the last epoch that stepped (a stopped epoch's losses are dropped with its gradient) and the line to print
+    after the iteration's (or None)."""
+    want = args.stats or args.target_kl is not None
+    stopped, st = None, None
+    for k in range(1, args.epochs + 1):
+        losses = mappo.train(tb, total_steps, return_numpy=False, allreduce=args.allreduce, stats=want)[:2]
+        if want:
+            st = mappo.last_train_stats.allreduce_()
+            if args.target_kl is not None and k >= 2 and st.approx_kl > args.target_kl:
+                stopped = k
+                break
+        mappo.update(total_steps)
+        obj_c, obj_a = losses
+    line = None
+    if args.stats:
+        fmt = lambda v: "-" if v is None else (str(v) if isinstance(v, int) else f"{v:.6g}")          # noqa: E731
+        hx = lambda v: "-" if v is None else float(v).hex()                                             # noqa: E731
+        vals = st.as_dict()
+        line = (f"stats {it:3d}  epoch {k}  kl_stop {stopped or '-'}  " + "  ".join(f"{f} {fmt(v)}" for f, v in vals.items())
+                + f"  hex {it} {k} {stopped or '-'} " + " ".join(hx(v) for v in vals.values()))
+    elif stopped:
+        line = f"kl_stop {it:3d}  epoch {stopped}  approx_kl {st.approx_kl:.6g}  target_kl {args.target_kl:g}  hex {it} {stopped} {st.approx_kl.hex()}"
+    return obj_c, obj_a, line
 
 
 def evaluate(args, it, total_steps, s):
@@ -271,9 +327,7 @@ def auto_reset_loop(args, rank, world, dev, cfg, env, arena, mappo, state_file):
             collided = float(env.collision.float().mean())
         total_steps += world * B * S
         carry = tb.carry
-        for _ in range(int(cfg.algo.epochs)):
-            obj_c, obj_a, _, _ = mappo.train(tb, total_steps, return_numpy=False, allreduce=args.allreduce)
-            mappo.update(total_steps)
+        obj_c, obj_a, stats_line = run_epochs(args, mappo, tb, total_steps, it)
         torch.cuda.synchronize()
         t3 = time.perf_counter()
         stats = torch.tensor([ep_reward, collided, obj_c, obj_a], device=dev, dtype=torch.float64)
@@ -290,6 +344,8 @@ def auto_reset_loop(args, rank, world, dev, cfg, env, arena, mappo, state_file):
             print(f"iter {it:3d}  steps {total_steps:9d}  ep_reward {rew}  collided {s[1]:5.2f}  objC {s[2]:8.4f}  "
                   f"objA {s[3]:8.4f}  reset {0.0:5.2f}s  rollout {1e3 * (t2 - t1):7.1f}ms  train {1e3 * (t3 - t2):7.1f}ms  "
                   f"exact {it} {total_steps} {rew_hex} {s[2].hex()} {s[3].hex()}", flush=True)
+            if stats_line:
+                print(stats_line, flush=True)
             if evaluation:
                 print(evaluation, flush=True)
     if world > 1:
