@@ -269,15 +269,19 @@ extern "C" int marl_gather_rows(const void *d_src, void *d_dst, const int64_t *d
                                 int64_t row_bytes, int64_t n_src_rows, void *stream)
 {
     (void)n_src_rows;
-    MARL_REQUIRE(d_src && d_dst && d_index && n_index > 0 && row_bytes > 0 && (row_bytes & 3) == 0,
+    MARL_REQUIRE(d_src && d_dst && d_index && n_index > 0 && row_bytes > 0,
                  "marl_gather_rows: bad argument (row_bytes=%lld)", (long long)row_bytes);
     cudaStream_t s = (cudaStream_t)stream;
-    const bool vec = ((row_bytes & 15) == 0) && (((uintptr_t)d_src & 15) == 0) && (((uintptr_t)d_dst & 15) == 0);
-    const int64_t row_vecs = vec ? row_bytes / 16 : row_bytes / 4;
+    // widest element that divides the row and both base addresses: 16 bytes, 4, or single bytes (e.g. the u8 e_adj rows of
+    // an odd-sized team)
+    const uintptr_t align = (uintptr_t)row_bytes | (uintptr_t)d_src | (uintptr_t)d_dst;
+    const int64_t elem = (align & 15) == 0 ? 16 : ((align & 3) == 0 ? 4 : 1);
+    const int64_t row_vecs = row_bytes / elem;
     const int64_t total = (int64_t)n_index * row_vecs;
     int nb = (int)((total + 255) / 256);
     if (nb > 148 * 16) nb = 148 * 16;
-    if (vec) gather_rows_kernel<uint4><<<nb, 256, 0, s>>>((const uint4 *)d_src, (uint4 *)d_dst, d_index, n_index, row_vecs);
-    else gather_rows_kernel<uint32_t><<<nb, 256, 0, s>>>((const uint32_t *)d_src, (uint32_t *)d_dst, d_index, n_index, row_vecs);
+    if (elem == 16) gather_rows_kernel<uint4><<<nb, 256, 0, s>>>((const uint4 *)d_src, (uint4 *)d_dst, d_index, n_index, row_vecs);
+    else if (elem == 4) gather_rows_kernel<uint32_t><<<nb, 256, 0, s>>>((const uint32_t *)d_src, (uint32_t *)d_dst, d_index, n_index, row_vecs);
+    else gather_rows_kernel<uint8_t><<<nb, 256, 0, s>>>((const uint8_t *)d_src, (uint8_t *)d_dst, d_index, n_index, row_vecs);
     return check_launch("gather_rows_kernel");
 }

@@ -195,8 +195,8 @@ int marl_gae_boundary(int32_t B, int32_t T, int32_t N, int32_t k, const float *d
 
 /* ---- kernel 4: minibatch gather ------------------------------------------------------------------
  * Replaces `batch[key][index]` (DHGN/mappo_parallel.py:665-679): copies rows d_index[i] (i < n_index) of a
- * [B,row_bytes] byte matrix into [n_index,row_bytes].  row_bytes must be a multiple of 4; 16-byte aligned
- * rows take the vectorised path. */
+ * [B,row_bytes] byte matrix into [n_index,row_bytes].  Any row_bytes > 0: 16-byte aligned rows take the
+ * vectorised path, 4-byte aligned rows copy words, others bytes. */
 int marl_gather_rows(const void *d_src, void *d_dst, const int64_t *d_index, int32_t n_index,
                      int64_t row_bytes, int64_t n_src_rows, void *stream);
 

@@ -93,7 +93,8 @@ def test_welford_kernel_matches_oracle(oracle):
     assert torch.equal(mean, before) and int(n[0]) == steps
 
 
-@pytest.mark.parametrize("row_elems,dtype", [(8 * 4, torch.float32), (150 * 8 * 176, torch.float32), (7, torch.int32), (150 * 8 * 6, torch.int32)])
+@pytest.mark.parametrize("row_elems,dtype", [(8 * 4, torch.float32), (150 * 8 * 176, torch.float32), (7, torch.int32), (150 * 8 * 6, torch.int32),
+                                             (33, torch.uint8), (3 * 33, torch.uint8)])
 def test_gather_rows(row_elems, dtype):
     from distributed_multi_agent_reinforcement_learning_b200 import _lib
     L = _lib.lib()
